@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- HER sample + DDPG update hot path on B200, next to the CPU port of the reference.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch: draw B positions of the HER buffer,
 gather + future-relabel + sparse reward, then one DDPG update (target forward, Bellman target,
@@ -14,7 +14,9 @@ hidden 256 x 3 layers, synthetic data (SURVEY 8d recipe).  N>1: every rank owns 
 1M-transition episode shard and samples its local batch of 256 (weak scaling); critic and actor
 gradients are averaged with NCCL between backward and optimiser phases.
 
-One JSON line on stdout (rank 0); progress on stderr.
+One JSON line on stdout (rank 0); progress on stderr.  ``--dump-outputs DIR`` also writes what the last timed
+step computed (its metrics and the weights of all four networks) as ``DIR/<name>.npy``: the inputs are seeded, so
+two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -34,16 +36,24 @@ for _p in (ROOT, os.path.join(ROOT, "goal-conditioned-rl-framework_b200")):
 
 METRIC = "her_relabelled_transitions_per_s"   # sampled+relabelled transitions consumed by DDPG updates
 UNIT = "transitions/s"
+DUMP_BYTES = 60 << 20      # payload cap of --dump-outputs: with the .npy headers the files stay under 64 MB
 
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
 
 
+def positive_int(text):
+    n = int(text)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {n}")
+    return n
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1000)
+    ap.add_argument("--steps", type=positive_int, default=1000, help="timed steps")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=256)
@@ -64,7 +74,27 @@ def parse():
                     help="also time the sampler on 100x the transitions (100M stored transitions, 23 GB; +1 min)")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     ap.add_argument("--spinup", type=int, default=80, help="extra untimed steps before the W warm-up steps")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (the 8 update metrics, the weights "
+                         "and biases of actor, critic and both targets) as DIR/<name>.npy in float32; rank 0 only")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Writes every named array as ``out_dir/<name>.npy`` in float32.  When they hold more than ``budget`` bytes in
+    all, each array is cut to the same fraction of its elements (flattened), at positions drawn from a fixed seed,
+    so that runs with the same arguments write the same positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    for name, v in arrays.items():
+        if total > budget:
+            keep = max(1, v.size * budget // total)
+            v = v.reshape(-1)[np.sort(np.random.default_rng(0).choice(v.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 # ------------------------------------------------------------------------------------------
@@ -773,6 +803,13 @@ def gpu_main(args):
     step += args.steps
     launches = int(lib.gcrl_kernel_launches()) - l0
     barrier()
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        # copied to the host before any later step changes the weights; written to disk after the measurements
+        outputs = {"metrics": np.array(agent.read_metrics(), np.float32)}
+        for tag in ("actor", "critic", "target_actor", "target_critic"):
+            for i, (w, b) in enumerate(getattr(agent, tag).layers()):
+                outputs[f"{tag}.{i}.weight"], outputs[f"{tag}.{i}.bias"] = w, b
     # keep the sampler alive over a short loaded stretch so that short runs still record clocks
     t_end = time.time() + 0.3
     while time.time() < t_end:
@@ -1079,6 +1116,9 @@ def gpu_main(args):
             "library": os.path.relpath(gcrl_b200.library_path(), ROOT),
             "kernel_launches_total": int(lib.gcrl_kernel_launches()) - launches0,
         }
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
+            log(f"[dump] {len(outputs)} arrays of the last timed step written to {args.dump_outputs}")
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

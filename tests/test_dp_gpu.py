@@ -95,7 +95,7 @@ def test_two_emulated_ranks_equal_one_rank_on_concatenated_batch():
 def test_two_gpu_nccl_run_matches_single_rank():
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     env = dict(os.environ, PYTHONPATH=ROOT + os.pathsep + os.path.join(ROOT, "goal-conditioned-rl-framework_b200"))
     out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
                           "--master-addr", "127.0.0.1", "--master-port", "29517",
