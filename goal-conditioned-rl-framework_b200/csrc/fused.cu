@@ -211,7 +211,7 @@ size_t fused_smem_bytes(int R, int D, int A, int H, int L, bool two_keeps) {
 // steps) and the critic forward (L + 1 steps) do not depend on each other, so CTA 0 runs the former while CTA 1
 // runs the latter; CTA 0 drops q' into CTA 1's shared memory (DSMEM), one cluster barrier, and CTA 1 goes on
 // with the loss and the backward pass.  Critical path 3L + 3 -> 2L + 2 + (L - 1) layer steps; used when both
-// CTAs of every slab fit in one wave.
+// CTAs of every slab fit in one wave (by default only at R = 8, see fused_rows_per_cta).
 template <int R, bool TD3, bool SPLIT>
 __global__ void __launch_bounds__(kFusedThreads, 1) fused_critic_kernel(FusedCriticArgs a) {
   extern __shared__ float4 fsm4[];
@@ -528,9 +528,16 @@ static void ensure_smem(K kernel, size_t bytes, int *flag) {
 // Rows per CTA.  The kernels are chains of dependent layer steps whose cost grows with R (16 FMAs per weight
 // load at R = 4, 8 at R = 2), so the smallest R whose slabs still fit in ONE wave of CTAs wins: at B = 256,
 // R = 2 (128 CTAs) runs the critic phase in 36.9 us and the actor phase in ~37 us, R = 4 (64 CTAs) in 48.9 / 45 us
-// (36.9 for the critic phase as 2-CTA clusters, see SPLIT).
+// (36.9 for the critic phase as 2-CTA clusters, see SPLIT, when forced with GCRL_FUSED_R=4).  The default rule
+// splits the critic phase only where both CTAs of every slab fit in one wave, 2 * ceil(B / R) <= SMs: at R = 8 for
+// 512 < B <= 4 * SMs (513..592 on 148 SMs); R = 4 starts above 2 * SMs rows, so it never splits.
+// GCRL_FUSED_R (experiments) forces R = 2, 4 or 8; any other value is ignored -- there are no other kernels, and
+// the grid is sized from R.
 int fused_rows_per_cta(int B) {
-  if (const char *e = getenv("GCRL_FUSED_R")) return atoi(e);
+  if (const char *e = getenv("GCRL_FUSED_R")) {
+    const int r = atoi(e);
+    if (r == 2 || r == 4 || r == 8) return r;
+  }
   if (B <= 2 * sm_count()) return 2;
   return B <= 512 ? 4 : 8;
 }

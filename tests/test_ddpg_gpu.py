@@ -143,7 +143,14 @@ def test_large_batch_update_matches_reference_fixture(case, precision, capsys):
 
 
 @pytest.mark.parametrize("B,H,L,D,A", [(1, 64, 3, 10, 3), (33, 100, 2, 22, 3), (1000, 256, 3, 23, 4),
-                                       (4096, 512, 3, 22, 3), (777, 64, 1, 7, 1)])
+                                       (4096, 512, 3, 22, 3), (777, 64, 1, 7, 1),
+                                       # one batch per rows-per-CTA variant of the row-slab kernels (148 SMs),
+                                       # each with a ragged last slab: R = 4; R = 8 as 2-CTA clusters; R = 8
+                                       (301, 256, 3, 21, 3), (517, 256, 3, 21, 3), (1021, 256, 3, 21, 3),
+                                       # R = 8 at H = 512: 194.5 KB of shared memory, the largest that fits
+                                       (517, 512, 3, 21, 3),
+                                       # K0 = 27 padded to 28; H = 100 leaves one column warp (16-way K split)
+                                       (301, 100, 2, 23, 4)])
 def test_update_matches_oracle_odd_shapes(B, H, L, D, A):
     """Ragged shapes (B not a tile multiple, H not a multiple of 16, A in 1..4), 4 updates
     spanning a Polyak step, versus the NumPy oracle on identical weights and batches."""
@@ -309,6 +316,23 @@ def test_save_weights_round_trip(tmp_path):
         assert np.array_equal(w, w2) and np.array_equal(b, b2)         # hard sync at init (:1251-1253)
 
 
+def synthetic_episodes(seed, n, D, A, G, T=50, k=4):
+    """Seeded episodes in the layout of tests.helpers.her_episodes: the last G state features are the desired
+    goal, ``fut`` holds apply_her's future offsets (randint(t + 1, T - 1), k per step)."""
+    rng = np.random.default_rng(seed)
+    eps = []
+    for _ in range(n):
+        obs = rng.standard_normal((T + 1, D)).astype(np.float32)
+        ag = np.cumsum(rng.normal(0, 0.05, (T + 1, G)), 0).astype(np.float32)
+        fut = np.zeros((T, k), np.uint8)
+        for t in range(T - 1):
+            fut[t] = rng.integers(t + 1, T, k)
+        eps.append({"s": obs[:-1], "a": rng.uniform(-1, 1, (T, A)).astype(np.float32), "ns": obs[1:],
+                    "r": -(rng.random(T) > 0.2).astype(np.float32), "d": np.zeros(T, np.float32),
+                    "ag": ag[1:], "fut": fut})
+    return eps
+
+
 def test_update_from_buffer_equals_sample_then_update():
     """The fused sample+update call == sample() followed by update(batch) on the same indices,
     bit for bit (same kernels, same order)."""
@@ -335,6 +359,54 @@ def test_update_from_buffer_equals_sample_then_update():
         assert [float(x) for x in i1] == [float(x) for x in i2]
     for n1, n2 in ((agents[0].actor, agents[1].actor), (agents[0].critic, agents[1].critic)):
         for (w, b), (w2, b2) in zip(n1.layers(), n2.layers()):
+            assert np.array_equal(w, w2) and np.array_equal(b, b2)
+
+
+@pytest.mark.parametrize("B,algo", [(128, "td3"), (301, "ddpg"), (301, "td3"), (517, "ddpg"), (517, "td3"),
+                                    (1021, "ddpg"), (1021, "td3")])
+def test_update_from_buffer_equals_sample_then_update_every_variant(B, algo):
+    """test_update_from_buffer_equals_sample_then_update (B = 128, DDPG) at the batches that reach every
+    rows-per-CTA variant of the critic kernel's in-kernel sampler (148 SMs: R = 2, 4, 8 as 2-CTA clusters, 8 with
+    a ragged last slab), for DDPG and TD3: bit for bit in metrics and in the weights of every network.  TD3's
+    critic-2 launch reuses the dense batch the critic-1 launch drew, and both agents get the same noise."""
+    import torch
+    from gcrl_b200 import DDPG, TD3Agent
+    from gcrl_b200.agent import NET_ACTOR, NET_CRITIC, NET_CRITIC2
+    from tests.helpers import her_episodes
+    D, A, G = 22, 3, 3
+    if B <= 777:
+        episodes, max_len = her_episodes(load("her_push_evict")), 777
+    else:             # the fixture's store is too small: seeded episodes, pushed until the store has evicted
+        max_len = 2 * B + 100
+        episodes = synthetic_episodes(B, max_len // 200 + 3, D, A, G)        # ~250 entries each (T = 50, k = 4)
+    cls = DDPG if algo == "ddpg" else TD3Agent
+    agents = []
+    for _ in range(2):
+        cfg = make_config(hidden_dim=64, batch_size=B, max_len=max_len, ac_update_freq=1 if algo == "ddpg" else 2)
+        ag = cls(D, A, cfg, None, 1, 40)
+        rng = np.random.default_rng(1)
+        ag._set_layers(NET_ACTOR, OD.init_mlp(rng, D, 64, A, 3))
+        ag._set_layers(NET_CRITIC, OD.init_mlp(rng, D + A, 64, 1, 3))
+        if algo == "td3":
+            ag._set_layers(NET_CRITIC2, OD.init_mlp(rng, D + A, 64, 1, 3))
+        ag.update_target_network()
+        growth = []
+        for ep in episodes:
+            n = len(ag.buffer)
+            ag.buffer.push_episode(ep["s"], ep["a"], ep["ns"], ep["r"], ep["d"], ep["ag"], ep["fut"])
+            growth.append(len(ag.buffer) - n)
+        # synthetic episodes all add the same number of entries until the store is full and evicts
+        assert len(ag.buffer) >= B and (B <= 777 or (min(growth) < max(growth) and len(ag.buffer) >= 2 * B))
+        agents.append(ag)
+    rng = np.random.default_rng(2)
+    for step in (39, 40, 41):
+        idx = rng.permutation(len(agents[0].buffer))[:B]
+        kw = {"noise": torch.randn((B, A), device="cuda")} if algo == "td3" else {}
+        i1 = agents[0].update(step, indices=idx, **kw)
+        i2 = agents[1].update(step, batch=agents[1].buffer.sample(B, indices=idx), **kw)
+        assert [float(x) for x in i1] == [float(x) for x in i2]
+    for n1, n2 in zip(agents[0]._all_nets(), agents[1]._all_nets()):
+        for (w, b), (w2, b2) in zip(agents[0]._get_layers(n1), agents[1]._get_layers(n2)):
             assert np.array_equal(w, w2) and np.array_equal(b, b2)
 
 
