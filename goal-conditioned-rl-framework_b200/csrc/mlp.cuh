@@ -176,11 +176,16 @@ bool tc_wgrad_supported(int M, int N, int K);
 // tensor-core version of launch_linear_wgrad (same partial-slab contract); returns the number of slabs
 int launch_tc_wgrad(const float *dZ, int lddz, const float *X, int ldx, float *pW, int ldw, int64_t w_split_stride,
                     float *pB, int64_t b_split_stride, int M, int N, int K, int max_splits, cudaStream_t st);
-// out[M, N] = epilogue(X[M, K] * W[N, K]^T); mode 0: leaky(. + bias), 1: . * leaky'(act), 2: . + bias
+// out[M, N] = epilogue(X[M, K] * W[N, K]^T); mode 0: leaky(. + bias), 1: . * leaky'(act), 2: . + bias, 3: . (bare)
 // W_lo != nullptr: the weights come pre-split (W = TF32 hi halves, W_lo = lo halves, same layout; launch_split_tf32)
 void launch_tc_dense(const float *X, int ldx, const float *W, int ldw, const float *bias, const float *act,
                      int ldact, float *out, int ldo, int M, int N, int K, int mode, cudaStream_t st,
                      const float *W_lo = nullptr);
+// the same for n <= 8 independent problems of one (M, N, K, mode) in one launch (e.g. the critics of an ensemble);
+// each member's output equals the single-CTA launch_tc_dense of that member bit for bit
+struct TcDenseProblem { const float *X; int ldx; const float *W_hi, *W_lo; int ldw; const float *bias, *act; float *out; };
+void launch_tc_dense_ensemble(const TcDenseProblem *pr, int n, int ldact, int ldo, int M, int N, int K, int mode,
+                              cudaStream_t st);
 void launch_split_tf32(const float *src, float *hi, float *lo, int n, cudaStream_t st);
 
 // ---- optimiser (optim.cu) --------------------------------------------------------------

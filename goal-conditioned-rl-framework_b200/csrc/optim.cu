@@ -305,7 +305,7 @@ __device__ __forceinline__ void adam_body(const AdamArgs &a) {
     if (a.polyak) {
       const float t = a.tau * p + a.one_minus_tau * a.target[e];
       a.target[e] = t;
-      if (tm >= 0) a.targetT[tm] = t;
+      if (tm >= 0 && a.targetT != nullptr) a.targetT[tm] = t;     // (SAC / TQC targets keep no W^T)
     }
   }
   if (blockIdx.x == 0 && threadIdx.x == 0) {

@@ -578,11 +578,59 @@ __global__ void alpha_step_kernel(const float *__restrict__ mean_in, const float
 
 
 // ---- parameter containers ----------------------------------------------------------------------
+// Weight copies of the tensor-core engine (precision >= 1): the TF32 hi / lo halves of the flat parameter buffer (the
+// forward operand arrives pre-split, tc_gemm.cu) and, for the listed Linear layers of a trainable network, a
+// transposed copy W^T[in][ldt] with its halves (the K-major operand of the input gradient dX = dZ W).  The optimiser
+// writes W^T through tmap with every step; the halves are refreshed after every optimiser / Polyak step of an update
+// that runs on the tensor cores, and before an update after weights changed in any other way (`stale`).
+struct TcCopies {
+  std::vector<int> t_off, ldt;   // per Linear layer (-1: no transposed copy)
+  int total = 0, total_t = 0;
+  int *tmap = nullptr;           // [total] -> index into pT, -1 elsewhere; nullptr when nothing is transposed
+  float *pT = nullptr, *p_hi = nullptr, *p_lo = nullptr, *pT_hi = nullptr, *pT_lo = nullptr;
+  bool stale = true;
+  // transpose: (Linear index, w_off, rows, cols, ldw) of the layers whose input gradient runs on the tensor cores
+  void init(int total_, int nlinear, const std::vector<std::vector<int>> &transpose) {
+    total = total_;
+    t_off.assign(size_t(nlinear), -1);
+    ldt.assign(size_t(nlinear), 0);
+    p_hi = dev_alloc<float>(total); p_lo = dev_alloc<float>(total);
+    if (transpose.empty()) return;
+    std::vector<int> map(size_t(total), -1);
+    for (const auto &t : transpose) {
+      const int l = t[0], w_off = t[1], rows = t[2], cols = t[3], ldw = t[4];
+      ldt[l] = pad4(rows);
+      t_off[l] = total_t;
+      for (int o = 0; o < rows; ++o)
+        for (int i = 0; i < cols; ++i) map[size_t(w_off) + size_t(o) * ldw + i] = total_t + i * ldt[l] + o;
+      total_t += cols * ldt[l];
+    }
+    tmap = dev_alloc<int>(total);
+    GCRL_CUDA(cudaMemcpy(tmap, map.data(), size_t(total) * sizeof(int), cudaMemcpyHostToDevice));
+    pT = dev_alloc<float>(total_t);
+    GCRL_CUDA(cudaMemset(pT, 0, size_t(total_t) * 4));
+    pT_hi = dev_alloc<float>(total_t); pT_lo = dev_alloc<float>(total_t);
+  }
+  bool on() const { return p_hi != nullptr; }
+  void split(const float *p, cudaStream_t st) {
+    launch_split_tf32(p, p_hi, p_lo, total, st);
+    if (pT != nullptr) launch_split_tf32(pT, pT_hi, pT_lo, total_t, st);
+  }
+  // weights written from outside an update: W^T follows now, the halves before the next tensor-core update
+  void weights_changed(const float *p, cudaStream_t st) {
+    if (!on()) return;
+    if (tmap != nullptr) launch_sync_transposed(p, pT, tmap, total, st);
+    stale = true;
+  }
+  void destroy() { for (void *q : {(void *)tmap, (void *)pT, (void *)p_hi, (void *)p_lo, (void *)pT_hi, (void *)pT_lo}) if (q) cudaFree(q); }
+};
+
 struct CriticNet {
   int layers = 0;
   std::vector<int> in_d, out_d, ldw, w_off, b_off;
   int total = 0;
   float *p = nullptr, *g = nullptr, *m = nullptr, *v = nullptr;
+  TcCopies tc;
   void init(int in, int hid, int L, bool trainable, float *grad_store = nullptr) {
     layers = L + 1;
     int off = 0;
@@ -609,7 +657,15 @@ struct CriticNet {
     }
     return off;
   }
-  void destroy() { for (float *q : {p, m, v}) if (q) cudaFree(q); }
+  // tensor-core engine: halves of every critic; W^T of the hidden layers 1..L-1 of a trainable one (the input
+  // gradient of layer 0 is only needed at the action columns, action_grad_acc_kernel)
+  void init_tc(bool trainable) {
+    std::vector<std::vector<int>> tr;
+    if (trainable)
+      for (int l = 1; l < layers - 1; ++l) tr.push_back({l, w_off[l], out_d[l], in_d[l], ldw[l]});
+    tc.init(total, layers, tr);
+  }
+  void destroy() { for (float *q : {p, m, v}) if (q) cudaFree(q); tc.destroy(); }
   const float *W(int l) const { return p + w_off[l]; }
   const float *b(int l) const { return p + b_off[l]; }
 };
@@ -621,6 +677,12 @@ struct ActorNet {
   int total = 0;
   float *p = nullptr, *g = nullptr, *m = nullptr, *v = nullptr;
   float *rmean = nullptr, *rvar = nullptr;                  // [L][ldh]
+  TcCopies tc;
+  void init_tc() {                                          // W^T of the hidden Linears 1..L-1 (input gradients)
+    std::vector<std::vector<int>> tr;
+    for (int l = 1; l < L; ++l) tr.push_back({l, w_off[l], H, H, ldw[l]});
+    tc.init(total, L, tr);
+  }
   void init(int D_, int H_, int A_, int L_) {
     L = L_; D = D_; H = H_; A = A_; ldh = pad4(H);
     int off = 0;
@@ -648,7 +710,7 @@ struct ActorNet {
     for (int l = 0; l < L; ++l)   // BatchNorm weight = 1 (torch default)
       GCRL_CUDA(cudaMemcpy(p + gam_off[l], ones.data(), size_t(H) * 4, cudaMemcpyHostToDevice));
   }
-  void destroy() { for (float *q : {p, g, m, v, rmean}) if (q) cudaFree(q); }
+  void destroy() { for (float *q : {p, g, m, v, rmean}) if (q) cudaFree(q); tc.destroy(); }
 };
 
 }  // namespace
@@ -663,6 +725,7 @@ struct gcrl_sac {
   CriticNet critic[kMaxCritics], target[kMaxCritics];
   int adam_t_c = 0, adam_t_a = 0, adam_t_alpha = 0;
   int dp_B = -1, dp_flags = -1;                  // the update the data-parallel phases belong to
+  bool tc_update = false;                        // the update being recorded / issued runs on the tensor-core engine
   bool use_graphs = true;
   cudaStream_t cap_stream = nullptr;             // capture-only stream (the caller's may be the legacy one)
   struct GraphRec { cudaGraphExec_t exec; uint64_t kernels; };
@@ -728,12 +791,78 @@ void seg_cut(gcrl_sac *ag, int collective, bool last = false) {
   if (!last) GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
 }
 
-// The whole ensemble on the same input rows: one launch per layer (blockIdx.z = critic) instead of n.
+// ---- tensor-core engine (tcgen05, 3xTF32; precision >= 1) --------------------------------------------
+// Hidden-layer forward, input-gradient and weight-gradient GEMMs of an update.  precision 2: every batch >= 128 rows;
+// precision 1: once B * H^2 reaches the break-even measured against the fp32 tiles for SAC / TQC on a B200 (DESIGN.md
+// 4, profiles/r03_sac_precision.json): between 1024 and 2048 rows at H = 256, at or below 512 rows at H = 512 (the
+// ensemble's launches fill the SMs at fewer rows per member when the layers are wider).
+constexpr int64_t kSacTcMinWork = int64_t(2048) * 256 * 256;
+bool use_tc(const gcrl_sac *ag, int B, int N, int K) {
+  if (!tc_dense_supported(B, N, K)) return false;
+  return ag->cfg.precision == 2 ? B >= 128
+                                : (ag->cfg.precision == 1 && int64_t(B) * ag->H * ag->H >= kSacTcMinWork);
+}
+// every hidden-layer shape of an update passes the same test (K = padded input widths, all multiples of 4)
+bool engine_tc(const gcrl_sac *ag, int B) { return use_tc(ag, B, ag->H, ag->ldh); }
+
+template <class F>
+void for_each_tc(gcrl_sac *ag, F f) {
+  f(ag->actor.tc, ag->actor.p);
+  for (int i = 0; i < ag->n; ++i) {
+    f(ag->critic[i].tc, ag->critic[i].p);
+    f(ag->target[i].tc, ag->target[i].p);
+  }
+}
+// eager, outside capture: the halves of every network whose weights changed since they were last split
+void ensure_split(gcrl_sac *ag, cudaStream_t st) {
+  for_each_tc(ag, [&](TcCopies &tc, const float *p) {
+    if (tc.on() && tc.stale) {
+      tc.split(p, st);
+      tc.stale = false;
+    }
+  });
+}
+void mark_split_stale(gcrl_sac *ag) {
+  for_each_tc(ag, [](TcCopies &tc, const float *) { tc.stale = true; });
+}
+
+// partial weight / bias gradients of one hidden Linear [H][ldw] on input X[B][K] (K: padded for layer 0)
+int linear_wgrad(gcrl_sac *ag, const float *dZ, const float *X, int ldx, int K, bool tc_ok, float *pW, int ldw,
+                 float *pB, int B, cudaStream_t st) {
+  const int Kp = pad4(K);     // operand rows and weight rows are zero-padded to ld
+  if (ag->tc_update && tc_ok && tc_wgrad_supported(B, ag->H, Kp))
+    return launch_tc_wgrad(dZ, ag->ldh, X, ldx, pW, ldw, ag->slab, pB, ag->slab, B, ag->H, Kp, kSplits, st);
+  return launch_linear_wgrad(dZ, ag->ldh, X, ldx, pW, ldw, ag->slab, pB, ag->slab, B, ag->H, K, kSplits, st);
+}
+
+// Tensor cores: dX = dZ W (.) leaky'(act) of hidden layer l >= 1 for the critics first .. first + m - 1 in one launch
+// (gradients dz_in[j] -> dz_out[j]), with the transposed weight copies as the K-major operand
+void critics_dgrad_tc(gcrl_sac *ag, int first, int m, int l, float *const *dz_in, float *const *dz_out, int B,
+                      cudaStream_t st) {
+  TcDenseProblem pr[kMaxBatchedLinear];
+  for (int j = 0; j < m; ++j) {
+    const TcCopies &tc = ag->critic[first + j].tc;
+    pr[j] = TcDenseProblem{dz_in[j], ag->ldh, tc.pT_hi + tc.t_off[l], tc.pT_lo + tc.t_off[l], tc.ldt[l], nullptr,
+                           ag->ch[first + j][l - 1], dz_out[j]};
+  }
+  launch_tc_dense_ensemble(pr, m, ag->ldh, ag->ldh, B, ag->H, ag->H, 1, st);
+}
+
+// The whole ensemble on the same input rows: one launch per layer (blockIdx.z = critic, or the members of the
+// tensor-core ensemble launch) instead of n.
 // Activations land in ag->ch[i][l] (the caches of the backward pass, or plain scratch for the targets).
 void critics_fwd(gcrl_sac *ag, const CriticNet *nets, const float *X, float *q_out, int B, cudaStream_t st) {
   const int n = ag->n, L = ag->L;
   LinearFwdProblem pr[kMaxBatchedLinear];
+  TcDenseProblem tp[kMaxBatchedLinear];
   for (int l = 0; l < L; ++l) {
+    if (ag->tc_update) {      // layer 0: K = ldc, the operand rows [s | a | 0] and the weight rows are zero-padded
+      for (int i = 0; i < n; ++i)
+        tp[i] = TcDenseProblem{l == 0 ? X : ag->ch[i][l - 1], l == 0 ? ag->ldc : ag->ldh, nets[i].tc.p_hi + nets[i].w_off[l],
+                               nets[i].tc.p_lo + nets[i].w_off[l], nets[i].ldw[l], nets[i].b(l), nullptr, ag->ch[i][l]};
+      launch_tc_dense_ensemble(tp, n, 0, ag->ldh, B, ag->H, l == 0 ? ag->ldc : ag->H, 0, st);
+      continue;
+    }
     for (int i = 0; i < n; ++i)
       pr[i] = LinearFwdProblem{l == 0 ? X : ag->ch[i][l - 1], l == 0 ? ag->ldc : ag->ldh, nets[i].W(l), nets[i].ldw[l],
                                nets[i].b(l), ag->ch[i][l], ag->ldh};
@@ -752,8 +881,12 @@ void actor_fwd(gcrl_sac *ag, float *rows, const float *eps, int B, bool train, b
   const float *in = rows;
   int ldin = ag->ldc, K = ag->D;
   for (int l = 0; l < ag->L; ++l) {
-    launch_linear_fwd(in, ldin, a.p + a.w_off[l], a.ldw[l], a.p + a.b_off[l], ag->xhat[l], ag->ldh, B, ag->H, K,
-                      ACT_NONE, st);
+    if (train && ag->tc_update)       // (select_action, train == false, stays on the fp32 path)
+      launch_tc_dense(in, ldin, a.tc.p_hi + a.w_off[l], a.ldw[l], a.p + a.b_off[l], nullptr, 0, ag->xhat[l], ag->ldh, B,
+                      ag->H, pad4(K), 2, st, a.tc.p_lo + a.w_off[l]);
+    else
+      launch_linear_fwd(in, ldin, a.p + a.w_off[l], a.ldw[l], a.p + a.b_off[l], ag->xhat[l], ag->ldh, B, ag->H, K,
+                        ACT_NONE, st);
     if (train && ag->sync_world > 0) {
       GCRL_REQUIRE(ag->seg_build != nullptr, "a sync-BN agent trains through gcrl_sac_update_segment only");
       bn_stats_kernel<<<(ag->H + 31) / 32, dim3(32, 32), 0, st>>>(
@@ -802,8 +935,9 @@ void reduce_critic(gcrl_sac *ag, CriticNet &c, const int *splits, int head_split
   launch_reduce_grads(r, st);
 }
 
+// tc / ttc: the tensor-core copies of the network and of its target (no W^T: targetT stays nullptr)
 void adam(gcrl_sac *ag, float *p, float *m, float *v, const float *g, int total, int which, float *target,
-          bool polyak, int slot_norm, cudaStream_t st) {
+          bool polyak, int slot_norm, cudaStream_t st, TcCopies &tc, TcCopies *ttc) {
   AdamArgs a{};
   a.p = p; a.m = m; a.v = v; a.g = g; a.n = total;
   a.sumsq_partials = ag->sumsq; a.nsumsq = reduce_grid(total);
@@ -813,8 +947,17 @@ void adam(gcrl_sac *ag, float *p, float *m, float *v, const float *g, int total,
   a.target = target; a.tau = ag->cfg.tau; a.one_minus_tau = float(1.0 - double(ag->cfg.tau));
   a.polyak = (polyak && target) ? 1 : 0;
   a.metrics = ag->mdev; a.slot_norm = slot_norm;
-  a.tmap = nullptr; a.pT = nullptr; a.targetT = nullptr;
+  a.tmap = tc.tmap; a.pT = tc.pT; a.targetT = nullptr;
   launch_adam(a, st);
+  if (ag->tc_update) {          // this update's later GEMMs read the stepped weights through the tensor cores
+    tc.split(p, st);
+    if (a.polyak && ttc != nullptr) ttc->split(target, st);
+  }
+}
+
+void adam_critic(gcrl_sac *ag, int i, int flags, cudaStream_t st) {
+  CriticNet &c = ag->critic[i];
+  adam(ag, c.p, c.m, c.v, c.g, c.total, 0, ag->target[i].p, (flags & 2) != 0, M_CGN + i, st, c.tc, &ag->target[i].tc);
 }
 
 // sums of squares of an (averaged) flat gradient that is already in place
@@ -879,8 +1022,18 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
         wp[i] = WgradProblem{ag->dzc[2 * i + cur], ag->ldh, l == 0 ? ag->sa : ag->ch[i][l - 1], l == 0 ? ag->ldc : ag->ldh,
                              part + c.w_off[l], c.ldw[l], part + c.b_off[l], ag->H, l == 0 ? K0 : ag->H};
       }
-      splits[l] = launch_multi_wgrad(wp, n, B, ag->slab, kSplits, st);
-      if (l > 0) {
+      if (ag->tc_update) {       // per critic: the slabs of one weight-gradient launch already fill the SMs
+        for (int i = 0; i < n; ++i)
+          splits[l] = linear_wgrad(ag, wp[i].dZ, wp[i].X, wp[i].ldx, wp[i].K, true, wp[i].pW, wp[i].ldw, wp[i].pB, B, st);
+      } else {
+        splits[l] = launch_multi_wgrad(wp, n, B, ag->slab, kSplits, st);
+      }
+      if (l > 0 && ag->tc_update) {
+        float *din[kMaxBatchedLinear], *dout[kMaxBatchedLinear];
+        for (int i = 0; i < n; ++i) { din[i] = ag->dzc[2 * i + cur]; dout[i] = ag->dzc[2 * i + (cur ^ 1)]; }
+        critics_dgrad_tc(ag, 0, n, l, din, dout, B, st);
+        cur ^= 1;
+      } else if (l > 0) {
         LinearDgradProblem dg[kMaxBatchedLinear];
         for (int i = 0; i < n; ++i) {
           const CriticNet &c = ag->critic[i];
@@ -894,7 +1047,7 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     for (int i = 0; i < n; ++i) {
       CriticNet &c = ag->critic[i];
       reduce_critic(ag, c, splits, head_splits, st, ag->partials + int64_t(i) * ag->pset);
-      if (!dp) adam(ag, c.p, c.m, c.v, c.g, c.total, 0, ag->target[i].p, (flags & 2) != 0, M_CGN + i, st);
+      if (!dp) adam_critic(ag, i, flags, st);
     }
   } else
   for (int i = 0; i < n; ++i) {
@@ -917,16 +1070,19 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
       const float *xin = l == 0 ? ag->sa : ag->ch[i][l - 1];
       const int ldin = l == 0 ? ag->ldc : ag->ldh;
       const int K = l == 0 ? K0 : ag->H;
-      splits[l] = launch_linear_wgrad(ag->dz[cur], ag->ldh, xin, ldin, ag->partials + c.w_off[l], c.ldw[l], ag->slab,
-                                      ag->partials + c.b_off[l], ag->slab, B, ag->H, K, kSplits, st);
+      splits[l] = linear_wgrad(ag, ag->dz[cur], xin, ldin, K, true, ag->partials + c.w_off[l], c.ldw[l],
+                               ag->partials + c.b_off[l], B, st);
       if (l > 0) {
-        launch_linear_dgrad(ag->dz[cur], ag->ldh, c.W(l), c.ldw[l], ag->ch[i][l - 1], ag->ldh, ag->dz[cur ^ 1],
-                            ag->ldh, B, ag->H, ag->H, st);
+        if (ag->tc_update)
+          critics_dgrad_tc(ag, i, 1, l, &ag->dz[cur], &ag->dz[cur ^ 1], B, st);
+        else
+          launch_linear_dgrad(ag->dz[cur], ag->ldh, c.W(l), c.ldw[l], ag->ch[i][l - 1], ag->ldh, ag->dz[cur ^ 1],
+                              ag->ldh, B, ag->H, ag->H, st);
         cur ^= 1;
       }
     }
     reduce_critic(ag, c, splits, head_splits, st);
-    if (!dp) adam(ag, c.p, c.m, c.v, c.g, c.total, 0, ag->target[i].p, (flags & 2) != 0, M_CGN + i, st);
+    if (!dp) adam_critic(ag, i, flags, st);
   }
   }
   if (ag->seg_build != nullptr) seg_cut(ag, COLL_AVG_CRITIC);
@@ -934,7 +1090,7 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     for (int i = 0; i < n; ++i) {
       CriticNet &c = ag->critic[i];
       rereduce(ag, c.g, c.total, st);
-      adam(ag, c.p, c.m, c.v, c.g, c.total, 0, ag->target[i].p, (flags & 2) != 0, M_CGN + i, st);
+      adam_critic(ag, i, flags, st);
     }
   }
   if (tqc && (mask & PH_CSTEP)) {   // logged Q = mean over the STEPPED critics (:1016-1019)
@@ -971,6 +1127,13 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     launch_head_bwd_batched(hs, n, kSplits, st);
     int cur = 0;
     for (int l = L - 1; l >= 1; --l) {
+      if (ag->tc_update) {
+        float *din[kMaxBatchedLinear], *dout[kMaxBatchedLinear];
+        for (int i = 0; i < n; ++i) { din[i] = ag->dzc[2 * i + cur]; dout[i] = ag->dzc[2 * i + (cur ^ 1)]; }
+        critics_dgrad_tc(ag, 0, n, l, din, dout, B, st);
+        cur ^= 1;
+        continue;
+      }
       LinearDgradProblem dg[kMaxBatchedLinear];
       for (int i = 0; i < n; ++i) {
         const CriticNet &c = ag->critic[i];
@@ -999,8 +1162,11 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     launch_head_bwd(h, kSplits, st);
     int cur = 0;
     for (int l = L - 1; l >= 1; --l) {
-      launch_linear_dgrad(ag->dz[cur], ag->ldh, c.W(l), c.ldw[l], ag->ch[i][l - 1], ag->ldh, ag->dz[cur ^ 1], ag->ldh,
-                          B, ag->H, ag->H, st);
+      if (ag->tc_update)
+        critics_dgrad_tc(ag, i, 1, l, &ag->dz[cur], &ag->dz[cur ^ 1], B, st);
+      else
+        launch_linear_dgrad(ag->dz[cur], ag->ldh, c.W(l), c.ldw[l], ag->ch[i][l - 1], ag->ldh, ag->dz[cur ^ 1], ag->ldh,
+                            B, ag->H, ag->H, st);
       cur ^= 1;
     }
     action_grad_acc_kernel<<<blocks_for(B, 8), 256, 0, st>>>(ag->dz[cur], ag->ldh, c.W(0), c.ldw[0], D, ag->dact, B,
@@ -1043,11 +1209,16 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     const float *xin = l == 0 ? ag->spi : ag->ah[l - 1];
     const int ldin = l == 0 ? ag->ldc : ag->ldh;
     const int K = l == 0 ? D : ag->H;
-    splits[l] = launch_linear_wgrad(ag->dz[cur], ag->ldh, xin, ldin, ag->partials + a.w_off[l], a.ldw[l], ag->slab,
-                                    ag->partials + a.b_off[l], ag->slab, B, ag->H, K, kSplits, st);
+    // layer 0 on the tensor cores only when K needs no padding: the columns D.. of spi hold the sampled action now
+    splits[l] = linear_wgrad(ag, ag->dz[cur], xin, ldin, K, l > 0 || D % 4 == 0, ag->partials + a.w_off[l], a.ldw[l],
+                             ag->partials + a.b_off[l], B, st);
     if (l > 0) {
-      launch_linear_dgrad(ag->dz[cur], ag->ldh, a.p + a.w_off[l], a.ldw[l], nullptr, 0, ag->dz[cur ^ 1], ag->ldh, B,
-                          ag->H, ag->H, st);
+      if (ag->tc_update)      // bare product: bn_bwd applies ReLU' itself
+        launch_tc_dense(ag->dz[cur], ag->ldh, a.tc.pT_hi + a.tc.t_off[l], a.tc.ldt[l], nullptr, nullptr, 0,
+                        ag->dz[cur ^ 1], ag->ldh, B, ag->H, ag->H, 3, st, a.tc.pT_lo + a.tc.t_off[l]);
+      else
+        launch_linear_dgrad(ag->dz[cur], ag->ldh, a.p + a.w_off[l], a.ldw[l], nullptr, 0, ag->dz[cur ^ 1], ag->ldh, B,
+                            ag->H, ag->H, st);
       cur ^= 1;
     }
   }
@@ -1073,7 +1244,7 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   if (ag->seg_build != nullptr) seg_cut(ag, COLL_AVG_ACTOR);
   if (mask & PH_ASTEP) {
     if (dp) rereduce(ag, a.g, a.total, st);
-    adam(ag, a.p, a.m, a.v, a.g, a.total, 1, nullptr, false, M_AGN, st);
+    adam(ag, a.p, a.m, a.v, a.g, a.total, 1, nullptr, false, M_AGN, st, a.tc, nullptr);
     if (flags & 4) {
       alpha_step_kernel<<<1, 1, 0, st>>>(a.g + a.total, reinterpret_cast<const float *>(ag->d_scalars + 1),
                                         ag->alpha_state, ag->mdev + M_ALPHA_LOSS);
@@ -1179,6 +1350,9 @@ void sac_update(gcrl_sac *ag, int phase, gcrl_her *buf, int64_t B64, const int64
   GCRL_REQUIRE(ag != nullptr, "agent handle is NULL");
   GCRL_REQUIRE(B64 >= 2 && B64 <= ag->maxB, "batch size outside [2, max_batch] (BatchNorm needs > 1 row)");
   const int B = int(B64);
+  ag->tc_update = engine_tc(ag, B);
+  if (ag->tc_update) ensure_split(ag, st);          // (the update itself re-splits what it steps)
+  else mark_split_stale(ag);                        // weights move without their split copies following
   if (seg > 0) {
     GCRL_REQUIRE(ag->dp_B == B && ag->dp_flags == flags, "segment > 0 must follow segment 0 of the same update");
     *collective = run_segment(ag, B, flags, seg, st);
@@ -1319,6 +1493,7 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
   GCRL_REQUIRE(cfg->n_critics >= 1 && cfg->n_critics <= kMaxCritics, "n_critics outside [1, 8]");
   GCRL_REQUIRE(cfg->drop_top >= 0 && cfg->drop_top < cfg->n_critics, "drop_top outside [0, n_critics)");
   GCRL_REQUIRE(cfg->max_batch >= 2 && cfg->max_batch <= kSplits * 256, "max_batch outside [2, 32768]");
+  GCRL_REQUIRE(cfg->precision >= 0 && cfg->precision <= 2, "precision must be 0 (fp32 FFMA), 1 (tensor cores for large batches) or 2 (tensor cores whenever supported)");
   GCRL_CUDA(cudaSetDevice(device));
   auto *ag = new gcrl_sac();
   try {
@@ -1361,6 +1536,14 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
     const float init_alpha[4] = {0.f, 1.f, 0.f, 0.f};       // log_alpha = 0 (:424)
     GCRL_CUDA(cudaMemcpy(ag->alpha_state, init_alpha, sizeof(init_alpha), cudaMemcpyHostToDevice));
     ag->d_scalars = dev_alloc<StepScalars>(2);
+    if (cfg->precision >= 1) {
+      tc_dense_init();
+      ag->actor.init_tc();
+      for (int i = 0; i < n; ++i) {
+        ag->critic[i].init_tc(true);
+        ag->target[i].init_tc(false);
+      }
+    }
     GCRL_CUDA(cudaStreamCreateWithFlags(&ag->cap_stream, cudaStreamNonBlocking));
     const char *ng = getenv("GCRL_B200_NO_GRAPH");
     ag->use_graphs = !(ng && ng[0] == '1');
@@ -1409,6 +1592,7 @@ int gcrl_sac_set_actor_linear(gcrl_sac *ag, int layer, const float *w, const flo
   actor_linear_geom(ag, layer, &rows, &cols, &ld, &woff, &boff);
   upload_padded(ag->actor.p + woff, w, rows, cols, ld, as_stream(stream));
   upload_padded(ag->actor.p + boff, b, 1, rows, rows, as_stream(stream));
+  ag->actor.tc.weights_changed(ag->actor.p, as_stream(stream));
   GCRL_API_END
 }
 
@@ -1463,6 +1647,7 @@ int gcrl_sac_set_critic_layer(gcrl_sac *ag, int critic, int target, int layer, c
   GCRL_CUDA(cudaSetDevice(ag->device));
   upload_padded(c.p + c.w_off[layer], w, c.out_d[layer], c.in_d[layer], c.ldw[layer], as_stream(stream));
   upload_padded(c.p + c.b_off[layer], b, 1, c.out_d[layer], c.out_d[layer], as_stream(stream));
+  c.tc.weights_changed(c.p, as_stream(stream));
   GCRL_API_END
 }
 
@@ -1483,9 +1668,11 @@ int gcrl_sac_hard_update(gcrl_sac *ag, void *stream) {
   require_handle(ag);
   GCRL_REQUIRE(ag != nullptr, "agent handle is NULL");
   GCRL_CUDA(cudaSetDevice(ag->device));
-  for (int i = 0; i < ag->n; ++i)
+  for (int i = 0; i < ag->n; ++i) {
     GCRL_CUDA(cudaMemcpyAsync(ag->target[i].p, ag->critic[i].p, size_t(ag->critic[i].total) * 4,
                               cudaMemcpyDeviceToDevice, as_stream(stream)));
+    ag->target[i].tc.weights_changed(ag->target[i].p, as_stream(stream));
+  }
   GCRL_API_END
 }
 

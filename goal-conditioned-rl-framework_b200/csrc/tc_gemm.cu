@@ -216,6 +216,7 @@ struct TcArgs {
   int acc_slabs;                 // kind 1: a CTA adds the later slabs of its (n, k) block onto the first one it wrote
   float *colsum;                 // kind 1: bias-gradient partials pB[slab][n] = column sums of the slab's dZ rows, taken
   long long colsum_stride;       // by the splitter warps from the tiles they split anyway (nullptr: separate kernel)
+  int members;                   // ensemble kernel (NMEM > 1): problems of this shape in the launch
   int full_items;                // pair kernel: tiles taken whole; the rest are split into two 256 x 128 halves
   long long *trace;              // GCRL_TC_TRACE: per-stage timestamps of the first CTA pair (pair kernel only)
   int dbg;                       // timing experiments only (GCRL_TC_DBG): 1 skip split, 2 skip stores, 4 one MMA per k
@@ -230,14 +231,25 @@ struct TcSmem {
   static constexpr int kBytes = STAGES * kStage + 1024 /*alignment slack*/ + 256 /*barriers*/ + 4 * 32 * kStgLd * 4 + kColsum;
 };
 
+// Operands of the launch: tensor maps A (activations), B (weights, or their TF32 hi halves), B lo halves (PRESPLIT)
+// per member.  NMEM = 1: one problem, epilogue pointers in TcArgs.  NMEM > 1 (ensemble, e.g. the critics of one
+// layer): a.members independent problems of the same (M, N, K, mode), each with its own epilogue pointers.
+template <int NMEM>
+struct TcOperands {
+  CUtensorMap map[NMEM][3];
+  float *out[NMEM];
+  const float *bias[NMEM];
+  const float *act[NMEM];
+};
+constexpr int kTcMaxMembers = 8;
+
 // PRESPLIT: the B operand (the layer's weights) arrives already split into TF32 hi / lo halves (two tensors, kept
 // next to the parameters and refreshed after every optimiser step): the producer loads both, the splitter warps only
 // handle the activation tile -- a third of the shared-memory passes they made over a stage, off the TMA -> MMA
 // critical path for 2/3 of the bytes.
-template <int BN, bool PRESPLIT>
+template <int BN, bool PRESPLIT, int NMEM>
 __global__ void __launch_bounds__(kTcThreads, 1)
-tc_dense_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                const __grid_constant__ CUtensorMap tmB2, TcArgs a) {
+tc_dense_kernel(const __grid_constant__ TcOperands<NMEM> ops, TcArgs a) {
   extern __shared__ uint8_t smem_raw[];
   using S = TcSmem<BN>;
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -275,13 +287,19 @@ tc_dense_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
 
   const bool wg = a.kind == 1;
-  const int total_tiles = wg ? a.nslabs * a.n_tiles * a.k_tiles : a.m_tiles * a.n_tiles;
-  // tile decode.  dense: (m block, n block), K tiles of BKF columns.  wgrad: (slab, n block, k block),
+  const int per_member = a.m_tiles * a.n_tiles;
+  const int total_tiles = wg ? a.nslabs * a.n_tiles * a.k_tiles : (NMEM > 1 ? a.members : 1) * per_member;
+  // tile decode.  dense: (member, m block, n block), K tiles of BKF columns.  wgrad: (slab, n block, k block),
   // "K tiles" = 16 batch rows each.
-  struct Tile { int m0, n0, nk, slab, out_slab, acc; };
+  struct Tile { int m0, n0, nk, slab, out_slab, acc, mem; };
   auto decode = [&](int t) {
     Tile ti;
+    ti.mem = 0;
     if (!wg) {
+      if (NMEM > 1) {
+        ti.mem = t / per_member;
+        t -= ti.mem * per_member;
+      }
       ti.m0 = (t / a.n_tiles) * BM; ti.n0 = (t % a.n_tiles) * BN; ti.nk = (a.K + BKF - 1) / BKF; ti.slab = 0;
       ti.out_slab = 0; ti.acc = 0;
     } else {
@@ -310,18 +328,19 @@ tc_dense_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         mbar_wait(empty(s), ((it / STAGES) & 1) ^ 1);
         const uint32_t st = base + s * S::kStage;
         if (elect_one()) {
+          const CUtensorMap *tm = ops.map[ti.mem];
           mbar_expect_tx(full(s), S::kA + (PRESPLIT ? 2 : 1) * S::kB);
           if (!wg) {
-            tma_load_2d(st, &tmA, full(s), kb * BKF, ti.m0);
-            tma_load_2d(st + 2 * S::kA, &tmB, full(s), kb * BKF, ti.n0);
-            if (PRESPLIT) tma_load_2d(st + 2 * S::kA + S::kB, &tmB2, full(s), kb * BKF, ti.n0);
+            tma_load_2d(st, &tm[0], full(s), kb * BKF, ti.m0);
+            tma_load_2d(st + 2 * S::kA, &tm[1], full(s), kb * BKF, ti.n0);
+            if (PRESPLIT) tma_load_2d(st + 2 * S::kA + S::kB, &tm[2], full(s), kb * BKF, ti.n0);
           } else {
             // boxes of 16 batch rows x 32 features (128-byte swizzle, 32-byte atoms), one per 32-feature MN block
             const int r = ti.slab * a.rows_per_slab + kb * 16;
 #pragma unroll 1
-            for (int b = 0; b < BM / 32; ++b) tma_load_2d(st + b * 2048, &tmA, full(s), ti.m0 + 32 * b, r);
+            for (int b = 0; b < BM / 32; ++b) tma_load_2d(st + b * 2048, &tm[0], full(s), ti.m0 + 32 * b, r);
 #pragma unroll 1
-            for (int b = 0; b < BN / 32; ++b) tma_load_2d(st + 2 * S::kA + b * 2048, &tmB, full(s), ti.n0 + 32 * b, r);
+            for (int b = 0; b < BN / 32; ++b) tma_load_2d(st + 2 * S::kA + b * 2048, &tm[1], full(s), ti.n0 + 32 * b, r);
           }
         }
         __syncwarp();
@@ -379,7 +398,10 @@ tc_dense_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       const Tile ti = decode(t);
       const int m0 = ti.m0, n0 = ti.n0;
       const int rows_valid = wg ? a.N : a.M, cols_valid = wg ? a.ldo : a.N;
-      float *const obase = a.out + (wg ? size_t(ti.out_slab) * size_t(a.split_stride) : size_t(0));
+      float *const out = NMEM > 1 ? ops.out[ti.mem] : a.out;
+      const float *const bias = NMEM > 1 ? ops.bias[ti.mem] : a.bias;
+      const float *const act = NMEM > 1 ? ops.act[ti.mem] : a.act;
+      float *const obase = out + (wg ? size_t(ti.out_slab) * size_t(a.split_stride) : size_t(0));
       const int emode = (wg && ti.acc) ? 4 : a.mode;
       const int as = tile_it & 1;
       mbar_wait(tfull(as), (tile_it >> 1) & 1);
@@ -404,7 +426,7 @@ tc_dense_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                        : "memory");
         __syncwarp();
         if (!(a.dbg & 2))
-          epilogue_store32(stg, lane, m0 + q * 32, n0 + c, rows_valid, cols_valid, emode, a.bias, a.act, a.ldact, obase,
+          epilogue_store32(stg, lane, m0 + q * 32, n0 + c, rows_valid, cols_valid, emode, bias, act, a.ldact, obase,
                            a.ldo);
       }
       tc_fence_before();
@@ -880,10 +902,12 @@ template <int BN>
 void set_attr() {
   static bool attr_set = false;
   if (!attr_set) {
-    GCRL_CUDA(cudaFuncSetAttribute(tc_dense_kernel<BN, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    GCRL_CUDA(cudaFuncSetAttribute(tc_dense_kernel<BN, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    TcSmem<BN>::kBytes));
-    GCRL_CUDA(cudaFuncSetAttribute(tc_dense_kernel<BN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    GCRL_CUDA(cudaFuncSetAttribute(tc_dense_kernel<BN, true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    TcSmem<BN>::kBytes));
+    GCRL_CUDA(cudaFuncSetAttribute(tc_dense_kernel<BN, true, kTcMaxMembers>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<BN>::kBytes));
     attr_set = true;
   }
 }
@@ -894,10 +918,22 @@ void launch_bn(const CUtensorMap &tmA, const CUtensorMap &tmB, const CUtensorMap
   set_attr<BN>();
   const int tiles = a.kind == 1 ? a.nslabs * a.n_tiles * a.k_tiles : a.m_tiles * a.n_tiles;
   const int grid = grid_wg > 0 ? grid_wg : std::min(tiles, sm_count());
+  TcOperands<1> ops{};
+  ops.map[0][0] = tmA;
+  ops.map[0][1] = tmB;
+  ops.map[0][2] = tmB2 != nullptr ? *tmB2 : tmB;
   if (tmB2 != nullptr)
-    tc_dense_kernel<BN, true><<<grid, kTcThreads, TcSmem<BN>::kBytes, st>>>(tmA, tmB, *tmB2, a);
+    tc_dense_kernel<BN, true, 1><<<grid, kTcThreads, TcSmem<BN>::kBytes, st>>>(ops, a);
   else
-    tc_dense_kernel<BN, false><<<grid, kTcThreads, TcSmem<BN>::kBytes, st>>>(tmA, tmB, tmB, a);
+    tc_dense_kernel<BN, false, 1><<<grid, kTcThreads, TcSmem<BN>::kBytes, st>>>(ops, a);
+  GCRL_LAUNCHED();
+}
+
+template <int BN>
+void launch_bn_ensemble(const TcOperands<kTcMaxMembers> &ops, const TcArgs &a, cudaStream_t st) {
+  set_attr<BN>();
+  const int grid = std::min(a.members * a.m_tiles * a.n_tiles, sm_count());
+  tc_dense_kernel<BN, true, kTcMaxMembers><<<grid, kTcThreads, TcSmem<BN>::kBytes, st>>>(ops, a);
   GCRL_LAUNCHED();
 }
 
@@ -943,19 +979,25 @@ bool tc_dense_supported(int M, int N, int K) {
   return M >= 1 && N >= 16 && (N % 16) == 0 && K >= 4 && (K % 4) == 0 && (N <= 256 || N % 256 == 0);
 }
 
+// Column tile of a dense launch of `members` problems: as wide as the layer when the row tiles of all members alone
+// fill the SMs (the activation tile is then loaded and split once), narrower when the batch is small so that more
+// CTAs share the work.
+static int dense_column_tile(int M, int N, int members) {
+  int BN = N <= 64 ? 64 : (N <= 128 ? 128 : 256);
+  const int m_tiles_ = (M + BM - 1) / BM;
+  while (BN > 64 && members * m_tiles_ * ((N + BN - 1) / BN) < (sm_count() * 3) / 4) BN >>= 1;
+  if (const char *e = getenv("GCRL_TC_BN")) BN = atoi(e);
+  return BN;
+}
+
 // out[M, N] = epilogue( X[M, K] * W[N, K]^T )
-//   mode 0: leaky(. + bias)   mode 1: . * leaky'(act)   mode 2: . + bias
+//   mode 0: leaky(. + bias)   mode 1: . * leaky'(act)   mode 2: . + bias   mode 3: . (bare product)
 void launch_tc_dense(const float *X, int ldx, const float *W, int ldw, const float *bias, const float *act,
                      int ldact, float *out, int ldo, int M, int N, int K, int mode, cudaStream_t st,
                      const float *W_lo) {
   GCRL_REQUIRE(tc_dense_supported(M, N, K), "shape not supported by the tensor-core dense kernel");
   GCRL_REQUIRE((ldx % 4) == 0 && (ldw % 4) == 0 && (ldo % 4) == 0, "leading dimensions must be multiples of 4");
-  // column tile: as wide as the layer when the row tiles alone fill the SMs (the activation tile is then
-  // loaded and split once), narrower when the batch is small so that more CTAs share the work
-  int BN = N <= 64 ? 64 : (N <= 128 ? 128 : 256);
-  const int m_tiles_ = (M + BM - 1) / BM;
-  while (BN > 64 && m_tiles_ * ((N + BN - 1) / BN) < (sm_count() * 3) / 4) BN >>= 1;
-  if (const char *e = getenv("GCRL_TC_BN")) BN = atoi(e);
+  const int BN = dense_column_tile(M, N, 1);
   TcArgs a{};
   a.out = out; a.ldo = ldo; a.bias = bias; a.act = act; a.ldact = ldact;
   a.M = M; a.N = N; a.K = K; a.mode = mode;
@@ -1006,6 +1048,39 @@ void launch_tc_dense(const float *X, int ldx, const float *W, int ldw, const flo
   if (BN == 64) launch_bn<64>(tmA, tmB, p2, a, st);
   else if (BN == 128) launch_bn<128>(tmA, tmB, p2, a, st);
   else launch_bn<256>(tmA, tmB, p2, a, st);
+}
+
+// n independent problems of one shape in one launch (pre-split weights); every member's output is what
+// launch_tc_dense computes for it alone.  One member goes through launch_tc_dense itself (CTA pairs included).
+void launch_tc_dense_ensemble(const TcDenseProblem *pr, int n, int ldact, int ldo, int M, int N, int K, int mode,
+                              cudaStream_t st) {
+  GCRL_REQUIRE(n >= 1 && n <= kTcMaxMembers, "ensemble of 1..8 problems");
+  if (n == 1) {
+    launch_tc_dense(pr[0].X, pr[0].ldx, pr[0].W_hi, pr[0].ldw, pr[0].bias, pr[0].act, ldact, pr[0].out, ldo, M, N, K,
+                    mode, st, pr[0].W_lo);
+    return;
+  }
+  GCRL_REQUIRE(tc_dense_supported(M, N, K), "shape not supported by the tensor-core dense kernel");
+  GCRL_REQUIRE((ldo % 4) == 0, "leading dimensions must be multiples of 4");
+  const int BN = dense_column_tile(M, N, n);
+  TcArgs a{};
+  a.ldo = ldo; a.ldact = ldact;
+  a.M = M; a.N = N; a.K = K; a.mode = mode;
+  a.m_tiles = (M + BM - 1) / BM;
+  a.n_tiles = (N + BN - 1) / BN;
+  a.members = n;
+  TcOperands<kTcMaxMembers> ops{};
+  for (int i = 0; i < n; ++i) {
+    GCRL_REQUIRE(pr[i].W_lo != nullptr && (pr[i].ldx % 4) == 0 && (pr[i].ldw % 4) == 0,
+                 "ensemble members need pre-split weights and leading dimensions that are multiples of 4");
+    ops.map[i][0] = make_map(pr[i].X, M, K, pr[i].ldx, BM);
+    ops.map[i][1] = make_map(pr[i].W_hi, N, K, pr[i].ldw, BN);
+    ops.map[i][2] = make_map(pr[i].W_lo, N, K, pr[i].ldw, BN);
+    ops.out[i] = pr[i].out; ops.bias[i] = pr[i].bias; ops.act[i] = pr[i].act;
+  }
+  if (BN == 64) launch_bn_ensemble<64>(ops, a, st);
+  else if (BN == 128) launch_bn_ensemble<128>(ops, a, st);
+  else launch_bn_ensemble<256>(ops, a, st);
 }
 
 // hi = rna_tf32(x), lo = rna_tf32(x - hi): the halves the 3xTF32 product is built from
@@ -1112,10 +1187,34 @@ extern "C" int gcrl_dense_layer_presplit(int device, int mode, int64_t M, int N,
   GCRL_API_BEGIN
   using namespace gcrl;
   GCRL_REQUIRE(x_dev && w_hi_dev && w_lo_dev && y_dev && M >= 1 && M < (int64_t(1) << 31), "bad argument");
-  GCRL_REQUIRE(mode >= 0 && mode <= 2 && (mode == 1 ? act_dev != nullptr : bias_dev != nullptr), "bad mode / operands");
+  GCRL_REQUIRE(mode >= 0 && mode <= 3 && (mode == 1 ? act_dev != nullptr : (mode == 3 || bias_dev != nullptr)),
+               "bad mode / operands");
   GCRL_CUDA(cudaSetDevice(device));
   launch_tc_dense(x_dev, ldx, w_hi_dev, ldw, bias_dev, act_dev, ldact, y_dev, ldy, int(M), N, K, mode, as_stream(stream),
                   w_lo_dev);
+  GCRL_API_END
+}
+
+extern "C" int gcrl_dense_layer_ensemble(int device, int n, int mode, int64_t M, int N, int K,
+                                         const float *const *x_dev, int ldx, const float *const *w_hi_dev,
+                                         const float *const *w_lo_dev, int ldw, const float *const *bias_dev,
+                                         const float *const *act_dev, int ldact, float *const *y_dev, int ldy,
+                                         void *stream) {
+  GCRL_API_BEGIN
+  using namespace gcrl;
+  GCRL_REQUIRE(n >= 1 && n <= 8 && x_dev && w_hi_dev && w_lo_dev && y_dev && M >= 1 && M < (int64_t(1) << 31),
+               "bad argument");
+  GCRL_REQUIRE(mode >= 0 && mode <= 3 && (mode == 1 ? act_dev != nullptr : (mode == 3 || bias_dev != nullptr)),
+               "bad mode / operands");
+  TcDenseProblem pr[8];
+  for (int i = 0; i < n; ++i) {
+    GCRL_REQUIRE(x_dev[i] && w_hi_dev[i] && w_lo_dev[i] && y_dev[i], "NULL member operand");
+    GCRL_REQUIRE(mode == 3 || (mode == 1 ? act_dev[i] != nullptr : bias_dev[i] != nullptr), "NULL member operand");
+    pr[i] = TcDenseProblem{x_dev[i], ldx, w_hi_dev[i], w_lo_dev[i], ldw, (mode == 0 || mode == 2) ? bias_dev[i] : nullptr,
+                           mode == 1 ? act_dev[i] : nullptr, y_dev[i]};
+  }
+  GCRL_CUDA(cudaSetDevice(device));
+  launch_tc_dense_ensemble(pr, n, ldact, ldy, int(M), N, K, mode, as_stream(stream));
   GCRL_API_END
 }
 

@@ -38,7 +38,7 @@ class SacConfig(C.Structure):
     _fields_ = [("algo", c_i32), ("state_dim", c_i32), ("act_dim", c_i32), ("hidden_dim", c_i32),
                 ("layer_count", c_i32), ("max_batch", c_i32), ("n_critics", c_i32), ("drop_top", c_i32),
                 ("gamma", c_f32), ("tau", c_f32), ("grad_clip", c_f32), ("weight_decay", c_f32),
-                ("entropy_coef", c_f32), ("target_entropy", c_f32), ("alpha_lr", c_f32), ("reserved", c_i32)]
+                ("entropy_coef", c_f32), ("target_entropy", c_f32), ("alpha_lr", c_f32), ("precision", c_i32)]
 
 
 # name -> (restype, argtypes); every symbol include/gcrl_b200.h declares
@@ -144,6 +144,8 @@ SIGNATURES = {
     "gcrl_split_tf32": (C.c_int, [C.c_int, vp, vp, vp, c_i64, vp]),
     "gcrl_dense_layer_presplit": (C.c_int, [C.c_int, C.c_int, c_i64, C.c_int, C.c_int, vp, C.c_int, vp, vp, C.c_int, vp, vp,
                                             C.c_int, vp, C.c_int, vp]),
+    "gcrl_dense_layer_ensemble": (C.c_int, [C.c_int, C.c_int, C.c_int, c_i64, C.c_int, C.c_int, pp, C.c_int, pp, pp,
+                                            C.c_int, pp, pp, C.c_int, pp, C.c_int, vp]),
     "gcrl_dense_wgrad": (C.c_int, [C.c_int, C.c_int, c_i64, C.c_int, C.c_int, vp, C.c_int, vp, C.c_int, vp, C.c_int, c_i64,
                                    vp, c_i64, C.c_int, C.POINTER(C.c_int), vp]),
     "gcrl_dense_layer": (C.c_int, [C.c_int, C.c_int, C.c_int, c_i64, C.c_int, C.c_int, vp, C.c_int, vp, C.c_int, vp,

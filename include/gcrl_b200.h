@@ -304,7 +304,12 @@ typedef struct gcrl_sac_config {
                               learned alpha = exp(log_alpha) (TQC, :928,:978)                  */
   float target_entropy;    /* SAC -A/2 (:423); TQC -A (:815)                                   */
   float alpha_lr;          /* SACAgentConfig.alpha_lr, src/utils.py:37                         */
-  int32_t reserved;
+  int32_t precision;       /* 0 = fp32 FFMA everywhere; 1 = the critics' and the actor's hidden-layer forward,
+                              input-gradient and weight-gradient GEMMs on tcgen05 tensor cores (3xTF32 split,
+                              fp32-level accuracy; the critic ensemble in one launch per layer) once
+                              B * H^2 >= 2048 * 256^2 (B = batch, H = hidden_dim: 2048 rows at H = 256, 512 at
+                              H = 512, 8192 at H = 128); 2 = the same for every batch >= 128 rows (tests).
+                              select_action stays on the fp32 path.  Other values: GCRL_ERR_INVALID          */
 } gcrl_sac_config;
 
 int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg);
@@ -475,11 +480,19 @@ int gcrl_dense_layer(int device, int engine, int mode, int64_t M, int N, int K, 
  * engine 0: fp32 FFMA tiles; engine 1: tcgen05, MN-major operands, 3xTF32 split. */
 /* The tensor-core dense layer as the agents call it: the weight operand pre-split into its TF32 hi / lo halves
  * (gcrl_split_tf32: hi = rna_tf32(w), lo = rna_tf32(w - hi); same layout as w), so that the kernel only splits the
- * activation tile.  Same modes as gcrl_dense_layer. */
+ * activation tile.  Same modes as gcrl_dense_layer, and mode 3: y = x w^T (bare product; bias and act unused). */
 int gcrl_split_tf32(int device, const float *src_dev, float *hi_dev, float *lo_dev, int64_t n, void *stream);
 int gcrl_dense_layer_presplit(int device, int mode, int64_t M, int N, int K, const float *x_dev, int ldx,
                               const float *w_hi_dev, const float *w_lo_dev, int ldw, const float *bias_dev,
                               const float *act_dev, int ldact, float *y_dev, int ldy, void *stream);
+/* n <= 8 independent pre-split dense layers of one shape and mode in ONE tcgen05 launch (the critic ensemble of the
+ * SAC / TQC tensor-core engine): member i reads x_dev[i], w_hi_dev[i], w_lo_dev[i], bias_dev[i] / act_dev[i] and
+ * writes y_dev[i] (host arrays of device pointers; bias_dev / act_dev may be NULL where the mode does not read them).
+ * Each member's y equals gcrl_dense_layer_presplit of that member on the single-CTA kernel, bit for bit. */
+int gcrl_dense_layer_ensemble(int device, int n, int mode, int64_t M, int N, int K, const float *const *x_dev,
+                              int ldx, const float *const *w_hi_dev, const float *const *w_lo_dev, int ldw,
+                              const float *const *bias_dev, const float *const *act_dev, int ldact,
+                              float *const *y_dev, int ldy, void *stream);
 
 int gcrl_dense_wgrad(int device, int engine, int64_t M, int N, int K, const float *dz_dev, int lddz,
                      const float *x_dev, int ldx, float *pw_dev, int ldw, int64_t w_split_stride,
