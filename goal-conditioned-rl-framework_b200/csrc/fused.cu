@@ -66,6 +66,10 @@ __device__ __forceinline__ void slab_matmul(const float *xT, int K, const float 
   const int Np = ncw * 128;
   const int cw = warp % ncw, ks = warp / ncw;
   const int j0 = (cw * 32 + lane) * 4;
+  // bias of this thread's first epilogue element, loaded now so that its L2 round trip overlaps the K loop instead
+  // of following the barrier (at H = 256, R = 2 that is the thread's only element)
+  float bias0 = 0.f;
+  if (EPI == EPI_BIAS_LEAKY && int(threadIdx.x) < N * R) bias0 = __ldg(bias + threadIdx.x / R);
   if (ks < ks_total) {
     const int kc = (K + ks_total - 1) / ks_total;
     const int kbeg = ks * kc, kend = min(K, kbeg + kc);
@@ -108,7 +112,7 @@ __device__ __forceinline__ void slab_matmul(const float *xT, int K, const float 
     float s = red[size_t(j) * R + r];
     for (int k2 = 1; k2 < ks_total; ++k2) s += red[(size_t(k2) * Np + j) * R + r];
     if (EPI == EPI_BIAS_LEAKY) {
-      s += bias[j];
+      s += e == int(threadIdx.x) ? bias0 : bias[j];
       s = s > 0.f ? s : s * kLeakySlope;
     } else {
       s = refT[e] > 0.f ? s : s * kLeakySlope;
@@ -125,12 +129,14 @@ __device__ __forceinline__ void slab_head(const float *hT, int K, const float *_
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int p = warp; p < nout * R; p += kFusedWarps) {
     const int j = p / R, r = p - j * R;
+    const float bj = __ldg(bh + j);              // issued with the weight loads, not after the shuffle tree
     float acc = 0.f;
+#pragma unroll 8
     for (int k = lane; k < K; k += 32) acc = fmaf(hT[k * R + r], __ldg(Wh + size_t(j) * ldw + k), acc);
 #pragma unroll
     for (int s = 16; s >= 1; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
     if (lane == 0) {
-      float v = acc + bh[j];
+      float v = acc + bj;
       out[p] = tanh_out ? tanhf(v) : v;
     }
   }
@@ -355,6 +361,9 @@ __global__ void __launch_bounds__(kFusedThreads, 1) fused_critic_kernel(FusedCri
     }
   }
   // ---- 3. q = critic([s, a]) (:1319), activations kept for the backward pass ----
+  // head weight of this thread's first element of step 5, loaded ahead of the forward so that step 5 starts from
+  // a register instead of an L2 round trip
+  const float wh0 = tid < H * R ? __ldg(a.c.Wh + tid / R) : 0.f;
   h = slab_forward<R>(a.c, L, H, x_sa, D + A, sp.keep1, nullptr, nullptr, sp.red, a.h_out, a.ldh, row0, B);
   slab_head<R>(h, H, a.c.Wh, a.c.ldwh, a.c.bh, 1, false, q);
   if (SPLIT) cooperative_groups::this_cluster().sync();      // q' has arrived
@@ -408,7 +417,7 @@ __global__ void __launch_bounds__(kFusedThreads, 1) fused_critic_kernel(FusedCri
   float *dz = sp.t0, *dzn = sp.t1;
   for (int e = tid; e < H * R; e += kFusedThreads) {
     const int k = e / R, r = e - k * R;
-    const float g = dzh[r] * __ldg(a.c.Wh + k);
+    const float g = dzh[r] * (e == tid ? wh0 : __ldg(a.c.Wh + k));
     dz[e] = sp.keep1[L - 1][e] > 0.f ? g : g * kLeakySlope;
   }
   __syncthreads();
@@ -452,6 +461,13 @@ __global__ void __launch_bounds__(kFusedThreads, 1) fused_actor_kernel(FusedActo
   for (int e = tid; e < A * R; e += kFusedThreads) x_sa[D * R + e] = act[e];
   __syncthreads();
   // ---- q = critic([s, a]) with the stepped critic (:1290) ----
+  // head weights of this thread's first element of the two backward elementwise steps below, loaded ahead so that
+  // those steps start from registers instead of L2 round trips
+  const float wh0 = tid < H * R ? __ldg(a.c.Wh + tid / R) : 0.f;
+  float awh0[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+  for (int j = 0; j < 4; ++j)
+    if (tid < H * R && j < A) awh0[j] = __ldg(a.actor.Wh + size_t(j) * a.actor.ldwh + tid / R);
   h = slab_forward<R>(a.c, L, H, x_sa, D + A, sp.keep2, nullptr, nullptr, sp.red, nullptr, 0, row0, B);
   slab_head<R>(h, H, a.c.Wh, a.c.ldwh, a.c.bh, 1, false, q);
   if (tid == 0) {
@@ -466,7 +482,7 @@ __global__ void __launch_bounds__(kFusedThreads, 1) fused_actor_kernel(FusedActo
   float *dz = sp.t0, *dzn = sp.t1;
   for (int e = tid; e < H * R; e += kFusedThreads) {
     const int k = e / R, r = e - k * R;
-    const float g = (row0 + r < B) ? -invB * __ldg(a.c.Wh + k) : 0.f;
+    const float g = (row0 + r < B) ? -invB * (e == tid ? wh0 : __ldg(a.c.Wh + k)) : 0.f;
     dz[e] = sp.keep2[L - 1][e] > 0.f ? g : g * kLeakySlope;
   }
   __syncthreads();
@@ -480,6 +496,7 @@ __global__ void __launch_bounds__(kFusedThreads, 1) fused_actor_kernel(FusedActo
     for (int p = warp; p < A * R; p += kFusedWarps) {
       const int j = p / R, r = p - j * R;
       float acc = 0.f;
+#pragma unroll 8
       for (int n = lane; n < H; n += 32) acc = fmaf(dz[n * R + r], __ldg(a.c.W[0] + size_t(n) * a.c.ldw[0] + D + j), acc);
 #pragma unroll
       for (int s = 16; s >= 1; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
@@ -499,7 +516,9 @@ __global__ void __launch_bounds__(kFusedThreads, 1) fused_actor_kernel(FusedActo
   for (int e = tid; e < H * R; e += kFusedThreads) {
     const int k = e / R, r = e - k * R;
     float g = 0.f;
-    for (int j = 0; j < A; ++j) g = fmaf(da[j * R + r], __ldg(a.actor.Wh + size_t(j) * a.actor.ldwh + k), g);
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (j < A) g = fmaf(da[j * R + r], e == tid ? awh0[j] : __ldg(a.actor.Wh + size_t(j) * a.actor.ldwh + k), g);
     dzn[e] = sp.keep1[L - 1][e] > 0.f ? g : g * kLeakySlope;
   }
   __syncthreads();

@@ -3,6 +3,9 @@
 //   mode 0: per-thread __ldg of 16-byte column slices (the round-1 scheme)
 //   mode 1: producer warp + cp.async.bulk ring in shared memory, consumers LDS.128 + FFMA
 //   mode 2: mode 1 with 2-CTA clusters, each CTA fetching half of every chunk and multicasting it to both
+//   mode 5: 2D split over a cluster of C CTAs sharing S rows: CTA c computes columns [c H/C, (c+1) H/C) of every
+//           layer for all S rows (the K chunks of fused.cu's slab_matmul at H = 256), then stores its slice into
+//           every peer's activation buffer (16-byte st.shared::cluster) and meets them at a split cluster barrier
 // Output: us per launch for a chain of `steps` 256x256 layer steps on R rows per CTA.
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -o slab_stream slab_stream.cu
 #include <cooperative_groups.h>
@@ -298,6 +301,100 @@ template <int R, int DEPTH> void run_ldg_pipe(const float *W, int nl, int steps,
   printf("ldg-pipelined R=%d depth=%2d grid=%3d steps=%d: %7.2f us  (%.2f us/step)\n", R, DEPTH, grid, steps, us, us / steps);
 }
 
+// mode 5: 2D split.  Thread = (4-column group, R = S / C row group, K chunk): 8 K chunks of 32 rows as in fused.cu at
+// H = 256, so a thread does the same R-row, 4-column, 32-deep FMA chain as the R-row kernel, but the 4 lanes of a
+// warp that share a column group load the same weight float4 (one L1 wavefront for 8 float4 per warp).
+// PF = 1: between the barrier's arrive and wait, the first 8 weight float4 of the next step go into registers.
+__device__ __forceinline__ void st_cluster4(uint32_t local, uint32_t cta, float4 v) {
+  uint32_t remote;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(local), "r"(cta));
+  asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(remote), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
+               : "memory");
+}
+template <int C, int S, int PF>
+__global__ void __launch_bounds__(kConsumers, 1) csplit_kernel(const float *W, int nlayers, int steps, float *out) {
+  constexpr int R = S / C, Nc = H / C, G = Nc / 4, KC = 32;
+  static_assert(G * C * (H / KC) == kConsumers, "one thread per (column group, row group, K chunk)");
+  extern __shared__ float4 dyn[];
+  float *xT = reinterpret_cast<float *>(dyn);            // [2][H][S]
+  float *red = xT + 2 * H * S;                           // [8][Nc][S]
+  const unsigned rank = cg::this_cluster().block_rank();
+  const int tid = threadIdx.x, cgp = tid % G, rg = (tid / G) % C, ks = tid / (G * C);
+  const int j0 = rank * Nc + cgp * 4;
+  for (int e = tid; e < H * S; e += kConsumers) xT[e] = 0.001f * (e % 7);
+  cg::this_cluster().sync();
+  float4 wpre[8];
+  auto preload = [&](int s) {
+    const float *M = W + size_t(s % nlayers) * H * H + size_t(ks * KC) * H + j0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) wpre[i] = __ldg(reinterpret_cast<const float4 *>(M + size_t(i) * H));
+  };
+  if (PF) preload(0);
+  for (int s = 0; s < steps; ++s) {
+    const float *M = W + size_t(s % nlayers) * H * H + size_t(ks * KC) * H + j0;
+    const float *x = xT + (s & 1) * H * S + ks * KC * S + rg * R;
+    float acc[4][R] = {};
+#pragma unroll
+    for (int i = 0; i < KC; ++i) {
+      const float4 w = (PF && i < 8) ? wpre[i & 7] : __ldg(reinterpret_cast<const float4 *>(M + size_t(i) * H));
+      float xv[R];
+      if constexpr (R == 1) xv[0] = x[i * S];
+      else if constexpr (R == 2) { const float2 t = *reinterpret_cast<const float2 *>(x + i * S); xv[0] = t.x; xv[1] = t.y; }
+      else {
+#pragma unroll
+        for (int q = 0; q < R / 4; ++q) {
+          const float4 t = *reinterpret_cast<const float4 *>(x + i * S + 4 * q);
+          xv[4 * q] = t.x; xv[4 * q + 1] = t.y; xv[4 * q + 2] = t.z; xv[4 * q + 3] = t.w;
+        }
+      }
+#pragma unroll
+      for (int r = 0; r < R; ++r) {
+        acc[0][r] = fmaf(w.x, xv[r], acc[0][r]); acc[1][r] = fmaf(w.y, xv[r], acc[1][r]);
+        acc[2][r] = fmaf(w.z, xv[r], acc[2][r]); acc[3][r] = fmaf(w.w, xv[r], acc[3][r]);
+      }
+    }
+#pragma unroll
+    for (int c = 0; c < 4; ++c)
+#pragma unroll
+      for (int r = 0; r < R; ++r) red[(ks * Nc + cgp * 4 + c) * S + rg * R + r] = acc[c][r];
+    __syncthreads();
+    const uint32_t ynext = smem_u32(xT + ((s + 1) & 1) * H * S + rank * Nc * S);
+    for (int e4 = tid; e4 < Nc * S / 4; e4 += kConsumers) {
+      float v[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        float t = red[e4 * 4 + q];
+#pragma unroll
+        for (int k2 = 1; k2 < H / KC; ++k2) t += red[k2 * Nc * S + e4 * 4 + q];
+        v[q] = t > 0.f ? t : 0.01f * t;
+      }
+      const float4 v4 = make_float4(v[0], v[1], v[2], v[3]);
+#pragma unroll
+      for (int p = 0; p < C; ++p) st_cluster4(ynext + e4 * 16, (rank + p) % C, v4);
+    }
+    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+    if (PF && s + 1 < steps) preload(s + 1);
+    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
+  }
+  if (tid < S) out[(blockIdx.x / C) * S + tid] = xT[(steps & 1) * H * S + tid];
+}
+template <int C, int S, int PF> void run_csplit(const float *W, int nl, int steps, float *out, int grid) {
+  const size_t smem = (size_t(2) * H * S + size_t(8) * (H / C) * S) * 4;
+  auto k = csplit_kernel<C, S, PF>;
+  CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  CK(cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+  cudaLaunchConfig_t cfg{}; cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kConsumers); cfg.dynamicSmemBytes = smem;
+  cudaLaunchAttribute attr[1]; attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = C; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  int nclusters = 0;
+  CK(cudaOccupancyMaxActiveClusters(&nclusters, k, &cfg));
+  const float us = time_it([&] { CK(cudaLaunchKernelEx(&cfg, k, W, nl, steps, out)); });
+  printf("csplit C=%d S=%2d R=%d prefetch=%d grid=%3d (%3d rows) steps=%d: %7.2f us  (%.2f us/step, smem %zu KB, "
+         "max active clusters %d, need %d)\n", C, S, S / C, PF, grid, grid / C * S, steps, us, us / steps, smem >> 10,
+         nclusters, grid / C);
+}
+
 template <typename F> float time_it(F f, int iters) {
   cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
   for (int i = 0; i < 3; ++i) f();
@@ -328,14 +425,33 @@ template <int R, int MODE = 0> void run_ldg(const float *W, int nl, int steps, f
   printf("ldg   R=%d mode=%d grid=%3d steps=%d: %7.2f us  (%.2f us/step)\n", R, MODE, grid, steps, us, us / steps);
 }
 
-int main() {
+int main(int argc, char **argv) {
   const int nl = 9, steps = 14;
+  const bool cluster_only = argc > 1 && argv[1][0] == 'c';   // `slab_stream c`: the mode-5 table + its baseline
   float *W, *out;
   CK(cudaMalloc(&W, size_t(nl) * H * H * 4));
   CK(cudaMalloc(&out, 4096 * 4));
   std::vector<float> h(size_t(nl) * H * H);
   for (size_t i = 0; i < h.size(); ++i) h[i] = float((i * 2654435761u) % 1000) * 1e-5f - 0.005f;
   CK(cudaMemcpy(W, h.data(), h.size() * 4, cudaMemcpyHostToDevice));
+  if (cluster_only) {
+    for (int rep = 0; rep < 2; ++rep) {
+      run_ldg<2, 0>(W, nl, steps, out, 128);
+      run_csplit<4, 8, 0>(W, nl, steps, out, 128);
+      run_csplit<4, 16, 0>(W, nl, steps, out, 128);
+      run_csplit<4, 32, 0>(W, nl, steps, out, 128);
+      run_csplit<8, 8, 0>(W, nl, steps, out, 128);
+      run_csplit<8, 16, 0>(W, nl, steps, out, 128);
+      run_csplit<8, 32, 0>(W, nl, steps, out, 128);
+      run_csplit<4, 8, 1>(W, nl, steps, out, 128);
+      run_csplit<8, 16, 1>(W, nl, steps, out, 128);
+      run_csplit<8, 16, 0>(W, nl, steps, out, 8);
+      run_csplit<8, 16, 0>(W, nl, steps, out, 64);
+      run_csplit<8, 16, 0>(W, nl, steps, out, 144);
+    }
+    printf("done\n");
+    return 0;
+  }
   for (int grid : {1, 16, 64, 128, 148}) {
     run_ldg<2, 0>(W, nl, steps, out, grid);
     run_ldg<2, 1>(W, nl, steps, out, grid);
