@@ -15,6 +15,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <initializer_list>
 #include <map>
 #include <tuple>
@@ -32,6 +33,9 @@ void her_sample_into(gcrl_her *h, int64_t B, const int64_t *idx_host, float *s, 
 int her_state_dim(const gcrl_her *h);
 int her_act_dim(const gcrl_her *h);
 int her_device(const gcrl_her *h);
+void her_sample_graphed(gcrl_her *h, int64_t B, const SampleScalars *sc_dev, const int64_t *idx_dev, float *s,
+                        float *a, float *r, float *ns, float *d, cudaStream_t st);
+unsigned long long &her_draw_epoch(gcrl_her *h);
 }  // namespace gcrl
 
 using namespace gcrl;
@@ -128,6 +132,8 @@ enum NetId { ACTOR = 0, CRITIC1 = 1, T_ACTOR = 2, T_CRITIC1 = 3, CRITIC2 = 4, T_
 enum Slot { S_CLOSS = 0, S_ALOSS = 1, S_TD = 2, S_Q = 3, S_CGRAD = 4, S_AGRAD = 5, S_C2LOSS = 6, S_C2GRAD = 7 };
 
 constexpr int kMaxSplits = 128;
+constexpr size_t kScalBytes = sizeof(StepScalars) + sizeof(SampleScalars);   // the per-update device scalars
+constexpr size_t kManyGraphCache = 8;    // n-update graphs kept per agent (one flag pattern per run is typical)
 
 }  // namespace
 
@@ -194,10 +200,20 @@ struct gcrl_agent {
     float **d_peer_g[NUM_NETS] = {};
     std::vector<void *> opened;                          // cudaIpcOpenMemHandle results
   } p2p;
+  bool dp_open = false;                    // a phase-wise data-parallel update: phase 0 issued, phase 3 not yet
   bool use_graphs = true;
   cudaStream_t cap_stream = nullptr;       // capture-only stream (the caller's may be the legacy one)
   struct GraphRec { cudaGraphExec_t exec; uint64_t kernels; };
   std::map<std::tuple<int64_t, int, int, uintptr_t>, GraphRec> graphs;   // (B, flags, phase mask, sampled buffer)
+  // n consecutive updates in one graph (gcrl_agent_update_many): everything a captured update reads that changes
+  // from one update to the next has one slot per update; allocated on first use
+  struct Many {
+    char *d = nullptr;                     // [GCRL_MAX_MANY_STEPS] x kScalBytes scalars, then positions [n][B] int64
+    float *noise = nullptr;                // TD3 smoothing noise [n][B][A]
+    float *h_pub = nullptr, *d_pub = nullptr;   // mapped publish blocks [GCRL_MAX_MANY_STEPS][16] of updates 0 .. n-2
+    // (B, flags of every update, buffer, engine path)
+    std::map<std::tuple<int64_t, std::vector<int>, uintptr_t, int>, GraphRec> graphs;
+  } many;
 };
 
 namespace {
@@ -648,7 +664,8 @@ void actor_phase_step(gcrl_agent *ag, bool rereduce, cudaStream_t st) {
   adam_step(ag, a, 1, ag->cfg.grad_clip, S_AGRAD, &ag->net[T_ACTOR], ag->td3, st, grad);
 }
 
-void write_scalars(gcrl_agent *ag, double lr_c, double lr_a, bool actor_steps, cudaStream_t st) {
+// The next update's Adam step counters and sequence number -> its StepScalars, followed by `ss`, at `out` (host)
+void fill_scalars(gcrl_agent *ag, double lr_c, double lr_a, bool actor_steps, const SampleScalars &ss, char *out) {
   auto fill = [&](int t, double lr, float *out) {
     const double bc1 = 1.0 - std::pow(0.9, double(t));
     const double bc2 = 1.0 - std::pow(0.999, double(t));
@@ -656,10 +673,8 @@ void write_scalars(gcrl_agent *ag, double lr_c, double lr_a, bool actor_steps, c
     out[1] = float(std::sqrt(bc2));
     out[2] = float(1.0 - lr * double(ag->cfg.weight_decay));
   };
-  int slot;
-  constexpr size_t kScalBytes = sizeof(StepScalars) + sizeof(SampleScalars);
-  auto *sc = reinterpret_cast<StepScalars *>(ag->scal_stage.acquire(kScalBytes, &slot));
-  std::memcpy(sc + 1, &ag->sample_sc, sizeof(SampleScalars));
+  auto *sc = reinterpret_cast<StepScalars *>(out);
+  std::memcpy(sc + 1, &ss, sizeof(SampleScalars));
   ag->net[CRITIC1].adam_t += 1;
   if (ag->td3) ag->net[CRITIC2].adam_t += 1;
   fill(ag->net[CRITIC1].adam_t, lr_c, &sc->step_size_c);
@@ -667,26 +682,40 @@ void write_scalars(gcrl_agent *ag, double lr_c, double lr_a, bool actor_steps, c
   fill(std::max(1, ag->net[ACTOR].adam_t), lr_a, &sc->step_size_a);
   sc->pad1 = 0.f;
   sc->seq = ++ag->pub_seq;
+}
+
+void write_scalars(gcrl_agent *ag, double lr_c, double lr_a, bool actor_steps, cudaStream_t st) {
+  int slot;
+  char *sc = ag->scal_stage.acquire(kScalBytes, &slot);
+  fill_scalars(ag, lr_c, lr_a, actor_steps, ag->sample_sc, sc);
   GCRL_CUDA(cudaMemcpyAsync(ag->d_scalars, sc, kScalBytes, cudaMemcpyHostToDevice, st));
   ag->scal_stage.release(slot, st);
 }
 
-// The Adam step counters advance in write_scalars, before the update is enqueued.  If anything after that throws
-// (argument checks, a CUDA error, graph capture), the Python schedulers do not step either, so the counters are
-// restored -- otherwise every later bias correction would be off by one step.
+// The Adam step counters and the update sequence number advance in write_scalars, before the update is enqueued.
+// If anything after that throws (argument checks, a CUDA error, graph capture), the Python schedulers do not step
+// either, so the counters are restored -- otherwise every later bias correction would be off by one step.
+// keep_draws: the device index-stream epoch of `buf` is restored too (an n-update call draws all its epochs first).
 struct AdamStepGuard {
   gcrl_agent *ag;
   int t[NUM_NETS];
   bool per_on; int dp_B, dp_flags;
+  unsigned int pub_seq;
+  gcrl_her *buf = nullptr;
+  unsigned long long draw_epoch = 0;
   bool done = false;
-  explicit AdamStepGuard(gcrl_agent *a) : ag(a), per_on(a->per_on), dp_B(a->dp_B), dp_flags(a->dp_flags) {
+  explicit AdamStepGuard(gcrl_agent *a)
+      : ag(a), per_on(a->per_on), dp_B(a->dp_B), dp_flags(a->dp_flags), pub_seq(a->pub_seq) {
     for (int i = 0; i < NUM_NETS; ++i) t[i] = a->net[i].adam_t;
   }
+  void keep_draws(gcrl_her *b) { buf = b; draw_epoch = her_draw_epoch(b); }
   void commit() { done = true; }
   ~AdamStepGuard() {
     if (done) return;
     for (int i = 0; i < NUM_NETS; ++i) ag->net[i].adam_t = t[i];
     ag->per_on = per_on; ag->dp_B = dp_B; ag->dp_flags = dp_flags;
+    ag->pub_seq = pub_seq;
+    if (buf != nullptr) her_draw_epoch(buf) = draw_epoch;
   }
 };
 
@@ -727,39 +756,115 @@ void run_update_body(gcrl_agent *ag, int B, const float *noise, int flags, int m
   }
 }
 
-// Replay (or capture on first use) the graph of (B, flags, phase mask).  TD3 noise pointers vary
-// per call, so the noise is first copied into an internal buffer by the caller.
-void run_update(gcrl_agent *ag, int B, const float *noise, int flags, int mask, cudaStream_t st) {
+// Record `body` on the capture stream into an instantiated graph; the kernels it records are not counted as
+// launches until the graph is replayed.
+gcrl_agent::GraphRec capture_graph(gcrl_agent *ag, const std::function<void(cudaStream_t)> &body) {
+  cudaGraph_t graph = nullptr;
+  const uint64_t before = launch_counter();
+  GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
+  try {
+    body(ag->cap_stream);
+  } catch (...) {
+    cudaStreamEndCapture(ag->cap_stream, &graph);
+    if (graph) cudaGraphDestroy(graph);
+    throw;
+  }
+  GCRL_CUDA(cudaStreamEndCapture(ag->cap_stream, &graph));
+  const uint64_t kernels = launch_counter() - before;   // recorded, not executed, by the capture
+  count_launch(uint64_t(0) - kernels);
+  cudaGraphExec_t exec = nullptr;
+  const cudaError_t e = cudaGraphInstantiate(&exec, graph, 0);
+  cudaGraphDestroy(graph);
+  GCRL_CUDA(e);
+  return gcrl_agent::GraphRec{exec, kernels};
+}
+
+void launch_graph(const gcrl_agent::GraphRec &g, cudaStream_t st) {
+  GCRL_CUDA(cudaGraphLaunch(g.exec, st));
+  count_launch(g.kernels);
+}
+
+// the engine an update at this batch runs on; the tensor-core one needs the split weight copies current
+void select_engine(gcrl_agent *ag, int B, cudaStream_t st) {
   ag->tc_update = !fused_ok(ag, B) && engine_tc(ag, B);
   if (ag->tc_update) ensure_split(ag, st);          // (the update itself re-splits what it steps)
   else mark_split_stale(ag);                        // weights move without their split copies following
+}
+
+// Replay (or capture on first use) the graph of (B, flags, phase mask).  TD3 noise pointers vary
+// per call, so the noise is first copied into an internal buffer by the caller.
+void run_update(gcrl_agent *ag, int B, const float *noise, int flags, int mask, cudaStream_t st) {
+  select_engine(ag, B, st);
   if (!ag->use_graphs) {
     run_update_body(ag, B, noise, flags, mask, st);
     return;
   }
   const auto key = std::make_tuple(int64_t(B), flags, mask, reinterpret_cast<uintptr_t>(ag->sample_buf));
   auto it = ag->graphs.find(key);
-  if (it == ag->graphs.end()) {
-    cudaGraph_t graph = nullptr;
-    const uint64_t before = launch_counter();
-    GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
-    try {
-      run_update_body(ag, B, noise, flags, mask, ag->cap_stream);
-    } catch (...) {
-      cudaStreamEndCapture(ag->cap_stream, &graph);
-      if (graph) cudaGraphDestroy(graph);
-      throw;
-    }
-    GCRL_CUDA(cudaStreamEndCapture(ag->cap_stream, &graph));
-    const uint64_t kernels = launch_counter() - before;   // recorded, not executed, by the capture
-    count_launch(uint64_t(0) - kernels);
-    cudaGraphExec_t exec = nullptr;
-    GCRL_CUDA(cudaGraphInstantiate(&exec, graph, 0));
-    GCRL_CUDA(cudaGraphDestroy(graph));
-    it = ag->graphs.emplace(key, gcrl_agent::GraphRec{exec, kernels}).first;
+  if (it == ag->graphs.end())
+    it = ag->graphs.emplace(key, capture_graph(ag, [&](cudaStream_t cs) { run_update_body(ag, B, noise, flags, mask, cs); })).first;
+  launch_graph(it->second, st);
+}
+
+// While update i of an n-update call is recorded (or issued eagerly), the agent's per-update inputs -- scalars,
+// sampler positions, TD3 noise, publish block -- point at slot i, so every argument builder picks the slot up.
+// The last update publishes through the single-update block: gcrl_agent_read_metrics then sees it as after
+// gcrl_agent_update_from_buffer.
+struct ManySlot {
+  gcrl_agent *ag;
+  StepScalars *sc; SampleScalars *ssc; int64_t *idx; float *noise, *pub;
+  ManySlot(gcrl_agent *a, int i, int n, int B)
+      : ag(a), sc(a->d_scalars), ssc(a->d_sample_sc), idx(a->d_idx), noise(a->noise), pub(a->d_pub) {
+    a->d_scalars = reinterpret_cast<StepScalars *>(a->many.d + size_t(i) * kScalBytes);
+    a->d_sample_sc = reinterpret_cast<SampleScalars *>(a->d_scalars + 1);
+    a->d_idx = reinterpret_cast<int64_t *>(a->many.d + size_t(n) * kScalBytes) + size_t(i) * B;
+    if (a->td3) a->noise = a->many.noise + size_t(i) * B * a->A;
+    if (i < n - 1) a->d_pub = a->many.d_pub + size_t(i) * 16;
   }
-  GCRL_CUDA(cudaGraphLaunch(it->second.exec, st));
-  count_launch(it->second.kernels);
+  ~ManySlot() { ag->d_scalars = sc; ag->d_sample_sc = ssc; ag->d_idx = idx; ag->noise = noise; ag->d_pub = pub; }
+  ManySlot(const ManySlot &) = delete;
+  ManySlot &operator=(const ManySlot &) = delete;
+};
+
+// n updates from `buf` back to back.  Where the sampler is a launch of its own (ag->sample_buf == nullptr) it is
+// part of every update here, reading that update's totals and positions from the slot.
+void run_many_body(gcrl_agent *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+  for (int i = 0; i < n; ++i) {
+    ManySlot slot(ag, i, n, B);
+    if (ag->sample_buf == nullptr) {
+      her_sample_graphed(buf, B, ag->d_sample_sc, ag->d_idx, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, st);
+      if (!fused_ok(ag, B))
+        launch_ingest_batch(ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->D, ag->A, B, ag->sa, ag->nsa, ag->spi, ag->ldc,
+                            ag->br, ag->bd, st);
+    }
+    run_update_body(ag, B, ag->td3 ? ag->noise : nullptr, flags[i], PH_ALL, st);
+  }
+}
+
+void run_many(gcrl_agent *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+  select_engine(ag, B, st);
+  if (!ag->use_graphs) {
+    run_many_body(ag, buf, B, n, flags, st);
+    return;
+  }
+  const int path = (ag->sample_buf != nullptr ? 1 : 0) | (fused_ok(ag, B) ? 2 : 0) | (ag->tc_update ? 4 : 0);
+  auto key = std::make_tuple(int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), path);
+  auto &cache = ag->many.graphs;
+  auto it = cache.find(key);
+  if (it == cache.end()) {
+    const gcrl_agent::GraphRec g = capture_graph(ag, [&](cudaStream_t cs) { run_many_body(ag, buf, B, n, flags, cs); });
+    if (cache.size() >= kManyGraphCache) {     // a replay still in flight is released when it completes
+      for (auto &kv : cache) cudaGraphExecDestroy(kv.second.exec);
+      cache.clear();
+    }
+    it = cache.emplace(std::move(key), g).first;
+  }
+  launch_graph(it->second, st);
+}
+
+// The row-slab critic kernel draws the batch itself from `buf` (else the sampler is a launch of its own)
+bool samples_in_kernel(const gcrl_agent *ag, const gcrl_her *buf, int64_t B) {
+  return fused_ok(ag, int(B)) && ag->fuse_sampler && fused_sample_supported(her_geom(buf));
 }
 
 // Stage one batch (sampled from `buf`, or the caller's dense device batch) into the operand rows.
@@ -770,7 +875,7 @@ void ingest(gcrl_agent *ag, gcrl_her *buf, int64_t B, const int64_t *idx_host, c
   if (buf != nullptr) {
     GCRL_REQUIRE(her_state_dim(buf) == ag->D && her_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
     GCRL_REQUIRE(her_device(buf) == ag->device, "buffer and agent live on different devices");
-    if (fused_ok(ag, int(B)) && ag->fuse_sampler && fused_sample_supported(her_geom(buf))) {
+    if (samples_in_kernel(ag, buf, B)) {
       // row-slab path: the critic-phase kernel draws its own rows; here only the positions (host index stream)
       // and the buffer's totals travel to the device
       if (her_len(buf) < B) throw Error(GCRL_ERR_UNDERFILLED, "[ERROR] Not enough in buffer to sample");
@@ -838,6 +943,28 @@ void ensure_io(gcrl_agent *ag, size_t floats, cudaStream_t st) {
   }
 }
 
+// Wait until the publish block `pub` (mapped host: float[8] metrics, uint32 seq, int32 err) carries sequence number
+// `seq`: the update's last optimiser kernel writes the metrics and then that word (no D2H copy, no stream
+// synchronisation, no driver call on the critical path), then copy the metrics out.
+void read_published(const float *pub, unsigned int want, float *metrics_host, cudaStream_t st) {
+  const volatile unsigned int *seq = reinterpret_cast<const volatile unsigned int *>(pub) + 8;
+  const auto t0 = std::chrono::steady_clock::now();
+  unsigned long spins = 0;
+  while (*seq != want) {
+    if ((++spins & 0xFFFF) == 0) {
+      if (cudaStreamQuery(st) != cudaErrorNotReady) {       // finished (or failed) without publishing this number
+        GCRL_CUDA(cudaStreamSynchronize(st));
+        if (*seq == want) break;
+        throw Error(GCRL_ERR_CUDA, "the update finished without publishing its metrics");
+      }
+      if (std::chrono::steady_clock::now() - t0 > std::chrono::seconds(120))
+        throw Error(GCRL_ERR_CUDA, "timed out waiting for the update's metrics");
+    }
+  }
+  std::atomic_thread_fence(std::memory_order_acquire);
+  std::memcpy(metrics_host, pub, 8 * sizeof(float));
+}
+
 void finish_metrics(gcrl_agent *ag, float *metrics_host, cudaStream_t st) {
   if (metrics_host == nullptr) return;
   auto dp_error = [](int err) {
@@ -845,24 +972,7 @@ void finish_metrics(gcrl_agent *ag, float *metrics_host, cudaStream_t st) {
                                     " never saw the flag of rank " + std::to_string((err - 1) % 16));
   };
   if (ag->pub_valid) {
-    // the update's last optimiser kernel wrote the metrics and then its sequence number into mapped host memory:
-    // poll that word (no D2H copy, no stream synchronisation, no driver call on the critical path)
-    volatile unsigned int *seq = reinterpret_cast<volatile unsigned int *>(ag->h_pub) + 8;
-    const auto t0 = std::chrono::steady_clock::now();
-    unsigned long spins = 0;
-    while (*seq != ag->pub_seq) {
-      if ((++spins & 0xFFFF) == 0) {
-        if (cudaStreamQuery(st) != cudaErrorNotReady) {       // finished (or failed) without publishing this number
-          GCRL_CUDA(cudaStreamSynchronize(st));
-          if (*seq == ag->pub_seq) break;
-          throw Error(GCRL_ERR_CUDA, "the update finished without publishing its metrics");
-        }
-        if (std::chrono::steady_clock::now() - t0 > std::chrono::seconds(120))
-          throw Error(GCRL_ERR_CUDA, "timed out waiting for the update's metrics");
-      }
-    }
-    std::atomic_thread_fence(std::memory_order_acquire);
-    std::memcpy(metrics_host, ag->h_pub, 8 * sizeof(float));
+    read_published(ag->h_pub, ag->pub_seq, metrics_host, st);
     const int err = reinterpret_cast<const int *>(ag->h_pub)[9];
     if (err) throw dp_error(err);
     return;
@@ -981,6 +1091,10 @@ int gcrl_agent_destroy(gcrl_agent *ag) {
   cudaSetDevice(ag->device);
   cudaDeviceSynchronize();
   for (auto &kv : ag->graphs) cudaGraphExecDestroy(kv.second.exec);
+  for (auto &kv : ag->many.graphs) cudaGraphExecDestroy(kv.second.exec);
+  if (ag->many.d) cudaFree(ag->many.d);
+  if (ag->many.noise) cudaFree(ag->many.noise);
+  if (ag->many.h_pub) cudaFreeHost(ag->many.h_pub);
   for (void *p : ag->p2p.opened) cudaIpcCloseMemHandle(p);
   for (void *p : {(void *)ag->p2p.flags, (void *)ag->p2p.epoch, (void *)ag->p2p.ticket, (void *)ag->p2p.wticket, (void *)ag->p2p.go, (void *)ag->p2p.tflags,
                   (void *)ag->p2p.d_peer_tflags, (void *)ag->p2p.err, (void *)ag->p2p.outbox,
@@ -1215,6 +1329,66 @@ int gcrl_agent_update_from_buffer(gcrl_agent *ag, gcrl_her *buf, int64_t B, cons
   GCRL_API_END
 }
 
+int gcrl_agent_update_many(gcrl_agent *ag, gcrl_her *buf, int64_t B, int n, const int *flags, const int64_t *idx_host,
+                           const float *noise_dev, const double *lr_critic, const double *lr_actor, float *metrics_host,
+                           void *stream) {
+  GCRL_API_BEGIN
+  GCRL_NVTX("gcrl_agent_update_many");
+  require_handle(ag);
+  check_batch(ag, B);
+  GCRL_REQUIRE(buf != nullptr, "buffer handle is NULL");
+  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
+  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
+  for (int i = 0; i < n; ++i) GCRL_REQUIRE((flags[i] & ~3) == 0, "flags of an n-update call may hold bit0 and bit1 only");
+  GCRL_REQUIRE(!ag->p2p.on, "n-update calls are not available under peer-memory data parallelism");
+  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
+  GCRL_REQUIRE(her_state_dim(buf) == ag->D && her_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
+  GCRL_REQUIRE(her_device(buf) == ag->device, "buffer and agent live on different devices");
+  GCRL_REQUIRE(!ag->td3 || noise_dev != nullptr, "TD3 update needs the [n, B, A] standard-normal noise tensor");
+  const int64_t len = her_len(buf);
+  if (len < B) throw Error(GCRL_ERR_UNDERFILLED, "[ERROR] Not enough in buffer to sample");
+  if (idx_host != nullptr)
+    for (int64_t i = 0; i < int64_t(n) * B; ++i)
+      if (idx_host[i] < 0 || idx_host[i] >= len) throw Error(GCRL_ERR_INVALID, "sample index out of range [0, len)");
+  GCRL_CUDA(cudaSetDevice(ag->device));
+  cudaStream_t st = as_stream(stream);
+  auto &mn = ag->many;
+  if (mn.d == nullptr) {
+    mn.d = dev_alloc<char>(GCRL_MAX_MANY_STEPS * (kScalBytes + size_t(ag->maxB) * sizeof(int64_t)));
+    if (ag->td3) mn.noise = dev_alloc<float>(size_t(GCRL_MAX_MANY_STEPS) * ag->maxB * ag->A);
+    GCRL_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&mn.h_pub), GCRL_MAX_MANY_STEPS * 64, cudaHostAllocMapped));
+    std::memset(mn.h_pub, 0, GCRL_MAX_MANY_STEPS * 64);
+    GCRL_CUDA(cudaHostGetDevicePointer(reinterpret_cast<void **>(&mn.d_pub), mn.h_pub, 0));
+  }
+  AdamStepGuard guard(ag);
+  guard.keep_draws(buf);
+  ag->per_on = false;
+  // every update's scalars (the device stream's draw epochs in order), then every update's positions: ONE copy
+  const size_t scal = size_t(n) * kScalBytes, pos = idx_host != nullptr ? size_t(n) * B * sizeof(int64_t) : 0;
+  int slot;
+  char *p = ag->io_stage.acquire(scal + pos, &slot);
+  for (int i = 0; i < n; ++i) {
+    ag->sample_sc = her_next_scalars(buf, idx_host != nullptr);
+    fill_scalars(ag, lr_critic[i], lr_actor[i], (flags[i] & 1) != 0, ag->sample_sc, p + size_t(i) * kScalBytes);
+  }
+  if (pos) std::memcpy(p + scal, idx_host, pos);
+  GCRL_CUDA(cudaMemcpyAsync(mn.d, p, scal + pos, cudaMemcpyHostToDevice, st));
+  ag->io_stage.release(slot, st);
+  if (ag->td3)   // stable addresses for the captured graph
+    GCRL_CUDA(cudaMemcpyAsync(mn.noise, noise_dev, size_t(n) * B * ag->A * 4, cudaMemcpyDeviceToDevice, st));
+  ag->sample_buf = samples_in_kernel(ag, buf, B) ? buf : nullptr;
+  run_many(ag, buf, int(B), n, flags, st);
+  ag->pub_valid = true;
+  guard.commit();
+  if (metrics_host != nullptr) {
+    // the last update publishes as a single one does; stream order then has the earlier blocks complete
+    finish_metrics(ag, metrics_host + size_t(n - 1) * 8, st);
+    for (int i = 0; i < n - 1; ++i)
+      read_published(mn.h_pub + size_t(i) * 16, ag->pub_seq - unsigned(n - 1 - i), metrics_host + size_t(i) * 8, st);
+  }
+  GCRL_API_END
+}
+
 int gcrl_agent_read_metrics(gcrl_agent *ag, float *metrics_host, void *stream) {
   GCRL_API_BEGIN
   require_handle(ag);
@@ -1302,10 +1476,12 @@ int gcrl_agent_update_phase(gcrl_agent *ag, int phase, gcrl_her *buf, int64_t B,
     ag->dp_flags = flags;
     run_update(ag, int(B), noise, flags, PH_CGRAD, st);
     ag->pub_valid = false;                 // phase-cut update: metrics through the D2H copy
+    ag->dp_open = true;
     guard.commit();
   } else {
     GCRL_REQUIRE(ag->dp_B == int(B) && ag->dp_flags == flags, "phase 1..3 must follow phase 0 of the same update");
     run_update(ag, int(B), ag->td3 ? ag->noise : nullptr, flags, phase == 1 ? PH_CSTEP : (phase == 2 ? PH_AGRAD : PH_ASTEP), st);
+    if (phase == 3) ag->dp_open = false;
   }
   GCRL_API_END
 }

@@ -114,9 +114,13 @@ __device__ __forceinline__ void write_field(float *__restrict__ out, const float
 
 template <bool VEC, int SPB>
 __global__ void __launch_bounds__(kSampleThreads)
-her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc, int64_t B, const int64_t *__restrict__ idx,
+her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg, const SampleScalars *__restrict__ sc_dev,
+                  int64_t B, const int64_t *__restrict__ idx,
                   float *__restrict__ out_s, float *__restrict__ out_a, float *__restrict__ out_r,
                   float *__restrict__ out_ns, float *__restrict__ out_d, int64_t *__restrict__ idx_out) {
+  // sc_dev: the totals and draw epoch of this launch's update, written by the host before a replayed graph runs
+  // (a value captured into the graph would freeze them); otherwise they come by value
+  const SampleScalars sc = sc_dev != nullptr ? *sc_dev : sc_arg;
   extern __shared__ float4 smem4[];
   float *tile = reinterpret_cast<float *>(smem4);
   uint32_t *m_row = reinterpret_cast<uint32_t *>(tile + SPB * g.row_f);
@@ -128,7 +132,7 @@ her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc, int
   // ---- round trip 1: deque position -> bucket record -> (episode, t, j) -> ring slot (her_device.cuh) ----
   SampleRef ref{0u, 0u, 0u, 0u};
   if (tid < n) {
-    ref = her_resolve(g, sc, base + tid, idx, idx_out);
+    ref = her_resolve(g, sc, base + tid, sc.use_idx ? idx : nullptr, idx_out);
     m_row[tid] = ref.slot;
   }
   __syncthreads();
@@ -249,22 +253,24 @@ int64_t her_len(const gcrl_her *h) { return h->len(); }
 static constexpr int kSmallTile = 32;      // samples per CTA while the batch is too small to fill the SMs with 128
 static size_t sample_smem(const gcrl_her *h, int spb) { return size_t(spb) * h->g.row_f * 4 + size_t(spb) * 4; }
 
+// sc_dev == nullptr: this call draws the scalars (her_next_scalars) and passes them by value
 static void her_launch_sample(gcrl_her *h, int64_t B, const int64_t *idx_dev, float *s, float *a,
-                              float *r, float *ns, float *d, int64_t *idx_out, cudaStream_t st) {
+                              float *r, float *ns, float *d, int64_t *idx_out, cudaStream_t st,
+                              const SampleScalars *sc_dev = nullptr) {
   auto aligned = [](const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
   const bool vec = aligned(s) && aligned(a) && aligned(r) && aligned(ns) && aligned(d);
-  const SampleScalars sc = her_next_scalars(h, idx_dev != nullptr);
+  const SampleScalars sc = sc_dev != nullptr ? SampleScalars{} : her_next_scalars(h, idx_dev != nullptr);
   // small batches: 32 samples per CTA (4x the CTAs, each row gather a single round of loads)
   const bool small = B <= int64_t(sm_count()) * 4 * kSmallTile;
   const int spb = small ? kSmallTile : kSamplesPerBlock;
   const unsigned blocks = unsigned((B + spb - 1) / spb);
   const size_t smem = sample_smem(h, spb);
   if (small) {
-    if (vec) her_sample_kernel<true, kSmallTile><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, B, idx_dev, s, a, r, ns, d, idx_out);
-    else her_sample_kernel<false, kSmallTile><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, B, idx_dev, s, a, r, ns, d, idx_out);
+    if (vec) her_sample_kernel<true, kSmallTile><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out);
+    else her_sample_kernel<false, kSmallTile><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out);
   } else {
-    if (vec) her_sample_kernel<true, kSamplesPerBlock><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, B, idx_dev, s, a, r, ns, d, idx_out);
-    else her_sample_kernel<false, kSamplesPerBlock><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, B, idx_dev, s, a, r, ns, d, idx_out);
+    if (vec) her_sample_kernel<true, kSamplesPerBlock><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out);
+    else her_sample_kernel<false, kSamplesPerBlock><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out);
   }
   GCRL_LAUNCHED();
 }
@@ -301,6 +307,13 @@ void her_sample_into(gcrl_her *h, int64_t B, const int64_t *idx_host, float *s, 
   const int64_t *idx_dev = her_stage_indices(h, B, idx_host, st);
   her_launch_sample(h, B, idx_dev, s, a, r, ns, d, idx_out, st);
 }
+// The sampler as a node of a captured graph: totals, draw epoch and index-buffer switch are read from `sc_dev`
+// (filled from her_next_scalars by the caller before every replay), positions from `idx_dev` when sc_dev->use_idx.
+void her_sample_graphed(gcrl_her *h, int64_t B, const SampleScalars *sc_dev, const int64_t *idx_dev, float *s,
+                        float *a, float *r, float *ns, float *d, cudaStream_t st) {
+  her_launch_sample(h, B, idx_dev, s, a, r, ns, d, nullptr, st, sc_dev);
+}
+unsigned long long &her_draw_epoch(gcrl_her *h) { return h->draw_epoch; }
 int her_state_dim(const gcrl_her *h) { return h->g.D; }
 int her_act_dim(const gcrl_her *h) { return h->g.A; }
 int her_device(const gcrl_her *h) { return h->device; }

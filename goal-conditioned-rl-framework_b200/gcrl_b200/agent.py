@@ -22,6 +22,7 @@ from .buffer import HERBuffer
 from .replay import PERBuffer, ReplayBuffer
 
 ALGO_DDPG, ALGO_TD3 = 0, 1
+MAX_MANY_STEPS = 64         # GCRL_MAX_MANY_STEPS: updates per n-update graph launch
 NET_ACTOR, NET_CRITIC, NET_T_ACTOR, NET_T_CRITIC, NET_CRITIC2, NET_T_CRITIC2 = range(6)
 
 
@@ -539,12 +540,73 @@ class _AgentBase:
         check(lib.gcrl_agent_read_metrics(self._h, C.cast(self._metrics, vp), self._stream()))
         return [float(x) for x in self._metrics]
 
+    # -- a training cycle's gradient steps in one call ---------------------------------------------------
+    _MANY_IN_ONE_GRAPH = False      # DDPG / TD3: n updates from a HER buffer replay as one CUDA graph
+
+    def update_many(self, steps):
+        """``[self.update(s) for s in steps]``: the same tuples, and afterwards the same state of every network,
+        optimiser, schedule, index stream and random generator.  ``steps`` need not be consecutive.
+
+        DDPG and TD3 sampling from a HER buffer on one GPU issue every 64 steps as ONE CUDA graph launch: the
+        positions (host index stream), learning rates and TD3 noise of all of them are drawn up front and
+        travel in one copy, so no interpreter, launch or metric read-back sits between the updates.  Every
+        other agent, buffer type and data-parallel mode runs the loop."""
+        steps = [int(s) for s in steps]
+        if not (self._MANY_IN_ONE_GRAPH and isinstance(self.buffer, HERBuffer) and self._dp is None
+                and getattr(self, "_peer_dp", None) is None):
+            return [self.update(s) for s in steps]
+        out = []
+        for lo in range(0, len(steps), MAX_MANY_STEPS):
+            out += self._update_chunk(steps[lo:lo + MAX_MANY_STEPS])
+        return out
+
+    def _many_noise(self, B, n):
+        return None
+
+    def _update_chunk(self, steps):
+        B, n = self.batch_size, len(steps)
+        assert len(self.buffer) >= B, "[ERROR] Not enough in buffer to sample"       # before any state moves
+        if B > self._max_batch:
+            raise ValueError(f"batch size {B} above max_batch {self._max_batch}")
+        noise = self._many_noise(B, n)
+        iptr = None
+        if self.index_source == "host":             # n draws of random.sample(range(len), B), in step order
+            self._pre = self._known_state = None
+            nlen = len(self.buffer)
+            idx = np.stack([_lib.py_sample_range(nlen, B) for _ in steps])
+            iptr = np_ptr(idx)
+        flags = (C.c_int * n)(*(self._flags(s) for s in steps))
+        lr_c, lr_a = (C.c_double * n)(), (C.c_double * n)()
+        schedules = (self.critic_scheduler, self.actor_scheduler)
+        saved = [(sch.last_epoch, sch.lr) for sch in schedules]
+        for i in range(n):                          # the schedules step as _run_update steps them
+            lr_c[i], lr_a[i] = self.critic_scheduler.lr, self.actor_scheduler.lr
+            self.critic_scheduler.step()
+            if flags[i] & 1:
+                self.actor_scheduler.step()
+        metrics = np.empty((n, 8), np.float32)
+        try:
+            check(lib.gcrl_agent_update_many(self._h, self.buffer.handle, B, n, flags, iptr,
+                                             vp(noise.data_ptr()) if noise is not None else None, lr_c, lr_a,
+                                             np_ptr(metrics), self._stream()))
+        except BaseException:
+            for sch, (epoch, lr) in zip(schedules, saved):
+                sch.last_epoch, sch.lr = epoch, lr
+            raise
+        self._last_td = None
+        out = []
+        for step, m in zip(steps, metrics.tolist()):
+            self.beta_scheduler(step)
+            out.append(self._result(step, m))
+        return out
+
 
 class DDPG(_AgentBase):
     """Reference src/agent.py:1173-1465."""
     ALGO = ALGO_DDPG
     WEIGHT_DECAY = 0.0          # torch.optim.Adam (:1201-1202)
     POLYAK_EVERY = 40           # literal at :1397
+    _MANY_IN_ONE_GRAPH = True
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw):
         super().__init__(obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw)
@@ -588,6 +650,9 @@ class DDPG(_AgentBase):
     def update(self, step: int, batch=None, indices=None):                    # :1378-1404
         m = self._run_update(step, batch=batch, indices=indices)
         self.beta_scheduler(step)
+        return self._result(step, m)
+
+    def _result(self, step, m):
         critic_loss, ac_loss, td, q, cg, agn = m[0], m[1], np.float32(m[2]), m[3], m[4], m[5]
         if self._last_td is not None:          # prioritised replay: the per-sample array (:1338-1340)
             td = self._last_td
@@ -613,6 +678,7 @@ class TD3Agent(_AgentBase):
     """Reference src/agent.py:12-386."""
     ALGO = ALGO_TD3
     WEIGHT_DECAY = 0.01         # torch.optim.AdamW default (:46-48)
+    _MANY_IN_ONE_GRAPH = True
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw):
         super().__init__(obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw)
@@ -665,6 +731,14 @@ class TD3Agent(_AgentBase):
             noise = torch.randn((B, self.ac_dim), dtype=torch.float32, device=self.device)
         m = self._run_update(step, batch=batch, indices=indices, noise=noise)
         self.beta_scheduler(step)
+        return self._result(step, m)
+
+    def _many_noise(self, B, n):
+        """n separate draws of update()'s noise, in step order: the CUDA generator advances as under the loop."""
+        import torch
+        return torch.stack([torch.randn((B, self.ac_dim), dtype=torch.float32, device=self.device) for _ in range(n)])
+
+    def _result(self, step, m):
         q1l, acl, td, q, c1g, acg, q2l, c2g = m
         td = np.float32(td) if self._last_td is None else self._last_td
         if step % self.ac_update_freq == 0:

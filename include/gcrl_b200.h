@@ -226,6 +226,19 @@ int gcrl_agent_update_from_buffer(gcrl_agent *h, gcrl_her *buf, int64_t B,
                                   const int64_t *idx_host, const float *noise_dev,
                                   double lr_critic, double lr_actor, int flags,
                                   float *metrics_host, void *stream);
+/* n consecutive updates from `buf`, issued as ONE graph launch.  Equivalent, bit for bit, to n calls of
+ * gcrl_agent_update_from_buffer with flags[i], lr_critic[i], lr_actor[i], the positions idx_host + i*B (or the
+ * device index stream's next n draws when idx_host is NULL) and the TD3 noise noise_dev + i*B*A.
+ * flags[i] may hold bit0 and bit1 only (no prioritised weights: a HER buffer has no priorities).
+ * metrics_host: float[n][8], row i = what update i would have returned; NULL leaves the call async, and
+ * gcrl_agent_read_metrics then returns the last row.  1 <= n <= GCRL_MAX_MANY_STEPS.
+ * Refused (GCRL_ERR_INVALID) on a handle connected for peer data parallelism and while a phase-wise
+ * data-parallel update is open (phase 0 issued, phase 3 not yet).  On any error no Adam step counter, update
+ * sequence number or device index-stream draw has advanced. */
+#define GCRL_MAX_MANY_STEPS 64
+int gcrl_agent_update_many(gcrl_agent *h, gcrl_her *buf, int64_t B, int n, const int *flags,
+                           const int64_t *idx_host, const float *noise_dev, const double *lr_critic,
+                           const double *lr_actor, float *metrics_host, void *stream);
 /* Device metrics of the most recent update (float[8], same order). */
 int gcrl_agent_read_metrics(gcrl_agent *h, float *metrics_host, void *stream);
 
