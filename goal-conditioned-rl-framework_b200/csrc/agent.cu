@@ -264,15 +264,18 @@ void forward_hidden(const gcrl_agent *ag, const Net &n, const float *X, int ldx,
 // Backward through the hidden stack given dz[cur] = grad wrt the pre-activation of the last hidden
 // layer.  Writes split partial weight/bias grads; returns per-layer split counts.  When
 // `to_input` the chain continues to dZ of layer 0 (left in dz[*cur_out]).
-void backward_hidden(gcrl_agent *ag, const Net &n, const float *X, int ldx, int K0, const Acts &acts, int B,
-                     int cur, bool want_wgrad, int *splits /*[layers]*/, int *cur_out, cudaStream_t st) {
+// x_pad_zero: X's columns K0 .. K0 padded to a multiple of 4 are zero.  The actor's input rows [s | a | 0] hold the
+// actions there, which the tensor-core weight gradient would sum into the padding columns of layer 0's gradient
+// (inflating its norm, hence the clip, and stepping the padding weights).
+void backward_hidden(gcrl_agent *ag, const Net &n, const float *X, int ldx, int K0, bool x_pad_zero, const Acts &acts,
+                     int B, int cur, bool want_wgrad, int *splits /*[layers]*/, int *cur_out, cudaStream_t st) {
   for (int l = ag->L - 1; l >= 0; --l) {
     const float *xin = l == 0 ? X : acts.h[l - 1];
     const int ldin = l == 0 ? ldx : ag->ldh;
     const int K = l == 0 ? K0 : ag->H;
     if (want_wgrad) {
-      const int Kp = (K + 3) & ~3;     // operand rows are zero-padded to ld (layer 0)
-      if (use_tc(ag, B, ag->H, Kp) && tc_wgrad_supported(B, ag->H, Kp))
+      const int Kp = (K + 3) & ~3;     // the tensor cores reduce over Kp columns of the operand rows
+      if ((Kp == K || x_pad_zero) && use_tc(ag, B, ag->H, Kp) && tc_wgrad_supported(B, ag->H, Kp))
         splits[l] = launch_tc_wgrad(ag->dz[cur], ag->ldh, xin, ldin, ag->partials + n.w_off[l], n.ldw[l], ag->slab,
                                     ag->partials + n.b_off[l], ag->slab, B, ag->H, Kp, kMaxSplits, st);
       else
@@ -376,7 +379,7 @@ void critic_forward_backward(gcrl_agent *ag, int which_critic, int B, int *split
   *head_splits = launch_head_bwd(h, kMaxSplits, st);
   *metric_splits = *head_splits;
   int cur;
-  backward_hidden(ag, c, ag->sa, ag->ldc, K0, acts, B, 0, true, splits, &cur, st);
+  backward_hidden(ag, c, ag->sa, ag->ldc, K0, true, acts, B, 0, true, splits, &cur, st);
 }
 
 void targets_and_critic_forward(gcrl_agent *ag, int B, const float *noise, cudaStream_t st) {
@@ -636,7 +639,7 @@ void actor_phase_grads(gcrl_agent *ag, int B, cudaStream_t st) {
   const int actor_metric_splits = launch_head_bwd(h, kMaxSplits, st);
   int cur;
   int dummy[8];
-  backward_hidden(ag, c, ag->spi, ag->ldc, K0, ag->acts_c1, B, 0, false, dummy, &cur, st);
+  backward_hidden(ag, c, ag->spi, ag->ldc, K0, true, ag->acts_c1, B, 0, false, dummy, &cur, st);
   launch_action_grad(ag->dz[cur], ag->ldh, c.W(0), c.ldw[0], ag->spi, ag->ldc, D, ag->dz_act, B, ag->H, A, st);
   // actor head + hidden stack backward
   HeadBwdArgs ha{};
@@ -648,7 +651,7 @@ void actor_phase_grads(gcrl_agent *ag, int B, cudaStream_t st) {
   ha.pB = ag->partials + actor.b_off[L]; ha.b_split_stride = ag->slab;
   ha.M = B; ha.K = ag->H;
   ps->head_splits = launch_head_bwd(ha, kMaxSplits, st);
-  backward_hidden(ag, actor, ag->spi, ag->ldc, D, ag->acts_actor, B, 0, true, ps->splits, &cur, st);
+  backward_hidden(ag, actor, ag->spi, ag->ldc, D, false, ag->acts_actor, B, 0, true, ps->splits, &cur, st);
   // the actor-loss metric partials (critic head pass) are still intact: the actor head pass has mode 2
   reduce_grads(ag, ag->net[ACTOR], ps->splits, ps->head_splits, false, S_ALOSS, -1, -1, actor_metric_splits, B,
                st);

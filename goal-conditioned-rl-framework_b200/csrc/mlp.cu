@@ -628,15 +628,18 @@ int launch_wgrad_sumsq(const WgradProblem *probs, int nprob, float *sumsq_partia
 template <int OP>
 static void launch_gemm(const GemmParams &p, int splits, cudaStream_t st) {
   const int sms = sm_count();
-  auto tiles = [&](int bm, int bn) { return ((p.M + bm - 1) / bm) * ((p.N + bn - 1) / bn) * splits; };
+  // weight-gradient slabs: the column tiles span the whole padded row (ldc), so that the epilogue writes its zeros
+  // beyond N even where ldc reaches past the last tile of the N columns
+  const int ncols = OP == OP_WGRAD ? std::max(p.N, p.ldc) : p.N;
+  auto tiles = [&](int bm, int bn) { return ((p.M + bm - 1) / bm) * ((ncols + bn - 1) / bn) * splits; };
   if (tiles(128, 128) >= sms) {
-    dim3 grid((p.N + 127) / 128, (p.M + 127) / 128, splits);
+    dim3 grid((ncols + 127) / 128, (p.M + 127) / 128, splits);
     gemm_kernel<128, 128, 8, 8, OP><<<grid, 256, 0, st>>>(p);
   } else if (tiles(64, 64) >= sms / 2) {
-    dim3 grid((p.N + 63) / 64, (p.M + 63) / 64, splits);
+    dim3 grid((ncols + 63) / 64, (p.M + 63) / 64, splits);
     gemm_kernel<64, 64, 4, 4, OP><<<grid, 256, 0, st>>>(p);
   } else {
-    dim3 grid((p.N + 31) / 32, (p.M + 31) / 32, splits);
+    dim3 grid((ncols + 31) / 32, (p.M + 31) / 32, splits);
     gemm_kernel<32, 32, 4, 4, OP><<<grid, 64, 0, st>>>(p);
   }
   GCRL_LAUNCHED();

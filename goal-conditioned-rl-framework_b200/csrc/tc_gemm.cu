@@ -1167,6 +1167,7 @@ extern "C" int gcrl_dense_layer(int device, int engine, int mode, int64_t M, int
     launch_tc_dense(x_dev, ldx, w_dev, ldw, bias_dev, act_dev, ldact, y_dev, ldy, int(M), N, K, mode, st);
   } else {
     GCRL_REQUIRE(engine == 0 && mode != 1, "engine 0 (fp32 FFMA) implements modes 0 and 2");
+    GCRL_REQUIRE((ldx % 4) == 0 && (ldw % 4) == 0 && (ldy % 4) == 0, "leading dimensions must be multiples of 4");
     launch_linear_fwd(x_dev, ldx, w_dev, ldw, bias_dev, y_dev, ldy, int(M), N, K, mode == 0 ? ACT_LEAKY : ACT_NONE, st);
   }
   GCRL_API_END
@@ -1227,10 +1228,13 @@ extern "C" int gcrl_dense_wgrad(int device, int engine, int64_t M, int N, int K,
   GCRL_REQUIRE(engine == 0 || engine == 1, "engine must be 0 (fp32 FFMA) or 1 (tensor cores)");
   GCRL_CUDA(cudaSetDevice(device));
   cudaStream_t st = as_stream(stream);
-  *splits_out = engine == 1
-                    ? launch_tc_wgrad(dz_dev, lddz, x_dev, ldx, pw_dev, ldw, w_split_stride, pb_dev, b_split_stride, int(M),
-                                      N, K, max_splits, st)
-                    : launch_linear_wgrad(dz_dev, lddz, x_dev, ldx, pw_dev, ldw, w_split_stride, pb_dev, b_split_stride,
-                                          int(M), N, K, max_splits, st);
+  if (engine == 1) {
+    *splits_out = launch_tc_wgrad(dz_dev, lddz, x_dev, ldx, pw_dev, ldw, w_split_stride, pb_dev, b_split_stride, int(M),
+                                  N, K, max_splits, st);
+  } else {
+    GCRL_REQUIRE((lddz % 4) == 0 && (ldx % 4) == 0 && (ldw % 4) == 0, "leading dimensions must be multiples of 4");
+    *splits_out = launch_linear_wgrad(dz_dev, lddz, x_dev, ldx, pw_dev, ldw, w_split_stride, pb_dev, b_split_stride,
+                                      int(M), N, K, max_splits, st);
+  }
   GCRL_API_END
 }

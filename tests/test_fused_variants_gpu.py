@@ -103,7 +103,7 @@ def init_nets(rng, algo, D, A, H, L):
     return [OD.init_mlp(rng, D, H, A, L)] + [OD.init_mlp(rng, D + A, H, 1, L) for _ in range(1 if algo == "ddpg" else 2)]
 
 
-def make_agent(algo, B, nets, monkeypatch, D, A, H, L, graphs=False, **over):
+def make_agent(algo, B, nets, monkeypatch, D, A, H, L, graphs=False, precision=1, **over):
     from gcrl_b200 import DDPG, TD3Agent
     from gcrl_b200.agent import NET_ACTOR, NET_CRITIC, NET_CRITIC2
     if graphs:
@@ -112,7 +112,7 @@ def make_agent(algo, B, nets, monkeypatch, D, A, H, L, graphs=False, **over):
         monkeypatch.setenv("GCRL_B200_NO_GRAPH", "1")             # read at creation
     cfg = make_config(hidden_dim=H, layer_count=L, batch_size=B, grad_clip=0.5, tau=0.05,
                       ac_update_freq=1 if algo == "ddpg" else 2, **over)
-    ag = (DDPG if algo == "ddpg" else TD3Agent)(D, A, cfg, None, 1, 40)
+    ag = (DDPG if algo == "ddpg" else TD3Agent)(D, A, cfg, None, 1, 40, precision=precision)
     for net, params in zip((NET_ACTOR, NET_CRITIC, NET_CRITIC2), nets):
         ag._set_layers(net, params)
     ag.update_target_network()
