@@ -157,7 +157,6 @@ struct gcrl_agent {
   float *metric_partials = nullptr;        // [kMaxSplits][4]
   float *sumsq = nullptr;                  // [max(reduce grid, wgrad tiles)]
   int nsumsq = 0;                          // how many sums of squares the pending optimiser step reads
-  int wtiles = 0;                          // upper bound of the weight-gradient tiles of any network
   float *metrics = nullptr;                // [8]
   StepScalars *d_scalars = nullptr;        // StepScalars, then the SampleScalars of the update (one H2D copy)
   SampleScalars *d_sample_sc = nullptr;
@@ -188,10 +187,6 @@ struct gcrl_agent {
     unsigned int *go = nullptr;                          // local release word: CTA 0 saw every peer's flag
     unsigned int *ticket = nullptr, *wticket = nullptr;  // CTA tickets of the barrier + average launch / the weight-gradient launch
     bool signalled = false;                              // capture-time: the gradient's producer raises the flag itself
-    bool averaged = false;                               // capture-time: ... or already left the average in gavg (tile-fused)
-    bool tile_fused = false;                             // GCRL_P2P_TILE_FUSED=1: average inside the weight-gradient kernel
-    unsigned int *tflags = nullptr;                      // per-tile flags [wtiles][32] written by the peers
-    unsigned int **d_peer_tflags = nullptr;
     int *err = nullptr;
     float *outbox = nullptr, *metrics_avg = nullptr;     // [2][8] metrics published to / [8] averaged over the ranks
     float *gavg[NUM_NETS] = {};                          // averaged gradient of every trainable network
@@ -446,7 +441,7 @@ unsigned int critic_metric_mask(const gcrl_agent *ag, int which) {
 // gradient n.g, the per-tile sums of squares and the batch-mean metrics (mlp.cu: multi_wgrad_kernel);
 // hidden-layer operands: dzl[l] and (l == 0 ? sa : acts.h[l-1]); head operand: dz_head [B][ld_head] and acts.h[L-1]
 void fused_wgrads(gcrl_agent *ag, Net &n, const Acts &acts, int K0, const float *dz_head, int ld_head, int B,
-                  int slot_loss, int slot_td, int slot_q, int metric_splits, unsigned int metric_mask, cudaStream_t st) {
+                  int slot_loss, int slot_td, int slot_q, int metric_splits, cudaStream_t st) {
   WgradProblem pr[kMaxWgradProblems];
   const int L = ag->L;
   for (int l = 0; l < L; ++l) {
@@ -463,21 +458,11 @@ void fused_wgrads(gcrl_agent *ag, Net &n, const Acts &acts, int K0, const float 
   fin.metric_scale = 1.0f / float(B);
   fin.metrics = ag->metrics;
   fin.slot_loss = slot_loss; fin.slot_td = slot_td; fin.slot_q = slot_q;
-  if (ag->p2p.on) {
+  if (ag->p2p.on) {         // the last CTA raises this rank's flag at every peer (p2p_average then only waits)
     auto &pp = ag->p2p;
-    const int id = int(&n - ag->net);
-    fin.epoch = pp.epoch; fin.ticket = pp.wticket; fin.outbox = pp.outbox;
+    fin.peer_flags = pp.d_peer_flags; fin.epoch = pp.epoch; fin.ticket = pp.wticket; fin.outbox = pp.outbox;
     fin.rank = pp.rank; fin.world = pp.world;
-    if (pp.tile_fused) {    // compute + all-reduce in one kernel: every CTA averages its own tile over the peers
-      fin.peers_g = pp.d_peer_g[id]; fin.g_base = n.g; fin.gavg = pp.gavg[id];
-      fin.peer_tflags = pp.d_peer_tflags; fin.tflags = pp.tflags;
-      fin.peer_outbox = pp.d_peer_outbox; fin.metrics_avg = pp.metrics_avg; fin.metric_mask = metric_mask;
-      fin.inv_world = 1.0f / float(pp.world); fin.err = pp.err; fin.timeout_cycles = p2p_timeout_cycles();
-      pp.averaged = true;
-    } else {                // the last CTA raises this rank's flag at every peer (p2p_average then only waits)
-      fin.peer_flags = pp.d_peer_flags;
-      pp.signalled = true;
-    }
+    pp.signalled = true;
   }
   ag->nsumsq = launch_wgrad_complete(pr, L + 1, B, fin, st);
 }
@@ -535,8 +520,7 @@ void fused_critic_phase_grads(gcrl_agent *ag, int B, int which, cudaStream_t st)
   // TD3: td error / Q metrics come from the critic-2 launch (they need both critics' Q)
   const bool metrics_here = !ag->td3 || which == 1;
   fused_wgrads(ag, c, which == 0 ? ag->acts_c1 : ag->acts_c2, ag->D + ag->A, ag->dzh, 1, B,
-               which == 0 ? S_CLOSS : S_C2LOSS, metrics_here ? S_TD : -1, metrics_here ? S_Q : -1, slabs,
-               critic_metric_mask(ag, which), st);
+               which == 0 ? S_CLOSS : S_C2LOSS, metrics_here ? S_TD : -1, metrics_here ? S_Q : -1, slabs, st);
 }
 
 void fused_actor_phase_grads(gcrl_agent *ag, int B, cudaStream_t st) {
@@ -549,7 +533,7 @@ void fused_actor_phase_grads(gcrl_agent *ag, int B, cudaStream_t st) {
   a.da_out = ag->dz_act;
   a.metric_partials = ag->metric_partials;
   const int slabs = launch_fused_actor(a, st);
-  fused_wgrads(ag, ag->net[ACTOR], ag->acts_actor, ag->D, ag->dz_act, 4, B, S_ALOSS, -1, -1, slabs, 1u << S_ALOSS, st);
+  fused_wgrads(ag, ag->net[ACTOR], ag->acts_actor, ag->D, ag->dz_act, 4, B, S_ALOSS, -1, -1, slabs, st);
 }
 
 // critic(s): forward, loss, backward, partials -> flat local-mean gradient(s) + metrics
@@ -596,8 +580,7 @@ void critic_phase_step(gcrl_agent *ag, int which, int flags, bool rereduce, cuda
   const float *grad = nullptr;
   // metrics final before this barrier: DDPG critic loss / td / q; TD3 critic 1: its loss; critic 2: loss, td, q
   const unsigned int mm = critic_metric_mask(ag, which);
-  if (ag->p2p.on && ag->p2p.averaged) { grad = ag->p2p.gavg[id]; ag->p2p.averaged = false; }   // done by the weight-gradient kernel
-  else if (ag->p2p.on) grad = p2p_average(ag, id, mm, st);
+  if (ag->p2p.on) grad = p2p_average(ag, id, mm, st);
   else if (rereduce && fused_ok(ag, ag->dp_B)) fused_grad_sumsq(ag, c, st);
   else if (rereduce) reduce_grads(ag, c, nullptr, 0, true, -1, -1, -1, 0, 1, st);
   // TD3 critic 1 is NOT clipped (:201 is commented out), critic 2 is
@@ -660,8 +643,7 @@ void actor_phase_grads(gcrl_agent *ag, int B, cudaStream_t st) {
 void actor_phase_step(gcrl_agent *ag, bool rereduce, cudaStream_t st) {
   Net &a = ag->net[ACTOR];
   const float *grad = nullptr;
-  if (ag->p2p.on && ag->p2p.averaged) { grad = ag->p2p.gavg[ACTOR]; ag->p2p.averaged = false; }
-  else if (ag->p2p.on) grad = p2p_average(ag, ACTOR, 1u << S_ALOSS, st);
+  if (ag->p2p.on) grad = p2p_average(ag, ACTOR, 1u << S_ALOSS, st);
   else if (rereduce && fused_ok(ag, ag->dp_B)) fused_grad_sumsq(ag, a, st);
   else if (rereduce) reduce_grads(ag, a, nullptr, 0, true, -1, -1, -1, 0, 1, st);
   adam_step(ag, a, 1, ag->cfg.grad_clip, S_AGRAD, &ag->net[T_ACTOR], ag->td3, st, grad);
@@ -1058,7 +1040,6 @@ int gcrl_agent_create(gcrl_agent **out, int device, const gcrl_agent_config *cfg
     ag->metric_partials = dev_alloc<float>(size_t(256) * 4);
     const int ht = (H + 31) / 32;              // 32 x 32 output tiles of the largest net (multi_wgrad_kernel)
     const int wtiles = ht * ((D + A + 31) / 32) + (L - 1) * ht * ht + ht + 8;
-    ag->wtiles = wtiles;
     ag->sumsq = dev_alloc<float>(size_t(std::max(reduce_grid(int(ag->slab)), wtiles)) + 8);
     ag->metrics = dev_alloc<float>(8);
     GCRL_CUDA(cudaMemset(ag->metrics, 0, 8 * sizeof(float)));
@@ -1099,8 +1080,8 @@ int gcrl_agent_destroy(gcrl_agent *ag) {
   if (ag->many.noise) cudaFree(ag->many.noise);
   if (ag->many.h_pub) cudaFreeHost(ag->many.h_pub);
   for (void *p : ag->p2p.opened) cudaIpcCloseMemHandle(p);
-  for (void *p : {(void *)ag->p2p.flags, (void *)ag->p2p.epoch, (void *)ag->p2p.ticket, (void *)ag->p2p.wticket, (void *)ag->p2p.go, (void *)ag->p2p.tflags,
-                  (void *)ag->p2p.d_peer_tflags, (void *)ag->p2p.err, (void *)ag->p2p.outbox,
+  for (void *p : {(void *)ag->p2p.flags, (void *)ag->p2p.epoch, (void *)ag->p2p.ticket, (void *)ag->p2p.wticket, (void *)ag->p2p.go,
+                  (void *)ag->p2p.err, (void *)ag->p2p.outbox,
                   (void *)ag->p2p.metrics_avg, (void *)ag->p2p.d_peer_flags, (void *)ag->p2p.d_peer_outbox})
     if (p) cudaFree(p);
   for (int i = 0; i < NUM_NETS; ++i) {
@@ -1524,7 +1505,6 @@ static int dp_items(gcrl_agent *ag, void **ptrs) {
   int n = 0;
   ptrs[n++] = ag->p2p.flags;
   ptrs[n++] = ag->p2p.outbox;
-  ptrs[n++] = ag->p2p.tflags;
   for (int id : {int(ACTOR), int(CRITIC1), int(CRITIC2)})
     if (ag->has[id]) ptrs[n++] = ag->net[id].g;
   return n;
@@ -1545,14 +1525,6 @@ int gcrl_agent_dp_export(gcrl_agent *ag, unsigned char *handles /*[n_items][64]*
     GCRL_CUDA(cudaMemset(pp.wticket, 0, sizeof(unsigned int)));
     pp.go = dev_alloc<unsigned int>(1);
     GCRL_CUDA(cudaMemset(pp.go, 0, sizeof(unsigned int)));
-    pp.tflags = dev_alloc<unsigned int>(size_t(ag->wtiles) * 32);
-    GCRL_CUDA(cudaMemset(pp.tflags, 0, size_t(ag->wtiles) * 32 * sizeof(unsigned int)));
-    // opt-in: compute + all-reduce in ONE kernel (every weight-gradient CTA averages its own tile over the peers).
-    // Parity-green at 2 and 8 GPUs but measured slower than the separate barrier + average launch (0.1533 vs 0.1511 ms
-    // per step at N = 2, 0.1697 vs 0.1640 at N = 8): the tiles finish together, so there is no transfer to hide
-    // behind arithmetic, and 144 CTAs each pay the flag round trip that one launch pays once.
-    const char *tf = getenv("GCRL_P2P_TILE_FUSED");
-    pp.tile_fused = tf && tf[0] == '1';
     pp.err = dev_alloc<int>(1);
     pp.outbox = dev_alloc<float>(16);
     pp.metrics_avg = dev_alloc<float>(8);
@@ -1603,8 +1575,7 @@ int gcrl_agent_dp_connect(gcrl_agent *ag, int rank, int world, const unsigned ch
   };
   pp.d_peer_flags = reinterpret_cast<unsigned int **>(upload(0));
   pp.d_peer_outbox = reinterpret_cast<float **>(upload(1));
-  pp.d_peer_tflags = reinterpret_cast<unsigned int **>(upload(2));
-  int item = 3;
+  int item = 2;
   for (int id : {int(ACTOR), int(CRITIC1), int(CRITIC2)})
     if (ag->has[id]) {
       pp.d_peer_g[id] = reinterpret_cast<float **>(upload(item++));

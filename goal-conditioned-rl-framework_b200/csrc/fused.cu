@@ -571,22 +571,13 @@ bool fused_supported(int B, int D, int A, int H, int L) {
   return fused_smem_bytes(R, D, A, H, L, true) <= size_t(200) * 1024;
 }
 
-static bool fused_split_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char *e = getenv("GCRL_FUSED_SPLIT");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
-
 int launch_fused_critic(const FusedCriticArgs &a, cudaStream_t st) {
   const int R = fused_rows_per_cta(a.B);
   const int grid = (a.B + R - 1) / R;
   const size_t smem = fused_smem_bytes(R, a.D, a.A, a.H, a.L, false);
   const bool td3 = a.has_tc2 || a.noise != nullptr || a.y_in != nullptr || a.loss_kind != 0 || a.q_other != nullptr;
   // two CTAs per slab (target path | critic path) when there is a target path and everything fits in one wave
-  const bool split = fused_split_enabled() && R != 2 && a.y_in == nullptr && 2 * grid <= sm_count();
+  const bool split = R != 2 && a.y_in == nullptr && 2 * grid <= sm_count();
   auto go = [&](auto kernel, int *flag, bool clustered) {
     ensure_smem(kernel, smem, flag);
     if (!clustered) {

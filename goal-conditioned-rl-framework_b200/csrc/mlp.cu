@@ -437,76 +437,8 @@ __global__ void __launch_bounds__(kWgThreads * GROUPS) wgrad_tile_kernel(const _
     const int slot = t == 0 ? mg.fin.slot_loss : (t == 1 ? mg.fin.slot_td : mg.fin.slot_q);
     if (slot >= 0) mg.fin.metrics[slot] = s * mg.fin.metric_scale;
   }
-  if (mg.fin.peers_g != nullptr) {
-    // ---- fused cross-rank average of THIS tile (peer-memory data parallelism) ----
-    const WgradFinal &f = mg.fin;
-    __shared__ unsigned int s_e;
-    if (t == 0) s_e = *f.epoch + 1u;          // advanced by the last CTA only after every CTA has taken its ticket
-    __syncthreads();                          // tile (and tile 0's metrics) written by this CTA's threads
-    const unsigned int e = s_e;
-    if (blockIdx.x == 0 && t < 8) f.outbox[(e & 1u) * 8 + t] = __ldcg(f.metrics + t);
-    __syncthreads();
-    if (t < f.world) {
-      __threadfence_system();                 // the CTA's tile is visible system-wide before its flag is
-      volatile unsigned int *dst = f.peer_tflags[t] + size_t(blockIdx.x) * 32 + f.rank;
-      *dst = e;
-      const unsigned int *src = f.tflags + size_t(blockIdx.x) * 32 + t;
-      const long long t0 = clock64();
-      unsigned int seen;
-      for (;;) {
-        asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(seen) : "l"(src) : "memory");
-        if (seen >= e) break;
-        if (clock64() - t0 > f.timeout_cycles) {             // a peer died: fail loudly instead of hanging
-          atomicExch(f.err, 1 + t + 16 * f.rank);
-          break;
-        }
-        __nanosleep(100);
-      }
-    }
-    __syncthreads();
-    sq = 0.f;
-    if (t < kWgFinish) {
-      const int r = t / (BN / 4), c = (t % (BN / 4)) * 4;
-      if (m0 + r < p.M && n0 + c < p.ldc) {
-        const size_t goff = size_t(mg.gW[pi] - f.g_base) + size_t(m0 + r) * p.ldc + n0 + c;
-        float4 v[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q)
-          if (q < f.world) v[q] = __ldcv(reinterpret_cast<const float4 *>(f.peers_g[q] + goff));
-        float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-        for (int q = 0; q < 8; ++q)
-          if (q < f.world) { a.x += v[q].x; a.y += v[q].y; a.z += v[q].z; a.w += v[q].w; }     // rank order: identical replicas
-        a.x *= f.inv_world; a.y *= f.inv_world; a.z *= f.inv_world; a.w *= f.inv_world;
-        *reinterpret_cast<float4 *>(f.gavg + goff) = a;
-        sq = fmaf(a.x, a.x, sq); sq = fmaf(a.y, a.y, sq); sq = fmaf(a.z, a.z, sq); sq = fmaf(a.w, a.w, sq);
-      }
-      if (bx == 0 && t < BM && m0 + t < p.M) {
-        const size_t goff = size_t(mg.gB[pi] - f.g_base) + m0 + t;
-        float a = 0.f;
-        for (int q = 0; q < f.world; ++q) a += __ldcv(f.peers_g[q] + goff);
-        a *= f.inv_world;
-        f.gavg[goff] = a;
-        sq = fmaf(a, a, sq);
-      }
-    }
-    if (blockIdx.x == 0 && t < 8 && ((f.metric_mask >> t) & 1u)) {
-      float s = 0.f;
-      for (int q = 0; q < f.world; ++q) s += __ldcv(f.peer_outbox[q] + (e & 1u) * 8 + t);
-      f.metrics_avg[t] = s * f.inv_world;
-    }
-  }
   tile_sumsq_store(sq, s_sq, mg.fin.sumsq_partials + blockIdx.x);
-  if (mg.fin.peers_g != nullptr) {
-    if (t == 0) {                              // (tile_sumsq_store ends with this thread past its barrier)
-      __threadfence();
-      const unsigned int k = atomicAdd(mg.fin.ticket, 1u);
-      if (k == gridDim.x - 1) {
-        *mg.fin.ticket = 0;
-        *mg.fin.epoch = *mg.fin.epoch + 1u;
-      }
-    }
-  } else if (mg.fin.peer_flags != nullptr) {
+  if (mg.fin.peer_flags != nullptr) {
     // every CTA: gradient tile (and tile 0's metrics) ordered before its ticket; the last one raises the flags
     __shared__ int s_last;
     __syncthreads();

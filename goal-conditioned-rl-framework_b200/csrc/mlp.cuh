@@ -95,16 +95,6 @@ struct WgradFinal {
   // (and publishes the metrics) -- the flag travels over NVLink while the averaging kernel is being launched
   unsigned int *const *peer_flags; unsigned int *epoch; unsigned int *ticket;
   float *outbox; int rank, world;
-  // ... or, fused with the collective: every CTA publishes ITS tile (a flag per tile and rank), waits for the
-  // same tile of every peer, reads the peers' tiles over NVLink, and leaves the rank-order AVERAGE in `gavg` with the
-  // average's sum of squares -- compute and all-reduce in one kernel, the transfer of finished tiles overlapping
-  // the arithmetic of the others (peers_g != nullptr selects this mode; peer_flags is then unused)
-  const float *const *peers_g;          // [world] flat gradient of this network on every rank (peers_g[rank] = g_base)
-  const float *g_base; float *gavg;
-  unsigned int *const *peer_tflags;     // [world] per-tile flag arrays, 32 words (128 B) per tile, word r = rank r
-  unsigned int *tflags;                 // this rank's own array
-  const float *const *peer_outbox; float *metrics_avg; unsigned int metric_mask;
-  float inv_world; int *err; long long timeout_cycles;
 };
 // Split-batch partial slabs (summed later by reduce_grads); returns the number of batch slabs S.
 int launch_multi_wgrad(const WgradProblem *probs, int nprob, int M, int64_t split_stride, int max_splits,

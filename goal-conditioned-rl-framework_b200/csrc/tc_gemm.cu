@@ -19,11 +19,8 @@
 // tile i overlaps the MMAs of tile i+1).
 #include <cuda.h>
 
-#include <cstdio>
-#include <cstdlib>
 #include <map>
 #include <tuple>
-#include <vector>
 
 #include "mlp.cuh"
 
@@ -215,12 +212,9 @@ struct TcArgs {
   long long split_stride;
   int acc_slabs;                 // kind 1: a CTA adds the later slabs of its (n, k) block onto the first one it wrote
   float *colsum;                 // kind 1: bias-gradient partials pB[slab][n] = column sums of the slab's dZ rows, taken
-  long long colsum_stride;       // by the splitter warps from the tiles they split anyway (nullptr: separate kernel)
+  long long colsum_stride;       // by the splitter warps from the tiles they split anyway (nullptr: no bias gradient)
   int members;                   // ensemble kernel (NMEM > 1): problems of this shape in the launch
   int full_items;                // pair kernel: tiles taken whole; the rest are split into two 256 x 128 halves
-  long long *trace;              // GCRL_TC_TRACE: per-stage timestamps of the first CTA pair (pair kernel only)
-  int dbg;                       // timing experiments only (GCRL_TC_DBG): 1 skip split, 2 skip stores, 4 one MMA per k
-                                 // step, 64 no epilogue, 128 epilogue stops after the TMEM load (wrong results)
 };
 
 template <int BN>
@@ -377,10 +371,8 @@ tc_dense_kernel(const __grid_constant__ TcOperands<NMEM> ops, TcArgs a) {
               // MN-major: the next 8-row group of every box (+1024 bytes)
               const uint64_t ko = wg ? uint64_t(k * (1024 >> 4)) : uint64_t(k * 2);
               umma_tf32(d, a_lo + ko, b_hi + ko, idesc, (kb | k) != 0 ? 1u : 0u);
-              if (!(a.dbg & 4)) {
-                umma_tf32(d, a_hi + ko, b_lo + ko, idesc, 1u);
-                umma_tf32(d, a_hi + ko, b_hi + ko, idesc, 1u);
-              }
+              umma_tf32(d, a_hi + ko, b_lo + ko, idesc, 1u);
+              umma_tf32(d, a_hi + ko, b_hi + ko, idesc, 1u);
             }
             umma_commit(empty(s));                      // smem stage reusable once these MMAs retire
           }
@@ -411,13 +403,9 @@ tc_dense_kernel(const __grid_constant__ TcOperands<NMEM> ops, TcArgs a) {
       // (lane = 4 columns of one of 4 rows) so that every global access is a full 128-byte row segment
       const uint32_t stg = stage_base + uint32_t(q) * (32 * kStgLd * 4);
 #pragma unroll 1
-      for (int c = 0; c < ((a.dbg & 64) ? 0 : BN); c += 32) {
+      for (int c = 0; c < BN; c += 32) {
         uint32_t v[32];
         tmem_ld32(taddr + uint32_t(c), v);
-        if (a.dbg & 128) {
-          asm volatile("" ::"r"(v[0]), "r"(v[31]));
-          continue;
-        }
         __syncwarp();
 #pragma unroll
         for (int j = 0; j < 32; j += 4)
@@ -425,9 +413,7 @@ tc_dense_kernel(const __grid_constant__ TcOperands<NMEM> ops, TcArgs a) {
                        "r"(v[j + 1]), "r"(v[j + 2]), "r"(v[j + 3])
                        : "memory");
         __syncwarp();
-        if (!(a.dbg & 2))
-          epilogue_store32(stg, lane, m0 + q * 32, n0 + c, rows_valid, cols_valid, emode, bias, act, a.ldact, obase,
-                           a.ldo);
+        epilogue_store32(stg, lane, m0 + q * 32, n0 + c, rows_valid, cols_valid, emode, bias, act, a.ldact, obase, a.ldo);
       }
       tc_fence_before();
       __syncwarp();
@@ -456,43 +442,41 @@ tc_dense_kernel(const __grid_constant__ TcOperands<NMEM> ops, TcArgs a) {
         // (hi at st + 2 kA, lo at + kB).  All loads of a thread are issued before the first store.
         constexpr int kChunksA = S::kA / 16, kChunks = PRESPLIT ? kChunksA : (S::kA + S::kB) / 16;
         constexpr int kPer = (kChunks + kSplitThreads - 1) / kSplitThreads;
-        if (!(a.dbg & 1)) {
-          float x[kPer][4];
-          uint32_t hi_addr[kPer], lo_addr[kPer];
+        float x[kPer][4];
+        uint32_t hi_addr[kPer], lo_addr[kPer];
 #pragma unroll
-          for (int u = 0; u < kPer; ++u) {
-            const int c = tid + u * kSplitThreads;
-            const bool isA = c < kChunksA;
-            hi_addr[u] = isA ? st + 16u * c : st + 2 * S::kA + 16u * (c - kChunksA);
-            lo_addr[u] = hi_addr[u] + (isA ? S::kA : S::kB);
-            if (c < kChunks)
-              asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
-                           : "=f"(x[u][0]), "=f"(x[u][1]), "=f"(x[u][2]), "=f"(x[u][3])
-                           : "r"(hi_addr[u]));
-          }
-          if (cs_tile) {
+        for (int u = 0; u < kPer; ++u) {
+          const int c = tid + u * kSplitThreads;
+          const bool isA = c < kChunksA;
+          hi_addr[u] = isA ? st + 16u * c : st + 2 * S::kA + 16u * (c - kChunksA);
+          lo_addr[u] = hi_addr[u] + (isA ? S::kA : S::kB);
+          if (c < kChunks)
+            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
+                         : "=f"(x[u][0]), "=f"(x[u][1]), "=f"(x[u][2]), "=f"(x[u][3])
+                         : "r"(hi_addr[u]));
+        }
+        if (cs_tile) {
 #pragma unroll
-            for (int u = 0; u < 2; ++u)
+          for (int u = 0; u < 2; ++u)
 #pragma unroll
-              for (int e = 0; e < 4; ++e) cs[u][e] += x[u][e];
-          }
+            for (int e = 0; e < 4; ++e) cs[u][e] += x[u][e];
+        }
 #pragma unroll
-          for (int u = 0; u < kPer; ++u) {
-            const int c = tid + u * kSplitThreads;
-            if (c < kChunks) {
-              uint32_t h[4], l[4];
+        for (int u = 0; u < kPer; ++u) {
+          const int c = tid + u * kSplitThreads;
+          if (c < kChunks) {
+            uint32_t h[4], l[4];
 #pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                h[e] = rna_tf32(x[u][e]);
-                l[e] = rna_tf32(x[u][e] - __uint_as_float(h[e]));
-              }
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(hi_addr[u]), "r"(h[0]), "r"(h[1]), "r"(h[2]),
-                           "r"(h[3])
-                           : "memory");
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(lo_addr[u]), "r"(l[0]), "r"(l[1]), "r"(l[2]),
-                           "r"(l[3])
-                           : "memory");
+            for (int e = 0; e < 4; ++e) {
+              h[e] = rna_tf32(x[u][e]);
+              l[e] = rna_tf32(x[u][e] - __uint_as_float(h[e]));
             }
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(hi_addr[u]), "r"(h[0]), "r"(h[1]), "r"(h[2]),
+                         "r"(h[3])
+                         : "memory");
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(lo_addr[u]), "r"(l[0]), "r"(l[1]), "r"(l[2]),
+                         "r"(l[3])
+                         : "memory");
           }
         }
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> visible to the MMA (async proxy)
@@ -609,14 +593,6 @@ tc_dense_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
   const bool leader = rank == 0;
-  // timeline of the first pair (GCRL_TC_TRACE=file): globaltimer at the hand-over points of every stage use
-  auto mark = [&](int role, uint32_t it) {
-    if (a.trace != nullptr && blockIdx.x < 2 && it < 64) {
-      long long t;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-      a.trace[(size_t(blockIdx.x) * 8 + role) * 64 + it] = t;
-    }
-  };
 
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < STAGES2; ++s) {
@@ -673,7 +649,6 @@ tc_dense_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
         mbar_wait(empty(s), ((it / STAGES2) & 1) ^ 1);
         const uint32_t st = base + s * S::kStage;
         if (elect_one()) {
-          mark(0, it);
           mbar_expect_tx(full(s), S::kA + 2 * rows_b * ROWB);
           tma_load_2d(st, &tmA, full(s), kb * BKF, wi.m0);
           for (int r = 0; r < rows_b; r += 64) {             // weight maps: boxes of 64 rows
@@ -704,18 +679,14 @@ tc_dense_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
           const uint64_t a_hi = umma_desc_sw(st), a_lo = umma_desc_sw(st + S::kA);
           const uint64_t b_hi = umma_desc_sw(st + 2 * S::kA), b_lo = umma_desc_sw(st + 2 * S::kA + S::kBh);
           if (elect_one()) {
-            mark(3, it);
 #pragma unroll
             for (int k = 0; k < BKF / 8; ++k) {
               const uint64_t ko = uint64_t(k * 2);
               umma_tf32_pair(d, a_lo + ko, b_hi + ko, idesc, (kb | k) != 0 ? 1u : 0u);
-              if (!(a.dbg & 4)) {
-                umma_tf32_pair(d, a_hi + ko, b_lo + ko, idesc, 1u);
-                umma_tf32_pair(d, a_hi + ko, b_hi + ko, idesc, 1u);
-              }
+              umma_tf32_pair(d, a_hi + ko, b_lo + ko, idesc, 1u);
+              umma_tf32_pair(d, a_hi + ko, b_hi + ko, idesc, 1u);
             }
             umma_commit_pair(empty(s));
-            mark(4, it);
           }
           __syncwarp();
         }
@@ -729,10 +700,7 @@ tc_dense_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
         for (int kb = 0; kb < nk; ++kb, ++it) {
           const int s = it % STAGES2;
           mbar_wait(split_done(s), (it / STAGES2) & 1);
-          if (elect_one()) {
-            mbar_arrive_cluster(map_to_cta(peer_ready(s), 0));
-            mark(5, it);
-          }
+          if (elect_one()) mbar_arrive_cluster(map_to_cta(peer_ready(s), 0));
           __syncwarp();
         }
     }
@@ -749,18 +717,13 @@ tc_dense_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       if (lane == 0) mbar_wait(tfull(as), (tile_it >> 1) & 1);
       __syncwarp();
       tc_fence_after();
-      if (q == 0 && part == 0 && lane == 0) mark(6, tile_it);
       const uint32_t taddr = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(as * BN);
       const uint32_t stg = stage_base + uint32_t(q + 4 * part) * (32 * kStgLd * 4);
       const int c_lo = part * (wi.ncols / 2), c_hi = c_lo + wi.ncols / 2;
 #pragma unroll 1
-      for (int c = c_lo; c < ((a.dbg & 64) ? 0 : c_hi); c += 32) {
+      for (int c = c_lo; c < c_hi; c += 32) {
         uint32_t v[32];
         tmem_ld32(taddr + uint32_t(c), v);
-        if (a.dbg & 128) {
-          asm volatile("" ::"r"(v[0]), "r"(v[31]));
-          continue;
-        }
         __syncwarp();
 #pragma unroll
         for (int j = 0; j < 32; j += 4)
@@ -768,13 +731,11 @@ tc_dense_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                        "r"(v[j + 1]), "r"(v[j + 2]), "r"(v[j + 3])
                        : "memory");
         __syncwarp();
-        if (!(a.dbg & 2))
-          epilogue_store32(stg, lane, m0 + q * 32, n0 + c, a.M, a.N, a.mode, a.bias, a.act, a.ldact, a.out, a.ldo);
+        epilogue_store32(stg, lane, m0 + q * 32, n0 + c, a.M, a.N, a.mode, a.bias, a.act, a.ldact, a.out, a.ldo);
       }
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(map_to_cta(tempty(as), 0));
-      if (q == 0 && part == 0 && lane == 0) mark(7, tile_it);
     }
   } else {
     // ===== hi / lo splitter (both CTAs): the activation tile only =====
@@ -785,12 +746,10 @@ tc_dense_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
         const int s = it % STAGES2;
         if (lane == 0) mbar_wait(full(s), (it / STAGES2) & 1);
         __syncwarp();
-        if (tid == 0) mark(1, it);
         const uint32_t st = base + s * S::kStage;
         constexpr int kChunks = S::kA / 16, kPer = kChunks / kSplitThreads;
         static_assert(kChunks % kSplitThreads == 0, "splitter threads must tile the activation stage");
         float x[kPer][4];
-        if (!(a.dbg & 1)) {
 #pragma unroll
         for (int u = 0; u < kPer; ++u)
           asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
@@ -811,11 +770,9 @@ tc_dense_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                        "r"(l[3])
                        : "memory");
         }
-        }
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();
         if (lane == 0) mbar_arrive(split_done(s));
-        if (tid == 0) mark(2, it);
       }
     }
   }
@@ -864,40 +821,6 @@ CUtensorMap make_map(const float *ptr, int64_t rows, int cols, int ld, int box_r
   return m;
 }
 
-// pB[slab][n] = sum over the slab's rows of dZ[m][n]   (bias gradient partials; fixed order).
-// One CTA per (slab, 32-column block): 8 row lanes x 32 columns, every warp reads whole 128-byte row segments,
-// 8 loads per thread in flight; the row lanes are summed through shared memory in lane order.  (The first version
-// -- 128 threads per 128 columns, 4 loads in flight, 256 CTAs -- kept 0.5 MB in flight and ran at 1.2 TB/s:
-// 11 % of the B = 65536 update.)
-__global__ void __launch_bounds__(256)
-colsum_partials_kernel(const float *__restrict__ dZ, int lddz, int M, int N, int rows_per_slab, float *__restrict__ pB,
-                       long long split_stride) {
-  __shared__ float sm[8][33];
-  const int lane = threadIdx.x & 31, rl = threadIdx.x >> 5;
-  const int n = blockIdx.y * 32 + lane;
-  const int r0 = blockIdx.x * rows_per_slab, r1 = min(M, r0 + rows_per_slab);
-  float s[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  if (n < N) {
-    int m = r0 + rl;
-    for (; m + 56 < r1; m += 64) {
-      float v[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) v[u] = dZ[size_t(m + 8 * u) * lddz + n];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) s[u] += v[u];
-    }
-    for (; m < r1; m += 8) s[0] += dZ[size_t(m) * lddz + n];
-  }
-  sm[rl][lane] = ((s[0] + s[1]) + (s[2] + s[3])) + ((s[4] + s[5]) + (s[6] + s[7]));
-  __syncthreads();
-  if (rl == 0 && n < N) {
-    float t = 0.f;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) t += sm[k][lane];
-    pB[(long long)blockIdx.x * split_stride + n] = t;
-  }
-}
-
 template <int BN>
 void set_attr() {
   static bool attr_set = false;
@@ -937,29 +860,26 @@ void launch_bn_ensemble(const TcOperands<kTcMaxMembers> &ops, const TcArgs &a, c
   GCRL_LAUNCHED();
 }
 
-// CTA pairs that can be co-resident (one per TPC); 0 = the pair kernel is switched off (GCRL_TC_PAIR=0) or the
-// device cannot host it.  Queried once, outside stream capture (tc_dense_init).
+// CTA pairs that can be co-resident (one per TPC); 0 = the device cannot host the pair kernel.  Queried once,
+// outside stream capture (tc_dense_init).
 int pair_capacity() {
   static int pairs = -1;
   if (pairs < 0) {
     pairs = 0;
-    const char *e = getenv("GCRL_TC_PAIR");
-    if (!(e && e[0] == '0')) {
-      GCRL_CUDA(cudaFuncSetAttribute(tc_dense_pair_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem2<5>::kBytes));
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(unsigned(sm_count() & ~1));
-      cfg.blockDim = dim3(kPairThreads);
-      cfg.dynamicSmemBytes = TcSmem2<5>::kBytes;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      cfg.attrs = at; cfg.numAttrs = 1;
-      int n = 0;
-      if (cudaOccupancyMaxActiveClusters(&n, tc_dense_pair_kernel<5>, &cfg) == cudaSuccess && n > 0)
-        pairs = std::min(n, sm_count() / 2);
-      else
-        cudaGetLastError();
-    }
+    GCRL_CUDA(cudaFuncSetAttribute(tc_dense_pair_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem2<5>::kBytes));
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(unsigned(sm_count() & ~1));
+    cfg.blockDim = dim3(kPairThreads);
+    cfg.dynamicSmemBytes = TcSmem2<5>::kBytes;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    int n = 0;
+    if (cudaOccupancyMaxActiveClusters(&n, tc_dense_pair_kernel<5>, &cfg) == cudaSuccess && n > 0)
+      pairs = std::min(n, sm_count() / 2);
+    else
+      cudaGetLastError();
   }
   return pairs;
 }
@@ -986,7 +906,6 @@ static int dense_column_tile(int M, int N, int members) {
   int BN = N <= 64 ? 64 : (N <= 128 ? 128 : 256);
   const int m_tiles_ = (M + BM - 1) / BM;
   while (BN > 64 && members * m_tiles_ * ((N + BN - 1) / BN) < (sm_count() * 3) / 4) BN >>= 1;
-  if (const char *e = getenv("GCRL_TC_BN")) BN = atoi(e);
   return BN;
 }
 
@@ -1003,10 +922,8 @@ void launch_tc_dense(const float *X, int ldx, const float *W, int ldw, const flo
   a.M = M; a.N = N; a.K = K; a.mode = mode;
   a.m_tiles = (M + BM - 1) / BM;
   a.n_tiles = (N + BN - 1) / BN;
-  if (const char *e = getenv("GCRL_TC_DBG")) a.dbg = atoi(e);
   // CTA pairs (256 x 256 tiles, each SM stages half of the weight tile) once they alone fill 3/4 of the TPCs
-  int pairs = (W_lo != nullptr && N % 256 == 0) ? pair_capacity() : 0;
-  if (const char *e = getenv("GCRL_TC_PAIR_RT")) if (e[0] == '0') pairs = 0;      // microbenchmarks: per-launch switch
+  const int pairs = (W_lo != nullptr && N % 256 == 0) ? pair_capacity() : 0;
   const int pair_tiles = ((M + 255) / 256) * (N / 256);
   // (M = 8192 as 64 half tiles on 64 pairs was tried: 20.5 us against 18.5 us for 128 single-CTA 128 x 128 tiles)
   if (pairs > 0 && 4 * pair_tiles >= 3 * pairs) {
@@ -1018,26 +935,9 @@ void launch_tc_dense(const float *X, int ldx, const float *W, int ldw, const flo
     const int used = std::min(pair_tiles, pairs);
     const int grid = 2 * used;
     const int rest = pair_tiles % used;                      // tiles of the last, partly filled round
-    a.full_items = (rest > 0 && 2 * rest <= used && !getenv("GCRL_TC_NO_HALVES")) ? pair_tiles - rest : pair_tiles;
-    if (getenv("GCRL_TC_VERBOSE")) fprintf(stderr, "[tc] pair kernel: %d pairs resident, %d tiles, grid %d\n", pairs, pair_tiles, grid);
-    const char *tr = getenv("GCRL_TC_TRACE");
-    constexpr size_t kTrace = 2 * 8 * 64;
-    if (tr != nullptr) {
-      GCRL_CUDA(cudaMalloc(&a.trace, kTrace * sizeof(long long)));
-      GCRL_CUDA(cudaMemsetAsync(a.trace, 0, kTrace * sizeof(long long), st));
-    }
+    a.full_items = (rest > 0 && 2 * rest <= used) ? pair_tiles - rest : pair_tiles;
     tc_dense_pair_kernel<5><<<grid, kPairThreads, TcSmem2<5>::kBytes, st>>>(tmA, tmBhi, tmBlo, a);
     GCRL_LAUNCHED();
-    if (tr != nullptr) {          // debug only: synchronous dump, [cta 0..1][role 0..7][stage use 0..63] nanoseconds
-      std::vector<long long> h(kTrace);
-      GCRL_CUDA(cudaStreamSynchronize(st));
-      GCRL_CUDA(cudaMemcpy(h.data(), a.trace, kTrace * sizeof(long long), cudaMemcpyDeviceToHost));
-      cudaFree(a.trace);
-      if (FILE *f = fopen(tr, "wb")) {
-        fwrite(h.data(), sizeof(long long), kTrace, f);
-        fclose(f);
-      }
-    }
     return;
   }
   const CUtensorMap tmA = make_map(X, M, K, ldx, BM);
@@ -1126,18 +1026,16 @@ int launch_tc_wgrad(const float *dZ, int lddz, const float *X, int ldx, float *p
   int rows = ((M + slabs - 1) / slabs + 15) & ~15;
   slabs = (M + rows - 1) / rows;
   a.rows_per_slab = rows; a.nslabs = slabs; a.split_stride = w_split_stride;
-  if (const char *e = getenv("GCRL_TC_DBG")) a.dbg = atoi(e);
-  // the bias-gradient partials ride on the splitter warps (unless a timing switch removes the split work)
-  const bool fused_colsum = pB != nullptr && !(a.dbg & 1) && !getenv("GCRL_TC_NO_FUSED_COLSUM");
-  if (fused_colsum) { a.colsum = pB; a.colsum_stride = b_split_stride; }
+  // the bias-gradient partials ride on the splitter warps
+  a.colsum = pB; a.colsum_stride = b_split_stride;
   const CUtensorMap tmA = make_map(dZ, M, N, lddz, 16, 32, true);
   const CUtensorMap tmB = make_map(X, M, K, ldx, 16, 32, true);
   // more tiles than SMs: a grid that is a multiple of the tiles per slab makes every CTA revisit the SAME (n, k) block
-  // in later slabs, and it accumulates them in place -- grid / per partial slabs for reduce_grads instead of `slabs`
-  // (74 instead of 128 at M = 65 536: 102 -> 59 MB per network).  Needs the bias sums in the same kernel.
+  // in later slabs, and it accumulates them in place (bias sums included) -- grid / per partial slabs for
+  // reduce_grads instead of `slabs` (74 instead of 128 at M = 65 536: 102 -> 59 MB per network)
   const int tiles = slabs * per;
   int grid = std::min(tiles, sm_count()), written = slabs;
-  if (tiles > grid && per <= sm_count() && (fused_colsum || pB == nullptr) && !getenv("GCRL_TC_NO_SLAB_ACC")) {
+  if (tiles > grid && per <= sm_count()) {
     grid = (sm_count() / per) * per;
     a.acc_slabs = 1;
     written = grid / per;
@@ -1145,10 +1043,6 @@ int launch_tc_wgrad(const float *dZ, int lddz, const float *X, int ldx, float *p
   if (BN == 64) launch_bn<64>(tmA, tmB, nullptr, a, st, grid);
   else if (BN == 128) launch_bn<128>(tmA, tmB, nullptr, a, st, grid);
   else launch_bn<256>(tmA, tmB, nullptr, a, st, grid);
-  if (pB != nullptr && !fused_colsum) {
-    colsum_partials_kernel<<<dim3(slabs, (N + 31) / 32), 256, 0, st>>>(dZ, lddz, M, N, rows, pB, b_split_stride);
-    GCRL_LAUNCHED();
-  }
   return written;
 }
 

@@ -43,9 +43,6 @@ def main():
             assert weights_close(w, ws, 1e-3, 4) and weights_close(b, bs, 1e-3, 4)
     tqc_section(rank, world, local)
     p2p_section(rank, world, local)
-    os.environ["GCRL_P2P_TILE_FUSED"] = "1"       # the one-kernel variant: every weight-gradient CTA averages its own tile
-    p2p_section(rank, world, local)
-    del os.environ["GCRL_P2P_TILE_FUSED"]
     normaliser_section(rank, world, local)
     if rank == 0:
         print("DP_OK", flush=True)

@@ -202,3 +202,49 @@ def test_tc_dense_presplit_weights_match_float64(M, N, K):
         assert torch.isfinite(y).all(), mode
         err = ((y.double() - want).abs().max() / want.abs().max()).item()
         assert err <= 1e-5, (mode, err)
+
+
+def test_tc_kernels_ignore_removed_timing_variables(monkeypatch):
+    """The tcgen05 dense and weight-gradient launches have no environment switches: variables that once forced kernel
+    variants or skipped work for timing experiments change no output bit.  A CTA-pair shape with a partly filled last
+    round (half tiles) and a weight gradient with bias sums and in-place slab accumulation (M = 65 536)."""
+    import ctypes as C
+    import torch
+    from gcrl_b200._lib import check, lib, vp
+    removed = {"GCRL_TC_DBG": "7", "GCRL_TC_BN": "64", "GCRL_TC_PAIR_RT": "0", "GCRL_TC_NO_HALVES": "1",
+               "GCRL_TC_NO_FUSED_COLSUM": "1", "GCRL_TC_NO_SLAB_ACC": "1"}
+    torch.manual_seed(11)
+    st = vp(torch.cuda.current_stream().cuda_stream)
+    M, N, K = 20000, 256, 256
+    x = torch.randn(M, K, device="cuda")
+    w = torch.randn(N, K, device="cuda") / K ** 0.5
+    b = torch.randn(N, device="cuda")
+    hi, lo = torch.empty_like(w), torch.empty_like(w)
+    check(lib.gcrl_split_tf32(0, vp(w.data_ptr()), vp(hi.data_ptr()), vp(lo.data_ptr()), w.numel(), st))
+    Mw = 65536
+    dz = torch.randn(Mw, N, device="cuda") / Mw ** 0.5
+    xw = torch.randn(Mw, K, device="cuda")
+    stride, max_splits = N * K + 8, 128
+
+    def run():
+        y = torch.full((M, N), float("nan"), device="cuda")           # fresh outputs: a skipped store stays NaN
+        check(lib.gcrl_dense_layer_presplit(0, 0, M, N, K, vp(x.data_ptr()), K, vp(hi.data_ptr()), vp(lo.data_ptr()), K,
+                                            vp(b.data_ptr()), None, 0, vp(y.data_ptr()), N, st))
+        pw = torch.full((max_splits, stride), float("nan"), device="cuda")
+        pb = torch.full((max_splits, N), float("nan"), device="cuda")
+        sp = C.c_int()
+        check(lib.gcrl_dense_wgrad(0, 1, Mw, N, K, vp(dz.data_ptr()), N, vp(xw.data_ptr()), K, vp(pw.data_ptr()), K,
+                                   stride, vp(pb.data_ptr()), N, max_splits, C.byref(sp), st))
+        torch.cuda.synchronize()
+        S = sp.value
+        return y, S, pw[:S, :N * K], pb[:S]
+
+    for name in removed:
+        monkeypatch.delenv(name, raising=False)
+    y0, s0, pw0, pb0 = run()
+    assert torch.isfinite(y0).all() and torch.isfinite(pw0).all() and torch.isfinite(pb0).all()
+    for name, value in removed.items():
+        monkeypatch.setenv(name, value)
+    y1, s1, pw1, pb1 = run()
+    assert torch.equal(y1, y0)
+    assert s1 == s0 and torch.equal(pw1, pw0) and torch.equal(pb1, pb0)
