@@ -14,6 +14,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <tuple>
 #include <vector>
@@ -27,6 +28,11 @@ void her_sample_into(gcrl_her *h, int64_t B, const int64_t *idx_host, float *s, 
 int her_state_dim(const gcrl_her *h);
 int her_act_dim(const gcrl_her *h);
 int her_device(const gcrl_her *h);
+SampleScalars her_next_scalars(gcrl_her *h, bool positions_given);
+int64_t her_len(const gcrl_her *h);
+void her_sample_graphed(gcrl_her *h, int64_t B, const SampleScalars *sc_dev, const int64_t *idx_dev, float *s,
+                        float *a, float *r, float *ns, float *d, cudaStream_t st);
+unsigned long long &her_draw_epoch(gcrl_her *h);
 }  // namespace gcrl
 
 using namespace gcrl;
@@ -40,6 +46,10 @@ constexpr int kEnsembleBatchMax = 4096;   // up to this batch the ensemble's bac
 constexpr float kBnEps = 1e-5f;        // nn.BatchNorm1d default
 constexpr float kBnMomentum = 0.1f;
 constexpr float kLogSqrt2Pi = 0.91893853320467274178f;
+constexpr int kMetricFloats = 36;         // the device metrics block [32], then the alpha state [4]
+// per-update scalars of an n-update call: critic / actor AdamW, alpha's AdamW, the sampler's totals and draw epoch
+constexpr size_t kManyScalBytes = 2 * sizeof(StepScalars) + sizeof(SampleScalars);
+constexpr size_t kManyGraphCache = 8;     // n-update graphs kept per agent (one flag pattern per run is typical)
 
 // ---- BatchNorm1d -----------------------------------------------------------------------------
 // One CTA per 32 feature columns, 32 x 32 threads: threadIdx.x = column (coalesced 128-byte row
@@ -725,11 +735,21 @@ struct gcrl_sac {
   CriticNet critic[kMaxCritics], target[kMaxCritics];
   int adam_t_c = 0, adam_t_a = 0, adam_t_alpha = 0;
   int dp_B = -1, dp_flags = -1;                  // the update the data-parallel phases belong to
+  bool dp_open = false;                          // a phase-wise data-parallel update: phase 0 issued, phase 3 not yet
   bool tc_update = false;                        // the update being recorded / issued runs on the tensor-core engine
   bool use_graphs = true;
   cudaStream_t cap_stream = nullptr;             // capture-only stream (the caller's may be the legacy one)
   struct GraphRec { cudaGraphExec_t exec; uint64_t kernels; };
   std::map<std::tuple<int, int, int>, GraphRec> graphs;   // (B, flags, phase mask)
+  // n consecutive updates in one graph (gcrl_sac_update_many): everything a captured update reads that changes from
+  // one update to the next has one slot per update, in one device allocation laid out for the call's (n, B):
+  // scalars [n] x kManyScalBytes | positions [n][B] int64 | eps_next [n][B][A] | eps_cur [n][B][A] | metrics [n][36]
+  struct Many {
+    char *d = nullptr;
+    size_t cap = 0;                              // bytes; growing it drops the cached graphs (their addresses move)
+    // (B, flags of every update, buffer, engine path)
+    std::map<std::tuple<int64_t, std::vector<int>, uintptr_t, int>, GraphRec> graphs;
+  } many;
   // sync-BN (gcrl_sac_set_sync_bn): the update is cut into graph segments, each ending in the collective the caller
   // runs before the next one (gcrl_sac_update_segment)
   int sync_world = 0, sync_rank = 0;
@@ -759,7 +779,7 @@ struct gcrl_sac {
   int64_t slab = 0;
   float *sumsq = nullptr;
   float *mdev = nullptr;                         // [32] device metrics block
-  float *alpha_state = nullptr;                  // [4] log_alpha, alpha, m, v
+  float *alpha_state = nullptr;                  // [4] log_alpha, alpha, m, v: mdev + 32 (one copy takes both)
   StepScalars *d_scalars = nullptr;
   PinnedRing scal_stage, io_stage;
   float *d_io = nullptr;
@@ -1263,6 +1283,41 @@ void run_body(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     actor_update(ag, B, flags, mask == PH_ALL ? PH_ALL : (mask & (PH_AGRAD | PH_ASTEP)), st);
 }
 
+// Record `body` on the capture stream into an instantiated graph; the kernels it records are not counted as
+// launches until the graph is replayed.
+gcrl_sac::GraphRec capture_graph(gcrl_sac *ag, const std::function<void(cudaStream_t)> &body) {
+  cudaGraph_t graph = nullptr;
+  const uint64_t before = launch_counter();
+  GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
+  try {
+    body(ag->cap_stream);
+  } catch (...) {
+    cudaStreamEndCapture(ag->cap_stream, &graph);
+    if (graph) cudaGraphDestroy(graph);
+    throw;
+  }
+  GCRL_CUDA(cudaStreamEndCapture(ag->cap_stream, &graph));
+  const uint64_t kernels = launch_counter() - before;   // recorded, not executed, by the capture
+  count_launch(uint64_t(0) - kernels);
+  cudaGraphExec_t exec = nullptr;
+  const cudaError_t e = cudaGraphInstantiate(&exec, graph, 0);
+  cudaGraphDestroy(graph);
+  GCRL_CUDA(e);
+  return gcrl_sac::GraphRec{exec, kernels};
+}
+
+void launch_graph(const gcrl_sac::GraphRec &g, cudaStream_t st) {
+  GCRL_CUDA(cudaGraphLaunch(g.exec, st));
+  count_launch(g.kernels);
+}
+
+// the engine an update at this batch runs on; the tensor-core one needs the split weight copies current
+void select_engine(gcrl_sac *ag, int B, cudaStream_t st) {
+  ag->tc_update = engine_tc(ag, B);
+  if (ag->tc_update) ensure_split(ag, st);          // (the update itself re-splits what it steps)
+  else mark_split_stale(ag);                        // weights move without their split copies following
+}
+
 // Replay (or capture on first use) the CUDA graph of (B, flags, phase mask): ~170 launches per TQC update
 // become one graph launch; everything that varies per step travels through device scalars.
 void run_phases(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
@@ -1275,27 +1330,80 @@ void run_phases(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   }
   const auto key = std::make_tuple(B, flags, mask);
   auto it = ag->graphs.find(key);
-  if (it == ag->graphs.end()) {
-    cudaGraph_t graph = nullptr;
-    const uint64_t before = launch_counter();
-    GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
-    try {
-      run_body(ag, B, flags, mask, ag->cap_stream);
-    } catch (...) {
-      cudaStreamEndCapture(ag->cap_stream, &graph);
-      if (graph) cudaGraphDestroy(graph);
-      throw;
-    }
-    GCRL_CUDA(cudaStreamEndCapture(ag->cap_stream, &graph));
-    const uint64_t kernels = launch_counter() - before;   // recorded, not executed, by the capture
-    count_launch(uint64_t(0) - kernels);
-    cudaGraphExec_t exec = nullptr;
-    GCRL_CUDA(cudaGraphInstantiate(&exec, graph, 0));
-    GCRL_CUDA(cudaGraphDestroy(graph));
-    it = ag->graphs.emplace(key, gcrl_sac::GraphRec{exec, kernels}).first;
+  if (it == ag->graphs.end())
+    it = ag->graphs.emplace(key, capture_graph(ag, [&](cudaStream_t cs) { run_body(ag, B, flags, mask, cs); })).first;
+  launch_graph(it->second, st);
+}
+
+// ---- n updates in one graph (gcrl_sac_update_many) -------------------------------------------------------------
+size_t many_bytes(const gcrl_sac *ag, int n, int64_t B) {
+  return size_t(n) * (kManyScalBytes + size_t(B) * (sizeof(int64_t) + 2 * ag->A * sizeof(float)) +
+                      kMetricFloats * sizeof(float));
+}
+char *many_scalars(const gcrl_sac *ag, int i) { return ag->many.d + size_t(i) * kManyScalBytes; }
+int64_t *many_positions(const gcrl_sac *ag, int n, int64_t B, int i) {
+  return reinterpret_cast<int64_t *>(ag->many.d + size_t(n) * kManyScalBytes) + size_t(i) * B;
+}
+float *many_eps(const gcrl_sac *ag, int n, int64_t B, int which /*0 next, 1 cur*/) {
+  return reinterpret_cast<float *>(many_positions(ag, n, B, n)) + size_t(which) * n * B * ag->A;
+}
+float *many_metrics(const gcrl_sac *ag, int n, int64_t B, int i) {
+  return many_eps(ag, n, B, 2) + size_t(i) * kMetricFloats;
+}
+
+// While update i of an n-update call is recorded (or issued eagerly), the agent's per-update inputs -- AdamW and
+// alpha scalars, rsample noise -- point at slot i, so every argument builder of critic_update / actor_update picks
+// the slot up; the sampler reads the slot's totals and positions.
+struct ManySlot {
+  gcrl_sac *ag;
+  StepScalars *sc; float *en, *ec;
+  const SampleScalars *ssc; const int64_t *idx; float *metrics;
+  ManySlot(gcrl_sac *a, int i, int n, int B)
+      : ag(a), sc(a->d_scalars), en(a->eps_next), ec(a->eps_cur),
+        ssc(reinterpret_cast<const SampleScalars *>(many_scalars(a, i) + 2 * sizeof(StepScalars))),
+        idx(many_positions(a, n, B, i)), metrics(many_metrics(a, n, B, i)) {
+    a->d_scalars = reinterpret_cast<StepScalars *>(many_scalars(a, i));
+    a->eps_next = many_eps(a, n, B, 0) + size_t(i) * B * a->A;
+    a->eps_cur = many_eps(a, n, B, 1) + size_t(i) * B * a->A;
   }
-  GCRL_CUDA(cudaGraphLaunch(it->second.exec, st));
-  count_launch(it->second.kernels);
+  ~ManySlot() { ag->d_scalars = sc; ag->eps_next = en; ag->eps_cur = ec; }
+  ManySlot(const ManySlot &) = delete;
+  ManySlot &operator=(const ManySlot &) = delete;
+};
+
+// n updates from `buf` back to back: sampler, operand rows, the update, then its metrics and alpha state into the
+// slot's row (a copy node, not a launch)
+void run_many_body(gcrl_sac *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+  for (int i = 0; i < n; ++i) {
+    ManySlot slot(ag, i, n, B);
+    her_sample_graphed(buf, B, slot.ssc, slot.idx, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, st);
+    launch_ingest_batch(ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->D, ag->A, B, ag->sa, ag->nsa, ag->spi, ag->ldc,
+                        ag->br, ag->bd, st);
+    run_body(ag, B, flags[i], PH_ALL, st);
+    GCRL_CUDA(cudaMemcpyAsync(slot.metrics, ag->mdev, kMetricFloats * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  }
+}
+
+void run_many(gcrl_sac *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+  select_engine(ag, B, st);
+  ag->per_on = false;
+  if (!ag->use_graphs) {
+    run_many_body(ag, buf, B, n, flags, st);
+    return;
+  }
+  auto key = std::make_tuple(int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf),
+                             ag->tc_update ? 1 : 0);
+  auto &cache = ag->many.graphs;
+  auto it = cache.find(key);
+  if (it == cache.end()) {
+    const gcrl_sac::GraphRec g = capture_graph(ag, [&](cudaStream_t cs) { run_many_body(ag, buf, B, n, flags, cs); });
+    if (cache.size() >= kManyGraphCache) {     // a replay still in flight is released when it completes
+      for (auto &kv : cache) cudaGraphExecDestroy(kv.second.exec);
+      cache.clear();
+    }
+    it = cache.emplace(std::move(key), g).first;
+  }
+  launch_graph(it->second, st);
 }
 
 // Segmented update (sync-BN): the body is captured ONCE per (B, flags) as a chain of graphs, cut wherever a
@@ -1341,6 +1449,46 @@ int run_segment(gcrl_sac *ag, int B, int flags, int seg, cudaStream_t st) {
   return r.collective;
 }
 
+// The next update's AdamW step counters -> sc[0] (critic / actor scalars) and the first 4 floats of sc[1] (alpha's)
+void fill_scalars(gcrl_sac *ag, double lr_c, double lr_a, int flags, StepScalars *sc) {
+  auto fill = [&](int t, double lr, float *out) {
+    out[0] = float(lr / (1.0 - std::pow(0.9, double(t))));
+    out[1] = float(std::sqrt(1.0 - std::pow(0.999, double(t))));
+    out[2] = float(1.0 - lr * double(ag->cfg.weight_decay));
+    out[3] = 0.f;
+  };
+  ag->adam_t_c += 1;
+  fill(ag->adam_t_c, lr_c, &sc->step_size_c);
+  if (flags & 1) ag->adam_t_a += 1;
+  fill(std::max(1, ag->adam_t_a), lr_a, &sc->step_size_a);
+  float *al = reinterpret_cast<float *>(sc + 1);
+  al[0] = 0.f; al[1] = 1.f; al[2] = 1.f; al[3] = 0.f;
+  if ((flags & 1) && (flags & 4)) {
+    ag->adam_t_alpha += 1;
+    fill(ag->adam_t_alpha, double(ag->cfg.alpha_lr), al);
+  }
+}
+
+// The step counters advance in fill_scalars, before the update is enqueued; unless commit() is reached they are
+// put back (and, after keep_draws, the device index-stream epoch of the sampled buffer with them).
+struct StepCounterGuard {
+  gcrl_sac *ag;
+  int t_c, t_a, t_al;
+  gcrl_her *buf = nullptr;
+  unsigned long long draw_epoch = 0;
+  bool done = false;
+  explicit StepCounterGuard(gcrl_sac *a) : ag(a), t_c(a->adam_t_c), t_a(a->adam_t_a), t_al(a->adam_t_alpha) {}
+  void keep_draws(gcrl_her *b) { buf = b; draw_epoch = her_draw_epoch(b); }
+  void commit() { done = true; }
+  ~StepCounterGuard() {
+    if (done) return;
+    ag->adam_t_c = t_c; ag->adam_t_a = t_a; ag->adam_t_alpha = t_al;
+    if (buf != nullptr) her_draw_epoch(buf) = draw_epoch;
+  }
+  StepCounterGuard(const StepCounterGuard &) = delete;
+  StepCounterGuard &operator=(const StepCounterGuard &) = delete;
+};
+
 // phase < 0: the whole update.  phase 0..3: the data-parallel cut (critic grads | critic steps | actor grads |
 // actor step), the caller averaging critic_grads / the actor gradient across ranks in between.
 void sac_update(gcrl_sac *ag, int phase, gcrl_her *buf, int64_t B64, const int64_t *idx_host, const float *s,
@@ -1350,9 +1498,7 @@ void sac_update(gcrl_sac *ag, int phase, gcrl_her *buf, int64_t B64, const int64
   GCRL_REQUIRE(ag != nullptr, "agent handle is NULL");
   GCRL_REQUIRE(B64 >= 2 && B64 <= ag->maxB, "batch size outside [2, max_batch] (BatchNorm needs > 1 row)");
   const int B = int(B64);
-  ag->tc_update = engine_tc(ag, B);
-  if (ag->tc_update) ensure_split(ag, st);          // (the update itself re-splits what it steps)
-  else mark_split_stale(ag);                        // weights move without their split copies following
+  select_engine(ag, B, st);
   if (seg > 0) {
     GCRL_REQUIRE(ag->dp_B == B && ag->dp_flags == flags, "segment > 0 must follow segment 0 of the same update");
     *collective = run_segment(ag, B, flags, seg, st);
@@ -1361,6 +1507,7 @@ void sac_update(gcrl_sac *ag, int phase, gcrl_her *buf, int64_t B64, const int64
   if (phase > 0) {
     GCRL_REQUIRE(ag->dp_B == B && ag->dp_flags == flags, "phase 1..3 must follow phase 0 of the same update");
     run_phases(ag, B, flags, phase == 1 ? PH_CSTEP : (phase == 2 ? PH_AGRAD : PH_ASTEP), st);
+    if (phase == 3) ag->dp_open = false;
     return;
   }
   GCRL_REQUIRE(eps_next != nullptr && (eps_cur != nullptr || !(flags & 1)), "NULL rsample noise tensor");
@@ -1376,47 +1523,52 @@ void sac_update(gcrl_sac *ag, int phase, gcrl_her *buf, int64_t B64, const int64
   GCRL_CUDA(cudaMemcpyAsync(ag->eps_next, eps_next, size_t(B) * ag->A * 4, cudaMemcpyDeviceToDevice, st));
   if (flags & 1)
     GCRL_CUDA(cudaMemcpyAsync(ag->eps_cur, eps_cur, size_t(B) * ag->A * 4, cudaMemcpyDeviceToDevice, st));
-  // per-step optimiser scalars
-  auto fill = [&](int t, double lr, float *out) {
-    out[0] = float(lr / (1.0 - std::pow(0.9, double(t))));
-    out[1] = float(std::sqrt(1.0 - std::pow(0.999, double(t))));
-    out[2] = float(1.0 - lr * double(ag->cfg.weight_decay));
-    out[3] = 0.f;
-  };
   // the step counters move only if the update is issued: a throw below (capture, CUDA error, a misuse check)
   // must not leave the bias corrections one step ahead of the Python schedulers
-  const int t_c0 = ag->adam_t_c, t_a0 = ag->adam_t_a, t_al0 = ag->adam_t_alpha;
-  try {
-  int slot;   // d_scalars[0] = critic / actor AdamW scalars, d_scalars[1] (first 3 floats) = alpha's
+  StepCounterGuard guard(ag);
+  int slot;
   auto *sc = reinterpret_cast<StepScalars *>(ag->scal_stage.acquire(2 * sizeof(StepScalars), &slot));
-  ag->adam_t_c += 1;
-  fill(ag->adam_t_c, lr_c, &sc->step_size_c);
-  if (flags & 1) ag->adam_t_a += 1;
-  fill(std::max(1, ag->adam_t_a), lr_a, &sc->step_size_a);
-  float *al = reinterpret_cast<float *>(sc + 1);
-  al[0] = 0.f; al[1] = 1.f; al[2] = 1.f; al[3] = 0.f;
-  if ((flags & 1) && (flags & 4)) {
-    ag->adam_t_alpha += 1;
-    fill(ag->adam_t_alpha, double(ag->cfg.alpha_lr), al);
-  }
+  fill_scalars(ag, lr_c, lr_a, flags, sc);
   GCRL_CUDA(cudaMemcpyAsync(ag->d_scalars, sc, sizeof(StepScalars) + 16, cudaMemcpyHostToDevice, st));
   ag->scal_stage.release(slot, st);
   if (seg == 0) {
     ag->dp_B = B; ag->dp_flags = flags;
     *collective = run_segment(ag, B, flags, 0, st);
+    guard.commit();
     return;
   }
   if (phase == 0) {
     ag->dp_B = B; ag->dp_flags = flags;
     run_phases(ag, B, flags, PH_CGRAD, st);
+    ag->dp_open = true;
+    guard.commit();
     return;
   }
   run_phases(ag, B, flags, PH_ALL, st);
   read_metrics(ag, flags, metrics_host, st);
-  } catch (...) {
-    ag->adam_t_c = t_c0; ag->adam_t_a = t_a0; ag->adam_t_alpha = t_al0;
-    throw;
+  guard.commit();
+}
+
+// the 12 floats an update returns (include/gcrl_b200.h), from its device metrics block hm[32] and alpha state hs[4]
+void metrics_tuple(const gcrl_sac *ag, int flags, const float *hm, const float *hs, float *metrics_host) {
+  const int n = ag->n;
+  if (ag->cfg.algo == GCRL_ALGO_SAC) {
+    metrics_host[0] = hm[M_CLOSS]; metrics_host[1] = hm[M_CLOSS + 1];
+    metrics_host[5] = hm[M_CGN]; metrics_host[6] = hm[M_CGN + 1];
+  } else {                                   // np.mean over the per-critic Python floats (:1013-1014)
+    double sl = 0.0, sg = 0.0;
+    for (int i = 0; i < n; ++i) { sl += double(hm[M_CLOSS + i]); sg += double(hm[M_CGN + i]); }
+    metrics_host[0] = metrics_host[1] = float(sl / n);
+    metrics_host[5] = metrics_host[6] = float(sg / n);
   }
+  metrics_host[2] = (flags & 1) ? hm[M_ALOSS] : 0.f;
+  metrics_host[3] = hm[M_TD];
+  metrics_host[4] = hm[M_Q];
+  metrics_host[7] = (flags & 1) ? hm[M_AGN] : 0.f;
+  metrics_host[8] = (flags & 1) ? hm[M_ALPHA_LOSS] : 0.f;
+  metrics_host[9] = hs[1];
+  metrics_host[10] = hs[0];
+  metrics_host[11] = 0.f;
 }
 
 void read_metrics(gcrl_sac *ag, int flags, float *metrics_host, cudaStream_t st) {
@@ -1425,24 +1577,7 @@ void read_metrics(gcrl_sac *ag, int flags, float *metrics_host, cudaStream_t st)
     GCRL_CUDA(cudaMemcpyAsync(hm, ag->mdev, sizeof(hm), cudaMemcpyDeviceToHost, st));
     GCRL_CUDA(cudaMemcpyAsync(hs, ag->alpha_state, sizeof(hs), cudaMemcpyDeviceToHost, st));
     GCRL_CUDA(cudaStreamSynchronize(st));
-    const int n = ag->n;
-    if (ag->cfg.algo == GCRL_ALGO_SAC) {
-      metrics_host[0] = hm[M_CLOSS]; metrics_host[1] = hm[M_CLOSS + 1];
-      metrics_host[5] = hm[M_CGN]; metrics_host[6] = hm[M_CGN + 1];
-    } else {                                   // np.mean over the per-critic Python floats (:1013-1014)
-      double sl = 0.0, sg = 0.0;
-      for (int i = 0; i < n; ++i) { sl += double(hm[M_CLOSS + i]); sg += double(hm[M_CGN + i]); }
-      metrics_host[0] = metrics_host[1] = float(sl / n);
-      metrics_host[5] = metrics_host[6] = float(sg / n);
-    }
-    metrics_host[2] = (flags & 1) ? hm[M_ALOSS] : 0.f;
-    metrics_host[3] = hm[M_TD];
-    metrics_host[4] = hm[M_Q];
-    metrics_host[7] = (flags & 1) ? hm[M_AGN] : 0.f;
-    metrics_host[8] = (flags & 1) ? hm[M_ALPHA_LOSS] : 0.f;
-    metrics_host[9] = hs[1];
-    metrics_host[10] = hs[0];
-    metrics_host[11] = 0.f;
+    metrics_tuple(ag, flags, hm, hs, metrics_host);
   }
 }
 
@@ -1530,9 +1665,9 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
     ag->pset = int64_t(kSplits) * ag->slab + int64_t(kSplits) * 4;
     ag->partials = dev_alloc<float>(size_t(ag->pset) * n);
     ag->sumsq = dev_alloc<float>(size_t(reduce_grid(int(ag->slab))) + 8);
-    ag->mdev = dev_alloc<float>(32);
-    GCRL_CUDA(cudaMemset(ag->mdev, 0, 32 * 4));
-    ag->alpha_state = dev_alloc<float>(4);
+    ag->mdev = dev_alloc<float>(kMetricFloats);
+    GCRL_CUDA(cudaMemset(ag->mdev, 0, kMetricFloats * 4));
+    ag->alpha_state = ag->mdev + 32;
     const float init_alpha[4] = {0.f, 1.f, 0.f, 0.f};       // log_alpha = 0 (:424)
     GCRL_CUDA(cudaMemcpy(ag->alpha_state, init_alpha, sizeof(init_alpha), cudaMemcpyHostToDevice));
     ag->d_scalars = dev_alloc<StepScalars>(2);
@@ -1569,10 +1704,12 @@ int gcrl_sac_destroy(gcrl_sac *ag) {
   for (float *p : ag->dzc) cudaFree(p);
   for (float *p : {ag->invstd, ag->dz[0], ag->dz[1], ag->sa, ag->nsa, ag->spi, ag->br, ag->bd, ag->bs, ag->ba, ag->bns,
                    ag->br0, ag->bd0, ag->q, ag->qt, ag->y, ag->dq, ag->logp, ag->act4, ag->std4, ag->gate4, ag->dact,
-                   ag->dzh, ag->eps_next, ag->eps_cur, ag->partials, ag->sumsq, ag->mdev, ag->alpha_state, ag->d_io,
+                   ag->dzh, ag->eps_next, ag->eps_cur, ag->partials, ag->sumsq, ag->mdev, ag->d_io,
                    ag->critic_grads, ag->per_w, ag->per_td})
     if (p) cudaFree(p);
   for (auto &kv : ag->graphs) cudaGraphExecDestroy(kv.second.exec);
+  for (auto &kv : ag->many.graphs) cudaGraphExecDestroy(kv.second.exec);
+  if (ag->many.d) cudaFree(ag->many.d);
   for (auto &kv : ag->seg_graphs) for (auto &r : kv.second) cudaGraphExecDestroy(r.exec);
   if (ag->bn_gather) cudaFree(ag->bn_gather);
   if (ag->cap_stream) cudaStreamDestroy(ag->cap_stream);
@@ -1721,6 +1858,78 @@ int gcrl_sac_update_from_buffer(gcrl_sac *ag, gcrl_her *buf, int64_t B, const in
   GCRL_CUDA(cudaSetDevice(ag->device));
   sac_update(ag, -1, buf, B, idx_host, nullptr, nullptr, nullptr, nullptr, nullptr, eps_next, eps_cur, lr_c, lr_a,
              flags, metrics_host, as_stream(stream));
+  GCRL_API_END
+}
+
+int gcrl_sac_update_many(gcrl_sac *ag, gcrl_her *buf, int64_t B, int n, const int *flags, const int64_t *idx_host,
+                         const float *eps_next_dev, const float *eps_cur_dev, const double *lr_critic,
+                         const double *lr_actor, float *metrics_host, void *stream) {
+  GCRL_API_BEGIN
+  GCRL_NVTX("gcrl_sac_update_many");
+  require_handle(ag);
+  GCRL_REQUIRE(buf != nullptr, "buffer handle is NULL");
+  GCRL_REQUIRE(B >= 2 && B <= ag->maxB, "batch size outside [2, max_batch] (BatchNorm needs > 1 row)");
+  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
+  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
+  bool any_actor = false;
+  for (int i = 0; i < n; ++i) {
+    GCRL_REQUIRE((flags[i] & ~7) == 0, "flags of an n-update call may hold bits 0-2 only");
+    any_actor = any_actor || (flags[i] & 1) != 0;
+  }
+  GCRL_REQUIRE(eps_next_dev != nullptr && (eps_cur_dev != nullptr || !any_actor), "NULL rsample noise tensor");
+  GCRL_REQUIRE(ag->sync_world == 0, "a sync-BN agent trains through gcrl_sac_update_segment only");
+  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
+  GCRL_REQUIRE(her_state_dim(buf) == ag->D && her_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
+  GCRL_REQUIRE(her_device(buf) == ag->device, "buffer and agent live on different devices");
+  const int64_t len = her_len(buf);
+  if (len < B) throw Error(GCRL_ERR_UNDERFILLED, "[ERROR] Not enough in buffer to sample");
+  if (idx_host != nullptr)
+    for (int64_t i = 0; i < int64_t(n) * B; ++i)
+      if (idx_host[i] < 0 || idx_host[i] >= len) throw Error(GCRL_ERR_INVALID, "sample index out of range [0, len)");
+  GCRL_CUDA(cudaSetDevice(ag->device));
+  cudaStream_t st = as_stream(stream);
+  auto &mn = ag->many;
+  const size_t need = many_bytes(ag, n, B);
+  if (need > mn.cap) {                       // cudaFree waits for replays still reading the old slots
+    for (auto &kv : mn.graphs) cudaGraphExecDestroy(kv.second.exec);
+    mn.graphs.clear();
+    if (mn.d) GCRL_CUDA(cudaFree(mn.d));
+    mn.d = nullptr;
+    mn.cap = 0;
+    mn.d = dev_alloc<char>(need);
+    mn.cap = need;
+  }
+  StepCounterGuard guard(ag);
+  guard.keep_draws(buf);
+  // every update's scalars (the device stream's draw epochs in order), then every update's positions: ONE copy
+  const size_t scal = size_t(n) * kManyScalBytes, pos = idx_host != nullptr ? size_t(n) * B * sizeof(int64_t) : 0;
+  int slot;
+  char *p = ag->io_stage.acquire(scal + pos, &slot);
+  for (int i = 0; i < n; ++i) {
+    char *s = p + size_t(i) * kManyScalBytes;
+    fill_scalars(ag, lr_critic[i], lr_actor[i], flags[i], reinterpret_cast<StepScalars *>(s));
+    const SampleScalars ss = her_next_scalars(buf, idx_host != nullptr);
+    std::memcpy(s + 2 * sizeof(StepScalars), &ss, sizeof(SampleScalars));
+  }
+  if (pos) std::memcpy(p + scal, idx_host, pos);
+  GCRL_CUDA(cudaMemcpyAsync(mn.d, p, scal + pos, cudaMemcpyHostToDevice, st));
+  ag->io_stage.release(slot, st);
+  // stable addresses for the captured graph
+  const size_t noise = size_t(n) * B * ag->A * sizeof(float);
+  GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 0), eps_next_dev, noise, cudaMemcpyDeviceToDevice, st));
+  if (any_actor) GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 1), eps_cur_dev, noise, cudaMemcpyDeviceToDevice, st));
+  run_many(ag, buf, int(B), n, flags, st);
+  guard.commit();
+  if (metrics_host != nullptr) {
+    // ONE read-back per call; to pageable memory the copy returns once it (and the updates before it) completed
+    std::vector<float> rows(size_t(n) * kMetricFloats);
+    GCRL_CUDA(cudaMemcpyAsync(rows.data(), many_metrics(ag, n, B, 0), rows.size() * sizeof(float),
+                              cudaMemcpyDeviceToHost, st));
+    for (int i = 0; i < n; ++i) {
+      const float *r = rows.data() + size_t(i) * kMetricFloats;
+      metrics_tuple(ag, flags[i], r, r + 32, metrics_host + size_t(i) * 12);
+    }
+  }
   GCRL_API_END
 }
 

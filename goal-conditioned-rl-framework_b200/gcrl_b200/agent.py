@@ -541,16 +541,16 @@ class _AgentBase:
         return [float(x) for x in self._metrics]
 
     # -- a training cycle's gradient steps in one call ---------------------------------------------------
-    _MANY_IN_ONE_GRAPH = False      # DDPG / TD3: n updates from a HER buffer replay as one CUDA graph
+    _MANY_IN_ONE_GRAPH = False      # n updates from a HER buffer replay as one CUDA graph (every agent sets it)
 
     def update_many(self, steps):
         """``[self.update(s) for s in steps]``: the same tuples, and afterwards the same state of every network,
         optimiser, schedule, index stream and random generator.  ``steps`` need not be consecutive.
 
-        DDPG and TD3 sampling from a HER buffer on one GPU issue every 64 steps as ONE CUDA graph launch: the
-        positions (host index stream), learning rates and TD3 noise of all of them are drawn up front and
-        travel in one copy, so no interpreter, launch or metric read-back sits between the updates.  Every
-        other agent, buffer type and data-parallel mode runs the loop."""
+        DDPG, TD3, SAC and TQC sampling from a HER buffer on one GPU issue every 64 steps as ONE CUDA graph
+        launch: the positions (host index stream), learning rates and noise (TD3 smoothing, SAC / TQC rsample)
+        of all of them are drawn up front and travel in one copy each, so no interpreter, launch or metric
+        read-back sits between the updates.  Every other buffer type and data-parallel mode runs the loop."""
         steps = [int(s) for s in steps]
         if not (self._MANY_IN_ONE_GRAPH and isinstance(self.buffer, HERBuffer) and self._dp is None
                 and getattr(self, "_peer_dp", None) is None):

@@ -324,6 +324,21 @@ class _SacBase(_AgentBase):
     def metrics_tensor(self):
         return self.grad_tensor(3)
 
+    def _flags(self, step):
+        """bit0 actor step, bit1 Polyak step, bit2 alpha step (an actor step past alpha_min_steps)."""
+        actor_step = step % self.ac_update_freq == 0
+        return (1 if actor_step else 0) | (2 if self._polyak_now(step) else 0) \
+            | (4 if (actor_step and step > self.alpha_min_steps) else 0)
+
+    def _result(self, step, m):
+        """The tuple update(step) returns, from the 12 metric floats of its update."""
+        flags = self._flags(step)
+        q1l, q2l, acl, td, qv, c1g, c2g, acg, all_ = m[:9]
+        td = np.float32(td) if self._last_td is None else self._last_td
+        if flags & 1:
+            return q1l, q2l, acl, td, qv, c1g, c2g, acg, (all_ if flags & 4 else 0.0)
+        return q1l, q2l, td, qv, c1g, c2g
+
     def update(self, step: int, batch=None, indices=None, eps_next=None, eps_cur=None):
         import torch
         B = self.batch_size if batch is None else batch[0].shape[0]
@@ -332,8 +347,7 @@ class _SacBase(_AgentBase):
             eps_next = torch.randn((B, self.ac_dim), dtype=torch.float32, device=self.device)
         if eps_cur is None and actor_step:
             eps_cur = torch.randn((B, self.ac_dim), dtype=torch.float32, device=self.device)
-        flags = (1 if actor_step else 0) | (2 if self._polyak_now(step) else 0) \
-            | (4 if (actor_step and step > self.alpha_min_steps) else 0)
+        flags = self._flags(step)
         lr_c, lr_a = self.critic_scheduler.lr, self.actor_scheduler.lr
         mptr = C.cast(self._metrics, vp)
         en = vp(eps_next.data_ptr())
@@ -392,12 +406,60 @@ class _SacBase(_AgentBase):
             self.actor_scheduler.step()
             self._bn_batches += 1
         self.beta_scheduler(step)
-        m = [float(x) for x in self._metrics]
-        q1l, q2l, acl, td, qv, c1g, c2g, acg, all_ = m[:9]
-        td = np.float32(td) if self._last_td is None else self._last_td
-        if actor_step:
-            return q1l, q2l, acl, td, qv, c1g, c2g, acg, (all_ if flags & 4 else 0.0)
-        return q1l, q2l, td, qv, c1g, c2g
+        return self._result(step, [float(x) for x in self._metrics])
+
+    # -- a training cycle's gradient steps in one call (_AgentBase.update_many) ------------------------------
+    _MANY_IN_ONE_GRAPH = True       # from a HER buffer on one GPU; REPLAY, PER and both data-parallel modes loop
+
+    def _update_chunk(self, steps):
+        """Up to MAX_MANY_STEPS updates through gcrl_sac_update_many: the noise, positions, flags and learning
+        rates of all of them are drawn up front, in the order the loop draws them."""
+        import torch
+        B, n = self.batch_size, len(steps)
+        assert len(self.buffer) >= B, "[ERROR] Not enough in buffer to sample"       # before any state moves
+        if not 2 <= B <= self._max_batch:
+            raise ValueError(f"batch size {B} outside [2, max_batch = {self._max_batch}]")
+        flags = [self._flags(s) for s in steps]
+        shape = (B, self.ac_dim)
+        eps_next, eps_cur = [], []
+        for f in flags:                             # update()'s torch.randn calls, in step order
+            eps_next.append(torch.randn(shape, dtype=torch.float32, device=self.device))
+            eps_cur.append(torch.randn(shape, dtype=torch.float32, device=self.device) if f & 1 else None)
+        any_actor = any(f & 1 for f in flags)
+        eps_next = torch.stack(eps_next)
+        if any_actor:                               # rows of critic-only steps are never read
+            unused = torch.zeros(shape, dtype=torch.float32, device=self.device)
+            eps_cur = torch.stack([unused if e is None else e for e in eps_cur])
+        iptr = None
+        if self.index_source == "host":             # n draws of random.sample(range(len), B), in step order
+            nlen = len(self.buffer)
+            idx = np.stack([_lib.py_sample_range(nlen, B) for _ in steps])
+            iptr = np_ptr(idx)
+        cflags = (C.c_int * n)(*flags)
+        lr_c, lr_a = (C.c_double * n)(), (C.c_double * n)()
+        schedules = (self.critic_scheduler, self.actor_scheduler)
+        saved = [(sch.last_epoch, sch.lr) for sch in schedules]
+        for i in range(n):                          # the schedules step as update() steps them
+            lr_c[i], lr_a[i] = self.critic_scheduler.lr, self.actor_scheduler.lr
+            self.critic_scheduler.step()
+            if flags[i] & 1:
+                self.actor_scheduler.step()
+        metrics = np.empty((n, 12), np.float32)
+        try:
+            check(lib.gcrl_sac_update_many(self._h, self.buffer.handle, B, n, cflags, iptr, vp(eps_next.data_ptr()),
+                                           vp(eps_cur.data_ptr()) if any_actor else None, lr_c, lr_a,
+                                           np_ptr(metrics), self._stream()))
+        except BaseException:
+            for sch, (epoch, lr) in zip(schedules, saved):
+                sch.last_epoch, sch.lr = epoch, lr
+            raise
+        self._last_td = None
+        out = []
+        for step, f, m in zip(steps, flags, metrics.tolist()):
+            self._bn_batches += 2 if f & 1 else 1
+            self.beta_scheduler(step)
+            out.append(self._result(step, m))
+        return out
 
     def _save_log_alpha(self, path):
         import torch

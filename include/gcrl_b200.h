@@ -366,6 +366,19 @@ int gcrl_sac_update_batch(gcrl_sac *h, int64_t B, const float *s_dev, const floa
 int gcrl_sac_update_from_buffer(gcrl_sac *h, gcrl_her *buf, int64_t B, const int64_t *idx_host,
                                 const float *eps_next_dev, const float *eps_cur_dev, double lr_critic,
                                 double lr_actor, int flags, float *metrics_host, void *stream);
+/* n consecutive SAC / TQC updates from `buf` as ONE graph launch.  Bit for bit equal to n calls of
+ * gcrl_sac_update_from_buffer with flags[i], lr_critic[i], lr_actor[i], the positions idx_host + i*B (or the device
+ * index stream's next n draws when idx_host is NULL), eps_next_dev + i*B*A and eps_cur_dev + i*B*A (row i of
+ * eps_cur read only when flags[i] bit0 is set; eps_cur_dev may be NULL when no flags[i] has it).
+ * flags[i]: bits 0-2 only (a HER buffer has no priorities).
+ * metrics_host: float[n][12], row i = what update i returns, read back once per call; NULL leaves the call async,
+ * and gcrl_sac_read_metrics then returns the last update's tuple.  1 <= n <= GCRL_MAX_MANY_STEPS.
+ * Refused (GCRL_ERR_INVALID) on a sync-BN agent (gcrl_sac_set_sync_bn world != 0) and while a phase-wise
+ * data-parallel update is open.  On any error, no AdamW step counter (critics, actor, alpha) and no device
+ * index-stream epoch has moved. */
+int gcrl_sac_update_many(gcrl_sac *h, gcrl_her *buf, int64_t B, int n, const int *flags, const int64_t *idx_host,
+                         const float *eps_next_dev, const float *eps_cur_dev, const double *lr_critic,
+                         const double *lr_actor, float *metrics_host, void *stream);
 /* Data-parallel hooks (one process per GPU, episode-sharded buffer, replicated weights): the update cut
  * at the points where gradients are averaged across ranks --
  *   phase 0: ingest the local batch, policy sample, targets, all critic forwards / backwards
