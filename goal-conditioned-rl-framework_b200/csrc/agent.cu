@@ -18,6 +18,7 @@
 #include <functional>
 #include <initializer_list>
 #include <map>
+#include <set>
 #include <tuple>
 #include <vector>
 
@@ -36,6 +37,17 @@ int her_device(const gcrl_her *h);
 void her_sample_graphed(gcrl_her *h, int64_t B, const SampleScalars *sc_dev, const int64_t *idx_dev, float *s,
                         float *a, float *r, float *ns, float *d, cudaStream_t st);
 unsigned long long &her_draw_epoch(gcrl_her *h);
+bool replay_prioritized(const gcrl_replay *h);
+int replay_state_dim(const gcrl_replay *h);
+int replay_act_dim(const gcrl_replay *h);
+int replay_device(const gcrl_replay *h);
+uint64_t replay_epoch(const gcrl_replay *h);
+int64_t replay_many_n(const gcrl_replay *h);
+void replay_many_stage(gcrl_replay *h, int64_t B, int n, const int64_t *pos_host, const double *u_host,
+                       const double *beta, cudaStream_t st);
+void replay_many_sample(gcrl_replay *h, int64_t B, int n, int i, float *s, float *a, float *r, float *ns, float *d,
+                        float *weights_dev, cudaStream_t st);
+void replay_many_write_back(gcrl_replay *h, int64_t B, const float *td_dev, cudaStream_t st);
 }  // namespace gcrl
 
 using namespace gcrl;
@@ -206,8 +218,12 @@ struct gcrl_agent {
     char *d = nullptr;                     // [GCRL_MAX_MANY_STEPS] x kScalBytes scalars, then positions [n][B] int64
     float *noise = nullptr;                // TD3 smoothing noise [n][B][A]
     float *h_pub = nullptr, *d_pub = nullptr;   // mapped publish blocks [GCRL_MAX_MANY_STEPS][16] of updates 0 .. n-2
-    // (B, flags of every update, buffer, engine path)
-    std::map<std::tuple<int64_t, std::vector<int>, uintptr_t, int>, GraphRec> graphs;
+    float *td = nullptr;                   // prioritised replay: every update's per-sample TD errors [n][B]
+    // (B, flags of every update, buffer, engine path, buffer epoch, length drawn from): a uniform or HER buffer has
+    // 0 for the last one, a graph serves any length; a HER buffer also has 0 for the epoch
+    using Key = std::tuple<int64_t, std::vector<int>, uintptr_t, int, uint64_t, int64_t>;
+    std::map<Key, GraphRec> graphs;
+    std::set<Key> seen;                    // keys issued eagerly once (prioritised: captured when one repeats)
   } many;
 };
 
@@ -826,18 +842,25 @@ void run_many_body(gcrl_agent *ag, gcrl_her *buf, int B, int n, const int *flags
   }
 }
 
-void run_many(gcrl_agent *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
-  select_engine(ag, B, st);
+// Replay the n-update graph of `key`, capturing it first when it is new -- or, with capture_new false, only when
+// the key was issued before (a key seen for the first time is issued eagerly: a prioritised buffer that is still
+// filling draws from a new length every call, and its graphs would never be replayed).
+void launch_many(gcrl_agent *ag, gcrl_agent::Many::Key key, bool capture_new,
+                 const std::function<void(cudaStream_t)> &body, cudaStream_t st) {
   if (!ag->use_graphs) {
-    run_many_body(ag, buf, B, n, flags, st);
+    body(st);
     return;
   }
-  const int path = (ag->sample_buf != nullptr ? 1 : 0) | (fused_ok(ag, B) ? 2 : 0) | (ag->tc_update ? 4 : 0);
-  auto key = std::make_tuple(int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), path);
   auto &cache = ag->many.graphs;
   auto it = cache.find(key);
+  if (it == cache.end() && !capture_new && ag->many.seen.count(key) == 0) {
+    if (ag->many.seen.size() >= 2 * kManyGraphCache) ag->many.seen.clear();
+    ag->many.seen.insert(std::move(key));
+    body(st);
+    return;
+  }
   if (it == cache.end()) {
-    const gcrl_agent::GraphRec g = capture_graph(ag, [&](cudaStream_t cs) { run_many_body(ag, buf, B, n, flags, cs); });
+    const gcrl_agent::GraphRec g = capture_graph(ag, body);
     if (cache.size() >= kManyGraphCache) {     // a replay still in flight is released when it completes
       for (auto &kv : cache) cudaGraphExecDestroy(kv.second.exec);
       cache.clear();
@@ -845,6 +868,40 @@ void run_many(gcrl_agent *ag, gcrl_her *buf, int B, int n, const int *flags, cud
     it = cache.emplace(std::move(key), g).first;
   }
   launch_graph(it->second, st);
+}
+
+int many_path(const gcrl_agent *ag, int B) {
+  return (ag->sample_buf != nullptr ? 1 : 0) | (fused_ok(ag, B) ? 2 : 0) | (ag->tc_update ? 4 : 0);
+}
+
+void run_many(gcrl_agent *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+  select_engine(ag, B, st);
+  launch_many(ag, {int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), many_path(ag, B), 0, 0},
+              true, [&](cudaStream_t cs) { run_many_body(ag, buf, B, n, flags, cs); }, st);
+}
+
+// n updates from a uniform / prioritised buffer: the slot's draw, the operand rows, the update and, prioritised, the
+// priority write-back and a copy of the TD errors into the update's row
+void run_many_replay_body(gcrl_agent *ag, gcrl_replay *buf, int B, int n, const int *flags, cudaStream_t st) {
+  for (int i = 0; i < n; ++i) {
+    ManySlot slot(ag, i, n, B);
+    replay_many_sample(buf, B, n, i, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->per_w, st);
+    if (!fused_ok(ag, B))
+      launch_ingest_batch(ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->D, ag->A, B, ag->sa, ag->nsa, ag->spi, ag->ldc,
+                          ag->br, ag->bd, st);
+    run_update_body(ag, B, ag->td3 ? ag->noise : nullptr, flags[i], PH_ALL, st);
+    if (ag->per_on) {
+      replay_many_write_back(buf, B, ag->per_td, st);
+      GCRL_CUDA(cudaMemcpyAsync(ag->many.td + size_t(i) * B, ag->per_td, size_t(B) * 4, cudaMemcpyDeviceToDevice, st));
+    }
+  }
+}
+
+void run_many_replay(gcrl_agent *ag, gcrl_replay *buf, int B, int n, const int *flags, cudaStream_t st) {
+  select_engine(ag, B, st);
+  launch_many(ag, {int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), many_path(ag, B),
+                   replay_epoch(buf), ag->per_on ? replay_many_n(buf) : 0},
+              !ag->per_on, [&](cudaStream_t cs) { run_many_replay_body(ag, buf, B, n, flags, cs); }, st);
 }
 
 // The row-slab critic kernel draws the batch itself from `buf` (else the sampler is a launch of its own)
@@ -902,6 +959,17 @@ void ingest(gcrl_agent *ag, gcrl_her *buf, int64_t B, const int64_t *idx_host, c
     GCRL_CUDA(cudaMemcpyAsync(ag->noise, noise_dev, size_t(B) * ag->A * 4, cudaMemcpyDeviceToDevice, st));
     *noise_out = ag->noise;
   }
+}
+
+// the per-update slots of n-update calls, on first use
+void ensure_many(gcrl_agent *ag) {
+  auto &mn = ag->many;
+  if (mn.d != nullptr) return;
+  mn.d = dev_alloc<char>(GCRL_MAX_MANY_STEPS * (kScalBytes + size_t(ag->maxB) * sizeof(int64_t)));
+  if (ag->td3) mn.noise = dev_alloc<float>(size_t(GCRL_MAX_MANY_STEPS) * ag->maxB * ag->A);
+  GCRL_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&mn.h_pub), GCRL_MAX_MANY_STEPS * 64, cudaHostAllocMapped));
+  std::memset(mn.h_pub, 0, GCRL_MAX_MANY_STEPS * 64);
+  GCRL_CUDA(cudaHostGetDevicePointer(reinterpret_cast<void **>(&mn.d_pub), mn.h_pub, 0));
 }
 
 void check_batch(const gcrl_agent *ag, int64_t B) {
@@ -970,6 +1038,15 @@ void finish_metrics(gcrl_agent *ag, float *metrics_host, cudaStream_t st) {
     GCRL_CUDA(cudaMemcpy(&err, ag->p2p.err, sizeof(int), cudaMemcpyDeviceToHost));
     if (err) throw dp_error(err);
   }
+}
+
+// metrics_host[n][8] of an n-update call: the last update publishes as a single one does; stream order then has the
+// earlier blocks complete
+void read_many_metrics(gcrl_agent *ag, int n, float *metrics_host, cudaStream_t st) {
+  if (metrics_host == nullptr) return;
+  finish_metrics(ag, metrics_host + size_t(n - 1) * 8, st);
+  for (int i = 0; i < n - 1; ++i)
+    read_published(ag->many.h_pub + size_t(i) * 16, ag->pub_seq - unsigned(n - 1 - i), metrics_host + size_t(i) * 8, st);
 }
 
 }  // namespace
@@ -1079,6 +1156,7 @@ int gcrl_agent_destroy(gcrl_agent *ag) {
   if (ag->many.d) cudaFree(ag->many.d);
   if (ag->many.noise) cudaFree(ag->many.noise);
   if (ag->many.h_pub) cudaFreeHost(ag->many.h_pub);
+  if (ag->many.td) cudaFree(ag->many.td);
   for (void *p : ag->p2p.opened) cudaIpcCloseMemHandle(p);
   for (void *p : {(void *)ag->p2p.flags, (void *)ag->p2p.epoch, (void *)ag->p2p.ticket, (void *)ag->p2p.wticket, (void *)ag->p2p.go,
                   (void *)ag->p2p.err, (void *)ag->p2p.outbox,
@@ -1337,13 +1415,7 @@ int gcrl_agent_update_many(gcrl_agent *ag, gcrl_her *buf, int64_t B, int n, cons
   GCRL_CUDA(cudaSetDevice(ag->device));
   cudaStream_t st = as_stream(stream);
   auto &mn = ag->many;
-  if (mn.d == nullptr) {
-    mn.d = dev_alloc<char>(GCRL_MAX_MANY_STEPS * (kScalBytes + size_t(ag->maxB) * sizeof(int64_t)));
-    if (ag->td3) mn.noise = dev_alloc<float>(size_t(GCRL_MAX_MANY_STEPS) * ag->maxB * ag->A);
-    GCRL_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&mn.h_pub), GCRL_MAX_MANY_STEPS * 64, cudaHostAllocMapped));
-    std::memset(mn.h_pub, 0, GCRL_MAX_MANY_STEPS * 64);
-    GCRL_CUDA(cudaHostGetDevicePointer(reinterpret_cast<void **>(&mn.d_pub), mn.h_pub, 0));
-  }
+  ensure_many(ag);
   AdamStepGuard guard(ag);
   guard.keep_draws(buf);
   ag->per_on = false;
@@ -1364,11 +1436,57 @@ int gcrl_agent_update_many(gcrl_agent *ag, gcrl_her *buf, int64_t B, int n, cons
   run_many(ag, buf, int(B), n, flags, st);
   ag->pub_valid = true;
   guard.commit();
-  if (metrics_host != nullptr) {
-    // the last update publishes as a single one does; stream order then has the earlier blocks complete
-    finish_metrics(ag, metrics_host + size_t(n - 1) * 8, st);
-    for (int i = 0; i < n - 1; ++i)
-      read_published(mn.h_pub + size_t(i) * 16, ag->pub_seq - unsigned(n - 1 - i), metrics_host + size_t(i) * 8, st);
+  read_many_metrics(ag, n, metrics_host, st);
+  GCRL_API_END
+}
+
+int gcrl_agent_update_many_replay(gcrl_agent *ag, gcrl_replay *buf, int64_t B, int n, const int *flags,
+                                  const int64_t *pos_host, const double *u_host, const double *beta,
+                                  const float *noise_dev, const double *lr_critic, const double *lr_actor,
+                                  float *metrics_host, float *td_host, void *stream) {
+  GCRL_API_BEGIN
+  GCRL_NVTX("gcrl_agent_update_many_replay");
+  require_handle(ag);
+  check_batch(ag, B);
+  GCRL_REQUIRE(buf != nullptr, "buffer handle is NULL");
+  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
+  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
+  const bool per = replay_prioritized(buf);
+  for (int i = 0; i < n; ++i) {
+    GCRL_REQUIRE((flags[i] & ~11) == 0, "flags of an n-update call from a replay buffer may hold bits 0, 1 and 3 only");
+    GCRL_REQUIRE(((flags[i] & 8) != 0) == per, "flags bit3 must be set exactly when the buffer is prioritised");
+  }
+  GCRL_REQUIRE(!ag->p2p.on, "n-update calls are not available under peer-memory data parallelism");
+  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
+  GCRL_REQUIRE(replay_state_dim(buf) == ag->D && replay_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
+  GCRL_REQUIRE(replay_device(buf) == ag->device, "buffer and agent live on different devices");
+  GCRL_REQUIRE(!ag->td3 || noise_dev != nullptr, "TD3 update needs the [n, B, A] standard-normal noise tensor");
+  GCRL_CUDA(cudaSetDevice(ag->device));
+  cudaStream_t st = as_stream(stream);
+  replay_many_stage(buf, B, n, pos_host, u_host, beta, st);      // the buffer's own checks come first
+  auto &mn = ag->many;
+  ensure_many(ag);
+  if (per && mn.td == nullptr) mn.td = dev_alloc<float>(size_t(GCRL_MAX_MANY_STEPS) * ag->maxB);
+  AdamStepGuard guard(ag);
+  ag->per_on = per;
+  int slot;
+  char *p = ag->io_stage.acquire(size_t(n) * kScalBytes, &slot);
+  for (int i = 0; i < n; ++i)
+    fill_scalars(ag, lr_critic[i], lr_actor[i], (flags[i] & 1) != 0, SampleScalars{}, p + size_t(i) * kScalBytes);
+  GCRL_CUDA(cudaMemcpyAsync(mn.d, p, size_t(n) * kScalBytes, cudaMemcpyHostToDevice, st));
+  ag->io_stage.release(slot, st);
+  if (ag->td3)   // stable addresses for the captured graph
+    GCRL_CUDA(cudaMemcpyAsync(mn.noise, noise_dev, size_t(n) * B * ag->A * 4, cudaMemcpyDeviceToDevice, st));
+  ag->sample_buf = nullptr;
+  run_many_replay(ag, buf, int(B), n, flags, st);
+  ag->pub_valid = true;
+  guard.commit();
+  read_many_metrics(ag, n, metrics_host, st);
+  if (per && td_host != nullptr) {
+    // ONE read-back per call; to pageable memory the copy returns once it (and the updates before it) completed
+    std::vector<float> rows(size_t(n) * B);
+    GCRL_CUDA(cudaMemcpyAsync(rows.data(), mn.td, rows.size() * sizeof(float), cudaMemcpyDeviceToHost, st));
+    std::memcpy(td_host, rows.data(), rows.size() * sizeof(float));
   }
   GCRL_API_END
 }

@@ -29,6 +29,7 @@
 // float32 power (importance weights, new priorities) is computed as float(pow(double)) -- within an ulp of
 // any libm / SIMD powf the reference may run on (DESIGN.md, prioritised replay).
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 #include <cstring>
 #include <functional>
@@ -556,13 +557,15 @@ __global__ void __launch_bounds__(1024) weight_norm_kernel(const float *__restri
   for (int i = threadIdx.x; i < B; i += 1024) w[i] = __fdiv_rn(w_raw[i], m);
 }
 
+// call != nullptr: the ring start is read from device memory (a replayed n-update graph follows the pushes made
+// between two calls); else `start` by value (gcrl_replay_sample)
 __global__ void __launch_bounds__(256)
-uniform_gather_kernel(ReplayGeom g, int64_t start, const int64_t *__restrict__ pos, int B, float *s, float *a, float *r,
-                      float *ns, float *d) {
+uniform_gather_kernel(ReplayGeom g, int64_t start, const PerCall *__restrict__ call, const int64_t *__restrict__ pos,
+                      int B, float *s, float *a, float *r, float *ns, float *d) {
   const int lane = threadIdx.x & 31;
   const int64_t b = (blockIdx.x * int64_t(blockDim.x) + threadIdx.x) >> 5;
   if (b >= B) return;
-  scatter_row(g, slot_of(start, pos[b], g.cap), b, lane, s, a, r, ns, d);
+  scatter_row(g, slot_of(call != nullptr ? call->start : start, pos[b], g.cap), b, lane, s, a, r, ns, d);
 }
 
 // ---- update_priorities (src/buffer.py:86-89): in draw order, so the LAST duplicate of a position wins ----
@@ -630,15 +633,26 @@ struct gcrl_replay {
   float *d_wraw = nullptr;
   int64_t *d_pos = nullptr, *d_slot = nullptr;
   PinnedRing stage;
+  // n-update calls (gcrl_agent_update_many_replay, gcrl_sac_update_many_replay): PerCall[n], then the uniforms
+  // (prioritised) or the positions (uniform) [n][B], 8 bytes each; many_n = the length the call draws from
+  char *d_many = nullptr;
+  size_t many_cap = 0;
+  int64_t many_n = 0;
+  // changes whenever a device array a captured n-update graph reads is reallocated (and differs between handles)
+  uint64_t epoch = 0;
   int64_t start() const { return (total - len) % g.cap; }
 };
 
 namespace {
 
+std::atomic<uint64_t> g_epoch{0};
+void new_epoch(gcrl_replay *h) { h->epoch = ++g_epoch; }
+
 void ensure_batch(gcrl_replay *h, int64_t B, cudaStream_t st) {
   if (B <= h->batch_cap) return;
   GCRL_CUDA(cudaStreamSynchronize(st));
   if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
+  new_epoch(h);
   for (void *p : {(void *)h->d_u, (void *)h->d_wraw, (void *)h->d_pos, (void *)h->d_slot})
     if (p) GCRL_CUDA(cudaFree(p));
   h->batch_cap = std::max<int64_t>(B, 1024);
@@ -685,6 +699,7 @@ void build_tree(gcrl_replay *h, int64_t n, cudaStream_t st) {
   if (need > h->tree_cap) {
     GCRL_CUDA(cudaStreamSynchronize(st));
     if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }   // it holds the old tables
+    new_epoch(h);
     for (void *p : {(void *)h->d_leaf_off, (void *)h->d_node_l, (void *)h->d_node_r, (void *)h->d_vals})
       if (p) GCRL_CUDA(cudaFree(p));
     h->tree_cap = need * 2;
@@ -706,13 +721,152 @@ void build_tree(gcrl_replay *h, int64_t n, cudaStream_t st) {
   h->n_leaves = L;
   h->n_groups = max_h;
   h->tree_n = n;
+  if (!h->fold_smem_set) {      // outside any capture: the fold's shared-memory form may need up to 200 KB
+    GCRL_CUDA(cudaFuncSetAttribute(tree_fold_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    h->fold_smem_set = true;
+  }
+}
+
+// The 11 launches of one prioritised draw from the first n entries: per-call scalars and uniforms from `call` / `u`
+void issue_draw(gcrl_replay *h, int64_t n, int64_t B, const PerCall *call, const double *u, float *s, float *a, float *r,
+                float *ns, float *d, float *weights_dev, cudaStream_t st) {
+  const int64_t cap = h->g.cap;
+  leaf_sum_kernel<<<blocks_for(int64_t(h->n_leaves) * 8, 256), 256, 0, st>>>(h->g.prio, call, cap, h->d_leaf_off,
+                                                                           h->n_leaves, h->d_vals, h->d_flags);
+  GCRL_LAUNCHED();
+  {
+    const size_t fold_smem = size_t(2 * h->n_leaves) * sizeof(float);
+    if (fold_smem <= size_t(200) * 1024) {
+      tree_fold_kernel<true><<<1, 1024, fold_smem, st>>>(h->d_vals, h->d_node_l, h->d_node_r, h->d_group_off,
+                                                         h->n_groups, h->n_leaves, h->d_psum);
+    } else {
+      tree_fold_kernel<false><<<1, 1024, 0, st>>>(h->d_vals, h->d_node_l, h->d_node_r, h->d_group_off, h->n_groups,
+                                                  h->n_leaves, h->d_psum);
+    }
+    GCRL_LAUNCHED();
+  }
+  const int tiles = blocks_for(n, kScanTile);
+  normalise_scan_kernel<<<tiles, kScanThreads, 0, st>>>(h->g.prio, call, cap, n, h->d_psum, h->pnorm, h->fixed,
+                                                        h->tile_sum, h->d_flags);
+  GCRL_LAUNCHED();
+  tile_scan_kernel<<<1, 1024, 0, st>>>(h->tile_sum, tiles, h->d_total, h->d_flags);
+  GCRL_LAUNCHED();
+  cdf_from_fixed_kernel<<<tiles, kScanThreads, 0, st>>>(h->fixed, h->tile_sum, h->d_total, n, h->d_flags);
+  GCRL_LAUNCHED();
+  double *cdf = reinterpret_cast<double *>(h->fixed);
+  {   // inexact additions: summarise the chunks, walk them in order, expand (all three return at once otherwise)
+    const int n_chunks = blocks_for(n, kChunk);
+    ChunkSum *sums = static_cast<ChunkSum *>(h->d_chunk_sums);
+    chunk_summary_kernel<<<blocks_for(int64_t(n_chunks) * 32, 256), 256, 0, st>>>(h->pnorm, h->fixed, h->tile_sum, n, n_chunks,
+                                                                               sums, h->d_flags);
+    GCRL_LAUNCHED();
+    chunk_walk_kernel<<<1, 32, 0, st>>>(h->pnorm, cdf, n, n_chunks, sums, h->d_chunk_in, h->d_chunk_expand, h->d_last,
+                                        h->d_flags);
+    GCRL_LAUNCHED();
+    chunk_expand_kernel<<<blocks_for(int64_t(n_chunks) * 32, 256), 256, 0, st>>>(h->pnorm, cdf, n, n_chunks, sums,
+                                                                              h->d_chunk_in, h->d_chunk_expand, h->d_flags);
+    GCRL_LAUNCHED();
+  }
+  cdf_divide_kernel<<<std::min(tiles, sm_count() * 8), 256, 0, st>>>(cdf, n, h->d_last, h->d_flags);
+  GCRL_LAUNCHED();
+  per_draw_kernel<<<blocks_for(B * 32, 256), 256, 0, st>>>(h->g, call, n, cdf, h->pnorm, u, int(B), s, a, r, ns, d,
+                                                          h->d_wraw, h->d_pos, h->d_slot);
+  GCRL_LAUNCHED();
+  weight_norm_kernel<<<1, 1024, 0, st>>>(h->d_wraw, weights_dev, int(B));
+  GCRL_LAUNCHED();
+}
+
+// update_priorities of the positions the preceding draw left in d_slot (winner is back to -1 after each write)
+void issue_write_back(gcrl_replay *h, int64_t B, const float *td_dev, cudaStream_t st) {
+  prio_winner_kernel<<<blocks_for(B, 256), 256, 0, st>>>(h->d_slot, int(B), h->winner);
+  GCRL_LAUNCHED();
+  prio_write_kernel<<<blocks_for(B, 256), 256, 0, st>>>(h->d_slot, td_dev, int(B), float(h->alpha), 1e-6f, h->g.prio,
+                                                       h->winner);
+  GCRL_LAUNCHED();
 }
 
 void require_outputs(const float *s, const float *a, const float *r, const float *ns, const float *d) {
   GCRL_REQUIRE(s && a && r && ns && d, "NULL batch pointer");
 }
 
+const PerCall *many_call(const gcrl_replay *h, int i) { return reinterpret_cast<const PerCall *>(h->d_many) + i; }
+const void *many_payload(const gcrl_replay *h, int n, int64_t B, int i) {
+  return h->d_many + size_t(n) * sizeof(PerCall) + size_t(i) * size_t(B) * 8;
+}
+
 }  // namespace
+
+// ---- graph-safe pieces of n-update calls (agent.cu, sac.cu) ------------------------------------------------------
+// The agent stages the call once (host), then records or issues, per update i, sample(i) -> its update ->
+// write_back(td) (prioritised).  Every launch reads what changes between calls -- ring start, beta, uniforms or
+// positions -- from the staged slots, and the priorities carry over from one update to the next in stream order.
+namespace gcrl {
+
+bool replay_prioritized(const gcrl_replay *h) { return h->prioritized; }
+int replay_state_dim(const gcrl_replay *h) { return h->g.D; }
+int replay_act_dim(const gcrl_replay *h) { return h->g.A; }
+int replay_device(const gcrl_replay *h) { return h->device; }
+uint64_t replay_epoch(const gcrl_replay *h) { return h->epoch; }
+int64_t replay_many_n(const gcrl_replay *h) { return h->many_n; }
+
+// Checks the call (moving nothing when it is refused), then moves every update's PerCall {ring start, -beta[i]} and
+// its uniforms u_host[i] (prioritised) or positions pos_host[i] (uniform) to the device in ONE pinned copy.  The
+// summation tree for the current length is built here, outside any capture.
+void replay_many_stage(gcrl_replay *h, int64_t B, int n, const int64_t *pos_host, const double *u_host,
+                       const double *beta, cudaStream_t st) {
+  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
+  if (h->prioritized) GCRL_REQUIRE(u_host != nullptr && beta != nullptr, "a prioritised buffer needs the uniforms and beta");
+  else GCRL_REQUIRE(pos_host != nullptr, "a uniform buffer needs the positions");
+  if (h->len < B) throw Error(GCRL_ERR_UNDERFILLED, "[ERROR] Not enough in buffer to sample");
+  if (!h->prioritized)
+    for (int64_t i = 0; i < int64_t(n) * B; ++i)
+      if (pos_host[i] < 0 || pos_host[i] >= h->len) throw Error(GCRL_ERR_INVALID, "sample index out of range [0, len)");
+  const size_t calls = size_t(n) * sizeof(PerCall), payload = size_t(n) * size_t(B) * 8;
+  if (calls + payload > h->many_cap) {
+    GCRL_CUDA(cudaStreamSynchronize(st));
+    if (h->d_many) GCRL_CUDA(cudaFree(h->d_many));
+    h->d_many = nullptr;
+    h->many_cap = 0;
+    new_epoch(h);
+    h->d_many = dev_alloc<char>((calls + payload) * 2);
+    h->many_cap = (calls + payload) * 2;
+  }
+  if (h->prioritized) {
+    ensure_batch(h, B, st);
+    build_tree(h, h->len, st);
+  }
+  int sl;
+  char *p = h->stage.acquire(calls + payload, &sl);
+  for (int i = 0; i < n; ++i) {
+    const PerCall c{h->start(), h->prioritized ? float(-beta[i]) : 0.f, 0};
+    std::memcpy(p + size_t(i) * sizeof(PerCall), &c, sizeof(PerCall));
+  }
+  std::memcpy(p + calls, h->prioritized ? static_cast<const void *>(u_host) : static_cast<const void *>(pos_host), payload);
+  GCRL_CUDA(cudaMemcpyAsync(h->d_many, p, calls + payload, cudaMemcpyHostToDevice, st));
+  h->stage.release(sl, st);
+  h->many_n = h->len;
+  if (h->prioritized) h->last_B = B;          // last_positions / update_priorities_last refer to this batch afterwards
+}
+
+// The batch of update i of the staged call into s .. d; the importance weights into weights_dev (prioritised)
+void replay_many_sample(gcrl_replay *h, int64_t B, int n, int i, float *s, float *a, float *r, float *ns, float *d,
+                        float *weights_dev, cudaStream_t st) {
+  if (h->prioritized) {
+    issue_draw(h, h->many_n, B, many_call(h, i), static_cast<const double *>(many_payload(h, n, B, i)), s, a, r, ns, d,
+               weights_dev, st);
+  } else {
+    uniform_gather_kernel<<<blocks_for(B * 32, 256), 256, 0, st>>>(
+        h->g, 0, many_call(h, i), static_cast<const int64_t *>(many_payload(h, n, B, i)), int(B), s, a, r, ns, d);
+    GCRL_LAUNCHED();
+  }
+}
+
+// update_priorities of update i's positions with its per-sample TD errors (prioritised)
+void replay_many_write_back(gcrl_replay *h, int64_t B, const float *td_dev, cudaStream_t st) {
+  issue_write_back(h, B, td_dev, st);
+}
+
+}  // namespace gcrl
 
 extern "C" {
 
@@ -762,6 +916,7 @@ int gcrl_replay_create(gcrl_replay **out, int device, int64_t capacity, int stat
       GCRL_CUDA(cudaDeviceSynchronize());
     }
     h->stage.init(size_t(1) << 16);
+    new_epoch(h);
   } catch (...) {
     delete h;
     throw;
@@ -783,6 +938,7 @@ int gcrl_replay_destroy(gcrl_replay *h) {
   if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
   if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
   if (h->d_call) cudaFree(h->d_call);
+  if (h->d_many) cudaFree(h->d_many);
   h->stage.destroy();
   delete h;
   GCRL_API_END
@@ -836,7 +992,8 @@ int gcrl_replay_sample(gcrl_replay *h, int64_t B, const int64_t *idx_host, float
   std::memcpy(p, idx_host, size_t(B) * 8);
   GCRL_CUDA(cudaMemcpyAsync(h->d_pos, p, size_t(B) * 8, cudaMemcpyHostToDevice, st));
   h->stage.release(sl, st);
-  uniform_gather_kernel<<<blocks_for(B * 32, 256), 256, 0, st>>>(h->g, h->start(), h->d_pos, int(B), s, a, r, ns, d);
+  uniform_gather_kernel<<<blocks_for(B * 32, 256), 256, 0, st>>>(h->g, h->start(), nullptr, h->d_pos, int(B), s, a, r,
+                                                                 ns, d);
   GCRL_LAUNCHED();
   GCRL_API_END
 }
@@ -852,7 +1009,7 @@ int gcrl_replay_sample_prioritized(gcrl_replay *h, int64_t B, const double *u_ho
   GCRL_CUDA(cudaSetDevice(h->device));
   cudaStream_t st = as_stream(stream);
   ensure_batch(h, B, st);
-  const int64_t n = h->len, start = h->start(), cap = h->g.cap;
+  const int64_t n = h->len, start = h->start();
   build_tree(h, n, st);
   {   // per-call scalars + the B uniforms: one pinned slot, two small copies
     int sl;
@@ -865,53 +1022,7 @@ int gcrl_replay_sample_prioritized(gcrl_replay *h, int64_t B, const double *u_ho
     h->stage.release(sl, st);
   }
   auto launch_all = [&](cudaStream_t st) {
-  leaf_sum_kernel<<<blocks_for(int64_t(h->n_leaves) * 8, 256), 256, 0, st>>>(h->g.prio, h->d_call, cap, h->d_leaf_off,
-                                                                           h->n_leaves, h->d_vals, h->d_flags);
-  GCRL_LAUNCHED();
-  {
-    const size_t fold_smem = size_t(2 * h->n_leaves) * sizeof(float);
-    if (fold_smem <= size_t(200) * 1024) {
-      if (!h->fold_smem_set) {
-        GCRL_CUDA(cudaFuncSetAttribute(tree_fold_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        h->fold_smem_set = true;
-      }
-      tree_fold_kernel<true><<<1, 1024, fold_smem, st>>>(h->d_vals, h->d_node_l, h->d_node_r, h->d_group_off,
-                                                         h->n_groups, h->n_leaves, h->d_psum);
-    } else {
-      tree_fold_kernel<false><<<1, 1024, 0, st>>>(h->d_vals, h->d_node_l, h->d_node_r, h->d_group_off, h->n_groups,
-                                                  h->n_leaves, h->d_psum);
-    }
-    GCRL_LAUNCHED();
-  }
-  const int tiles = blocks_for(n, kScanTile);
-  normalise_scan_kernel<<<tiles, kScanThreads, 0, st>>>(h->g.prio, h->d_call, cap, n, h->d_psum, h->pnorm, h->fixed,
-                                                        h->tile_sum, h->d_flags);
-  GCRL_LAUNCHED();
-  tile_scan_kernel<<<1, 1024, 0, st>>>(h->tile_sum, tiles, h->d_total, h->d_flags);
-  GCRL_LAUNCHED();
-  cdf_from_fixed_kernel<<<tiles, kScanThreads, 0, st>>>(h->fixed, h->tile_sum, h->d_total, n, h->d_flags);
-  GCRL_LAUNCHED();
-  double *cdf = reinterpret_cast<double *>(h->fixed);
-  {   // inexact additions: summarise the chunks, walk them in order, expand (all three return at once otherwise)
-    const int n_chunks = blocks_for(n, kChunk);
-    ChunkSum *sums = static_cast<ChunkSum *>(h->d_chunk_sums);
-    chunk_summary_kernel<<<blocks_for(int64_t(n_chunks) * 32, 256), 256, 0, st>>>(h->pnorm, h->fixed, h->tile_sum, n, n_chunks,
-                                                                               sums, h->d_flags);
-    GCRL_LAUNCHED();
-    chunk_walk_kernel<<<1, 32, 0, st>>>(h->pnorm, cdf, n, n_chunks, sums, h->d_chunk_in, h->d_chunk_expand, h->d_last,
-                                        h->d_flags);
-    GCRL_LAUNCHED();
-    chunk_expand_kernel<<<blocks_for(int64_t(n_chunks) * 32, 256), 256, 0, st>>>(h->pnorm, cdf, n, n_chunks, sums,
-                                                                              h->d_chunk_in, h->d_chunk_expand, h->d_flags);
-    GCRL_LAUNCHED();
-  }
-  cdf_divide_kernel<<<std::min(tiles, sm_count() * 8), 256, 0, st>>>(cdf, n, h->d_last, h->d_flags);
-  GCRL_LAUNCHED();
-  per_draw_kernel<<<blocks_for(B * 32, 256), 256, 0, st>>>(h->g, h->d_call, n, cdf, h->pnorm, h->d_u, int(B), s, a, r, ns, d,
-                                                          h->d_wraw, h->d_pos, h->d_slot);
-  GCRL_LAUNCHED();
-  weight_norm_kernel<<<1, 1024, 0, st>>>(h->d_wraw, weights_dev, int(B));
-  GCRL_LAUNCHED();
+    issue_draw(h, n, B, h->d_call, h->d_u, s, a, r, ns, d, weights_dev, st);
   };
   // The draw is 11 small launches: replayed as one graph once the same (length, batch, outputs) repeats -- i.e.
   // as soon as the ring is full; while it is still filling every call has a new length and launches directly.
@@ -974,11 +1085,7 @@ int gcrl_replay_update_priorities(gcrl_replay *h, int64_t B, const int64_t *idx_
   } else {
     GCRL_REQUIRE(B == h->last_B, "update_priorities without positions must follow the sample() of the same batch");
   }
-  prio_winner_kernel<<<blocks_for(B, 256), 256, 0, st>>>(h->d_slot, int(B), h->winner);
-  GCRL_LAUNCHED();
-  prio_write_kernel<<<blocks_for(B, 256), 256, 0, st>>>(h->d_slot, td_dev, int(B), float(h->alpha), 1e-6f, h->g.prio,
-                                                       h->winner);
-  GCRL_LAUNCHED();
+  issue_write_back(h, B, td_dev, st);
   h->last_B = idx_host != nullptr ? 0 : h->last_B;
   GCRL_API_END
 }

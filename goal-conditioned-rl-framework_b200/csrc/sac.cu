@@ -16,6 +16,7 @@
 #include <cstring>
 #include <functional>
 #include <map>
+#include <set>
 #include <tuple>
 #include <vector>
 
@@ -33,6 +34,17 @@ int64_t her_len(const gcrl_her *h);
 void her_sample_graphed(gcrl_her *h, int64_t B, const SampleScalars *sc_dev, const int64_t *idx_dev, float *s,
                         float *a, float *r, float *ns, float *d, cudaStream_t st);
 unsigned long long &her_draw_epoch(gcrl_her *h);
+bool replay_prioritized(const gcrl_replay *h);
+int replay_state_dim(const gcrl_replay *h);
+int replay_act_dim(const gcrl_replay *h);
+int replay_device(const gcrl_replay *h);
+uint64_t replay_epoch(const gcrl_replay *h);
+int64_t replay_many_n(const gcrl_replay *h);
+void replay_many_stage(gcrl_replay *h, int64_t B, int n, const int64_t *pos_host, const double *u_host,
+                       const double *beta, cudaStream_t st);
+void replay_many_sample(gcrl_replay *h, int64_t B, int n, int i, float *s, float *a, float *r, float *ns, float *d,
+                        float *weights_dev, cudaStream_t st);
+void replay_many_write_back(gcrl_replay *h, int64_t B, const float *td_dev, cudaStream_t st);
 }  // namespace gcrl
 
 using namespace gcrl;
@@ -744,11 +756,14 @@ struct gcrl_sac {
   // n consecutive updates in one graph (gcrl_sac_update_many): everything a captured update reads that changes from
   // one update to the next has one slot per update, in one device allocation laid out for the call's (n, B):
   // scalars [n] x kManyScalBytes | positions [n][B] int64 | eps_next [n][B][A] | eps_cur [n][B][A] | metrics [n][36]
+  // | TD errors [n][B] (prioritised replay; read back with the metric rows in one copy)
   struct Many {
     char *d = nullptr;
     size_t cap = 0;                              // bytes; growing it drops the cached graphs (their addresses move)
-    // (B, flags of every update, buffer, engine path)
-    std::map<std::tuple<int64_t, std::vector<int>, uintptr_t, int>, GraphRec> graphs;
+    // (B, flags of every update, buffer, engine path, buffer epoch, length drawn from): as in agent.cu
+    using Key = std::tuple<int64_t, std::vector<int>, uintptr_t, int, uint64_t, int64_t>;
+    std::map<Key, GraphRec> graphs;
+    std::set<Key> seen;                          // keys issued eagerly once (prioritised: captured when one repeats)
   } many;
   // sync-BN (gcrl_sac_set_sync_bn): the update is cut into graph segments, each ending in the collective the caller
   // runs before the next one (gcrl_sac_update_segment)
@@ -1337,7 +1352,7 @@ void run_phases(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
 
 // ---- n updates in one graph (gcrl_sac_update_many) -------------------------------------------------------------
 size_t many_bytes(const gcrl_sac *ag, int n, int64_t B) {
-  return size_t(n) * (kManyScalBytes + size_t(B) * (sizeof(int64_t) + 2 * ag->A * sizeof(float)) +
+  return size_t(n) * (kManyScalBytes + size_t(B) * (sizeof(int64_t) + 2 * ag->A * sizeof(float) + sizeof(float)) +
                       kMetricFloats * sizeof(float));
 }
 char *many_scalars(const gcrl_sac *ag, int i) { return ag->many.d + size_t(i) * kManyScalBytes; }
@@ -1350,6 +1365,7 @@ float *many_eps(const gcrl_sac *ag, int n, int64_t B, int which /*0 next, 1 cur*
 float *many_metrics(const gcrl_sac *ag, int n, int64_t B, int i) {
   return many_eps(ag, n, B, 2) + size_t(i) * kMetricFloats;
 }
+float *many_td(const gcrl_sac *ag, int n, int64_t B, int i) { return many_metrics(ag, n, B, n) + size_t(i) * B; }
 
 // While update i of an n-update call is recorded (or issued eagerly), the agent's per-update inputs -- AdamW and
 // alpha scalars, rsample noise -- point at slot i, so every argument builder of critic_update / actor_update picks
@@ -1358,10 +1374,11 @@ struct ManySlot {
   gcrl_sac *ag;
   StepScalars *sc; float *en, *ec;
   const SampleScalars *ssc; const int64_t *idx; float *metrics;
+  float *td;
   ManySlot(gcrl_sac *a, int i, int n, int B)
       : ag(a), sc(a->d_scalars), en(a->eps_next), ec(a->eps_cur),
         ssc(reinterpret_cast<const SampleScalars *>(many_scalars(a, i) + 2 * sizeof(StepScalars))),
-        idx(many_positions(a, n, B, i)), metrics(many_metrics(a, n, B, i)) {
+        idx(many_positions(a, n, B, i)), metrics(many_metrics(a, n, B, i)), td(many_td(a, n, B, i)) {
     a->d_scalars = reinterpret_cast<StepScalars *>(many_scalars(a, i));
     a->eps_next = many_eps(a, n, B, 0) + size_t(i) * B * a->A;
     a->eps_cur = many_eps(a, n, B, 1) + size_t(i) * B * a->A;
@@ -1384,19 +1401,25 @@ void run_many_body(gcrl_sac *ag, gcrl_her *buf, int B, int n, const int *flags, 
   }
 }
 
-void run_many(gcrl_sac *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
-  select_engine(ag, B, st);
-  ag->per_on = false;
+// Replay the n-update graph of `key`, capturing it first when it is new -- or, with capture_new false, only when
+// the key was issued before (a key seen for the first time is issued eagerly: a prioritised buffer that is still
+// filling draws from a new length every call, and its graphs would never be replayed).
+void launch_many(gcrl_sac *ag, gcrl_sac::Many::Key key, bool capture_new, const std::function<void(cudaStream_t)> &body,
+                 cudaStream_t st) {
   if (!ag->use_graphs) {
-    run_many_body(ag, buf, B, n, flags, st);
+    body(st);
     return;
   }
-  auto key = std::make_tuple(int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf),
-                             ag->tc_update ? 1 : 0);
   auto &cache = ag->many.graphs;
   auto it = cache.find(key);
+  if (it == cache.end() && !capture_new && ag->many.seen.count(key) == 0) {
+    if (ag->many.seen.size() >= 2 * kManyGraphCache) ag->many.seen.clear();
+    ag->many.seen.insert(std::move(key));
+    body(st);
+    return;
+  }
   if (it == cache.end()) {
-    const gcrl_sac::GraphRec g = capture_graph(ag, [&](cudaStream_t cs) { run_many_body(ag, buf, B, n, flags, cs); });
+    const gcrl_sac::GraphRec g = capture_graph(ag, body);
     if (cache.size() >= kManyGraphCache) {     // a replay still in flight is released when it completes
       for (auto &kv : cache) cudaGraphExecDestroy(kv.second.exec);
       cache.clear();
@@ -1404,6 +1427,39 @@ void run_many(gcrl_sac *ag, gcrl_her *buf, int B, int n, const int *flags, cudaS
     it = cache.emplace(std::move(key), g).first;
   }
   launch_graph(it->second, st);
+}
+
+void run_many(gcrl_sac *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+  select_engine(ag, B, st);
+  ag->per_on = false;
+  launch_many(ag, {int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), ag->tc_update ? 1 : 0,
+                   0, 0},
+              true, [&](cudaStream_t cs) { run_many_body(ag, buf, B, n, flags, cs); }, st);
+}
+
+// n updates from a uniform / prioritised buffer: the slot's draw, operand rows, the update, then -- prioritised -- the
+// priority write-back and the TD errors into the slot's row, and the metrics into the slot's row
+void run_many_replay_body(gcrl_sac *ag, gcrl_replay *buf, int B, int n, const int *flags, cudaStream_t st) {
+  for (int i = 0; i < n; ++i) {
+    ManySlot slot(ag, i, n, B);
+    replay_many_sample(buf, B, n, i, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->per_w, st);
+    launch_ingest_batch(ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->D, ag->A, B, ag->sa, ag->nsa, ag->spi, ag->ldc,
+                        ag->br, ag->bd, st);
+    run_body(ag, B, flags[i], PH_ALL, st);
+    if (ag->per_on) {
+      replay_many_write_back(buf, B, ag->per_td, st);
+      GCRL_CUDA(cudaMemcpyAsync(slot.td, ag->per_td, size_t(B) * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    }
+    GCRL_CUDA(cudaMemcpyAsync(slot.metrics, ag->mdev, kMetricFloats * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  }
+}
+
+void run_many_replay(gcrl_sac *ag, gcrl_replay *buf, int B, int n, const int *flags, cudaStream_t st) {
+  select_engine(ag, B, st);
+  ag->per_on = replay_prioritized(buf);
+  launch_many(ag, {int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), ag->tc_update ? 1 : 0,
+                   replay_epoch(buf), ag->per_on ? replay_many_n(buf) : 0},
+              !ag->per_on, [&](cudaStream_t cs) { run_many_replay_body(ag, buf, B, n, flags, cs); }, st);
 }
 
 // Segmented update (sync-BN): the body is captured ONCE per (B, flags) as a chain of graphs, cut wherever a
@@ -1579,6 +1635,37 @@ void read_metrics(gcrl_sac *ag, int flags, float *metrics_host, cudaStream_t st)
     GCRL_CUDA(cudaStreamSynchronize(st));
     metrics_tuple(ag, flags, hm, hs, metrics_host);
   }
+}
+
+// the per-update slots of an n-update call laid out for (n, B)
+void ensure_many(gcrl_sac *ag, int n, int64_t B) {
+  auto &mn = ag->many;
+  const size_t need = many_bytes(ag, n, B);
+  if (need <= mn.cap) return;
+  for (auto &kv : mn.graphs) cudaGraphExecDestroy(kv.second.exec);   // cudaFree waits for replays still reading them
+  mn.graphs.clear();
+  if (mn.d) GCRL_CUDA(cudaFree(mn.d));
+  mn.d = nullptr;
+  mn.cap = 0;
+  mn.d = dev_alloc<char>(need);
+  mn.cap = need;
+}
+
+// The metric rows [n][36] and, when td_host is given, the TD rows [n][B] that follow them: ONE read-back per call;
+// to pageable memory the copy returns once it (and the updates before it) completed
+void read_many_rows(gcrl_sac *ag, int n, int64_t B, const int *flags, float *metrics_host, float *td_host,
+                    cudaStream_t st) {
+  if (metrics_host == nullptr && td_host == nullptr) return;
+  const size_t m = size_t(n) * kMetricFloats;
+  std::vector<float> rows(m + (td_host != nullptr ? size_t(n) * B : 0));
+  GCRL_CUDA(cudaMemcpyAsync(rows.data(), many_metrics(ag, n, B, 0), rows.size() * sizeof(float), cudaMemcpyDeviceToHost,
+                            st));
+  if (metrics_host != nullptr)
+    for (int i = 0; i < n; ++i) {
+      const float *r = rows.data() + size_t(i) * kMetricFloats;
+      metrics_tuple(ag, flags[i], r, r + 32, metrics_host + size_t(i) * 12);
+    }
+  if (td_host != nullptr) std::memcpy(td_host, rows.data() + m, size_t(n) * B * sizeof(float));
 }
 
 void upload_padded(float *dst, const float *w, int rows, int cols, int ld, cudaStream_t st) {
@@ -1889,16 +1976,7 @@ int gcrl_sac_update_many(gcrl_sac *ag, gcrl_her *buf, int64_t B, int n, const in
   GCRL_CUDA(cudaSetDevice(ag->device));
   cudaStream_t st = as_stream(stream);
   auto &mn = ag->many;
-  const size_t need = many_bytes(ag, n, B);
-  if (need > mn.cap) {                       // cudaFree waits for replays still reading the old slots
-    for (auto &kv : mn.graphs) cudaGraphExecDestroy(kv.second.exec);
-    mn.graphs.clear();
-    if (mn.d) GCRL_CUDA(cudaFree(mn.d));
-    mn.d = nullptr;
-    mn.cap = 0;
-    mn.d = dev_alloc<char>(need);
-    mn.cap = need;
-  }
+  ensure_many(ag, n, B);
   StepCounterGuard guard(ag);
   guard.keep_draws(buf);
   // every update's scalars (the device stream's draw epochs in order), then every update's positions: ONE copy
@@ -1920,16 +1998,54 @@ int gcrl_sac_update_many(gcrl_sac *ag, gcrl_her *buf, int64_t B, int n, const in
   if (any_actor) GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 1), eps_cur_dev, noise, cudaMemcpyDeviceToDevice, st));
   run_many(ag, buf, int(B), n, flags, st);
   guard.commit();
-  if (metrics_host != nullptr) {
-    // ONE read-back per call; to pageable memory the copy returns once it (and the updates before it) completed
-    std::vector<float> rows(size_t(n) * kMetricFloats);
-    GCRL_CUDA(cudaMemcpyAsync(rows.data(), many_metrics(ag, n, B, 0), rows.size() * sizeof(float),
-                              cudaMemcpyDeviceToHost, st));
-    for (int i = 0; i < n; ++i) {
-      const float *r = rows.data() + size_t(i) * kMetricFloats;
-      metrics_tuple(ag, flags[i], r, r + 32, metrics_host + size_t(i) * 12);
-    }
+  read_many_rows(ag, n, B, flags, metrics_host, nullptr, st);
+  GCRL_API_END
+}
+
+int gcrl_sac_update_many_replay(gcrl_sac *ag, gcrl_replay *buf, int64_t B, int n, const int *flags,
+                                const int64_t *pos_host, const double *u_host, const double *beta,
+                                const float *eps_next_dev, const float *eps_cur_dev, const double *lr_critic,
+                                const double *lr_actor, float *metrics_host, float *td_host, void *stream) {
+  GCRL_API_BEGIN
+  GCRL_NVTX("gcrl_sac_update_many_replay");
+  require_handle(ag);
+  GCRL_REQUIRE(buf != nullptr, "buffer handle is NULL");
+  GCRL_REQUIRE(B >= 2 && B <= ag->maxB, "batch size outside [2, max_batch] (BatchNorm needs > 1 row)");
+  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
+  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
+  const bool per = replay_prioritized(buf);
+  bool any_actor = false;
+  for (int i = 0; i < n; ++i) {
+    GCRL_REQUIRE((flags[i] & ~15) == 0, "flags of an n-update call from a replay buffer may hold bits 0-3 only");
+    GCRL_REQUIRE(((flags[i] & 8) != 0) == per, "flags bit3 must be set exactly when the buffer is prioritised");
+    any_actor = any_actor || (flags[i] & 1) != 0;
   }
+  GCRL_REQUIRE(eps_next_dev != nullptr && (eps_cur_dev != nullptr || !any_actor), "NULL rsample noise tensor");
+  GCRL_REQUIRE(ag->sync_world == 0, "a sync-BN agent trains through gcrl_sac_update_segment only");
+  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
+  GCRL_REQUIRE(replay_state_dim(buf) == ag->D && replay_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
+  GCRL_REQUIRE(replay_device(buf) == ag->device, "buffer and agent live on different devices");
+  GCRL_CUDA(cudaSetDevice(ag->device));
+  cudaStream_t st = as_stream(stream);
+  replay_many_stage(buf, B, n, pos_host, u_host, beta, st);      // the buffer's own checks come first
+  ensure_many(ag, n, B);
+  StepCounterGuard guard(ag);
+  int slot;
+  char *p = ag->io_stage.acquire(size_t(n) * kManyScalBytes, &slot);
+  for (int i = 0; i < n; ++i) {
+    char *s = p + size_t(i) * kManyScalBytes;
+    fill_scalars(ag, lr_critic[i], lr_actor[i], flags[i], reinterpret_cast<StepScalars *>(s));
+    std::memset(s + 2 * sizeof(StepScalars), 0, sizeof(SampleScalars));
+  }
+  GCRL_CUDA(cudaMemcpyAsync(ag->many.d, p, size_t(n) * kManyScalBytes, cudaMemcpyHostToDevice, st));
+  ag->io_stage.release(slot, st);
+  // stable addresses for the captured graph
+  const size_t noise = size_t(n) * B * ag->A * sizeof(float);
+  GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 0), eps_next_dev, noise, cudaMemcpyDeviceToDevice, st));
+  if (any_actor) GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 1), eps_cur_dev, noise, cudaMemcpyDeviceToDevice, st));
+  run_many_replay(ag, buf, int(B), n, flags, st);
+  guard.commit();
+  read_many_rows(ag, n, B, flags, metrics_host, per ? td_host : nullptr, st);
   GCRL_API_END
 }
 

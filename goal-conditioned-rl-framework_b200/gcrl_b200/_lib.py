@@ -91,6 +91,7 @@ SIGNATURES = {
     "gcrl_agent_update_batch": (C.c_int, [vp, c_i64, vp, vp, vp, vp, vp, vp, c_f64, c_f64, C.c_int, vp, vp]),
     "gcrl_agent_update_from_buffer": (C.c_int, [vp, vp, c_i64, vp, vp, c_f64, c_f64, C.c_int, vp, vp]),
     "gcrl_agent_update_many": (C.c_int, [vp, vp, c_i64, C.c_int, vp, vp, vp, vp, vp, vp, vp]),
+    "gcrl_agent_update_many_replay": (C.c_int, [vp, vp, c_i64, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "gcrl_agent_read_metrics": (C.c_int, [vp, vp, vp]),
     "gcrl_agent_act": (C.c_int, [vp, c_i64, vp, vp, vp]),
     "gcrl_agent_q": (C.c_int, [vp, c_i64, vp, vp, vp, vp]),
@@ -116,6 +117,7 @@ SIGNATURES = {
     "gcrl_sac_update_batch": (C.c_int, [vp, c_i64, vp, vp, vp, vp, vp, vp, vp, c_f64, c_f64, C.c_int, vp, vp]),
     "gcrl_sac_update_from_buffer": (C.c_int, [vp, vp, c_i64, vp, vp, vp, c_f64, c_f64, C.c_int, vp, vp]),
     "gcrl_sac_update_many": (C.c_int, [vp, vp, c_i64, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "gcrl_sac_update_many_replay": (C.c_int, [vp, vp, c_i64, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "gcrl_sac_act": (C.c_int, [vp, c_i64, vp, vp, vp, vp]),
     "gcrl_sac_update_phase": (C.c_int, [vp, C.c_int, vp, c_i64, vp, vp, vp, vp, vp, vp, vp, vp, c_f64, c_f64, C.c_int,
                                         vp]),

@@ -225,8 +225,11 @@ class _AgentBase:
         pass
 
     def beta_scheduler(self, step: int):
+        self.beta = self._beta_at(step)
+
+    def _beta_at(self, step):
         ratio = step / self.beta_end
-        self.beta = min(self.beta_max, self.beta_start + ratio * (self.beta_max - self.beta_start))
+        return min(self.beta_max, self.beta_start + ratio * (self.beta_max - self.beta_start))
 
     def update_normalizers(self, obs_list, dg_list, obs_normalize, g_normalize):
         if getattr(self.buffer, "obs_normalizer", None) is not None and obs_list and obs_normalize:
@@ -541,27 +544,93 @@ class _AgentBase:
         return [float(x) for x in self._metrics]
 
     # -- a training cycle's gradient steps in one call ---------------------------------------------------
-    _MANY_IN_ONE_GRAPH = False      # n updates from a HER buffer replay as one CUDA graph (every agent sets it)
+    _MANY_IN_ONE_GRAPH = False      # n updates replay as one CUDA graph (every agent sets it)
 
     def update_many(self, steps):
         """``[self.update(s) for s in steps]``: the same tuples, and afterwards the same state of every network,
-        optimiser, schedule, index stream and random generator.  ``steps`` need not be consecutive.
+        optimiser, schedule, beta, buffer (ring, priorities, last positions), index stream and random generator.
+        ``steps`` need not be consecutive.
 
-        DDPG, TD3, SAC and TQC sampling from a HER buffer on one GPU issue every 64 steps as ONE CUDA graph
-        launch: the positions (host index stream), learning rates and noise (TD3 smoothing, SAC / TQC rsample)
-        of all of them are drawn up front and travel in one copy each, so no interpreter, launch or metric
-        read-back sits between the updates.  Every other buffer type and data-parallel mode runs the loop."""
+        DDPG, TD3, SAC and TQC on one GPU issue every 64 steps as ONE CUDA graph launch, whatever the buffer: the
+        positions (HER host index stream, ``random.sample`` of REPLAY), the uniforms and beta of every PER draw,
+        the learning rates and the noise (TD3 smoothing, SAC / TQC rsample) of all of them are drawn up front in
+        the loop's order and travel in one copy each, so no interpreter, launch, priority round trip or metric
+        read-back sits between the updates.  With PER, each update's draw reads the priorities the previous one
+        wrote; while the ring is still filling, each call issues its updates without a graph.  Both data-parallel
+        modes run the loop."""
         steps = [int(s) for s in steps]
-        if not (self._MANY_IN_ONE_GRAPH and isinstance(self.buffer, HERBuffer) and self._dp is None
-                and getattr(self, "_peer_dp", None) is None):
+        if not (self._MANY_IN_ONE_GRAPH and self._dp is None and getattr(self, "_peer_dp", None) is None):
             return [self.update(s) for s in steps]
+        chunk = self._update_chunk if isinstance(self.buffer, HERBuffer) else self._update_chunk_replay
         out = []
         for lo in range(0, len(steps), MAX_MANY_STEPS):
-            out += self._update_chunk(steps[lo:lo + MAX_MANY_STEPS])
+            out += chunk(steps[lo:lo + MAX_MANY_STEPS])
         return out
 
     def _many_noise(self, B, n):
         return None
+
+    def _step_schedules(self, flags):
+        """The learning rates of n updates with these flags: the schedules step as update() steps them.  Returns
+        (lr_critic[n], lr_actor[n], the schedules' state before) for _restore_schedules on a refused call."""
+        n = len(flags)
+        lr_c, lr_a = (C.c_double * n)(), (C.c_double * n)()
+        saved = [(sch.last_epoch, sch.lr) for sch in (self.critic_scheduler, self.actor_scheduler)]
+        for i, f in enumerate(flags):
+            lr_c[i], lr_a[i] = self.critic_scheduler.lr, self.actor_scheduler.lr
+            self.critic_scheduler.step()
+            if f & 1:
+                self.actor_scheduler.step()
+        return lr_c, lr_a, saved
+
+    def _restore_schedules(self, saved):
+        for sch, (epoch, lr) in zip((self.critic_scheduler, self.actor_scheduler), saved):
+            sch.last_epoch, sch.lr = epoch, lr
+
+    def _check_replay_chunk(self, B, min_batch=1):
+        """What update() checks from a REPLAY / PER buffer, before any generator is touched."""
+        assert len(self.buffer) >= B, "Not enough in buffer to sample"
+        if not min_batch <= B <= self._max_batch:
+            raise ValueError(f"batch size {B} outside [{min_batch}, max_batch = {self._max_batch}]")
+
+    def _replay_draws(self, B, steps):
+        """update()'s host draws from a REPLAY / PER buffer for every step, in step order: the positions
+        ``random.sample(range(len), B)`` (REPLAY), or the uniforms ``np.random.random_sample(B)`` and the beta each
+        draw uses -- the one beta_scheduler(step) left after the update before (PER).  Returns (flags bit3,
+        positions, uniforms, betas); the arrays not used are None."""
+        if isinstance(self.buffer, PERBuffer):
+            u = np.stack([np.random.random_sample(B) for _ in steps])
+            betas, beta = [], self.beta
+            for s in steps:
+                betas.append(beta)
+                beta = self._beta_at(s)
+            return 8, None, u, np.array(betas, np.float64)
+        nlen = len(self.buffer)
+        return 0, np.stack([_lib.py_sample_range(nlen, B) for _ in steps]), None, None
+
+    def _update_chunk_replay(self, steps):
+        B, n = self.batch_size, len(steps)
+        self._check_replay_chunk(B)
+        noise = self._many_noise(B, n)
+        per, pos, u, beta = self._replay_draws(B, steps)
+        flags = (C.c_int * n)(*(self._flags(s) | per for s in steps))
+        lr_c, lr_a, saved = self._step_schedules(flags)
+        metrics = np.empty((n, 8), np.float32)
+        td = np.empty((n, B), np.float32) if per else None
+        try:
+            check(lib.gcrl_agent_update_many_replay(
+                self._h, self.buffer.handle, B, n, flags, *(None if x is None else np_ptr(x) for x in (pos, u, beta)),
+                vp(noise.data_ptr()) if noise is not None else None, lr_c, lr_a, np_ptr(metrics),
+                np_ptr(td) if per else None, self._stream()))
+        except BaseException:
+            self._restore_schedules(saved)
+            raise
+        out = []
+        for i, (step, m) in enumerate(zip(steps, metrics.tolist())):
+            self._last_td = td[i].reshape(B, 1) if per else None
+            self.beta_scheduler(step)
+            out.append(self._result(step, m))
+        return out
 
     def _update_chunk(self, steps):
         B, n = self.batch_size, len(steps)
@@ -576,22 +645,14 @@ class _AgentBase:
             idx = np.stack([_lib.py_sample_range(nlen, B) for _ in steps])
             iptr = np_ptr(idx)
         flags = (C.c_int * n)(*(self._flags(s) for s in steps))
-        lr_c, lr_a = (C.c_double * n)(), (C.c_double * n)()
-        schedules = (self.critic_scheduler, self.actor_scheduler)
-        saved = [(sch.last_epoch, sch.lr) for sch in schedules]
-        for i in range(n):                          # the schedules step as _run_update steps them
-            lr_c[i], lr_a[i] = self.critic_scheduler.lr, self.actor_scheduler.lr
-            self.critic_scheduler.step()
-            if flags[i] & 1:
-                self.actor_scheduler.step()
+        lr_c, lr_a, saved = self._step_schedules(flags)
         metrics = np.empty((n, 8), np.float32)
         try:
             check(lib.gcrl_agent_update_many(self._h, self.buffer.handle, B, n, flags, iptr,
                                              vp(noise.data_ptr()) if noise is not None else None, lr_c, lr_a,
                                              np_ptr(metrics), self._stream()))
         except BaseException:
-            for sch, (epoch, lr) in zip(schedules, saved):
-                sch.last_epoch, sch.lr = epoch, lr
+            self._restore_schedules(saved)
             raise
         self._last_td = None
         out = []

@@ -481,6 +481,28 @@ int gcrl_replay_last_tables(gcrl_replay *h, float *p_host, double *cdf_host, voi
 int gcrl_agent_per_buffers(gcrl_agent *h, float **weights_dev, float **td_dev);
 int gcrl_sac_per_buffers(gcrl_sac *h, float **weights_dev, float **td_dev);
 
+/* n consecutive updates sampling from a uniform or prioritised buffer, issued as ONE graph launch (prioritised:
+ * once the same (B, flags, length) repeats; while the ring is still filling every call issues its updates directly).
+ * Equivalent, bit for bit, to n rounds of
+ *   uniform:     gcrl_replay_sample(pos_host + i*B) -> gcrl_agent_update_batch / gcrl_sac_update_batch;
+ *   prioritised: gcrl_replay_sample_prioritized(u_host + i*B, beta[i]) -> the update with flags[i] bit3 ->
+ *                gcrl_replay_update_priorities(NULL, td) -> TD errors into td_host + i*B,
+ * with flags[i], lr_critic[i], lr_actor[i] and the noise rows of update i as in gcrl_agent_update_many /
+ * gcrl_sac_update_many.  flags[i] bit3 must be set exactly when the buffer is prioritised; beyond it, the flag bits of
+ * those calls.  pos_host [n][B] (uniform) or u_host [n][B] and beta [n] (prioritised); the other pointers may be NULL.
+ * metrics_host: float[n][8] / float[n][12] as in those calls; td_host (prioritised, may be NULL): float[n][B], read
+ * back with one copy at the end of the call.  Afterwards the buffer's last positions and sample info are those of
+ * update n - 1.  Refused as gcrl_agent_update_many / gcrl_sac_update_many are, and GCRL_ERR_UNDERFILLED when len < B;
+ * on any error no step counter, sequence number or priority has moved. */
+int gcrl_agent_update_many_replay(gcrl_agent *h, gcrl_replay *buf, int64_t B, int n, const int *flags,
+                                  const int64_t *pos_host, const double *u_host, const double *beta,
+                                  const float *noise_dev, const double *lr_critic, const double *lr_actor,
+                                  float *metrics_host, float *td_host, void *stream);
+int gcrl_sac_update_many_replay(gcrl_sac *h, gcrl_replay *buf, int64_t B, int n, const int *flags,
+                                const int64_t *pos_host, const double *u_host, const double *beta,
+                                const float *eps_next_dev, const float *eps_cur_dev, const double *lr_critic,
+                                const double *lr_actor, float *metrics_host, float *td_host, void *stream);
+
 /* ------------------------------------------------------------------------------------
  * Diagnostics / micro-benchmarks
  * ------------------------------------------------------------------------------------
