@@ -319,6 +319,7 @@ __global__ void __launch_bounds__((BM / TM) * (BN / TN)) multi_wgrad_kernel(cons
 // together with the tile's sum of squares for the global-norm clip.  No partial slabs in HBM, no reduction
 // launch, no atomics.  Tile 0 also finalises the batch-mean metrics of the phase.
 constexpr int kWgThreads = 64, kWgTile = 32, kWgFinish = 256;
+constexpr int kWgMaxMetricSlabs = 256;                       // row-slab kernels run <= 256 CTAs (fused_supported)
 constexpr int kWgStageFloats = 2 * 2 * BK * (kWgTile + SPAD);      // As[2][BK][36] + Bs[2][BK][36] per group
 
 __device__ __forceinline__ void bar_group(int grp) { asm volatile("bar.sync %0, %1;" ::"r"(grp + 1), "n"(kWgThreads) : "memory"); }
@@ -348,8 +349,16 @@ __global__ void __launch_bounds__(kWgThreads * GROUPS) wgrad_tile_kernel(const _
   extern __shared__ float4 wg_sm4[];
   __shared__ float s_sq[kWgFinish / 32];
   float *sm = reinterpret_cast<float *>(wg_sm4);
+  __shared__ __align__(16) float s_met[kWgMaxMetricSlabs * 4];
   pdl_wait();
   pdl_launch_dependents();
+  // tile 0 sums the row-slab kernel's metric partials slab after slab at the end; copied here in one round trip,
+  // they are no longer a chain of loads at the end of the kernel (B = 256: 128 slabs, 8 round trips of 16 loads)
+  const bool metrics_here = blockIdx.x == 0 && mg.fin.metric_partials != nullptr;
+  if (metrics_here && int(threadIdx.x) < mg.fin.metric_splits) {
+    const unsigned int d = static_cast<unsigned int>(__cvta_generic_to_shared(s_met + threadIdx.x * 4));
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(mg.fin.metric_partials + threadIdx.x * 4) : "memory");
+  }
   int pi, bx, by;
   locate_tile(mg, pi, bx, by);
   const GemmParams &p = mg.p[pi];
@@ -407,6 +416,7 @@ __global__ void __launch_bounds__(kWgThreads * GROUPS) wgrad_tile_kernel(const _
   for (int i = 0; i < 4; ++i)
     *reinterpret_cast<float4 *>(red + (ty * 4 + i) * BN + tx * 4) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
   if (tid < BM) red[BM * BN + tid] = bsum;
+  asm volatile("cp.async.wait_all;" ::: "memory");           // (the metric partials)
   __syncthreads();
   float sq = 0.f;
   const int t = threadIdx.x;
@@ -431,9 +441,9 @@ __global__ void __launch_bounds__(kWgThreads * GROUPS) wgrad_tile_kernel(const _
       sq = fmaf(gb, gb, sq);
     }
   }
-  if (blockIdx.x == 0 && mg.fin.metric_partials != nullptr && t < 3) {
+  if (metrics_here && t < 3) {
     float s = 0.f;
-    for (int k = 0; k < mg.fin.metric_splits; ++k) s += mg.fin.metric_partials[size_t(k) * 4 + t];
+    for (int k = 0; k < mg.fin.metric_splits; ++k) s += s_met[k * 4 + t];
     const int slot = t == 0 ? mg.fin.slot_loss : (t == 1 ? mg.fin.slot_td : mg.fin.slot_q);
     if (slot >= 0) mg.fin.metrics[slot] = s * mg.fin.metric_scale;
   }
@@ -530,7 +540,9 @@ static void launch_wgrad_tiles(const MultiGemm &mg, int tiles, cudaStream_t st) 
     GCRL_CUDA(cudaFuncSetAttribute(wgrad_tile_kernel<GROUPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     attr_set = true;
   }
-  // no early launch: the small CTAs would pile onto the SMs the preceding row-slab kernel leaves free
+  // no early launch: the small CTAs would pile onto the SMs the preceding row-slab kernel leaves free.  Measured again
+  // with the metric partials prefetched (profiles/r04_update_tail.json, B = 256 flushed step on one B200 at 1000 W):
+  // PDL_WGRAD on 0.1209 ms, off 0.1147 ms; each weight-gradient launch adds 10.6-11.0 instead of 7.2-7.3 us
   launch_pdl<PDL_WGRAD>(wgrad_tile_kernel<GROUPS>, dim3(tiles), dim3(kWgThreads * GROUPS), smem, st, mg);
 }
 
@@ -539,6 +551,9 @@ int launch_wgrad_complete(const WgradProblem *probs, int nprob, int M, const Wgr
   const int groups = M > 256 ? 8 : 4;
   int chunk = (M + groups - 1) / groups;
   chunk = (chunk + BK - 1) / BK * BK;
+  GCRL_REQUIRE(fin.metric_partials == nullptr ||
+                   (fin.metric_splits <= kWgMaxMetricSlabs && (reinterpret_cast<uintptr_t>(fin.metric_partials) & 15) == 0),
+               "wgrad metrics: at most 256 16-byte aligned partial slabs");
   MultiGemm mg{};
   mg.fin = fin;
   const int tiles = fill_multi(mg, probs, nprob, M, 0, chunk, true);

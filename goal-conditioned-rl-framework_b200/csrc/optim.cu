@@ -263,8 +263,35 @@ void launch_p2p_reduce(const P2PReduceHost &h, cudaStream_t st) {
 //   p *= 1 - lr*wd (AdamW only);  m += (1-b1)(g-m);  v = v*b2 + (1-b2) g g;
 //   p -= (lr/bc1) * m / (sqrt(v)/sqrt(bc2) + eps)
 // preceded by clip_grad_norm_: g *= min(1, max_norm / (||g|| + 1e-6)).
+//
+// Only g and the sums of squares come from the kernel this one depends on (weight-gradient kernel, gradient
+// reduction, sums-of-squares kernel or peer average -- p2p_reduce_kernel writes gavg and sumsq).  p, m, v, tmap,
+// target and the step scalars of a thread's first element are loaded BEFORE pdl_wait(), so that their DRAM round
+// trip overlaps the tail of that kernel:
+//   - p, m, v and pT are written only by this kernel, and the target it blends only by this kernel's own Polyak
+//     (polyak_kernel writes the DDPG actor target, which no Adam launch blends, and the targets in
+//     gcrl_agent_soft_update, which no Adam launch follows directly).  The actor-target Polyak that may directly
+//     precede the DDPG critic step writes nothing the critic step reads.  tmap never changes; the step scalars are
+//     a host copy made before the update.
+//   - Every kernel launched with the PDL attribute executes pdl_launch_dependents() only after its own pdl_wait()
+//     (p2p_reduce_kernel not at all: it releases this one when it exits), and a kernel launched without it starts
+//     after its predecessor has completed.  So when this kernel starts, every launch two or more back has completed
+//     and its writes are visible: the other critic's step (TD3), the previous update's steps (update_many).
+//     Keep pdl_launch_dependents() below pdl_wait() everywhere, or these loads may read stale values.
+// At B = 256 one grid-stride pass covers every element; later passes load after the wait as before.
 __device__ __forceinline__ void adam_body(const AdamArgs &a) {
   __shared__ float s_coef, s_norm;
+  const int e0 = blockIdx.x * blockDim.x + threadIdx.x, stride = gridDim.x * blockDim.x;
+  float p0 = 0.f, m0 = 0.f, v0 = 0.f, t0 = 0.f;
+  int tm0 = -1;
+  if (e0 < a.n) {
+    p0 = a.p[e0]; m0 = a.m[e0]; v0 = a.v[e0];
+    if (a.tmap != nullptr) tm0 = a.tmap[e0];
+    if (a.polyak) t0 = a.target[e0];
+  }
+  const float step_size = a.which == 0 ? a.sc->step_size_c : a.sc->step_size_a;
+  const float bc2_sqrt = a.which == 0 ? a.sc->bc2_sqrt_c : a.sc->bc2_sqrt_a;
+  const float decay = a.which == 0 ? a.sc->decay_c : a.sc->decay_a;
   pdl_wait();
   pdl_launch_dependents();
   if (threadIdx.x < 32) {
@@ -282,32 +309,30 @@ __device__ __forceinline__ void adam_body(const AdamArgs &a) {
   }
   __syncthreads();
   const float coef = s_coef;
-  const float step_size = a.which == 0 ? a.sc->step_size_c : a.sc->step_size_a;
-  const float bc2_sqrt = a.which == 0 ? a.sc->bc2_sqrt_c : a.sc->bc2_sqrt_a;
-  const float decay = a.which == 0 ? a.sc->decay_c : a.sc->decay_a;
   // scalar arguments exactly as torch narrows them: float(1 - 0.9), float(0.999), float(1 - 0.999)
   const float omb1 = float(1.0 - 0.9), b2 = float(0.999), omb2 = float(1.0 - 0.999), eps = 1e-8f;
-  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < a.n; e += gridDim.x * blockDim.x) {
-    const float g = a.g[e] * coef;
-    float p = a.p[e];
-    if (a.weight_decay != 0.f) p *= decay;
-    float m = a.m[e], v = a.v[e];
-    m = m + omb1 * (g - m);
-    v = v * b2;
-    v = v + omb2 * g * g;
-    const float denom = sqrtf(v) / bc2_sqrt + eps;
-    p = p - step_size * (m / denom);
+  // the roundings spelled out (the contractions the compiler chose for this kernel before its loads were hoisted),
+  // so that moving a load cannot change which products are fused
+  auto step = [&](int e, float p, float m, float v, int tm, float tgt) {
+    const float g = __fmul_rn(a.g[e], coef);
+    if (a.weight_decay != 0.f) p = __fmul_rn(p, decay);
+    m = __fmaf_rn(__fsub_rn(g, m), omb1, m);
+    v = __fmaf_rn(__fmul_rn(omb2, g), g, __fmul_rn(v, b2));
+    const float denom = __fadd_rn(sqrtf(v) / bc2_sqrt, eps);
+    p = __fmaf_rn(-step_size, m / denom, p);
     a.m[e] = m;
     a.v[e] = v;
     a.p[e] = p;
-    const int tm = a.tmap != nullptr ? a.tmap[e] : -1;
     if (tm >= 0) a.pT[tm] = p;
     if (a.polyak) {
-      const float t = a.tau * p + a.one_minus_tau * a.target[e];
+      const float t = __fmaf_rn(a.tau, p, __fmul_rn(a.one_minus_tau, tgt));
       a.target[e] = t;
       if (tm >= 0 && a.targetT != nullptr) a.targetT[tm] = t;     // (SAC / TQC targets keep no W^T)
     }
-  }
+  };
+  if (e0 < a.n) step(e0, p0, m0, v0, tm0, t0);
+  for (int e = e0 + stride; e < a.n; e += stride)
+    step(e, a.p[e], a.m[e], a.v[e], a.tmap != nullptr ? a.tmap[e] : -1, a.polyak ? a.target[e] : 0.f);
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     const float post = s_norm * coef;         // norm after clipping (src/agent.py:1332,:1300)
     if (a.metrics != nullptr && a.slot_norm >= 0) a.metrics[a.slot_norm] = post;
