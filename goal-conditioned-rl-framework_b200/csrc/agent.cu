@@ -15,40 +15,14 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
-#include <functional>
 #include <initializer_list>
 #include <map>
-#include <set>
 #include <tuple>
 #include <vector>
 
+#include "buffer_api.cuh"
+#include "graphs.cuh"
 #include "mlp.cuh"
-
-struct gcrl_her;
-namespace gcrl {
-SampleScalars her_next_scalars(gcrl_her *h, bool positions_given);
-const HerGeom &her_geom(const gcrl_her *h);
-int64_t her_len(const gcrl_her *h);
-void her_sample_into(gcrl_her *h, int64_t B, const int64_t *idx_host, float *s, float *a, float *r,
-                     float *ns, float *d, int64_t *idx_out, cudaStream_t st);
-int her_state_dim(const gcrl_her *h);
-int her_act_dim(const gcrl_her *h);
-int her_device(const gcrl_her *h);
-void her_sample_graphed(gcrl_her *h, int64_t B, const SampleScalars *sc_dev, const int64_t *idx_dev, float *s,
-                        float *a, float *r, float *ns, float *d, cudaStream_t st);
-unsigned long long &her_draw_epoch(gcrl_her *h);
-bool replay_prioritized(const gcrl_replay *h);
-int replay_state_dim(const gcrl_replay *h);
-int replay_act_dim(const gcrl_replay *h);
-int replay_device(const gcrl_replay *h);
-uint64_t replay_epoch(const gcrl_replay *h);
-int64_t replay_many_n(const gcrl_replay *h);
-void replay_many_stage(gcrl_replay *h, int64_t B, int n, const int64_t *pos_host, const double *u_host,
-                       const double *beta, cudaStream_t st);
-void replay_many_sample(gcrl_replay *h, int64_t B, int n, int i, float *s, float *a, float *r, float *ns, float *d,
-                        float *weights_dev, cudaStream_t st);
-void replay_many_write_back(gcrl_replay *h, int64_t B, const float *td_dev, cudaStream_t st);
-}  // namespace gcrl
 
 using namespace gcrl;
 
@@ -145,7 +119,6 @@ enum Slot { S_CLOSS = 0, S_ALOSS = 1, S_TD = 2, S_Q = 3, S_CGRAD = 4, S_AGRAD = 
 
 constexpr int kMaxSplits = 128;
 constexpr size_t kScalBytes = sizeof(StepScalars) + sizeof(SampleScalars);   // the per-update device scalars
-constexpr size_t kManyGraphCache = 8;    // n-update graphs kept per agent (one flag pattern per run is typical)
 
 }  // namespace
 
@@ -210,7 +183,6 @@ struct gcrl_agent {
   bool dp_open = false;                    // a phase-wise data-parallel update: phase 0 issued, phase 3 not yet
   bool use_graphs = true;
   cudaStream_t cap_stream = nullptr;       // capture-only stream (the caller's may be the legacy one)
-  struct GraphRec { cudaGraphExec_t exec; uint64_t kernels; };
   std::map<std::tuple<int64_t, int, int, uintptr_t>, GraphRec> graphs;   // (B, flags, phase mask, sampled buffer)
   // n consecutive updates in one graph (gcrl_agent_update_many): everything a captured update reads that changes
   // from one update to the next has one slot per update; allocated on first use
@@ -222,8 +194,7 @@ struct gcrl_agent {
     // (B, flags of every update, buffer, engine path, buffer epoch, length drawn from): a uniform or HER buffer has
     // 0 for the last one, a graph serves any length; a HER buffer also has 0 for the epoch
     using Key = std::tuple<int64_t, std::vector<int>, uintptr_t, int, uint64_t, int64_t>;
-    std::map<Key, GraphRec> graphs;
-    std::set<Key> seen;                    // keys issued eagerly once (prioritised: captured when one repeats)
+    ManyGraphs<Key> graphs;
   } many;
 };
 
@@ -757,34 +728,6 @@ void run_update_body(gcrl_agent *ag, int B, const float *noise, int flags, int m
   }
 }
 
-// Record `body` on the capture stream into an instantiated graph; the kernels it records are not counted as
-// launches until the graph is replayed.
-gcrl_agent::GraphRec capture_graph(gcrl_agent *ag, const std::function<void(cudaStream_t)> &body) {
-  cudaGraph_t graph = nullptr;
-  const uint64_t before = launch_counter();
-  GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
-  try {
-    body(ag->cap_stream);
-  } catch (...) {
-    cudaStreamEndCapture(ag->cap_stream, &graph);
-    if (graph) cudaGraphDestroy(graph);
-    throw;
-  }
-  GCRL_CUDA(cudaStreamEndCapture(ag->cap_stream, &graph));
-  const uint64_t kernels = launch_counter() - before;   // recorded, not executed, by the capture
-  count_launch(uint64_t(0) - kernels);
-  cudaGraphExec_t exec = nullptr;
-  const cudaError_t e = cudaGraphInstantiate(&exec, graph, 0);
-  cudaGraphDestroy(graph);
-  GCRL_CUDA(e);
-  return gcrl_agent::GraphRec{exec, kernels};
-}
-
-void launch_graph(const gcrl_agent::GraphRec &g, cudaStream_t st) {
-  GCRL_CUDA(cudaGraphLaunch(g.exec, st));
-  count_launch(g.kernels);
-}
-
 // the engine an update at this batch runs on; the tensor-core one needs the split weight copies current
 void select_engine(gcrl_agent *ag, int B, cudaStream_t st) {
   ag->tc_update = !fused_ok(ag, B) && engine_tc(ag, B);
@@ -803,7 +746,7 @@ void run_update(gcrl_agent *ag, int B, const float *noise, int flags, int mask, 
   const auto key = std::make_tuple(int64_t(B), flags, mask, reinterpret_cast<uintptr_t>(ag->sample_buf));
   auto it = ag->graphs.find(key);
   if (it == ag->graphs.end())
-    it = ag->graphs.emplace(key, capture_graph(ag, [&](cudaStream_t cs) { run_update_body(ag, B, noise, flags, mask, cs); })).first;
+    it = ag->graphs.emplace(key, capture_graph(ag->cap_stream, [&](cudaStream_t cs) { run_update_body(ag, B, noise, flags, mask, cs); })).first;
   launch_graph(it->second, st);
 }
 
@@ -827,81 +770,42 @@ struct ManySlot {
   ManySlot &operator=(const ManySlot &) = delete;
 };
 
-// n updates from `buf` back to back.  Where the sampler is a launch of its own (ag->sample_buf == nullptr) it is
-// part of every update here, reading that update's totals and positions from the slot.
-void run_many_body(gcrl_agent *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+// n updates back to back from the HER buffer `her` or the uniform / prioritised buffer `rb` (the other is NULL).
+// Update i draws its batch from slot i -- HER: from the slot's totals and positions, unless the row-slab critic kernel
+// draws it (ag->sample_buf set) -- and, prioritised, writes its priorities back and copies its TD errors into row i.
+void run_many_body(gcrl_agent *ag, gcrl_her *her, gcrl_replay *rb, int B, int n, const int *flags, cudaStream_t st) {
   for (int i = 0; i < n; ++i) {
     ManySlot slot(ag, i, n, B);
     if (ag->sample_buf == nullptr) {
-      her_sample_graphed(buf, B, ag->d_sample_sc, ag->d_idx, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, st);
+      if (rb != nullptr)
+        replay_many_sample(rb, B, n, i, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->per_w, st);
+      else
+        her_sample_graphed(her, B, ag->d_sample_sc, ag->d_idx, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, st);
       if (!fused_ok(ag, B))
         launch_ingest_batch(ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->D, ag->A, B, ag->sa, ag->nsa, ag->spi, ag->ldc,
                             ag->br, ag->bd, st);
     }
     run_update_body(ag, B, ag->td3 ? ag->noise : nullptr, flags[i], PH_ALL, st);
-  }
-}
-
-// Replay the n-update graph of `key`, capturing it first when it is new -- or, with capture_new false, only when
-// the key was issued before (a key seen for the first time is issued eagerly: a prioritised buffer that is still
-// filling draws from a new length every call, and its graphs would never be replayed).
-void launch_many(gcrl_agent *ag, gcrl_agent::Many::Key key, bool capture_new,
-                 const std::function<void(cudaStream_t)> &body, cudaStream_t st) {
-  if (!ag->use_graphs) {
-    body(st);
-    return;
-  }
-  auto &cache = ag->many.graphs;
-  auto it = cache.find(key);
-  if (it == cache.end() && !capture_new && ag->many.seen.count(key) == 0) {
-    if (ag->many.seen.size() >= 2 * kManyGraphCache) ag->many.seen.clear();
-    ag->many.seen.insert(std::move(key));
-    body(st);
-    return;
-  }
-  if (it == cache.end()) {
-    const gcrl_agent::GraphRec g = capture_graph(ag, body);
-    if (cache.size() >= kManyGraphCache) {     // a replay still in flight is released when it completes
-      for (auto &kv : cache) cudaGraphExecDestroy(kv.second.exec);
-      cache.clear();
+    if (ag->per_on) {
+      replay_many_write_back(rb, B, ag->per_td, st);
+      GCRL_CUDA(cudaMemcpyAsync(ag->many.td + size_t(i) * B, ag->per_td, size_t(B) * 4, cudaMemcpyDeviceToDevice, st));
     }
-    it = cache.emplace(std::move(key), g).first;
   }
-  launch_graph(it->second, st);
 }
 
 int many_path(const gcrl_agent *ag, int B) {
   return (ag->sample_buf != nullptr ? 1 : 0) | (fused_ok(ag, B) ? 2 : 0) | (ag->tc_update ? 4 : 0);
 }
 
-void run_many(gcrl_agent *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+// A prioritised call is captured when its key repeats only (see ManyGraphs::launch); a HER buffer has 0 for the
+// key's epoch and length.
+void run_many(gcrl_agent *ag, gcrl_her *her, gcrl_replay *rb, int B, int n, const int *flags, cudaStream_t st) {
   select_engine(ag, B, st);
-  launch_many(ag, {int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), many_path(ag, B), 0, 0},
-              true, [&](cudaStream_t cs) { run_many_body(ag, buf, B, n, flags, cs); }, st);
-}
-
-// n updates from a uniform / prioritised buffer: the slot's draw, the operand rows, the update and, prioritised, the
-// priority write-back and a copy of the TD errors into the update's row
-void run_many_replay_body(gcrl_agent *ag, gcrl_replay *buf, int B, int n, const int *flags, cudaStream_t st) {
-  for (int i = 0; i < n; ++i) {
-    ManySlot slot(ag, i, n, B);
-    replay_many_sample(buf, B, n, i, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->per_w, st);
-    if (!fused_ok(ag, B))
-      launch_ingest_batch(ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->D, ag->A, B, ag->sa, ag->nsa, ag->spi, ag->ldc,
-                          ag->br, ag->bd, st);
-    run_update_body(ag, B, ag->td3 ? ag->noise : nullptr, flags[i], PH_ALL, st);
-    if (ag->per_on) {
-      replay_many_write_back(buf, B, ag->per_td, st);
-      GCRL_CUDA(cudaMemcpyAsync(ag->many.td + size_t(i) * B, ag->per_td, size_t(B) * 4, cudaMemcpyDeviceToDevice, st));
-    }
-  }
-}
-
-void run_many_replay(gcrl_agent *ag, gcrl_replay *buf, int B, int n, const int *flags, cudaStream_t st) {
-  select_engine(ag, B, st);
-  launch_many(ag, {int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), many_path(ag, B),
-                   replay_epoch(buf), ag->per_on ? replay_many_n(buf) : 0},
-              !ag->per_on, [&](cudaStream_t cs) { run_many_replay_body(ag, buf, B, n, flags, cs); }, st);
+  const uintptr_t buf = rb != nullptr ? reinterpret_cast<uintptr_t>(rb) : reinterpret_cast<uintptr_t>(her);
+  ag->many.graphs.launch({int64_t(B), std::vector<int>(flags, flags + n), buf, many_path(ag, B),
+                          rb != nullptr ? replay_epoch(rb) : 0, ag->per_on ? replay_many_n(rb) : 0},
+                         !ag->per_on, [&](cudaStream_t cs) { run_many_body(ag, her, rb, B, n, flags, cs); }, st,
+                         ag->use_graphs, ag->cap_stream);
 }
 
 // The row-slab critic kernel draws the batch itself from `buf` (else the sampler is a launch of its own)
@@ -1058,6 +962,79 @@ static inline void require_handle(const gcrl_agent *h) {
   if (h->magic != 0x544E4741u) throw ::gcrl::Error(GCRL_ERR_INVALID, "handle is not a DDPG / TD3 agent (gcrl_agent_create)");
 }
 
+// gcrl_agent_update_many (HER buffer `her`) and gcrl_agent_update_many_replay (uniform / prioritised buffer `rb`): one
+// of the two is NULL.  Nothing moves before the last refusal: the buffer's own checks (replay_many_stage) come first.
+static void update_many(gcrl_agent *ag, gcrl_her *her, gcrl_replay *rb, int64_t B, int n, const int *flags,
+                        const int64_t *idx_host, const int64_t *pos_host, const double *u_host, const double *beta,
+                        const float *noise_dev, const double *lr_critic, const double *lr_actor, float *metrics_host,
+                        float *td_host, void *stream) {
+  require_handle(ag);
+  check_batch(ag, B);
+  GCRL_REQUIRE(her != nullptr || rb != nullptr, "buffer handle is NULL");
+  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
+  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
+  const bool per = rb != nullptr && replay_prioritized(rb);
+  for (int i = 0; i < n; ++i) {
+    if (her != nullptr) {
+      GCRL_REQUIRE((flags[i] & ~3) == 0, "flags of an n-update call may hold bit0 and bit1 only");
+    } else {
+      GCRL_REQUIRE((flags[i] & ~11) == 0, "flags of an n-update call from a replay buffer may hold bits 0, 1 and 3 only");
+      GCRL_REQUIRE(((flags[i] & 8) != 0) == per, "flags bit3 must be set exactly when the buffer is prioritised");
+    }
+  }
+  GCRL_REQUIRE(!ag->p2p.on, "n-update calls are not available under peer-memory data parallelism");
+  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
+  if (her != nullptr) {
+    GCRL_REQUIRE(her_state_dim(her) == ag->D && her_act_dim(her) == ag->A, "buffer / agent shape mismatch");
+    GCRL_REQUIRE(her_device(her) == ag->device, "buffer and agent live on different devices");
+  } else {
+    GCRL_REQUIRE(replay_state_dim(rb) == ag->D && replay_act_dim(rb) == ag->A, "buffer / agent shape mismatch");
+    GCRL_REQUIRE(replay_device(rb) == ag->device, "buffer and agent live on different devices");
+  }
+  GCRL_REQUIRE(!ag->td3 || noise_dev != nullptr, "TD3 update needs the [n, B, A] standard-normal noise tensor");
+  if (her != nullptr) {
+    const int64_t len = her_len(her);
+    if (len < B) throw Error(GCRL_ERR_UNDERFILLED, "[ERROR] Not enough in buffer to sample");
+    if (idx_host != nullptr)
+      for (int64_t i = 0; i < int64_t(n) * B; ++i)
+        if (idx_host[i] < 0 || idx_host[i] >= len) throw Error(GCRL_ERR_INVALID, "sample index out of range [0, len)");
+  }
+  GCRL_CUDA(cudaSetDevice(ag->device));
+  cudaStream_t st = as_stream(stream);
+  if (rb != nullptr) replay_many_stage(rb, B, n, pos_host, u_host, beta, st);
+  auto &mn = ag->many;
+  ensure_many(ag);
+  if (per && mn.td == nullptr) mn.td = dev_alloc<float>(size_t(GCRL_MAX_MANY_STEPS) * ag->maxB);
+  AdamStepGuard guard(ag);
+  if (her != nullptr) guard.keep_draws(her);
+  ag->per_on = per;
+  // every update's scalars (HER: the device stream's draw epochs in order), then every update's positions: ONE copy
+  const size_t scal = size_t(n) * kScalBytes, pos = idx_host != nullptr ? size_t(n) * B * sizeof(int64_t) : 0;
+  int slot;
+  char *p = ag->io_stage.acquire(scal + pos, &slot);
+  for (int i = 0; i < n; ++i) {
+    if (her != nullptr) ag->sample_sc = her_next_scalars(her, idx_host != nullptr);
+    fill_scalars(ag, lr_critic[i], lr_actor[i], (flags[i] & 1) != 0, her != nullptr ? ag->sample_sc : SampleScalars{},
+                 p + size_t(i) * kScalBytes);
+  }
+  if (pos) std::memcpy(p + scal, idx_host, pos);
+  GCRL_CUDA(cudaMemcpyAsync(mn.d, p, scal + pos, cudaMemcpyHostToDevice, st));
+  ag->io_stage.release(slot, st);
+  if (ag->td3)   // stable addresses for the captured graph
+    GCRL_CUDA(cudaMemcpyAsync(mn.noise, noise_dev, size_t(n) * B * ag->A * 4, cudaMemcpyDeviceToDevice, st));
+  ag->sample_buf = her != nullptr && samples_in_kernel(ag, her, B) ? her : nullptr;
+  run_many(ag, her, rb, int(B), n, flags, st);
+  ag->pub_valid = true;
+  guard.commit();
+  read_many_metrics(ag, n, metrics_host, st);
+  if (per && td_host != nullptr) {
+    // ONE read-back per call; to pageable memory the copy returns once it (and the updates before it) completed
+    std::vector<float> rows(size_t(n) * B);
+    GCRL_CUDA(cudaMemcpyAsync(rows.data(), mn.td, rows.size() * sizeof(float), cudaMemcpyDeviceToHost, st));
+    std::memcpy(td_host, rows.data(), rows.size() * sizeof(float));
+  }
+}
+
 extern "C" {
 
 int gcrl_agent_create(gcrl_agent **out, int device, const gcrl_agent_config *cfg) {
@@ -1130,8 +1107,7 @@ int gcrl_agent_create(gcrl_agent **out, int device, const gcrl_agent_config *cfg
     ag->fuse_sampler = !(nfs && nfs[0] == '1');
     ag->scal_stage.init(256);
     GCRL_CUDA(cudaStreamCreateWithFlags(&ag->cap_stream, cudaStreamNonBlocking));
-    const char *ng = getenv("GCRL_B200_NO_GRAPH");
-    ag->use_graphs = !(ng && ng[0] == '1');
+    ag->use_graphs = graphs_enabled();
     ag->io_stage.init(size_t(1) << 16);
     if (ag->cfg.precision >= 1) {
       tc_dense_init();
@@ -1152,7 +1128,7 @@ int gcrl_agent_destroy(gcrl_agent *ag) {
   cudaSetDevice(ag->device);
   cudaDeviceSynchronize();
   for (auto &kv : ag->graphs) cudaGraphExecDestroy(kv.second.exec);
-  for (auto &kv : ag->many.graphs) cudaGraphExecDestroy(kv.second.exec);
+  ag->many.graphs.clear();
   if (ag->many.d) cudaFree(ag->many.d);
   if (ag->many.noise) cudaFree(ag->many.noise);
   if (ag->many.h_pub) cudaFreeHost(ag->many.h_pub);
@@ -1396,47 +1372,8 @@ int gcrl_agent_update_many(gcrl_agent *ag, gcrl_her *buf, int64_t B, int n, cons
                            void *stream) {
   GCRL_API_BEGIN
   GCRL_NVTX("gcrl_agent_update_many");
-  require_handle(ag);
-  check_batch(ag, B);
-  GCRL_REQUIRE(buf != nullptr, "buffer handle is NULL");
-  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
-  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
-  for (int i = 0; i < n; ++i) GCRL_REQUIRE((flags[i] & ~3) == 0, "flags of an n-update call may hold bit0 and bit1 only");
-  GCRL_REQUIRE(!ag->p2p.on, "n-update calls are not available under peer-memory data parallelism");
-  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
-  GCRL_REQUIRE(her_state_dim(buf) == ag->D && her_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
-  GCRL_REQUIRE(her_device(buf) == ag->device, "buffer and agent live on different devices");
-  GCRL_REQUIRE(!ag->td3 || noise_dev != nullptr, "TD3 update needs the [n, B, A] standard-normal noise tensor");
-  const int64_t len = her_len(buf);
-  if (len < B) throw Error(GCRL_ERR_UNDERFILLED, "[ERROR] Not enough in buffer to sample");
-  if (idx_host != nullptr)
-    for (int64_t i = 0; i < int64_t(n) * B; ++i)
-      if (idx_host[i] < 0 || idx_host[i] >= len) throw Error(GCRL_ERR_INVALID, "sample index out of range [0, len)");
-  GCRL_CUDA(cudaSetDevice(ag->device));
-  cudaStream_t st = as_stream(stream);
-  auto &mn = ag->many;
-  ensure_many(ag);
-  AdamStepGuard guard(ag);
-  guard.keep_draws(buf);
-  ag->per_on = false;
-  // every update's scalars (the device stream's draw epochs in order), then every update's positions: ONE copy
-  const size_t scal = size_t(n) * kScalBytes, pos = idx_host != nullptr ? size_t(n) * B * sizeof(int64_t) : 0;
-  int slot;
-  char *p = ag->io_stage.acquire(scal + pos, &slot);
-  for (int i = 0; i < n; ++i) {
-    ag->sample_sc = her_next_scalars(buf, idx_host != nullptr);
-    fill_scalars(ag, lr_critic[i], lr_actor[i], (flags[i] & 1) != 0, ag->sample_sc, p + size_t(i) * kScalBytes);
-  }
-  if (pos) std::memcpy(p + scal, idx_host, pos);
-  GCRL_CUDA(cudaMemcpyAsync(mn.d, p, scal + pos, cudaMemcpyHostToDevice, st));
-  ag->io_stage.release(slot, st);
-  if (ag->td3)   // stable addresses for the captured graph
-    GCRL_CUDA(cudaMemcpyAsync(mn.noise, noise_dev, size_t(n) * B * ag->A * 4, cudaMemcpyDeviceToDevice, st));
-  ag->sample_buf = samples_in_kernel(ag, buf, B) ? buf : nullptr;
-  run_many(ag, buf, int(B), n, flags, st);
-  ag->pub_valid = true;
-  guard.commit();
-  read_many_metrics(ag, n, metrics_host, st);
+  update_many(ag, buf, nullptr, B, n, flags, idx_host, nullptr, nullptr, nullptr, noise_dev, lr_critic, lr_actor,
+              metrics_host, nullptr, stream);
   GCRL_API_END
 }
 
@@ -1446,48 +1383,8 @@ int gcrl_agent_update_many_replay(gcrl_agent *ag, gcrl_replay *buf, int64_t B, i
                                   float *metrics_host, float *td_host, void *stream) {
   GCRL_API_BEGIN
   GCRL_NVTX("gcrl_agent_update_many_replay");
-  require_handle(ag);
-  check_batch(ag, B);
-  GCRL_REQUIRE(buf != nullptr, "buffer handle is NULL");
-  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
-  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
-  const bool per = replay_prioritized(buf);
-  for (int i = 0; i < n; ++i) {
-    GCRL_REQUIRE((flags[i] & ~11) == 0, "flags of an n-update call from a replay buffer may hold bits 0, 1 and 3 only");
-    GCRL_REQUIRE(((flags[i] & 8) != 0) == per, "flags bit3 must be set exactly when the buffer is prioritised");
-  }
-  GCRL_REQUIRE(!ag->p2p.on, "n-update calls are not available under peer-memory data parallelism");
-  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
-  GCRL_REQUIRE(replay_state_dim(buf) == ag->D && replay_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
-  GCRL_REQUIRE(replay_device(buf) == ag->device, "buffer and agent live on different devices");
-  GCRL_REQUIRE(!ag->td3 || noise_dev != nullptr, "TD3 update needs the [n, B, A] standard-normal noise tensor");
-  GCRL_CUDA(cudaSetDevice(ag->device));
-  cudaStream_t st = as_stream(stream);
-  replay_many_stage(buf, B, n, pos_host, u_host, beta, st);      // the buffer's own checks come first
-  auto &mn = ag->many;
-  ensure_many(ag);
-  if (per && mn.td == nullptr) mn.td = dev_alloc<float>(size_t(GCRL_MAX_MANY_STEPS) * ag->maxB);
-  AdamStepGuard guard(ag);
-  ag->per_on = per;
-  int slot;
-  char *p = ag->io_stage.acquire(size_t(n) * kScalBytes, &slot);
-  for (int i = 0; i < n; ++i)
-    fill_scalars(ag, lr_critic[i], lr_actor[i], (flags[i] & 1) != 0, SampleScalars{}, p + size_t(i) * kScalBytes);
-  GCRL_CUDA(cudaMemcpyAsync(mn.d, p, size_t(n) * kScalBytes, cudaMemcpyHostToDevice, st));
-  ag->io_stage.release(slot, st);
-  if (ag->td3)   // stable addresses for the captured graph
-    GCRL_CUDA(cudaMemcpyAsync(mn.noise, noise_dev, size_t(n) * B * ag->A * 4, cudaMemcpyDeviceToDevice, st));
-  ag->sample_buf = nullptr;
-  run_many_replay(ag, buf, int(B), n, flags, st);
-  ag->pub_valid = true;
-  guard.commit();
-  read_many_metrics(ag, n, metrics_host, st);
-  if (per && td_host != nullptr) {
-    // ONE read-back per call; to pageable memory the copy returns once it (and the updates before it) completed
-    std::vector<float> rows(size_t(n) * B);
-    GCRL_CUDA(cudaMemcpyAsync(rows.data(), mn.td, rows.size() * sizeof(float), cudaMemcpyDeviceToHost, st));
-    std::memcpy(td_host, rows.data(), rows.size() * sizeof(float));
-  }
+  update_many(ag, nullptr, buf, B, n, flags, nullptr, pos_host, u_host, beta, noise_dev, lr_critic, lr_actor,
+              metrics_host, td_host, stream);
   GCRL_API_END
 }
 

@@ -1,5 +1,6 @@
-// Error plumbing, pinned staging ring, misc C-ABI entry points.
+// Error plumbing, pinned staging ring, CUDA-graph capture (graphs.cuh), misc C-ABI entry points.
 #include "common.cuh"
+#include "graphs.cuh"
 
 #include <atomic>
 #include <cstdlib>
@@ -73,6 +74,50 @@ char *PinnedRing::acquire(size_t bytes, int *slot) {
 void PinnedRing::release(int slot, cudaStream_t st) {
   GCRL_CUDA(cudaEventRecord(ev[slot], st));
   used[slot] = true;
+}
+
+bool graphs_enabled() {
+  const char *ng = getenv("GCRL_B200_NO_GRAPH");
+  return !(ng && ng[0] == '1');
+}
+
+void begin_capture(cudaStream_t cap) { GCRL_CUDA(cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal)); }
+
+GraphRec end_capture(cudaStream_t cap, uint64_t kernels) {
+  cudaGraph_t graph = nullptr;
+  GCRL_CUDA(cudaStreamEndCapture(cap, &graph));
+  count_launch(uint64_t(0) - kernels);
+  cudaGraphExec_t exec = nullptr;
+  const cudaError_t e = cudaGraphInstantiate(&exec, graph, 0);
+  cudaGraphDestroy(graph);
+  GCRL_CUDA(e);
+  return GraphRec{exec, kernels};
+}
+
+void abort_capture(cudaStream_t cap) {
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  cudaStreamIsCapturing(cap, &cs);
+  if (cs == cudaStreamCaptureStatusNone) return;
+  cudaGraph_t graph = nullptr;
+  cudaStreamEndCapture(cap, &graph);
+  if (graph) cudaGraphDestroy(graph);
+}
+
+GraphRec capture_graph(cudaStream_t cap, const std::function<void(cudaStream_t)> &body) {
+  const uint64_t before = launch_counter();
+  begin_capture(cap);
+  try {
+    body(cap);
+  } catch (...) {
+    abort_capture(cap);
+    throw;
+  }
+  return end_capture(cap, launch_counter() - before);
+}
+
+void launch_graph(const GraphRec &g, cudaStream_t st) {
+  GCRL_CUDA(cudaGraphLaunch(g.exec, st));
+  count_launch(g.kernels);
 }
 
 }  // namespace gcrl

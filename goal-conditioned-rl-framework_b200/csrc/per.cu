@@ -36,6 +36,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "graphs.cuh"
 
 namespace gcrl {
 namespace {
@@ -619,8 +620,7 @@ struct gcrl_replay {
       return n == o.n && B == o.B && std::memcmp(ptr, o.ptr, sizeof(ptr)) == 0;
     }
   } graph_key, last_key;
-  cudaGraphExec_t graph_exec = nullptr;
-  uint64_t graph_kernels = 0;
+  GraphRec graph{nullptr, 0};
   cudaStream_t cap_stream = nullptr;
   bool use_graphs = true;
   int n_leaves = 0, n_groups = 0;
@@ -651,7 +651,7 @@ void new_epoch(gcrl_replay *h) { h->epoch = ++g_epoch; }
 void ensure_batch(gcrl_replay *h, int64_t B, cudaStream_t st) {
   if (B <= h->batch_cap) return;
   GCRL_CUDA(cudaStreamSynchronize(st));
-  if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
+  if (h->graph.exec) { cudaGraphExecDestroy(h->graph.exec); h->graph.exec = nullptr; }
   new_epoch(h);
   for (void *p : {(void *)h->d_u, (void *)h->d_wraw, (void *)h->d_pos, (void *)h->d_slot})
     if (p) GCRL_CUDA(cudaFree(p));
@@ -698,7 +698,7 @@ void build_tree(gcrl_replay *h, int64_t n, cudaStream_t st) {
   const size_t need = size_t(L) + 2;
   if (need > h->tree_cap) {
     GCRL_CUDA(cudaStreamSynchronize(st));
-    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }   // it holds the old tables
+    if (h->graph.exec) { cudaGraphExecDestroy(h->graph.exec); h->graph.exec = nullptr; }   // it holds the old tables
     new_epoch(h);
     for (void *p : {(void *)h->d_leaf_off, (void *)h->d_node_l, (void *)h->d_node_r, (void *)h->d_vals})
       if (p) GCRL_CUDA(cudaFree(p));
@@ -905,10 +905,7 @@ int gcrl_replay_create(gcrl_replay **out, int device, int64_t capacity, int stat
       h->d_flags = dev_alloc<int>(1);
       h->d_call = dev_alloc<PerCall>(1);
       GCRL_CUDA(cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking));
-      {
-        const char *ng = getenv("GCRL_B200_NO_GRAPH");
-        h->use_graphs = !(ng && ng[0] == '1');
-      }
+      h->use_graphs = graphs_enabled();
       h->winner = dev_alloc<int>(size_t(capacity));
       fill_i32_kernel<<<blocks_for(capacity, 256 * 8), 256>>>(h->winner, capacity, -1);
       GCRL_LAUNCHED();
@@ -935,7 +932,7 @@ int gcrl_replay_destroy(gcrl_replay *h) {
                   (void *)h->d_leaf_off, (void *)h->d_node_l, (void *)h->d_node_r, (void *)h->d_group_off,
                   (void *)h->d_vals, (void *)h->d_u, (void *)h->d_wraw, (void *)h->d_pos, (void *)h->d_slot})
     if (p) cudaFree(p);
-  if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
+  if (h->graph.exec) cudaGraphExecDestroy(h->graph.exec);
   if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
   if (h->d_call) cudaFree(h->d_call);
   if (h->d_many) cudaFree(h->d_many);
@@ -1030,29 +1027,13 @@ int gcrl_replay_sample_prioritized(gcrl_replay *h, int64_t B, const double *u_ho
   key.n = n; key.B = B;
   const void *ptrs[6] = {s, a, r, ns, d, weights_dev};
   std::memcpy(key.ptr, ptrs, sizeof(ptrs));
-  if (h->use_graphs && h->graph_exec != nullptr && key == h->graph_key) {
-    GCRL_CUDA(cudaGraphLaunch(h->graph_exec, st));
-    count_launch(h->graph_kernels);
+  if (h->use_graphs && h->graph.exec != nullptr && key == h->graph_key) {
+    launch_graph(h->graph, st);
   } else if (h->use_graphs && key == h->last_key) {
-    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
-    cudaGraph_t graph = nullptr;
-    const uint64_t before = launch_counter();
-    GCRL_CUDA(cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeThreadLocal));
-    try {
-      launch_all(h->cap_stream);
-    } catch (...) {
-      cudaStreamEndCapture(h->cap_stream, &graph);
-      if (graph) cudaGraphDestroy(graph);
-      throw;
-    }
-    GCRL_CUDA(cudaStreamEndCapture(h->cap_stream, &graph));
-    h->graph_kernels = launch_counter() - before;          // recorded, not executed, by the capture
-    count_launch(uint64_t(0) - h->graph_kernels);
-    GCRL_CUDA(cudaGraphInstantiate(&h->graph_exec, graph, 0));
-    GCRL_CUDA(cudaGraphDestroy(graph));
+    if (h->graph.exec) { cudaGraphExecDestroy(h->graph.exec); h->graph.exec = nullptr; }
+    h->graph = capture_graph(h->cap_stream, launch_all);
     h->graph_key = key;
-    GCRL_CUDA(cudaGraphLaunch(h->graph_exec, st));
-    count_launch(h->graph_kernels);
+    launch_graph(h->graph, st);
   } else {
     launch_all(st);
   }

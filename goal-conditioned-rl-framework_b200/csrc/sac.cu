@@ -14,38 +14,13 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
-#include <functional>
 #include <map>
-#include <set>
 #include <tuple>
 #include <vector>
 
+#include "buffer_api.cuh"
+#include "graphs.cuh"
 #include "mlp.cuh"
-
-struct gcrl_her;
-namespace gcrl {
-void her_sample_into(gcrl_her *h, int64_t B, const int64_t *idx_host, float *s, float *a, float *r,
-                     float *ns, float *d, int64_t *idx_out, cudaStream_t st);
-int her_state_dim(const gcrl_her *h);
-int her_act_dim(const gcrl_her *h);
-int her_device(const gcrl_her *h);
-SampleScalars her_next_scalars(gcrl_her *h, bool positions_given);
-int64_t her_len(const gcrl_her *h);
-void her_sample_graphed(gcrl_her *h, int64_t B, const SampleScalars *sc_dev, const int64_t *idx_dev, float *s,
-                        float *a, float *r, float *ns, float *d, cudaStream_t st);
-unsigned long long &her_draw_epoch(gcrl_her *h);
-bool replay_prioritized(const gcrl_replay *h);
-int replay_state_dim(const gcrl_replay *h);
-int replay_act_dim(const gcrl_replay *h);
-int replay_device(const gcrl_replay *h);
-uint64_t replay_epoch(const gcrl_replay *h);
-int64_t replay_many_n(const gcrl_replay *h);
-void replay_many_stage(gcrl_replay *h, int64_t B, int n, const int64_t *pos_host, const double *u_host,
-                       const double *beta, cudaStream_t st);
-void replay_many_sample(gcrl_replay *h, int64_t B, int n, int i, float *s, float *a, float *r, float *ns, float *d,
-                        float *weights_dev, cudaStream_t st);
-void replay_many_write_back(gcrl_replay *h, int64_t B, const float *td_dev, cudaStream_t st);
-}  // namespace gcrl
 
 using namespace gcrl;
 
@@ -61,7 +36,6 @@ constexpr float kLogSqrt2Pi = 0.91893853320467274178f;
 constexpr int kMetricFloats = 36;         // the device metrics block [32], then the alpha state [4]
 // per-update scalars of an n-update call: critic / actor AdamW, alpha's AdamW, the sampler's totals and draw epoch
 constexpr size_t kManyScalBytes = 2 * sizeof(StepScalars) + sizeof(SampleScalars);
-constexpr size_t kManyGraphCache = 8;     // n-update graphs kept per agent (one flag pattern per run is typical)
 
 // ---- BatchNorm1d -----------------------------------------------------------------------------
 // One CTA per 32 feature columns, 32 x 32 threads: threadIdx.x = column (coalesced 128-byte row
@@ -751,7 +725,6 @@ struct gcrl_sac {
   bool tc_update = false;                        // the update being recorded / issued runs on the tensor-core engine
   bool use_graphs = true;
   cudaStream_t cap_stream = nullptr;             // capture-only stream (the caller's may be the legacy one)
-  struct GraphRec { cudaGraphExec_t exec; uint64_t kernels; };
   std::map<std::tuple<int, int, int>, GraphRec> graphs;   // (B, flags, phase mask)
   // n consecutive updates in one graph (gcrl_sac_update_many): everything a captured update reads that changes from
   // one update to the next has one slot per update, in one device allocation laid out for the call's (n, B):
@@ -762,14 +735,13 @@ struct gcrl_sac {
     size_t cap = 0;                              // bytes; growing it drops the cached graphs (their addresses move)
     // (B, flags of every update, buffer, engine path, buffer epoch, length drawn from): as in agent.cu
     using Key = std::tuple<int64_t, std::vector<int>, uintptr_t, int, uint64_t, int64_t>;
-    std::map<Key, GraphRec> graphs;
-    std::set<Key> seen;                          // keys issued eagerly once (prioritised: captured when one repeats)
+    ManyGraphs<Key> graphs;
   } many;
   // sync-BN (gcrl_sac_set_sync_bn): the update is cut into graph segments, each ending in the collective the caller
   // runs before the next one (gcrl_sac_update_segment)
   int sync_world = 0, sync_rank = 0;
   float *bn_gather = nullptr;                    // [world][2 ldh]: per-rank BatchNorm partial statistics
-  struct SegRec { cudaGraphExec_t exec; uint64_t kernels; int collective; };
+  struct SegRec { GraphRec graph; int collective; };
   std::map<std::tuple<int, int>, std::vector<SegRec>> seg_graphs;     // (B, flags)
   std::vector<SegRec> *seg_build = nullptr;      // the segment list being captured
   uint64_t seg_mark = 0;
@@ -814,16 +786,9 @@ enum : int { COLL_DONE = 0, COLL_GATHER_BN = 1, COLL_AVG_CRITIC = 2, COLL_AVG_AC
 
 // Close the graph segment being captured and open the next one.  Only the segmented capture reaches this.
 void seg_cut(gcrl_sac *ag, int collective, bool last = false) {
-  cudaGraph_t graph = nullptr;
-  GCRL_CUDA(cudaStreamEndCapture(ag->cap_stream, &graph));
-  const uint64_t now = launch_counter();
-  cudaGraphExec_t exec = nullptr;
-  const cudaError_t e = cudaGraphInstantiate(&exec, graph, 0);
-  cudaGraphDestroy(graph);
-  GCRL_CUDA(e);
-  ag->seg_build->push_back(gcrl_sac::SegRec{exec, now - ag->seg_mark, collective});
-  ag->seg_mark = now;
-  if (!last) GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
+  ag->seg_build->push_back(gcrl_sac::SegRec{end_capture(ag->cap_stream, launch_counter() - ag->seg_mark), collective});
+  ag->seg_mark = launch_counter();
+  if (!last) begin_capture(ag->cap_stream);
 }
 
 // ---- tensor-core engine (tcgen05, 3xTF32; precision >= 1) --------------------------------------------
@@ -1298,34 +1263,6 @@ void run_body(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     actor_update(ag, B, flags, mask == PH_ALL ? PH_ALL : (mask & (PH_AGRAD | PH_ASTEP)), st);
 }
 
-// Record `body` on the capture stream into an instantiated graph; the kernels it records are not counted as
-// launches until the graph is replayed.
-gcrl_sac::GraphRec capture_graph(gcrl_sac *ag, const std::function<void(cudaStream_t)> &body) {
-  cudaGraph_t graph = nullptr;
-  const uint64_t before = launch_counter();
-  GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
-  try {
-    body(ag->cap_stream);
-  } catch (...) {
-    cudaStreamEndCapture(ag->cap_stream, &graph);
-    if (graph) cudaGraphDestroy(graph);
-    throw;
-  }
-  GCRL_CUDA(cudaStreamEndCapture(ag->cap_stream, &graph));
-  const uint64_t kernels = launch_counter() - before;   // recorded, not executed, by the capture
-  count_launch(uint64_t(0) - kernels);
-  cudaGraphExec_t exec = nullptr;
-  const cudaError_t e = cudaGraphInstantiate(&exec, graph, 0);
-  cudaGraphDestroy(graph);
-  GCRL_CUDA(e);
-  return gcrl_sac::GraphRec{exec, kernels};
-}
-
-void launch_graph(const gcrl_sac::GraphRec &g, cudaStream_t st) {
-  GCRL_CUDA(cudaGraphLaunch(g.exec, st));
-  count_launch(g.kernels);
-}
-
 // the engine an update at this batch runs on; the tensor-core one needs the split weight copies current
 void select_engine(gcrl_sac *ag, int B, cudaStream_t st) {
   ag->tc_update = engine_tc(ag, B);
@@ -1346,7 +1283,7 @@ void run_phases(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   const auto key = std::make_tuple(B, flags, mask);
   auto it = ag->graphs.find(key);
   if (it == ag->graphs.end())
-    it = ag->graphs.emplace(key, capture_graph(ag, [&](cudaStream_t cs) { run_body(ag, B, flags, mask, cs); })).first;
+    it = ag->graphs.emplace(key, capture_graph(ag->cap_stream, [&](cudaStream_t cs) { run_body(ag, B, flags, mask, cs); })).first;
   launch_graph(it->second, st);
 }
 
@@ -1388,78 +1325,37 @@ struct ManySlot {
   ManySlot &operator=(const ManySlot &) = delete;
 };
 
-// n updates from `buf` back to back: sampler, operand rows, the update, then its metrics and alpha state into the
-// slot's row (a copy node, not a launch)
-void run_many_body(gcrl_sac *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
+// n updates back to back from the HER buffer `her` or the uniform / prioritised buffer `rb` (the other is NULL): the
+// slot's draw, operand rows, the update, then -- prioritised -- the priority write-back and the TD errors into the
+// slot's row, and the metrics and alpha state into the slot's row (copy nodes, not launches)
+void run_many_body(gcrl_sac *ag, gcrl_her *her, gcrl_replay *rb, int B, int n, const int *flags, cudaStream_t st) {
   for (int i = 0; i < n; ++i) {
     ManySlot slot(ag, i, n, B);
-    her_sample_graphed(buf, B, slot.ssc, slot.idx, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, st);
-    launch_ingest_batch(ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->D, ag->A, B, ag->sa, ag->nsa, ag->spi, ag->ldc,
-                        ag->br, ag->bd, st);
-    run_body(ag, B, flags[i], PH_ALL, st);
-    GCRL_CUDA(cudaMemcpyAsync(slot.metrics, ag->mdev, kMetricFloats * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  }
-}
-
-// Replay the n-update graph of `key`, capturing it first when it is new -- or, with capture_new false, only when
-// the key was issued before (a key seen for the first time is issued eagerly: a prioritised buffer that is still
-// filling draws from a new length every call, and its graphs would never be replayed).
-void launch_many(gcrl_sac *ag, gcrl_sac::Many::Key key, bool capture_new, const std::function<void(cudaStream_t)> &body,
-                 cudaStream_t st) {
-  if (!ag->use_graphs) {
-    body(st);
-    return;
-  }
-  auto &cache = ag->many.graphs;
-  auto it = cache.find(key);
-  if (it == cache.end() && !capture_new && ag->many.seen.count(key) == 0) {
-    if (ag->many.seen.size() >= 2 * kManyGraphCache) ag->many.seen.clear();
-    ag->many.seen.insert(std::move(key));
-    body(st);
-    return;
-  }
-  if (it == cache.end()) {
-    const gcrl_sac::GraphRec g = capture_graph(ag, body);
-    if (cache.size() >= kManyGraphCache) {     // a replay still in flight is released when it completes
-      for (auto &kv : cache) cudaGraphExecDestroy(kv.second.exec);
-      cache.clear();
-    }
-    it = cache.emplace(std::move(key), g).first;
-  }
-  launch_graph(it->second, st);
-}
-
-void run_many(gcrl_sac *ag, gcrl_her *buf, int B, int n, const int *flags, cudaStream_t st) {
-  select_engine(ag, B, st);
-  ag->per_on = false;
-  launch_many(ag, {int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), ag->tc_update ? 1 : 0,
-                   0, 0},
-              true, [&](cudaStream_t cs) { run_many_body(ag, buf, B, n, flags, cs); }, st);
-}
-
-// n updates from a uniform / prioritised buffer: the slot's draw, operand rows, the update, then -- prioritised -- the
-// priority write-back and the TD errors into the slot's row, and the metrics into the slot's row
-void run_many_replay_body(gcrl_sac *ag, gcrl_replay *buf, int B, int n, const int *flags, cudaStream_t st) {
-  for (int i = 0; i < n; ++i) {
-    ManySlot slot(ag, i, n, B);
-    replay_many_sample(buf, B, n, i, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->per_w, st);
+    if (rb != nullptr)
+      replay_many_sample(rb, B, n, i, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->per_w, st);
+    else
+      her_sample_graphed(her, B, slot.ssc, slot.idx, ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, st);
     launch_ingest_batch(ag->bs, ag->ba, ag->br0, ag->bns, ag->bd0, ag->D, ag->A, B, ag->sa, ag->nsa, ag->spi, ag->ldc,
                         ag->br, ag->bd, st);
     run_body(ag, B, flags[i], PH_ALL, st);
     if (ag->per_on) {
-      replay_many_write_back(buf, B, ag->per_td, st);
+      replay_many_write_back(rb, B, ag->per_td, st);
       GCRL_CUDA(cudaMemcpyAsync(slot.td, ag->per_td, size_t(B) * sizeof(float), cudaMemcpyDeviceToDevice, st));
     }
     GCRL_CUDA(cudaMemcpyAsync(slot.metrics, ag->mdev, kMetricFloats * sizeof(float), cudaMemcpyDeviceToDevice, st));
   }
 }
 
-void run_many_replay(gcrl_sac *ag, gcrl_replay *buf, int B, int n, const int *flags, cudaStream_t st) {
+// A prioritised call is captured when its key repeats only (see ManyGraphs::launch); a HER buffer has 0 for the
+// key's epoch and length.
+void run_many(gcrl_sac *ag, gcrl_her *her, gcrl_replay *rb, int B, int n, const int *flags, cudaStream_t st) {
   select_engine(ag, B, st);
-  ag->per_on = replay_prioritized(buf);
-  launch_many(ag, {int64_t(B), std::vector<int>(flags, flags + n), reinterpret_cast<uintptr_t>(buf), ag->tc_update ? 1 : 0,
-                   replay_epoch(buf), ag->per_on ? replay_many_n(buf) : 0},
-              !ag->per_on, [&](cudaStream_t cs) { run_many_replay_body(ag, buf, B, n, flags, cs); }, st);
+  ag->per_on = rb != nullptr && replay_prioritized(rb);
+  const uintptr_t buf = rb != nullptr ? reinterpret_cast<uintptr_t>(rb) : reinterpret_cast<uintptr_t>(her);
+  ag->many.graphs.launch({int64_t(B), std::vector<int>(flags, flags + n), buf, ag->tc_update ? 1 : 0,
+                          rb != nullptr ? replay_epoch(rb) : 0, ag->per_on ? replay_many_n(rb) : 0},
+                         !ag->per_on, [&](cudaStream_t cs) { run_many_body(ag, her, rb, B, n, flags, cs); }, st,
+                         ag->use_graphs, ag->cap_stream);
 }
 
 // Segmented update (sync-BN): the body is captured ONCE per (B, flags) as a chain of graphs, cut wherever a
@@ -1474,34 +1370,25 @@ int run_segment(gcrl_sac *ag, int B, int flags, int seg, cudaStream_t st) {
   auto it = ag->seg_graphs.find(key);
   if (it == ag->seg_graphs.end()) {
     std::vector<gcrl_sac::SegRec> segs;
-    const uint64_t before = launch_counter();
     ag->seg_build = &segs;
-    ag->seg_mark = before;
-    GCRL_CUDA(cudaStreamBeginCapture(ag->cap_stream, cudaStreamCaptureModeThreadLocal));
+    ag->seg_mark = launch_counter();
+    begin_capture(ag->cap_stream);
     try {
       run_body(ag, B, flags, PH_SEGMENTED, ag->cap_stream);
       seg_cut(ag, COLL_DONE, true);
     } catch (...) {
-      cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-      cudaStreamIsCapturing(ag->cap_stream, &cs);
-      if (cs != cudaStreamCaptureStatusNone) {
-        cudaGraph_t g = nullptr;
-        cudaStreamEndCapture(ag->cap_stream, &g);
-        if (g) cudaGraphDestroy(g);
-      }
-      for (auto &r : segs) cudaGraphExecDestroy(r.exec);
+      abort_capture(ag->cap_stream);
+      for (auto &r : segs) cudaGraphExecDestroy(r.graph.exec);
       ag->seg_build = nullptr;
-      count_launch(before - launch_counter());
+      count_launch(ag->seg_mark - launch_counter());     // what the open segment recorded (each cut took its own)
       throw;
     }
     ag->seg_build = nullptr;
-    count_launch(before - launch_counter());              // recorded, not executed, by the capture
     it = ag->seg_graphs.emplace(key, std::move(segs)).first;
   }
   GCRL_REQUIRE(seg >= 0 && seg < int(it->second.size()), "segment index past the end of the update");
   const auto &r = it->second[size_t(seg)];
-  GCRL_CUDA(cudaGraphLaunch(r.exec, st));
-  count_launch(r.kernels);
+  launch_graph(r.graph, st);
   return r.collective;
 }
 
@@ -1642,8 +1529,7 @@ void ensure_many(gcrl_sac *ag, int n, int64_t B) {
   auto &mn = ag->many;
   const size_t need = many_bytes(ag, n, B);
   if (need <= mn.cap) return;
-  for (auto &kv : mn.graphs) cudaGraphExecDestroy(kv.second.exec);   // cudaFree waits for replays still reading them
-  mn.graphs.clear();
+  mn.graphs.clear();   // cudaFree waits for replays still reading them
   if (mn.d) GCRL_CUDA(cudaFree(mn.d));
   mn.d = nullptr;
   mn.cap = 0;
@@ -1701,6 +1587,71 @@ void actor_linear_geom(const gcrl_sac *ag, int layer, int *rows, int *cols, int 
 static inline void require_handle(const gcrl_sac *h) {
   if (h == nullptr) throw ::gcrl::Error(GCRL_ERR_INVALID, "handle is NULL");
   if (h->magic != 0x54434153u) throw ::gcrl::Error(GCRL_ERR_INVALID, "handle is not a SAC / TQC agent (gcrl_sac_create)");
+}
+
+// gcrl_sac_update_many (HER buffer `her`) and gcrl_sac_update_many_replay (uniform / prioritised buffer `rb`): one of
+// the two is NULL.  Nothing moves before the last refusal: the buffer's own checks (replay_many_stage) come first.
+static void update_many(gcrl_sac *ag, gcrl_her *her, gcrl_replay *rb, int64_t B, int n, const int *flags,
+                        const int64_t *idx_host, const int64_t *pos_host, const double *u_host, const double *beta,
+                        const float *eps_next_dev, const float *eps_cur_dev, const double *lr_critic,
+                        const double *lr_actor, float *metrics_host, float *td_host, void *stream) {
+  require_handle(ag);
+  GCRL_REQUIRE(her != nullptr || rb != nullptr, "buffer handle is NULL");
+  GCRL_REQUIRE(B >= 2 && B <= ag->maxB, "batch size outside [2, max_batch] (BatchNorm needs > 1 row)");
+  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
+  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
+  const bool per = rb != nullptr && replay_prioritized(rb);
+  bool any_actor = false;
+  for (int i = 0; i < n; ++i) {
+    if (her != nullptr) {
+      GCRL_REQUIRE((flags[i] & ~7) == 0, "flags of an n-update call may hold bits 0-2 only");
+    } else {
+      GCRL_REQUIRE((flags[i] & ~15) == 0, "flags of an n-update call from a replay buffer may hold bits 0-3 only");
+      GCRL_REQUIRE(((flags[i] & 8) != 0) == per, "flags bit3 must be set exactly when the buffer is prioritised");
+    }
+    any_actor = any_actor || (flags[i] & 1) != 0;
+  }
+  GCRL_REQUIRE(eps_next_dev != nullptr && (eps_cur_dev != nullptr || !any_actor), "NULL rsample noise tensor");
+  GCRL_REQUIRE(ag->sync_world == 0, "a sync-BN agent trains through gcrl_sac_update_segment only");
+  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
+  if (her != nullptr) {
+    GCRL_REQUIRE(her_state_dim(her) == ag->D && her_act_dim(her) == ag->A, "buffer / agent shape mismatch");
+    GCRL_REQUIRE(her_device(her) == ag->device, "buffer and agent live on different devices");
+    const int64_t len = her_len(her);
+    if (len < B) throw Error(GCRL_ERR_UNDERFILLED, "[ERROR] Not enough in buffer to sample");
+    if (idx_host != nullptr)
+      for (int64_t i = 0; i < int64_t(n) * B; ++i)
+        if (idx_host[i] < 0 || idx_host[i] >= len) throw Error(GCRL_ERR_INVALID, "sample index out of range [0, len)");
+  } else {
+    GCRL_REQUIRE(replay_state_dim(rb) == ag->D && replay_act_dim(rb) == ag->A, "buffer / agent shape mismatch");
+    GCRL_REQUIRE(replay_device(rb) == ag->device, "buffer and agent live on different devices");
+  }
+  GCRL_CUDA(cudaSetDevice(ag->device));
+  cudaStream_t st = as_stream(stream);
+  if (rb != nullptr) replay_many_stage(rb, B, n, pos_host, u_host, beta, st);
+  ensure_many(ag, n, B);
+  StepCounterGuard guard(ag);
+  if (her != nullptr) guard.keep_draws(her);
+  // every update's scalars (HER: the device stream's draw epochs in order), then every update's positions: ONE copy
+  const size_t scal = size_t(n) * kManyScalBytes, pos = idx_host != nullptr ? size_t(n) * B * sizeof(int64_t) : 0;
+  int slot;
+  char *p = ag->io_stage.acquire(scal + pos, &slot);
+  for (int i = 0; i < n; ++i) {
+    char *s = p + size_t(i) * kManyScalBytes;
+    fill_scalars(ag, lr_critic[i], lr_actor[i], flags[i], reinterpret_cast<StepScalars *>(s));
+    const SampleScalars ss = her != nullptr ? her_next_scalars(her, idx_host != nullptr) : SampleScalars{};
+    std::memcpy(s + 2 * sizeof(StepScalars), &ss, sizeof(SampleScalars));
+  }
+  if (pos) std::memcpy(p + scal, idx_host, pos);
+  GCRL_CUDA(cudaMemcpyAsync(ag->many.d, p, scal + pos, cudaMemcpyHostToDevice, st));
+  ag->io_stage.release(slot, st);
+  // stable addresses for the captured graph
+  const size_t noise = size_t(n) * B * ag->A * sizeof(float);
+  GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 0), eps_next_dev, noise, cudaMemcpyDeviceToDevice, st));
+  if (any_actor) GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 1), eps_cur_dev, noise, cudaMemcpyDeviceToDevice, st));
+  run_many(ag, her, rb, int(B), n, flags, st);
+  guard.commit();
+  read_many_rows(ag, n, B, flags, metrics_host, per ? td_host : nullptr, st);
 }
 
 extern "C" {
@@ -1767,8 +1718,7 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
       }
     }
     GCRL_CUDA(cudaStreamCreateWithFlags(&ag->cap_stream, cudaStreamNonBlocking));
-    const char *ng = getenv("GCRL_B200_NO_GRAPH");
-    ag->use_graphs = !(ng && ng[0] == '1');
+    ag->use_graphs = graphs_enabled();
     ag->scal_stage.init(256);
     ag->io_stage.init(size_t(1) << 16);
   } catch (...) {
@@ -1795,9 +1745,9 @@ int gcrl_sac_destroy(gcrl_sac *ag) {
                    ag->critic_grads, ag->per_w, ag->per_td})
     if (p) cudaFree(p);
   for (auto &kv : ag->graphs) cudaGraphExecDestroy(kv.second.exec);
-  for (auto &kv : ag->many.graphs) cudaGraphExecDestroy(kv.second.exec);
+  ag->many.graphs.clear();
   if (ag->many.d) cudaFree(ag->many.d);
-  for (auto &kv : ag->seg_graphs) for (auto &r : kv.second) cudaGraphExecDestroy(r.exec);
+  for (auto &kv : ag->seg_graphs) for (auto &r : kv.second) cudaGraphExecDestroy(r.graph.exec);
   if (ag->bn_gather) cudaFree(ag->bn_gather);
   if (ag->cap_stream) cudaStreamDestroy(ag->cap_stream);
   cudaFree(ag->d_scalars);
@@ -1953,52 +1903,8 @@ int gcrl_sac_update_many(gcrl_sac *ag, gcrl_her *buf, int64_t B, int n, const in
                          const double *lr_actor, float *metrics_host, void *stream) {
   GCRL_API_BEGIN
   GCRL_NVTX("gcrl_sac_update_many");
-  require_handle(ag);
-  GCRL_REQUIRE(buf != nullptr, "buffer handle is NULL");
-  GCRL_REQUIRE(B >= 2 && B <= ag->maxB, "batch size outside [2, max_batch] (BatchNorm needs > 1 row)");
-  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
-  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
-  bool any_actor = false;
-  for (int i = 0; i < n; ++i) {
-    GCRL_REQUIRE((flags[i] & ~7) == 0, "flags of an n-update call may hold bits 0-2 only");
-    any_actor = any_actor || (flags[i] & 1) != 0;
-  }
-  GCRL_REQUIRE(eps_next_dev != nullptr && (eps_cur_dev != nullptr || !any_actor), "NULL rsample noise tensor");
-  GCRL_REQUIRE(ag->sync_world == 0, "a sync-BN agent trains through gcrl_sac_update_segment only");
-  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
-  GCRL_REQUIRE(her_state_dim(buf) == ag->D && her_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
-  GCRL_REQUIRE(her_device(buf) == ag->device, "buffer and agent live on different devices");
-  const int64_t len = her_len(buf);
-  if (len < B) throw Error(GCRL_ERR_UNDERFILLED, "[ERROR] Not enough in buffer to sample");
-  if (idx_host != nullptr)
-    for (int64_t i = 0; i < int64_t(n) * B; ++i)
-      if (idx_host[i] < 0 || idx_host[i] >= len) throw Error(GCRL_ERR_INVALID, "sample index out of range [0, len)");
-  GCRL_CUDA(cudaSetDevice(ag->device));
-  cudaStream_t st = as_stream(stream);
-  auto &mn = ag->many;
-  ensure_many(ag, n, B);
-  StepCounterGuard guard(ag);
-  guard.keep_draws(buf);
-  // every update's scalars (the device stream's draw epochs in order), then every update's positions: ONE copy
-  const size_t scal = size_t(n) * kManyScalBytes, pos = idx_host != nullptr ? size_t(n) * B * sizeof(int64_t) : 0;
-  int slot;
-  char *p = ag->io_stage.acquire(scal + pos, &slot);
-  for (int i = 0; i < n; ++i) {
-    char *s = p + size_t(i) * kManyScalBytes;
-    fill_scalars(ag, lr_critic[i], lr_actor[i], flags[i], reinterpret_cast<StepScalars *>(s));
-    const SampleScalars ss = her_next_scalars(buf, idx_host != nullptr);
-    std::memcpy(s + 2 * sizeof(StepScalars), &ss, sizeof(SampleScalars));
-  }
-  if (pos) std::memcpy(p + scal, idx_host, pos);
-  GCRL_CUDA(cudaMemcpyAsync(mn.d, p, scal + pos, cudaMemcpyHostToDevice, st));
-  ag->io_stage.release(slot, st);
-  // stable addresses for the captured graph
-  const size_t noise = size_t(n) * B * ag->A * sizeof(float);
-  GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 0), eps_next_dev, noise, cudaMemcpyDeviceToDevice, st));
-  if (any_actor) GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 1), eps_cur_dev, noise, cudaMemcpyDeviceToDevice, st));
-  run_many(ag, buf, int(B), n, flags, st);
-  guard.commit();
-  read_many_rows(ag, n, B, flags, metrics_host, nullptr, st);
+  update_many(ag, buf, nullptr, B, n, flags, idx_host, nullptr, nullptr, nullptr, eps_next_dev, eps_cur_dev, lr_critic,
+              lr_actor, metrics_host, nullptr, stream);
   GCRL_API_END
 }
 
@@ -2008,44 +1914,8 @@ int gcrl_sac_update_many_replay(gcrl_sac *ag, gcrl_replay *buf, int64_t B, int n
                                 const double *lr_actor, float *metrics_host, float *td_host, void *stream) {
   GCRL_API_BEGIN
   GCRL_NVTX("gcrl_sac_update_many_replay");
-  require_handle(ag);
-  GCRL_REQUIRE(buf != nullptr, "buffer handle is NULL");
-  GCRL_REQUIRE(B >= 2 && B <= ag->maxB, "batch size outside [2, max_batch] (BatchNorm needs > 1 row)");
-  GCRL_REQUIRE(n >= 1 && n <= GCRL_MAX_MANY_STEPS, "n must be in [1, GCRL_MAX_MANY_STEPS]");
-  GCRL_REQUIRE(flags != nullptr && lr_critic != nullptr && lr_actor != nullptr, "NULL flags / learning rates");
-  const bool per = replay_prioritized(buf);
-  bool any_actor = false;
-  for (int i = 0; i < n; ++i) {
-    GCRL_REQUIRE((flags[i] & ~15) == 0, "flags of an n-update call from a replay buffer may hold bits 0-3 only");
-    GCRL_REQUIRE(((flags[i] & 8) != 0) == per, "flags bit3 must be set exactly when the buffer is prioritised");
-    any_actor = any_actor || (flags[i] & 1) != 0;
-  }
-  GCRL_REQUIRE(eps_next_dev != nullptr && (eps_cur_dev != nullptr || !any_actor), "NULL rsample noise tensor");
-  GCRL_REQUIRE(ag->sync_world == 0, "a sync-BN agent trains through gcrl_sac_update_segment only");
-  GCRL_REQUIRE(!ag->dp_open, "a phase-wise data-parallel update is open (phase 3 not issued)");
-  GCRL_REQUIRE(replay_state_dim(buf) == ag->D && replay_act_dim(buf) == ag->A, "buffer / agent shape mismatch");
-  GCRL_REQUIRE(replay_device(buf) == ag->device, "buffer and agent live on different devices");
-  GCRL_CUDA(cudaSetDevice(ag->device));
-  cudaStream_t st = as_stream(stream);
-  replay_many_stage(buf, B, n, pos_host, u_host, beta, st);      // the buffer's own checks come first
-  ensure_many(ag, n, B);
-  StepCounterGuard guard(ag);
-  int slot;
-  char *p = ag->io_stage.acquire(size_t(n) * kManyScalBytes, &slot);
-  for (int i = 0; i < n; ++i) {
-    char *s = p + size_t(i) * kManyScalBytes;
-    fill_scalars(ag, lr_critic[i], lr_actor[i], flags[i], reinterpret_cast<StepScalars *>(s));
-    std::memset(s + 2 * sizeof(StepScalars), 0, sizeof(SampleScalars));
-  }
-  GCRL_CUDA(cudaMemcpyAsync(ag->many.d, p, size_t(n) * kManyScalBytes, cudaMemcpyHostToDevice, st));
-  ag->io_stage.release(slot, st);
-  // stable addresses for the captured graph
-  const size_t noise = size_t(n) * B * ag->A * sizeof(float);
-  GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 0), eps_next_dev, noise, cudaMemcpyDeviceToDevice, st));
-  if (any_actor) GCRL_CUDA(cudaMemcpyAsync(many_eps(ag, n, B, 1), eps_cur_dev, noise, cudaMemcpyDeviceToDevice, st));
-  run_many_replay(ag, buf, int(B), n, flags, st);
-  guard.commit();
-  read_many_rows(ag, n, B, flags, metrics_host, per ? td_host : nullptr, st);
+  update_many(ag, nullptr, buf, B, n, flags, nullptr, pos_host, u_host, beta, eps_next_dev, eps_cur_dev, lr_critic,
+              lr_actor, metrics_host, td_host, stream);
   GCRL_API_END
 }
 
@@ -2069,7 +1939,7 @@ int gcrl_sac_set_sync_bn(gcrl_sac *ag, int world, int rank) {
                "need 0 <= world <= 1024 and 0 <= rank < world (world 0 switches sync-BN off)");
   GCRL_CUDA(cudaSetDevice(ag->device));
   GCRL_CUDA(cudaDeviceSynchronize());
-  for (auto &kv : ag->seg_graphs) for (auto &r : kv.second) cudaGraphExecDestroy(r.exec);
+  for (auto &kv : ag->seg_graphs) for (auto &r : kv.second) cudaGraphExecDestroy(r.graph.exec);
   ag->seg_graphs.clear();
   if (ag->bn_gather) { cudaFree(ag->bn_gather); ag->bn_gather = nullptr; }
   ag->sync_world = world; ag->sync_rank = world > 0 ? rank : 0;

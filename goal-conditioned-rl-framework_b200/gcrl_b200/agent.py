@@ -544,7 +544,12 @@ class _AgentBase:
         return [float(x) for x in self._metrics]
 
     # -- a training cycle's gradient steps in one call ---------------------------------------------------
-    _MANY_IN_ONE_GRAPH = False      # n updates replay as one CUDA graph (every agent sets it)
+    # What the family's n-update calls take: their C functions (HER buffer, REPLAY / PER buffer), the metric floats of
+    # an update, the smallest batch, and (SAC / TQC) the BatchNorm batches an update counts without / with an actor step
+    _MANY_FNS = ("gcrl_agent_update_many", "gcrl_agent_update_many_replay")
+    _METRIC_WIDTH = 8
+    _MIN_BATCH = 1
+    _BN_BATCHES = None
 
     def update_many(self, steps):
         """``[self.update(s) for s in steps]``: the same tuples, and afterwards the same state of every network,
@@ -559,16 +564,17 @@ class _AgentBase:
         wrote; while the ring is still filling, each call issues its updates without a graph.  Both data-parallel
         modes run the loop."""
         steps = [int(s) for s in steps]
-        if not (self._MANY_IN_ONE_GRAPH and self._dp is None and getattr(self, "_peer_dp", None) is None):
+        if self._dp is not None or getattr(self, "_peer_dp", None) is not None:
             return [self.update(s) for s in steps]
-        chunk = self._update_chunk if isinstance(self.buffer, HERBuffer) else self._update_chunk_replay
         out = []
         for lo in range(0, len(steps), MAX_MANY_STEPS):
-            out += chunk(steps[lo:lo + MAX_MANY_STEPS])
+            out += self._update_chunk(steps[lo:lo + MAX_MANY_STEPS])
         return out
 
-    def _many_noise(self, B, n):
-        return None
+    def _many_noise(self, B, flags):
+        """The device noise update() draws for each of these updates, in step order: the tensors the n-update call
+        takes (None: a NULL pointer)."""
+        return (None,)
 
     def _step_schedules(self, flags):
         """The learning rates of n updates with these flags: the schedules step as update() steps them.  Returns
@@ -587,76 +593,59 @@ class _AgentBase:
         for sch, (epoch, lr) in zip((self.critic_scheduler, self.actor_scheduler), saved):
             sch.last_epoch, sch.lr = epoch, lr
 
-    def _check_replay_chunk(self, B, min_batch=1):
-        """What update() checks from a REPLAY / PER buffer, before any generator is touched."""
-        assert len(self.buffer) >= B, "Not enough in buffer to sample"
-        if not min_batch <= B <= self._max_batch:
-            raise ValueError(f"batch size {B} outside [{min_batch}, max_batch = {self._max_batch}]")
-
-    def _replay_draws(self, B, steps):
-        """update()'s host draws from a REPLAY / PER buffer for every step, in step order: the positions
-        ``random.sample(range(len), B)`` (REPLAY), or the uniforms ``np.random.random_sample(B)`` and the beta each
-        draw uses -- the one beta_scheduler(step) left after the update before (PER).  Returns (flags bit3,
-        positions, uniforms, betas); the arrays not used are None."""
-        if isinstance(self.buffer, PERBuffer):
-            u = np.stack([np.random.random_sample(B) for _ in steps])
-            betas, beta = [], self.beta
-            for s in steps:
-                betas.append(beta)
-                beta = self._beta_at(s)
-            return 8, None, u, np.array(betas, np.float64)
-        nlen = len(self.buffer)
-        return 0, np.stack([_lib.py_sample_range(nlen, B) for _ in steps]), None, None
-
-    def _update_chunk_replay(self, steps):
-        B, n = self.batch_size, len(steps)
-        self._check_replay_chunk(B)
-        noise = self._many_noise(B, n)
-        per, pos, u, beta = self._replay_draws(B, steps)
-        flags = (C.c_int * n)(*(self._flags(s) | per for s in steps))
-        lr_c, lr_a, saved = self._step_schedules(flags)
-        metrics = np.empty((n, 8), np.float32)
-        td = np.empty((n, B), np.float32) if per else None
-        try:
-            check(lib.gcrl_agent_update_many_replay(
-                self._h, self.buffer.handle, B, n, flags, *(None if x is None else np_ptr(x) for x in (pos, u, beta)),
-                vp(noise.data_ptr()) if noise is not None else None, lr_c, lr_a, np_ptr(metrics),
-                np_ptr(td) if per else None, self._stream()))
-        except BaseException:
-            self._restore_schedules(saved)
-            raise
-        out = []
-        for i, (step, m) in enumerate(zip(steps, metrics.tolist())):
-            self._last_td = td[i].reshape(B, 1) if per else None
-            self.beta_scheduler(step)
-            out.append(self._result(step, m))
-        return out
-
     def _update_chunk(self, steps):
+        """Up to MAX_MANY_STEPS updates in one C call.  update()'s host draws for every step are made up front, each
+        generator in step order: the noise, then the positions ``random.sample(range(len), B)`` (REPLAY, HER with the
+        host index stream) or the uniforms ``np.random.random_sample(B)`` and the beta each draw uses -- the one
+        beta_scheduler(step) left after the update before (PER)."""
         B, n = self.batch_size, len(steps)
-        assert len(self.buffer) >= B, "[ERROR] Not enough in buffer to sample"       # before any state moves
-        if B > self._max_batch:
-            raise ValueError(f"batch size {B} above max_batch {self._max_batch}")
-        noise = self._many_noise(B, n)
-        iptr = None
-        if self.index_source == "host":             # n draws of random.sample(range(len), B), in step order
-            self._pre = self._known_state = None
+        her, per = isinstance(self.buffer, HERBuffer), isinstance(self.buffer, PERBuffer)
+        # what update() checks, before any generator is touched
+        assert len(self.buffer) >= B, ("[ERROR] " if her else "") + "Not enough in buffer to sample"
+        if not self._MIN_BATCH <= B <= self._max_batch:
+            raise ValueError(f"batch size {B} outside [{self._MIN_BATCH}, max_batch = {self._max_batch}]")
+        flags = [self._flags(s) | (8 if per else 0) for s in steps]
+        noise = self._many_noise(B, flags)       # referenced until the call has copied it
+        pos = u = beta = None
+        if per:
+            u = np.stack([np.random.random_sample(B) for _ in steps])
+            betas, b = [], self.beta
+            for s in steps:
+                betas.append(b)
+                b = self._beta_at(s)
+            beta = np.array(betas, np.float64)
+        elif not her or self.index_source == "host":
+            self._pre = self._known_state = None        # the host index stream's pre-drawn positions are stale
             nlen = len(self.buffer)
-            idx = np.stack([_lib.py_sample_range(nlen, B) for _ in steps])
-            iptr = np_ptr(idx)
-        flags = (C.c_int * n)(*(self._flags(s) for s in steps))
+            pos = np.stack([_lib.py_sample_range(nlen, B) for _ in steps])
+        cflags = (C.c_int * n)(*flags)
         lr_c, lr_a, saved = self._step_schedules(flags)
-        metrics = np.empty((n, 8), np.float32)
+        metrics = np.empty((n, self._METRIC_WIDTH), np.float32)
+        td = np.empty((n, B), np.float32) if per else None
+
+        def ptr(x):
+            return None if x is None else np_ptr(x)
+        nptrs = [None if t is None else vp(t.data_ptr()) for t in noise]
+        if her:
+            fn, draws, tail = self._MANY_FNS[0], (ptr(pos),), ()
+        else:
+            fn, draws, tail = self._MANY_FNS[1], (ptr(pos), ptr(u), ptr(beta)), (ptr(td),)
         try:
-            check(lib.gcrl_agent_update_many(self._h, self.buffer.handle, B, n, flags, iptr,
-                                             vp(noise.data_ptr()) if noise is not None else None, lr_c, lr_a,
-                                             np_ptr(metrics), self._stream()))
+            check(getattr(lib, fn)(self._h, self.buffer.handle, B, n, cflags, *draws, *nptrs, lr_c, lr_a,
+                                   np_ptr(metrics), *tail, self._stream()))
         except BaseException:
             self._restore_schedules(saved)
             raise
-        self._last_td = None
+        return self._many_results(steps, flags, metrics, td)
+
+    def _many_results(self, steps, flags, metrics, td):
+        """What update() does after its call, for every step in order: the TD array (PER), the BatchNorm batch count
+        (SAC / TQC), beta and the returned tuple."""
         out = []
-        for step, m in zip(steps, metrics.tolist()):
+        for i, (step, f, m) in enumerate(zip(steps, flags, metrics.tolist())):
+            self._last_td = td[i].reshape(-1, 1) if td is not None else None
+            if self._BN_BATCHES is not None:
+                self._bn_batches += self._BN_BATCHES[f & 1]
             self.beta_scheduler(step)
             out.append(self._result(step, m))
         return out
@@ -667,7 +656,6 @@ class DDPG(_AgentBase):
     ALGO = ALGO_DDPG
     WEIGHT_DECAY = 0.0          # torch.optim.Adam (:1201-1202)
     POLYAK_EVERY = 40           # literal at :1397
-    _MANY_IN_ONE_GRAPH = True
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw):
         super().__init__(obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw)
@@ -739,7 +727,6 @@ class TD3Agent(_AgentBase):
     """Reference src/agent.py:12-386."""
     ALGO = ALGO_TD3
     WEIGHT_DECAY = 0.01         # torch.optim.AdamW default (:46-48)
-    _MANY_IN_ONE_GRAPH = True
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw):
         super().__init__(obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw)
@@ -794,10 +781,10 @@ class TD3Agent(_AgentBase):
         self.beta_scheduler(step)
         return self._result(step, m)
 
-    def _many_noise(self, B, n):
+    def _many_noise(self, B, flags):
         """n separate draws of update()'s noise, in step order: the CUDA generator advances as under the loop."""
         import torch
-        return torch.stack([torch.randn((B, self.ac_dim), dtype=torch.float32, device=self.device) for _ in range(n)])
+        return (torch.stack([torch.randn((B, self.ac_dim), dtype=torch.float32, device=self.device) for _ in flags]),)
 
     def _result(self, step, m):
         q1l, acl, td, q, c1g, acg, q2l, c2g = m

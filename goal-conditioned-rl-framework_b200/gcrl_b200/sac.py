@@ -19,7 +19,6 @@ from . import _lib
 from ._lib import SacConfig, check, lib, np_ptr, vp
 from .agent import CosineAnnealingLR, _AgentBase
 from .buffer import HERBuffer
-from .replay import PERBuffer
 
 ALGO_SAC, ALGO_TQC = 2, 3
 
@@ -410,9 +409,12 @@ class _SacBase(_AgentBase):
         return self._result(step, [float(x) for x in self._metrics])
 
     # -- a training cycle's gradient steps in one call (_AgentBase.update_many) ------------------------------
-    _MANY_IN_ONE_GRAPH = True       # on one GPU, from every buffer type; both data-parallel modes loop
+    _MANY_FNS = ("gcrl_sac_update_many", "gcrl_sac_update_many_replay")
+    _METRIC_WIDTH = 12
+    _MIN_BATCH = 2              # BatchNorm needs more than one row
+    _BN_BATCHES = (1, 2)        # num_batches_tracked grows as update() grows it: 1, or 2 with an actor step
 
-    def _many_eps(self, B, flags):
+    def _many_noise(self, B, flags):
         """update()'s torch.randn calls for n updates, in step order: (eps_next [n][B][A], eps_cur [n][B][A] or None
         when no update steps the actor)."""
         import torch
@@ -426,67 +428,6 @@ class _SacBase(_AgentBase):
             return eps_next, None
         unused = torch.zeros(shape, dtype=torch.float32, device=self.device)    # rows of critic-only steps: never read
         return eps_next, torch.stack([unused if e is None else e for e in eps_cur])
-
-    def _update_chunk(self, steps):
-        """Up to MAX_MANY_STEPS updates through gcrl_sac_update_many: the noise, positions, flags and learning
-        rates of all of them are drawn up front, in the order the loop draws them."""
-        B, n = self.batch_size, len(steps)
-        assert len(self.buffer) >= B, "[ERROR] Not enough in buffer to sample"       # before any state moves
-        if not 2 <= B <= self._max_batch:
-            raise ValueError(f"batch size {B} outside [2, max_batch = {self._max_batch}]")
-        flags = [self._flags(s) for s in steps]
-        eps_next, eps_cur = self._many_eps(B, flags)
-        iptr = None
-        if self.index_source == "host":             # n draws of random.sample(range(len), B), in step order
-            nlen = len(self.buffer)
-            idx = np.stack([_lib.py_sample_range(nlen, B) for _ in steps])
-            iptr = np_ptr(idx)
-        cflags = (C.c_int * n)(*flags)
-        lr_c, lr_a, saved = self._step_schedules(flags)
-        metrics = np.empty((n, 12), np.float32)
-        try:
-            check(lib.gcrl_sac_update_many(self._h, self.buffer.handle, B, n, cflags, iptr, vp(eps_next.data_ptr()),
-                                           vp(eps_cur.data_ptr()) if eps_cur is not None else None, lr_c, lr_a,
-                                           np_ptr(metrics), self._stream()))
-        except BaseException:
-            self._restore_schedules(saved)
-            raise
-        return self._many_results(steps, flags, metrics, None)
-
-    def _update_chunk_replay(self, steps):
-        """Up to MAX_MANY_STEPS updates from a REPLAY / PER buffer through gcrl_sac_update_many_replay: the noise,
-        positions or uniforms and betas, flags and learning rates of all of them are drawn up front, in the order
-        the loop draws them."""
-        B, n = self.batch_size, len(steps)
-        self._check_replay_chunk(B, min_batch=2)
-        per = 8 if isinstance(self.buffer, PERBuffer) else 0
-        flags = [self._flags(s) | per for s in steps]
-        eps_next, eps_cur = self._many_eps(B, flags)
-        _, pos, u, beta = self._replay_draws(B, steps)
-        cflags = (C.c_int * n)(*flags)
-        lr_c, lr_a, saved = self._step_schedules(flags)
-        metrics = np.empty((n, 12), np.float32)
-        td = np.empty((n, B), np.float32) if per else None
-        try:
-            check(lib.gcrl_sac_update_many_replay(
-                self._h, self.buffer.handle, B, n, cflags, *(None if x is None else np_ptr(x) for x in (pos, u, beta)),
-                vp(eps_next.data_ptr()), vp(eps_cur.data_ptr()) if eps_cur is not None else None, lr_c, lr_a,
-                np_ptr(metrics), np_ptr(td) if per else None, self._stream()))
-        except BaseException:
-            self._restore_schedules(saved)
-            raise
-        return self._many_results(steps, flags, metrics, td)
-
-    def _many_results(self, steps, flags, metrics, td):
-        """What update() does after its call, for every step in order: TD array (PER), BatchNorm batch count, beta
-        and the returned tuple."""
-        out = []
-        for i, (step, f, m) in enumerate(zip(steps, flags, metrics.tolist())):
-            self._last_td = td[i].reshape(-1, 1) if td is not None else None
-            self._bn_batches += 2 if f & 1 else 1
-            self.beta_scheduler(step)
-            out.append(self._result(step, m))
-        return out
 
     def _save_log_alpha(self, path):
         import torch
