@@ -10,6 +10,7 @@
 // rows (sa, nsa, spi) fold torch.cat: the actor heads write their tanh output straight into
 // the action columns.  An update is captured once per (batch, flags) into a CUDA graph and
 // replayed; per-step scalars (lr / bias corrections) travel through a small device struct.
+#include <algorithm>
 #include <atomic>
 #include <chrono>
 #include <cmath>
@@ -23,88 +24,11 @@
 #include "buffer_api.cuh"
 #include "graphs.cuh"
 #include "mlp.cuh"
+#include "params.cuh"
 
 using namespace gcrl;
 
 namespace {
-
-inline int pad4(int x) { return (x + 3) & ~3; }
-
-struct Net {
-  int layers = 0;  // number of Linear layers = layer_count + 1
-  int in_dim = 0, hidden = 0, out_dim = 0;
-  std::vector<int> in_d, out_d, ldw, w_off, b_off;
-  std::vector<int> ldt, t_off;   // transposed copy Wt[in][ldt] per layer (forward operand of fused.cu)
-  int total = 0, total_t = 0;
-  float *p = nullptr, *g = nullptr, *m = nullptr, *v = nullptr;
-  float *pT = nullptr;
-  int *tmap = nullptr;           // [total] -> index into pT, -1 for bias / padding
-  // TF32 hi / lo halves of p and pT (tensor-core engine: the weight operand arrives pre-split, tc_gemm.cu);
-  // refreshed after every optimiser / Polyak step of an update that uses that engine, lazily otherwise
-  float *p_hi = nullptr, *p_lo = nullptr, *pT_hi = nullptr, *pT_lo = nullptr;
-  bool split_stale = true;
-  int adam_t = 0;
-
-  void init(int in, int hid, int out, int layer_count, bool trainable) {
-    layers = layer_count + 1;
-    in_dim = in; hidden = hid; out_dim = out;
-    int off = 0;
-    for (int l = 0; l < layers; ++l) {
-      in_d.push_back(l == 0 ? in : hid);
-      out_d.push_back(l == layers - 1 ? out : hid);
-      ldw.push_back(pad4(in_d[l]));
-      w_off.push_back(off);
-      off += out_d[l] * ldw[l];
-      b_off.push_back(off);
-      off += pad4(out_d[l]);
-    }
-    total = off;
-    int toff = 0;
-    for (int l = 0; l < layers; ++l) {
-      ldt.push_back(pad4(out_d[l]));
-      t_off.push_back(toff);
-      toff += in_d[l] * ldt[l];
-    }
-    total_t = toff;
-    std::vector<int> map(size_t(total), -1);
-    for (int l = 0; l < layers; ++l)
-      for (int o = 0; o < out_d[l]; ++o)
-        for (int i = 0; i < in_d[l]; ++i) map[size_t(w_off[l]) + size_t(o) * ldw[l] + i] = t_off[l] + i * ldt[l] + o;
-    tmap = dev_alloc<int>(total);
-    GCRL_CUDA(cudaMemcpy(tmap, map.data(), size_t(total) * sizeof(int), cudaMemcpyHostToDevice));
-    pT = dev_alloc<float>(total_t);
-    GCRL_CUDA(cudaMemset(pT, 0, size_t(total_t) * 4));
-    p = dev_alloc<float>(total);
-    GCRL_CUDA(cudaMemset(p, 0, size_t(total) * 4));
-    if (trainable) {
-      g = dev_alloc<float>(total);
-      m = dev_alloc<float>(total);
-      v = dev_alloc<float>(total);
-      GCRL_CUDA(cudaMemset(g, 0, size_t(total) * 4));
-      GCRL_CUDA(cudaMemset(m, 0, size_t(total) * 4));
-      GCRL_CUDA(cudaMemset(v, 0, size_t(total) * 4));
-    }
-  }
-  void alloc_split() {
-    if (p_hi != nullptr) return;
-    p_hi = dev_alloc<float>(total); p_lo = dev_alloc<float>(total);
-    pT_hi = dev_alloc<float>(total_t); pT_lo = dev_alloc<float>(total_t);
-  }
-  void split(cudaStream_t st) {
-    launch_split_tf32(p, p_hi, p_lo, total, st);
-    launch_split_tf32(pT, pT_hi, pT_lo, total_t, st);
-  }
-  void destroy() {
-    cudaFree(p);
-    cudaFree(pT);
-    cudaFree(tmap);
-    for (float *q : {p_hi, p_lo, pT_hi, pT_lo})
-      if (q) cudaFree(q);
-    if (g) { cudaFree(g); cudaFree(m); cudaFree(v); }
-  }
-  const float *W(int l) const { return p + w_off[l]; }
-  const float *b(int l) const { return p + b_off[l]; }
-};
 
 struct Acts {  // post-activation outputs of the hidden layers, [max_batch, ldh] each
   std::vector<float *> h;
@@ -129,8 +53,9 @@ struct gcrl_agent {
   int D = 0, A = 0, H = 0, L = 0, ldh = 0, ldc = 0;
   int64_t maxB = 0;
   bool td3 = false;
-  Net net[NUM_NETS];
+  MlpParams net[NUM_NETS];
   bool has[NUM_NETS] = {};
+  int adam_t[NUM_NETS] = {};               // Adam step counters
   Acts acts_actor, acts_c1, acts_c2, acts_tgt;
   float *dz[2] = {nullptr, nullptr};       // ping-pong grad-wrt-preactivation buffers [maxB, ldh]
   float *sa = nullptr, *nsa = nullptr, *spi = nullptr;
@@ -214,18 +139,15 @@ bool engine_tc(const gcrl_agent *ag, int B) { return use_tc(ag, B, ag->H, (ag->H
 // the TF32 hi / lo copies of every network whose parameters changed since they were last split (eager, outside capture)
 void ensure_split(gcrl_agent *ag, cudaStream_t st) {
   for (int i = 0; i < NUM_NETS; ++i)
-    if (ag->has[i] && ag->net[i].p_hi != nullptr && ag->net[i].split_stale) {
-      ag->net[i].split(st);
-      ag->net[i].split_stale = false;
-    }
+    if (ag->has[i]) ag->net[i].copies.split_if_stale(ag->net[i].p, st);
 }
 void mark_split_stale(gcrl_agent *ag) {
-  for (int i = 0; i < NUM_NETS; ++i) ag->net[i].split_stale = true;
+  for (int i = 0; i < NUM_NETS; ++i) ag->net[i].copies.stale = true;
 }
 
 // ---- forward / backward building blocks ----------------------------------------------------
 // hidden stack: X[B, K0] -> acts.h[0..L-1]
-void forward_hidden(const gcrl_agent *ag, const Net &n, const float *X, int ldx, int K0, const Acts &acts,
+void forward_hidden(const gcrl_agent *ag, const MlpParams &n, const float *X, int ldx, int K0, const Acts &acts,
                     int B, cudaStream_t st) {
   const float *in = X;
   int ldin = ldx, K = K0;
@@ -233,8 +155,8 @@ void forward_hidden(const gcrl_agent *ag, const Net &n, const float *X, int ldx,
     // layer 0: the operand rows and the weight rows are zero-padded to ld, so the padded K is exact
     const int Kp = (K + 3) & ~3;
     if (use_tc(ag, B, ag->H, Kp))
-      launch_tc_dense(in, ldin, n.p_hi + n.w_off[l], n.ldw[l], n.b(l), nullptr, 0, acts.h[l], ag->ldh, B, ag->H, Kp, 0, st,
-                      n.p_lo + n.w_off[l]);
+      launch_tc_dense(in, ldin, n.copies.p_hi + n.w_off[l], n.ldw[l], n.b(l), nullptr, 0, acts.h[l], ag->ldh, B, ag->H, Kp,
+                      0, st, n.copies.p_lo + n.w_off[l]);
     else
       launch_linear_fwd(in, ldin, n.W(l), n.ldw[l], n.b(l), acts.h[l], ag->ldh, B, ag->H, K, ACT_LEAKY, st);
     in = acts.h[l];
@@ -249,8 +171,9 @@ void forward_hidden(const gcrl_agent *ag, const Net &n, const float *X, int ldx,
 // x_pad_zero: X's columns K0 .. K0 padded to a multiple of 4 are zero.  The actor's input rows [s | a | 0] hold the
 // actions there, which the tensor-core weight gradient would sum into the padding columns of layer 0's gradient
 // (inflating its norm, hence the clip, and stepping the padding weights).
-void backward_hidden(gcrl_agent *ag, const Net &n, const float *X, int ldx, int K0, bool x_pad_zero, const Acts &acts,
-                     int B, int cur, bool want_wgrad, int *splits /*[layers]*/, int *cur_out, cudaStream_t st) {
+void backward_hidden(gcrl_agent *ag, const MlpParams &n, const float *X, int ldx, int K0, bool x_pad_zero,
+                     const Acts &acts, int B, int cur, bool want_wgrad, int *splits /*[layers]*/, int *cur_out,
+                     cudaStream_t st) {
   for (int l = ag->L - 1; l >= 0; --l) {
     const float *xin = l == 0 ? X : acts.h[l - 1];
     const int ldin = l == 0 ? ldx : ag->ldh;
@@ -267,8 +190,9 @@ void backward_hidden(gcrl_agent *ag, const Net &n, const float *X, int ldx, int 
     }
     if (l > 0) {
       if (use_tc(ag, B, ag->H, ag->H))   // dX = dZ Wt^T with the transposed weight copy as the K-major operand
-        launch_tc_dense(ag->dz[cur], ag->ldh, n.pT_hi + n.t_off[l], n.ldt[l], nullptr, acts.h[l - 1], ag->ldh,
-                        ag->dz[cur ^ 1], ag->ldh, B, ag->H, ag->H, 1, st, n.pT_lo + n.t_off[l]);
+        launch_tc_dense(ag->dz[cur], ag->ldh, n.copies.pT_hi + n.copies.t_off[l], n.copies.ldt[l], nullptr,
+                        acts.h[l - 1], ag->ldh, ag->dz[cur ^ 1], ag->ldh, B, ag->H, ag->H, 1, st,
+                        n.copies.pT_lo + n.copies.t_off[l]);
       else
         launch_linear_dgrad(ag->dz[cur], ag->ldh, n.W(l), n.ldw[l], acts.h[l - 1], ag->ldh, ag->dz[cur ^ 1],
                             ag->ldh, B, ag->H, ag->H, st);
@@ -281,7 +205,7 @@ void backward_hidden(gcrl_agent *ag, const Net &n, const float *X, int ldx, int 
 // partial slabs -> flat gradient of `n` (+ per-CTA sums of squares, + batch-mean metrics).
 // rereduce: the gradient is already in n.g (it was averaged across ranks); only the sums of
 // squares for the global-norm clip are recomputed.
-void reduce_grads(gcrl_agent *ag, Net &n, const int *splits, int head_splits, bool rereduce, int slot_loss,
+void reduce_grads(gcrl_agent *ag, MlpParams &n, const int *splits, int head_splits, bool rereduce, int slot_loss,
                   int slot_td, int slot_q, int metric_splits, int B, cudaStream_t st) {
   ReduceArgs r{};
   r.nseg = 0;
@@ -306,7 +230,7 @@ void reduce_grads(gcrl_agent *ag, Net &n, const int *splits, int head_splits, bo
 }
 
 // global-norm clip + Adam(W) (+ fused Polyak of `target` with the stepped parameters)
-void adam_step(gcrl_agent *ag, Net &n, int which, float max_norm, int slot_norm, Net *target, bool polyak,
+void adam_step(gcrl_agent *ag, MlpParams &n, int which, float max_norm, int slot_norm, MlpParams *target, bool polyak,
                cudaStream_t st, const float *grad = nullptr) {
   AdamArgs a{};
   a.p = n.p; a.m = n.m; a.v = n.v; a.g = grad ? grad : n.g; a.n = n.total;
@@ -318,7 +242,7 @@ void adam_step(gcrl_agent *ag, Net &n, int which, float max_norm, int slot_norm,
   a.polyak = (polyak && target) ? 1 : 0;
   a.metrics = ag->p2p.on ? ag->p2p.metrics_avg : ag->metrics;   // the norm of the averaged gradient is global already
   a.slot_norm = slot_norm;
-  a.tmap = n.tmap; a.pT = n.pT; a.targetT = target ? target->pT : nullptr;
+  a.tmap = n.copies.tmap; a.pT = n.copies.pT; a.targetT = target ? target->copies.pT : nullptr;
   if (ag->publish_now) {
     a.publish = ag->d_pub;
     a.publish_src = a.metrics;
@@ -326,8 +250,8 @@ void adam_step(gcrl_agent *ag, Net &n, int which, float max_norm, int slot_norm,
   }
   launch_adam(a, st);
   if (ag->tc_update) {          // this update's later layers read the stepped weights through the tensor cores
-    n.split(st);
-    if (a.polyak) target->split(st);
+    n.copies.split(n.p, st);
+    if (a.polyak) target->copies.split(target->p, st);
   }
 }
 
@@ -335,7 +259,7 @@ void adam_step(gcrl_agent *ag, Net &n, int which, float max_norm, int slot_norm,
 // phase 0/1: critic(s).  Operands sa / nsa / br / bd must be resident.
 void critic_forward_backward(gcrl_agent *ag, int which_critic, int B, int *splits, int *head_splits,
                              int *metric_splits, cudaStream_t st) {
-  const Net &c = ag->net[which_critic == 0 ? CRITIC1 : CRITIC2];
+  const MlpParams &c = ag->net[which_critic == 0 ? CRITIC1 : CRITIC2];
   const Acts &acts = which_critic == 0 ? ag->acts_c1 : ag->acts_c2;
   float *q = which_critic == 0 ? ag->q1 : ag->q2;
   const int K0 = ag->D + ag->A;
@@ -405,15 +329,16 @@ bool fused_ok(const gcrl_agent *ag, int B) {
   return ag->use_fused && fused_supported(B, ag->D, ag->A, ag->H, ag->L);
 }
 
-FusedNet fused_net(const gcrl_agent *ag, const Net &n) {
+FusedNet fused_net(const gcrl_agent *ag, const MlpParams &n) {
   FusedNet f{};
+  const WeightCopies &c = n.copies;
   for (int l = 0; l < ag->L; ++l) {
-    f.Wt[l] = n.pT + n.t_off[l]; f.ldt[l] = n.ldt[l];
+    f.Wt[l] = c.pT + c.t_off[l]; f.ldt[l] = c.ldt[l];
     f.W[l] = n.p + n.w_off[l];   f.ldw[l] = n.ldw[l];
     f.b[l] = n.p + n.b_off[l];
   }
   f.Wh = n.p + n.w_off[ag->L]; f.ldwh = n.ldw[ag->L]; f.bh = n.p + n.b_off[ag->L];
-  f.flat = n.p; f.nflat = n.total; f.flatT = n.pT; f.nflatT = n.total_t;
+  f.flat = n.p; f.nflat = n.total; f.flatT = c.pT; f.nflatT = c.total_t;
   return f;
 }
 
@@ -427,7 +352,7 @@ unsigned int critic_metric_mask(const gcrl_agent *ag, int which) {
 // weight gradients of all layers of `n` in ONE launch that also completes the split-batch sums into the flat
 // gradient n.g, the per-tile sums of squares and the batch-mean metrics (mlp.cu: multi_wgrad_kernel);
 // hidden-layer operands: dzl[l] and (l == 0 ? sa : acts.h[l-1]); head operand: dz_head [B][ld_head] and acts.h[L-1]
-void fused_wgrads(gcrl_agent *ag, Net &n, const Acts &acts, int K0, const float *dz_head, int ld_head, int B,
+void fused_wgrads(gcrl_agent *ag, MlpParams &n, const Acts &acts, int K0, const float *dz_head, int ld_head, int B,
                   int slot_loss, int slot_td, int slot_q, int metric_splits, cudaStream_t st) {
   WgradProblem pr[kMaxWgradProblems];
   const int L = ag->L;
@@ -456,7 +381,7 @@ void fused_wgrads(gcrl_agent *ag, Net &n, const Acts &acts, int K0, const float 
 
 // the same per-tile sums of squares for a gradient that is already complete in n.g (data-parallel phases: the
 // cross-rank average replaced it) -- bit-identical to what fused_wgrads leaves for the same values
-void fused_grad_sumsq(gcrl_agent *ag, Net &n, cudaStream_t st) {
+void fused_grad_sumsq(gcrl_agent *ag, MlpParams &n, cudaStream_t st) {
   WgradProblem pr[kMaxWgradProblems];
   for (int l = 0; l < n.layers; ++l) {
     pr[l] = WgradProblem{};
@@ -503,7 +428,7 @@ FusedCriticArgs fused_critic_args(gcrl_agent *ag, int B, int which = 0) {
 void fused_critic_phase_grads(gcrl_agent *ag, int B, int which, cudaStream_t st) {
   const FusedCriticArgs a = fused_critic_args(ag, B, which);
   const int slabs = launch_fused_critic(a, st);
-  Net &c = ag->net[which == 0 ? CRITIC1 : CRITIC2];
+  MlpParams &c = ag->net[which == 0 ? CRITIC1 : CRITIC2];
   // TD3: td error / Q metrics come from the critic-2 launch (they need both critics' Q)
   const bool metrics_here = !ag->td3 || which == 1;
   fused_wgrads(ag, c, which == 0 ? ag->acts_c1 : ag->acts_c2, ag->D + ag->A, ag->dzh, 1, B,
@@ -563,7 +488,7 @@ const float *p2p_average(gcrl_agent *ag, int net, unsigned int metric_mask, cuda
 void critic_phase_step(gcrl_agent *ag, int which, int flags, bool rereduce, cudaStream_t st) {
   const bool polyak = ag->td3 ? true : ((flags & 2) != 0);
   const int id = which == 0 ? CRITIC1 : CRITIC2;
-  Net &c = ag->net[id];
+  MlpParams &c = ag->net[id];
   const float *grad = nullptr;
   // metrics final before this barrier: DDPG critic loss / td / q; TD3 critic 1: its loss; critic 2: loss, td, q
   const unsigned int mm = critic_metric_mask(ag, which);
@@ -579,9 +504,10 @@ void critic_phase_step(gcrl_agent *ag, int which, int flags, bool rereduce, cuda
 // DDPG: the actor target blends the PRE-step actor, before the actor step (:1397-1401)
 void ddpg_actor_target_polyak(gcrl_agent *ag, int flags, cudaStream_t st) {
   if (!ag->td3 && (flags & 2)) {
-    launch_polyak(ag->net[T_ACTOR].p, ag->net[ACTOR].p, ag->net[ACTOR].total, ag->cfg.tau,
-                  float(1.0 - double(ag->cfg.tau)), ag->net[ACTOR].tmap, ag->net[T_ACTOR].pT, st);
-    if (ag->tc_update) ag->net[T_ACTOR].split(st);
+    MlpParams &t = ag->net[T_ACTOR];
+    launch_polyak(t.p, ag->net[ACTOR].p, ag->net[ACTOR].total, ag->cfg.tau, float(1.0 - double(ag->cfg.tau)),
+                  ag->net[ACTOR].copies.tmap, t.copies.pT, st);
+    if (ag->tc_update) t.copies.split(t.p, st);
   }
 }
 
@@ -589,8 +515,8 @@ void actor_phase_grads(gcrl_agent *ag, int B, cudaStream_t st) {
   if (fused_ok(ag, B)) { fused_actor_phase_grads(ag, B, st); return; }
   PhaseState pstate, *ps = &pstate;
   const int D = ag->D, A = ag->A, K0 = D + A, L = ag->L;
-  const Net &actor = ag->net[ACTOR];
-  const Net &c = ag->net[CRITIC1];
+  const MlpParams &actor = ag->net[ACTOR];
+  const MlpParams &c = ag->net[CRITIC1];
   // a = actor(s) -> action columns of spi; q = critic([s, a]) with the stepped critic (:1289-1290)
   forward_hidden(ag, actor, ag->spi, ag->ldc, D, ag->acts_actor, B, st);
   launch_head_fwd(ag->acts_actor.h[L - 1], ag->ldh, actor.W(L), actor.ldw[L], actor.b(L), ag->spi, ag->ldc, D,
@@ -628,7 +554,7 @@ void actor_phase_grads(gcrl_agent *ag, int B, cudaStream_t st) {
 }
 
 void actor_phase_step(gcrl_agent *ag, bool rereduce, cudaStream_t st) {
-  Net &a = ag->net[ACTOR];
+  MlpParams &a = ag->net[ACTOR];
   const float *grad = nullptr;
   if (ag->p2p.on) grad = p2p_average(ag, ACTOR, 1u << S_ALOSS, st);
   else if (rereduce && fused_ok(ag, ag->dp_B)) fused_grad_sumsq(ag, a, st);
@@ -647,11 +573,11 @@ void fill_scalars(gcrl_agent *ag, double lr_c, double lr_a, bool actor_steps, co
   };
   auto *sc = reinterpret_cast<StepScalars *>(out);
   std::memcpy(sc + 1, &ss, sizeof(SampleScalars));
-  ag->net[CRITIC1].adam_t += 1;
-  if (ag->td3) ag->net[CRITIC2].adam_t += 1;
-  fill(ag->net[CRITIC1].adam_t, lr_c, &sc->step_size_c);
-  if (actor_steps) ag->net[ACTOR].adam_t += 1;
-  fill(std::max(1, ag->net[ACTOR].adam_t), lr_a, &sc->step_size_a);
+  ag->adam_t[CRITIC1] += 1;
+  if (ag->td3) ag->adam_t[CRITIC2] += 1;
+  fill(ag->adam_t[CRITIC1], lr_c, &sc->step_size_c);
+  if (actor_steps) ag->adam_t[ACTOR] += 1;
+  fill(std::max(1, ag->adam_t[ACTOR]), lr_a, &sc->step_size_a);
   sc->pad1 = 0.f;
   sc->seq = ++ag->pub_seq;
 }
@@ -678,13 +604,13 @@ struct AdamStepGuard {
   bool done = false;
   explicit AdamStepGuard(gcrl_agent *a)
       : ag(a), per_on(a->per_on), dp_B(a->dp_B), dp_flags(a->dp_flags), pub_seq(a->pub_seq) {
-    for (int i = 0; i < NUM_NETS; ++i) t[i] = a->net[i].adam_t;
+    std::copy(a->adam_t, a->adam_t + NUM_NETS, t);
   }
   void keep_draws(gcrl_her *b) { buf = b; draw_epoch = her_draw_epoch(b); }
   void commit() { done = true; }
   ~AdamStepGuard() {
     if (done) return;
-    for (int i = 0; i < NUM_NETS; ++i) ag->net[i].adam_t = t[i];
+    std::copy(t, t + NUM_NETS, ag->adam_t);
     ag->per_on = per_on; ag->dp_B = dp_B; ag->dp_flags = dp_flags;
     ag->pub_seq = pub_seq;
     if (buf != nullptr) her_draw_epoch(buf) = draw_epoch;
@@ -1059,13 +985,20 @@ int gcrl_agent_create(gcrl_agent **out, int device, const gcrl_agent_config *cfg
     ag->td3 = cfg->algo == GCRL_ALGO_TD3;
     GCRL_REQUIRE(ag->maxB <= int64_t(kMaxSplits) * 512, "max_batch too large for the partial buffers");
     const int D = ag->D, A = ag->A, H = ag->H, L = ag->L;
-    ag->net[ACTOR].init(D, H, A, L, true);       ag->has[ACTOR] = true;
-    ag->net[CRITIC1].init(D + A, H, 1, L, true); ag->has[CRITIC1] = true;
-    ag->net[T_ACTOR].init(D, H, A, L, false);    ag->has[T_ACTOR] = true;
-    ag->net[T_CRITIC1].init(D + A, H, 1, L, false); ag->has[T_CRITIC1] = true;
+    auto init_net = [&](int id, int in, int out, bool trainable) {
+      MlpParams &n = ag->net[id];
+      n.layout(in, H, out, L);
+      n.init_copies(0, n.layers, false);   // W^T of every layer: the row-slab kernels read Wt, prefetch all of flatT
+      n.alloc(trainable);
+      ag->has[id] = true;
+    };
+    init_net(ACTOR, D, A, true);
+    init_net(CRITIC1, D + A, 1, true);
+    init_net(T_ACTOR, D, A, false);
+    init_net(T_CRITIC1, D + A, 1, false);
     if (ag->td3) {
-      ag->net[CRITIC2].init(D + A, H, 1, L, true);    ag->has[CRITIC2] = true;
-      ag->net[T_CRITIC2].init(D + A, H, 1, L, false); ag->has[T_CRITIC2] = true;
+      init_net(CRITIC2, D + A, 1, true);
+      init_net(T_CRITIC2, D + A, 1, false);
     }
     const int64_t mb = ag->maxB;
     ag->acts_actor.init(L, mb, ag->ldh);
@@ -1110,9 +1043,11 @@ int gcrl_agent_create(gcrl_agent **out, int device, const gcrl_agent_config *cfg
     ag->use_graphs = graphs_enabled();
     ag->io_stage.init(size_t(1) << 16);
     if (ag->cfg.precision >= 1) {
+      // the TF32 halves of tcgen05 come last: the row-slab kernels' buffers keep their places (next to each other,
+      // in the order tmap, Wt, p, g, m, v), without which B = 256 steps ran 0.5 % slower on a B200
       tc_dense_init();
       for (int i = 0; i < NUM_NETS; ++i)
-        if (ag->has[i]) ag->net[i].alloc_split();
+        if (ag->has[i]) ag->net[i].copies.alloc_halves();
     }
   } catch (...) {
     delete ag;
@@ -1180,17 +1115,13 @@ int gcrl_agent_set_layer(gcrl_agent *ag, int net, int layer, const float *weight
   GCRL_API_BEGIN
   require_handle(ag);
   GCRL_REQUIRE(ag && net >= 0 && net < NUM_NETS && ag->has[net], "bad network id");
-  Net &n = ag->net[net];
+  MlpParams &n = ag->net[net];
   GCRL_REQUIRE(layer >= 0 && layer < n.layers && weight_host && bias_host, "bad layer / NULL data");
   GCRL_CUDA(cudaSetDevice(ag->device));
   cudaStream_t st = as_stream(stream);
-  const int o = n.out_d[layer], i = n.in_d[layer], ld = n.ldw[layer];
-  std::vector<float> padded(size_t(o) * ld + pad4(o), 0.f);
-  for (int r = 0; r < o; ++r) std::memcpy(&padded[size_t(r) * ld], weight_host + size_t(r) * i, size_t(i) * 4);
-  std::memcpy(&padded[size_t(o) * ld], bias_host, size_t(o) * 4);
-  GCRL_CUDA(cudaMemcpyAsync(n.p + n.w_off[layer], padded.data(), padded.size() * 4, cudaMemcpyHostToDevice, st));
-  launch_sync_transposed(n.p, n.pT, n.tmap, n.total, st);
-  n.split_stale = true;
+  upload_rows(n.p + n.w_off[layer], weight_host, n.out_d[layer], n.in_d[layer], n.ldw[layer], st);
+  upload_rows(n.p + n.b_off[layer], bias_host, 1, n.out_d[layer], n.out_d[layer], st);
+  n.copies.weights_changed(n.p, st);
   GCRL_CUDA(cudaStreamSynchronize(st));
   GCRL_API_END
 }
@@ -1200,17 +1131,12 @@ int gcrl_agent_get_layer(gcrl_agent *ag, int net, int layer, float *weight_host,
   GCRL_API_BEGIN
   require_handle(ag);
   GCRL_REQUIRE(ag && net >= 0 && net < NUM_NETS && ag->has[net], "bad network id");
-  Net &n = ag->net[net];
+  MlpParams &n = ag->net[net];
   GCRL_REQUIRE(layer >= 0 && layer < n.layers, "bad layer index");
   GCRL_CUDA(cudaSetDevice(ag->device));
   cudaStream_t st = as_stream(stream);
-  const int o = n.out_d[layer], i = n.in_d[layer], ld = n.ldw[layer];
-  std::vector<float> padded(size_t(o) * ld + pad4(o));
-  GCRL_CUDA(cudaMemcpyAsync(padded.data(), n.p + n.w_off[layer], padded.size() * 4, cudaMemcpyDeviceToHost, st));
-  GCRL_CUDA(cudaStreamSynchronize(st));
-  if (weight_host)
-    for (int r = 0; r < o; ++r) std::memcpy(weight_host + size_t(r) * i, &padded[size_t(r) * ld], size_t(i) * 4);
-  if (bias_host) std::memcpy(bias_host, &padded[size_t(o) * ld], size_t(o) * 4);
+  if (weight_host) download_rows(weight_host, n.p + n.w_off[layer], n.out_d[layer], n.in_d[layer], n.ldw[layer], st);
+  if (bias_host) download_rows(bias_host, n.p + n.b_off[layer], 1, n.out_d[layer], n.out_d[layer], st);
   GCRL_API_END
 }
 
@@ -1221,26 +1147,20 @@ static int adam_layer_io(gcrl_agent *ag, int net, int layer, float *m_w, float *
   GCRL_API_BEGIN
   require_handle(ag);
   GCRL_REQUIRE(ag && net >= 0 && net < NUM_NETS && ag->has[net] && ag->net[net].m, "bad (or non-trainable) network id");
-  Net &n = ag->net[net];
+  MlpParams &n = ag->net[net];
   GCRL_REQUIRE(layer >= 0 && layer < n.layers && m_w && m_b && v_w && v_b, "bad layer / NULL data");
   GCRL_CUDA(cudaSetDevice(ag->device));
   cudaStream_t st = as_stream(stream);
   const int o = n.out_d[layer], i = n.in_d[layer], ld = n.ldw[layer];
-  std::vector<float> padded(size_t(o) * ld + pad4(o), 0.f);
   float *dev[2] = {n.m, n.v};
   float *hw[2] = {m_w, v_w}, *hb[2] = {m_b, v_b};
   for (int k = 0; k < 2; ++k) {
     if (set) {
-      std::fill(padded.begin(), padded.end(), 0.f);
-      for (int r = 0; r < o; ++r) std::memcpy(&padded[size_t(r) * ld], hw[k] + size_t(r) * i, size_t(i) * 4);
-      std::memcpy(&padded[size_t(o) * ld], hb[k], size_t(o) * 4);
-      GCRL_CUDA(cudaMemcpyAsync(dev[k] + n.w_off[layer], padded.data(), padded.size() * 4, cudaMemcpyHostToDevice, st));
-      GCRL_CUDA(cudaStreamSynchronize(st));
+      upload_rows(dev[k] + n.w_off[layer], hw[k], o, i, ld, st);
+      upload_rows(dev[k] + n.b_off[layer], hb[k], 1, o, o, st);
     } else {
-      GCRL_CUDA(cudaMemcpyAsync(padded.data(), dev[k] + n.w_off[layer], padded.size() * 4, cudaMemcpyDeviceToHost, st));
-      GCRL_CUDA(cudaStreamSynchronize(st));
-      for (int r = 0; r < o; ++r) std::memcpy(hw[k] + size_t(r) * i, &padded[size_t(r) * ld], size_t(i) * 4);
-      std::memcpy(hb[k], &padded[size_t(o) * ld], size_t(o) * 4);
+      download_rows(hw[k], dev[k] + n.w_off[layer], o, i, ld, st);
+      download_rows(hb[k], dev[k] + n.b_off[layer], 1, o, o, st);
     }
   }
   GCRL_API_END
@@ -1259,14 +1179,14 @@ int gcrl_agent_get_adam_step(gcrl_agent *ag, int net, int *step) {
   GCRL_API_BEGIN
   require_handle(ag);
   GCRL_REQUIRE(ag && step && net >= 0 && net < NUM_NETS && ag->has[net] && ag->net[net].m, "bad network id");
-  *step = ag->net[net].adam_t;
+  *step = ag->adam_t[net];
   GCRL_API_END
 }
 int gcrl_agent_set_adam_step(gcrl_agent *ag, int net, int step) {
   GCRL_API_BEGIN
   require_handle(ag);
   GCRL_REQUIRE(ag && step >= 0 && net >= 0 && net < NUM_NETS && ag->has[net] && ag->net[net].m, "bad network id");
-  ag->net[net].adam_t = step;
+  ag->adam_t[net] = step;
   GCRL_API_END
 }
 
@@ -1279,11 +1199,12 @@ int gcrl_agent_hard_update(gcrl_agent *ag, void *stream) {
   const int pairs[3][2] = {{T_ACTOR, ACTOR}, {T_CRITIC1, CRITIC1}, {T_CRITIC2, CRITIC2}};
   for (auto &pr : pairs)
     if (ag->has[pr[0]]) {
-      GCRL_CUDA(cudaMemcpyAsync(ag->net[pr[0]].p, ag->net[pr[1]].p, size_t(ag->net[pr[1]].total) * 4,
-                                cudaMemcpyDeviceToDevice, st));
-      GCRL_CUDA(cudaMemcpyAsync(ag->net[pr[0]].pT, ag->net[pr[1]].pT, size_t(ag->net[pr[1]].total_t) * 4,
-                                cudaMemcpyDeviceToDevice, st));
-      ag->net[pr[0]].split_stale = true;
+      MlpParams &t = ag->net[pr[0]];
+      const MlpParams &src = ag->net[pr[1]];
+      GCRL_CUDA(cudaMemcpyAsync(t.p, src.p, size_t(src.total) * 4, cudaMemcpyDeviceToDevice, st));
+      GCRL_CUDA(cudaMemcpyAsync(t.copies.pT, src.copies.pT, size_t(src.copies.total_t) * 4, cudaMemcpyDeviceToDevice,
+                                st));
+      t.copies.stale = true;
     }
   GCRL_API_END
 }
@@ -1300,10 +1221,10 @@ int gcrl_agent_soft_update(gcrl_agent *ag, int which, double tau, void *stream) 
   const int pairs[3][3] = {{T_ACTOR, ACTOR, 1}, {T_CRITIC1, CRITIC1, 2}, {T_CRITIC2, CRITIC2, 2}};
   for (auto &pr : pairs)
     if ((which & pr[2]) && ag->has[pr[0]]) {
-      Net &t = ag->net[pr[0]];
-      const Net &srcn = ag->net[pr[1]];
-      launch_polyak(t.p, srcn.p, srcn.total, float(tau), float(1.0 - tau), srcn.tmap, t.pT, st);
-      t.split_stale = true;
+      MlpParams &t = ag->net[pr[0]];
+      const MlpParams &srcn = ag->net[pr[1]];
+      launch_polyak(t.p, srcn.p, srcn.total, float(tau), float(1.0 - tau), srcn.copies.tmap, t.copies.pT, st);
+      t.copies.stale = true;
     }
   GCRL_API_END
 }
@@ -1318,7 +1239,7 @@ int gcrl_agent_reset_optim(gcrl_agent *ag, void *stream) {
     if (ag->has[i]) {
       GCRL_CUDA(cudaMemsetAsync(ag->net[i].m, 0, size_t(ag->net[i].total) * 4, st));
       GCRL_CUDA(cudaMemsetAsync(ag->net[i].v, 0, size_t(ag->net[i].total) * 4, st));
-      ag->net[i].adam_t = 0;
+      ag->adam_t[i] = 0;
     }
   GCRL_API_END
 }
@@ -1411,7 +1332,7 @@ int gcrl_agent_act(gcrl_agent *ag, int64_t n, const float *obs_host, float *act_
   // uses the actor-phase scratch (spi / acts_actor): select_action never overlaps an update
   launch_pack_rows(obs, D, nullptr, A, ag->spi, ag->ldc, int(n), st);
   if (engine_tc(ag, int(n))) ensure_split(ag, st);
-  const Net &actor = ag->net[ACTOR];
+  const MlpParams &actor = ag->net[ACTOR];
   forward_hidden(ag, actor, ag->spi, ag->ldc, D, ag->acts_actor, int(n), st);
   float *out = ag->d_io + size_t(n) * D;
   launch_head_fwd(ag->acts_actor.h[L - 1], ag->ldh, actor.W(L), actor.ldw[L], actor.b(L), out, A, 0, int(n),
@@ -1435,7 +1356,7 @@ int gcrl_agent_q(gcrl_agent *ag, int64_t n, const float *obs_host, const float *
   float *act = stage_to_device(ag, act_host, size_t(n) * A, size_t(n) * D, st);
   launch_pack_rows(obs, D, act, A, ag->spi, ag->ldc, int(n), st);
   if (engine_tc(ag, int(n))) ensure_split(ag, st);
-  const Net &c = ag->net[CRITIC1];
+  const MlpParams &c = ag->net[CRITIC1];
   forward_hidden(ag, c, ag->spi, ag->ldc, D + A, ag->acts_c1, int(n), st);
   float *out = ag->d_io + size_t(n) * (D + A);
   launch_head_fwd(ag->acts_c1.h[L - 1], ag->ldh, c.W(L), c.ldw[L], c.b(L), out, 1, 0, int(n), ag->H, 1, 0, st);

@@ -75,7 +75,9 @@ __host__ __device__ inline int64_t feistel_position(uint64_t x, uint64_t n, uint
   const uint32_t keys[4] = {uint32_t(k0), uint32_t(k0 >> 32), uint32_t(k1), uint32_t(k1 >> 32)};
   do {
     uint32_t L = uint32_t(x >> half) & mask, R = uint32_t(x) & mask;
+#ifdef __CUDA_ARCH__   // (the host compiler does not know the pragma and warns)
 #pragma unroll
+#endif
     for (int r = 0; r < 4; ++r) {
       uint32_t nl = R;
       R = L ^ (mix32(R ^ keys[r]) & mask);

@@ -21,12 +21,12 @@
 #include "buffer_api.cuh"
 #include "graphs.cuh"
 #include "mlp.cuh"
+#include "params.cuh"
 
 using namespace gcrl;
 
 namespace {
 
-inline int pad4(int x) { return (x + 3) & ~3; }
 constexpr int kMaxCritics = 8;
 constexpr int kSplits = 128;
 constexpr int kEnsembleBatchMax = 4096;   // up to this batch the ensemble's backward passes share their launches
@@ -573,99 +573,8 @@ __global__ void alpha_step_kernel(const float *__restrict__ mean_in, const float
 }
 
 
-// ---- parameter containers ----------------------------------------------------------------------
-// Weight copies of the tensor-core engine (precision >= 1): the TF32 hi / lo halves of the flat parameter buffer (the
-// forward operand arrives pre-split, tc_gemm.cu) and, for the listed Linear layers of a trainable network, a
-// transposed copy W^T[in][ldt] with its halves (the K-major operand of the input gradient dX = dZ W).  The optimiser
-// writes W^T through tmap with every step; the halves are refreshed after every optimiser / Polyak step of an update
-// that runs on the tensor cores, and before an update after weights changed in any other way (`stale`).
-struct TcCopies {
-  std::vector<int> t_off, ldt;   // per Linear layer (-1: no transposed copy)
-  int total = 0, total_t = 0;
-  int *tmap = nullptr;           // [total] -> index into pT, -1 elsewhere; nullptr when nothing is transposed
-  float *pT = nullptr, *p_hi = nullptr, *p_lo = nullptr, *pT_hi = nullptr, *pT_lo = nullptr;
-  bool stale = true;
-  // transpose: (Linear index, w_off, rows, cols, ldw) of the layers whose input gradient runs on the tensor cores
-  void init(int total_, int nlinear, const std::vector<std::vector<int>> &transpose) {
-    total = total_;
-    t_off.assign(size_t(nlinear), -1);
-    ldt.assign(size_t(nlinear), 0);
-    p_hi = dev_alloc<float>(total); p_lo = dev_alloc<float>(total);
-    if (transpose.empty()) return;
-    std::vector<int> map(size_t(total), -1);
-    for (const auto &t : transpose) {
-      const int l = t[0], w_off = t[1], rows = t[2], cols = t[3], ldw = t[4];
-      ldt[l] = pad4(rows);
-      t_off[l] = total_t;
-      for (int o = 0; o < rows; ++o)
-        for (int i = 0; i < cols; ++i) map[size_t(w_off) + size_t(o) * ldw + i] = total_t + i * ldt[l] + o;
-      total_t += cols * ldt[l];
-    }
-    tmap = dev_alloc<int>(total);
-    GCRL_CUDA(cudaMemcpy(tmap, map.data(), size_t(total) * sizeof(int), cudaMemcpyHostToDevice));
-    pT = dev_alloc<float>(total_t);
-    GCRL_CUDA(cudaMemset(pT, 0, size_t(total_t) * 4));
-    pT_hi = dev_alloc<float>(total_t); pT_lo = dev_alloc<float>(total_t);
-  }
-  bool on() const { return p_hi != nullptr; }
-  void split(const float *p, cudaStream_t st) {
-    launch_split_tf32(p, p_hi, p_lo, total, st);
-    if (pT != nullptr) launch_split_tf32(pT, pT_hi, pT_lo, total_t, st);
-  }
-  // weights written from outside an update: W^T follows now, the halves before the next tensor-core update
-  void weights_changed(const float *p, cudaStream_t st) {
-    if (!on()) return;
-    if (tmap != nullptr) launch_sync_transposed(p, pT, tmap, total, st);
-    stale = true;
-  }
-  void destroy() { for (void *q : {(void *)tmap, (void *)pT, (void *)p_hi, (void *)p_lo, (void *)pT_hi, (void *)pT_lo}) if (q) cudaFree(q); }
-};
-
-struct CriticNet {
-  int layers = 0;
-  std::vector<int> in_d, out_d, ldw, w_off, b_off;
-  int total = 0;
-  float *p = nullptr, *g = nullptr, *m = nullptr, *v = nullptr;
-  TcCopies tc;
-  void init(int in, int hid, int L, bool trainable, float *grad_store = nullptr) {
-    layers = L + 1;
-    int off = 0;
-    for (int l = 0; l < layers; ++l) {
-      in_d.push_back(l == 0 ? in : hid);
-      out_d.push_back(l == layers - 1 ? 1 : hid);
-      ldw.push_back(pad4(in_d[l]));
-      w_off.push_back(off); off += out_d[l] * ldw[l];
-      b_off.push_back(off); off += pad4(out_d[l]);
-    }
-    total = off;
-    p = dev_alloc<float>(total);
-    GCRL_CUDA(cudaMemset(p, 0, size_t(total) * 4));
-    if (trainable) {
-      for (float **q : {&m, &v}) { *q = dev_alloc<float>(total); GCRL_CUDA(cudaMemset(*q, 0, size_t(total) * 4)); }
-      g = grad_store;          // slice of gcrl_sac::critic_grads (one all-reduce covers the ensemble)
-    }
-  }
-  static int layout_total(int in, int hid, int L) {
-    int off = 0;
-    for (int l = 0; l <= L; ++l) {
-      const int i = l == 0 ? in : hid, o = l == L ? 1 : hid;
-      off += o * pad4(i) + pad4(o);
-    }
-    return off;
-  }
-  // tensor-core engine: halves of every critic; W^T of the hidden layers 1..L-1 of a trainable one (the input
-  // gradient of layer 0 is only needed at the action columns, action_grad_acc_kernel)
-  void init_tc(bool trainable) {
-    std::vector<std::vector<int>> tr;
-    if (trainable)
-      for (int l = 1; l < layers - 1; ++l) tr.push_back({l, w_off[l], out_d[l], in_d[l], ldw[l]});
-    tc.init(total, layers, tr);
-  }
-  void destroy() { for (float *q : {p, m, v}) if (q) cudaFree(q); tc.destroy(); }
-  const float *W(int l) const { return p + w_off[l]; }
-  const float *b(int l) const { return p + b_off[l]; }
-};
-
+// ---- actor parameters ----------------------------------------------------------------------------
+// A layout of its own (BatchNorm parameters, two heads); the critics are MlpParams (params.cuh).
 struct ActorNet {
   int L = 0, D = 0, H = 0, A = 0, ldh = 0;
   std::vector<int> ldw, w_off, b_off, gam_off, bet_off;     // hidden layers
@@ -673,11 +582,11 @@ struct ActorNet {
   int total = 0;
   float *p = nullptr, *g = nullptr, *m = nullptr, *v = nullptr;
   float *rmean = nullptr, *rvar = nullptr;                  // [L][ldh]
-  TcCopies tc;
-  void init_tc() {                                          // W^T of the hidden Linears 1..L-1 (input gradients)
-    std::vector<std::vector<int>> tr;
+  WeightCopies copies;
+  void init_copies() {                                      // W^T of the hidden Linears 1..L-1 (input gradients)
+    std::vector<WeightCopies::Linear> tr;
     for (int l = 1; l < L; ++l) tr.push_back({l, w_off[l], H, H, ldw[l]});
-    tc.init(total, L, tr);
+    copies.init(total, L, tr, true);
   }
   void init(int D_, int H_, int A_, int L_) {
     L = L_; D = D_; H = H_; A = A_; ldh = pad4(H);
@@ -706,7 +615,7 @@ struct ActorNet {
     for (int l = 0; l < L; ++l)   // BatchNorm weight = 1 (torch default)
       GCRL_CUDA(cudaMemcpy(p + gam_off[l], ones.data(), size_t(H) * 4, cudaMemcpyHostToDevice));
   }
-  void destroy() { for (float *q : {p, g, m, v, rmean}) if (q) cudaFree(q); tc.destroy(); }
+  void destroy() { for (float *q : {p, g, m, v, rmean}) if (q) cudaFree(q); copies.destroy(); }
 };
 
 }  // namespace
@@ -718,7 +627,7 @@ struct gcrl_sac {
   int D = 0, A = 0, H = 0, L = 0, n = 0, keep = 0, ldh = 0, ldc = 0;
   int64_t maxB = 0;
   ActorNet actor;
-  CriticNet critic[kMaxCritics], target[kMaxCritics];
+  MlpParams critic[kMaxCritics], target[kMaxCritics];
   int adam_t_c = 0, adam_t_a = 0, adam_t_alpha = 0;
   int dp_B = -1, dp_flags = -1;                  // the update the data-parallel phases belong to
   bool dp_open = false;                          // a phase-wise data-parallel update: phase 0 issued, phase 3 not yet
@@ -805,25 +714,17 @@ bool use_tc(const gcrl_sac *ag, int B, int N, int K) {
 // every hidden-layer shape of an update passes the same test (K = padded input widths, all multiples of 4)
 bool engine_tc(const gcrl_sac *ag, int B) { return use_tc(ag, B, ag->H, ag->ldh); }
 
-template <class F>
-void for_each_tc(gcrl_sac *ag, F f) {
-  f(ag->actor.tc, ag->actor.p);
-  for (int i = 0; i < ag->n; ++i) {
-    f(ag->critic[i].tc, ag->critic[i].p);
-    f(ag->target[i].tc, ag->target[i].p);
-  }
-}
 // eager, outside capture: the halves of every network whose weights changed since they were last split
 void ensure_split(gcrl_sac *ag, cudaStream_t st) {
-  for_each_tc(ag, [&](TcCopies &tc, const float *p) {
-    if (tc.on() && tc.stale) {
-      tc.split(p, st);
-      tc.stale = false;
-    }
-  });
+  ag->actor.copies.split_if_stale(ag->actor.p, st);
+  for (int i = 0; i < ag->n; ++i) {
+    ag->critic[i].copies.split_if_stale(ag->critic[i].p, st);
+    ag->target[i].copies.split_if_stale(ag->target[i].p, st);
+  }
 }
 void mark_split_stale(gcrl_sac *ag) {
-  for_each_tc(ag, [](TcCopies &tc, const float *) { tc.stale = true; });
+  ag->actor.copies.stale = true;
+  for (int i = 0; i < ag->n; ++i) ag->critic[i].copies.stale = ag->target[i].copies.stale = true;
 }
 
 // partial weight / bias gradients of one hidden Linear [H][ldw] on input X[B][K] (K: padded for layer 0)
@@ -841,7 +742,7 @@ void critics_dgrad_tc(gcrl_sac *ag, int first, int m, int l, float *const *dz_in
                       cudaStream_t st) {
   TcDenseProblem pr[kMaxBatchedLinear];
   for (int j = 0; j < m; ++j) {
-    const TcCopies &tc = ag->critic[first + j].tc;
+    const WeightCopies &tc = ag->critic[first + j].copies;
     pr[j] = TcDenseProblem{dz_in[j], ag->ldh, tc.pT_hi + tc.t_off[l], tc.pT_lo + tc.t_off[l], tc.ldt[l], nullptr,
                            ag->ch[first + j][l - 1], dz_out[j]};
   }
@@ -851,15 +752,15 @@ void critics_dgrad_tc(gcrl_sac *ag, int first, int m, int l, float *const *dz_in
 // The whole ensemble on the same input rows: one launch per layer (blockIdx.z = critic, or the members of the
 // tensor-core ensemble launch) instead of n.
 // Activations land in ag->ch[i][l] (the caches of the backward pass, or plain scratch for the targets).
-void critics_fwd(gcrl_sac *ag, const CriticNet *nets, const float *X, float *q_out, int B, cudaStream_t st) {
+void critics_fwd(gcrl_sac *ag, const MlpParams *nets, const float *X, float *q_out, int B, cudaStream_t st) {
   const int n = ag->n, L = ag->L;
   LinearFwdProblem pr[kMaxBatchedLinear];
   TcDenseProblem tp[kMaxBatchedLinear];
   for (int l = 0; l < L; ++l) {
     if (ag->tc_update) {      // layer 0: K = ldc, the operand rows [s | a | 0] and the weight rows are zero-padded
       for (int i = 0; i < n; ++i)
-        tp[i] = TcDenseProblem{l == 0 ? X : ag->ch[i][l - 1], l == 0 ? ag->ldc : ag->ldh, nets[i].tc.p_hi + nets[i].w_off[l],
-                               nets[i].tc.p_lo + nets[i].w_off[l], nets[i].ldw[l], nets[i].b(l), nullptr, ag->ch[i][l]};
+        tp[i] = TcDenseProblem{l == 0 ? X : ag->ch[i][l - 1], l == 0 ? ag->ldc : ag->ldh, nets[i].copies.p_hi + nets[i].w_off[l],
+                               nets[i].copies.p_lo + nets[i].w_off[l], nets[i].ldw[l], nets[i].b(l), nullptr, ag->ch[i][l]};
       launch_tc_dense_ensemble(tp, n, 0, ag->ldh, B, ag->H, l == 0 ? ag->ldc : ag->H, 0, st);
       continue;
     }
@@ -882,8 +783,8 @@ void actor_fwd(gcrl_sac *ag, float *rows, const float *eps, int B, bool train, b
   int ldin = ag->ldc, K = ag->D;
   for (int l = 0; l < ag->L; ++l) {
     if (train && ag->tc_update)       // (select_action, train == false, stays on the fp32 path)
-      launch_tc_dense(in, ldin, a.tc.p_hi + a.w_off[l], a.ldw[l], a.p + a.b_off[l], nullptr, 0, ag->xhat[l], ag->ldh, B,
-                      ag->H, pad4(K), 2, st, a.tc.p_lo + a.w_off[l]);
+      launch_tc_dense(in, ldin, a.copies.p_hi + a.w_off[l], a.ldw[l], a.p + a.b_off[l], nullptr, 0, ag->xhat[l], ag->ldh, B,
+                      ag->H, pad4(K), 2, st, a.copies.p_lo + a.w_off[l]);
     else
       launch_linear_fwd(in, ldin, a.p + a.w_off[l], a.ldw[l], a.p + a.b_off[l], ag->xhat[l], ag->ldh, B, ag->H, K,
                         ACT_NONE, st);
@@ -920,7 +821,7 @@ void actor_fwd(gcrl_sac *ag, float *rows, const float *eps, int B, bool train, b
   GCRL_LAUNCHED();
 }
 
-void reduce_critic(gcrl_sac *ag, CriticNet &c, const int *splits, int head_splits, cudaStream_t st,
+void reduce_critic(gcrl_sac *ag, MlpParams &c, const int *splits, int head_splits, cudaStream_t st,
                    const float *partials = nullptr) {
   if (partials == nullptr) partials = ag->partials;
   ReduceArgs r{};
@@ -937,7 +838,7 @@ void reduce_critic(gcrl_sac *ag, CriticNet &c, const int *splits, int head_split
 
 // tc / ttc: the tensor-core copies of the network and of its target (no W^T: targetT stays nullptr)
 void adam(gcrl_sac *ag, float *p, float *m, float *v, const float *g, int total, int which, float *target,
-          bool polyak, int slot_norm, cudaStream_t st, TcCopies &tc, TcCopies *ttc) {
+          bool polyak, int slot_norm, cudaStream_t st, WeightCopies &tc, WeightCopies *ttc) {
   AdamArgs a{};
   a.p = p; a.m = m; a.v = v; a.g = g; a.n = total;
   a.sumsq_partials = ag->sumsq; a.nsumsq = reduce_grid(total);
@@ -956,8 +857,9 @@ void adam(gcrl_sac *ag, float *p, float *m, float *v, const float *g, int total,
 }
 
 void adam_critic(gcrl_sac *ag, int i, int flags, cudaStream_t st) {
-  CriticNet &c = ag->critic[i];
-  adam(ag, c.p, c.m, c.v, c.g, c.total, 0, ag->target[i].p, (flags & 2) != 0, M_CGN + i, st, c.tc, &ag->target[i].tc);
+  MlpParams &c = ag->critic[i];
+  adam(ag, c.p, c.m, c.v, c.g, c.total, 0, ag->target[i].p, (flags & 2) != 0, M_CGN + i, st, c.copies,
+       &ag->target[i].copies);
 }
 
 // sums of squares of an (averaged) flat gradient that is already in place
@@ -996,7 +898,7 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     // input-gradient launch per layer (per-critic gradient buffers and partial sets), then reduce + AdamW per critic
     HeadBwdArgs hs[kMaxBatchedLinear];
     for (int i = 0; i < n; ++i) {
-      const CriticNet &c = ag->critic[i];
+      const MlpParams &c = ag->critic[i];
       float *part = ag->partials + int64_t(i) * ag->pset;
       HeadBwdArgs h{};
       h.mode = 0; h.loss_kind = 0; h.clamp_y = 0; h.nout = 1;
@@ -1017,7 +919,7 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     for (int l = L - 1; l >= 0; --l) {
       WgradProblem wp[kMaxWgradProblems];
       for (int i = 0; i < n; ++i) {
-        const CriticNet &c = ag->critic[i];
+        const MlpParams &c = ag->critic[i];
         float *part = ag->partials + int64_t(i) * ag->pset;
         wp[i] = WgradProblem{ag->dzc[2 * i + cur], ag->ldh, l == 0 ? ag->sa : ag->ch[i][l - 1], l == 0 ? ag->ldc : ag->ldh,
                              part + c.w_off[l], c.ldw[l], part + c.b_off[l], ag->H, l == 0 ? K0 : ag->H};
@@ -1036,7 +938,7 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
       } else if (l > 0) {
         LinearDgradProblem dg[kMaxBatchedLinear];
         for (int i = 0; i < n; ++i) {
-          const CriticNet &c = ag->critic[i];
+          const MlpParams &c = ag->critic[i];
           dg[i] = LinearDgradProblem{ag->dzc[2 * i + cur], ag->ldh, c.W(l), c.ldw[l], ag->ch[i][l - 1], ag->ldh,
                                      ag->dzc[2 * i + (cur ^ 1)], ag->ldh};
         }
@@ -1045,13 +947,13 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
       }
     }
     for (int i = 0; i < n; ++i) {
-      CriticNet &c = ag->critic[i];
+      MlpParams &c = ag->critic[i];
       reduce_critic(ag, c, splits, head_splits, st, ag->partials + int64_t(i) * ag->pset);
       if (!dp) adam_critic(ag, i, flags, st);
     }
   } else
   for (int i = 0; i < n; ++i) {
-    CriticNet &c = ag->critic[i];
+    MlpParams &c = ag->critic[i];
     HeadBwdArgs h{};
     h.mode = 0; h.loss_kind = 0; h.clamp_y = 0; h.nout = 1;
     h.q = ag->q + int64_t(i) * ag->maxB; h.y_in = ag->y;
@@ -1088,7 +990,7 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   if (ag->seg_build != nullptr) seg_cut(ag, COLL_AVG_CRITIC);
   if (dp && (mask & PH_CSTEP)) {
     for (int i = 0; i < n; ++i) {
-      CriticNet &c = ag->critic[i];
+      MlpParams &c = ag->critic[i];
       rereduce(ag, c.g, c.total, st);
       adam_critic(ag, i, flags, st);
     }
@@ -1114,7 +1016,7 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   if (B <= kEnsembleBatchMax) {        // the ensemble's input-gradient chains share their launches
     HeadBwdArgs hs[kMaxBatchedLinear];
     for (int i = 0; i < n; ++i) {
-      const CriticNet &c = ag->critic[i];
+      const MlpParams &c = ag->critic[i];
       HeadBwdArgs h{};
       h.mode = 2; h.nout = 1; h.dz_in = ag->dq + int64_t(i) * ag->maxB * 4;
       h.Hact = ag->ch[i][L - 1]; h.ldh = ag->ldh;
@@ -1136,7 +1038,7 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
       }
       LinearDgradProblem dg[kMaxBatchedLinear];
       for (int i = 0; i < n; ++i) {
-        const CriticNet &c = ag->critic[i];
+        const MlpParams &c = ag->critic[i];
         dg[i] = LinearDgradProblem{ag->dzc[2 * i + cur], ag->ldh, c.W(l), c.ldw[l], ag->ch[i][l - 1], ag->ldh,
                                    ag->dzc[2 * i + (cur ^ 1)], ag->ldh};
       }
@@ -1144,14 +1046,14 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
       cur ^= 1;
     }
     for (int i = 0; i < n; ++i) {                // summed over the critics in index order
-      const CriticNet &c = ag->critic[i];
+      const MlpParams &c = ag->critic[i];
       action_grad_acc_kernel<<<blocks_for(B, 8), 256, 0, st>>>(ag->dzc[2 * i + cur], ag->ldh, c.W(0), c.ldw[0], D,
                                                               ag->dact, B, ag->H, A, i > 0 ? 1 : 0);
       GCRL_LAUNCHED();
     }
   } else
   for (int i = 0; i < n; ++i) {
-    const CriticNet &c = ag->critic[i];
+    const MlpParams &c = ag->critic[i];
     HeadBwdArgs h{};
     h.mode = 2; h.nout = 1; h.dz_in = ag->dq + int64_t(i) * ag->maxB * 4;
     h.Hact = ag->ch[i][L - 1]; h.ldh = ag->ldh;
@@ -1214,8 +1116,8 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
                              ag->partials + a.b_off[l], B, st);
     if (l > 0) {
       if (ag->tc_update)      // bare product: bn_bwd applies ReLU' itself
-        launch_tc_dense(ag->dz[cur], ag->ldh, a.tc.pT_hi + a.tc.t_off[l], a.tc.ldt[l], nullptr, nullptr, 0,
-                        ag->dz[cur ^ 1], ag->ldh, B, ag->H, ag->H, 3, st, a.tc.pT_lo + a.tc.t_off[l]);
+        launch_tc_dense(ag->dz[cur], ag->ldh, a.copies.pT_hi + a.copies.t_off[l], a.copies.ldt[l], nullptr, nullptr, 0,
+                        ag->dz[cur ^ 1], ag->ldh, B, ag->H, ag->H, 3, st, a.copies.pT_lo + a.copies.t_off[l]);
       else
         launch_linear_dgrad(ag->dz[cur], ag->ldh, a.p + a.w_off[l], a.ldw[l], nullptr, 0, ag->dz[cur ^ 1], ag->ldh, B,
                             ag->H, ag->H, st);
@@ -1244,7 +1146,7 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   if (ag->seg_build != nullptr) seg_cut(ag, COLL_AVG_ACTOR);
   if (mask & PH_ASTEP) {
     if (dp) rereduce(ag, a.g, a.total, st);
-    adam(ag, a.p, a.m, a.v, a.g, a.total, 1, nullptr, false, M_AGN, st, a.tc, nullptr);
+    adam(ag, a.p, a.m, a.v, a.g, a.total, 1, nullptr, false, M_AGN, st, a.copies, nullptr);
     if (flags & 4) {
       alpha_step_kernel<<<1, 1, 0, st>>>(a.g + a.total, reinterpret_cast<const float *>(ag->d_scalars + 1),
                                         ag->alpha_state, ag->mdev + M_ALPHA_LOSS);
@@ -1554,18 +1456,6 @@ void read_many_rows(gcrl_sac *ag, int n, int64_t B, const int *flags, float *met
   if (td_host != nullptr) std::memcpy(td_host, rows.data() + m, size_t(n) * B * sizeof(float));
 }
 
-void upload_padded(float *dst, const float *w, int rows, int cols, int ld, cudaStream_t st) {
-  std::vector<float> padded(size_t(rows) * ld, 0.f);
-  for (int r = 0; r < rows; ++r) std::memcpy(&padded[size_t(r) * ld], w + size_t(r) * cols, size_t(cols) * 4);
-  GCRL_CUDA(cudaMemcpyAsync(dst, padded.data(), padded.size() * 4, cudaMemcpyHostToDevice, st));
-  GCRL_CUDA(cudaStreamSynchronize(st));
-}
-void download_padded(float *w, const float *src, int rows, int cols, int ld, cudaStream_t st) {
-  std::vector<float> padded(size_t(rows) * ld);
-  GCRL_CUDA(cudaMemcpyAsync(padded.data(), src, padded.size() * 4, cudaMemcpyDeviceToHost, st));
-  GCRL_CUDA(cudaStreamSynchronize(st));
-  for (int r = 0; r < rows; ++r) std::memcpy(w + size_t(r) * cols, &padded[size_t(r) * ld], size_t(cols) * 4);
-}
 
 // (rows, cols, ld, weight offset, bias offset) of actor Linear `layer`
 void actor_linear_geom(const gcrl_sac *ag, int layer, int *rows, int *cols, int *ld, int *woff, int *boff) {
@@ -1678,12 +1568,13 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
     const int D = ag->D, A = ag->A, H = ag->H, L = ag->L, n = ag->n;
     const size_t mb = size_t(ag->maxB), act = mb * ag->ldh;
     ag->actor.init(D, H, A, L);
-    ag->critic_stride = CriticNet::layout_total(D + A, H, L);
+    for (int i = 0; i < n; ++i) { ag->critic[i].layout(D + A, H, 1, L); ag->target[i].layout(D + A, H, 1, L); }
+    ag->critic_stride = ag->critic[0].total;
     ag->critic_grads = dev_alloc<float>(size_t(n) * ag->critic_stride);
     GCRL_CUDA(cudaMemset(ag->critic_grads, 0, size_t(n) * ag->critic_stride * 4));
-    for (int i = 0; i < n; ++i) {
-      ag->critic[i].init(D + A, H, L, true, ag->critic_grads + size_t(i) * ag->critic_stride);
-      ag->target[i].init(D + A, H, L, false);
+    for (int i = 0; i < n; ++i) {     // the critics' gradients: one buffer, so one all-reduce covers the ensemble
+      ag->critic[i].alloc(true, ag->critic_grads + size_t(i) * ag->critic_stride);
+      ag->target[i].alloc(false);
     }
     for (int l = 0; l < L; ++l) { ag->xhat.push_back(dev_alloc<float>(act)); ag->ah.push_back(dev_alloc<float>(act)); }
     ag->invstd = dev_alloc<float>(size_t(L) * ag->ldh);
@@ -1710,11 +1601,13 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
     GCRL_CUDA(cudaMemcpy(ag->alpha_state, init_alpha, sizeof(init_alpha), cudaMemcpyHostToDevice));
     ag->d_scalars = dev_alloc<StepScalars>(2);
     if (cfg->precision >= 1) {
+      // tensor-core engine: halves of every network; W^T of the hidden layers 1..L-1 of a trainable one (the input
+      // gradient of a critic's layer 0 is only needed at the action columns, action_grad_acc_kernel)
       tc_dense_init();
-      ag->actor.init_tc();
+      ag->actor.init_copies();
       for (int i = 0; i < n; ++i) {
-        ag->critic[i].init_tc(true);
-        ag->target[i].init_tc(false);
+        ag->critic[i].init_copies(1, L, true);
+        ag->target[i].init_copies(0, 0, true);
       }
     }
     GCRL_CUDA(cudaStreamCreateWithFlags(&ag->cap_stream, cudaStreamNonBlocking));
@@ -1764,9 +1657,9 @@ int gcrl_sac_set_actor_linear(gcrl_sac *ag, int layer, const float *w, const flo
   GCRL_CUDA(cudaSetDevice(ag->device));
   int rows, cols, ld, woff, boff;
   actor_linear_geom(ag, layer, &rows, &cols, &ld, &woff, &boff);
-  upload_padded(ag->actor.p + woff, w, rows, cols, ld, as_stream(stream));
-  upload_padded(ag->actor.p + boff, b, 1, rows, rows, as_stream(stream));
-  ag->actor.tc.weights_changed(ag->actor.p, as_stream(stream));
+  upload_rows(ag->actor.p + woff, w, rows, cols, ld, as_stream(stream));
+  upload_rows(ag->actor.p + boff, b, 1, rows, rows, as_stream(stream));
+  ag->actor.copies.weights_changed(ag->actor.p, as_stream(stream));
   GCRL_API_END
 }
 
@@ -1777,8 +1670,8 @@ int gcrl_sac_get_actor_linear(gcrl_sac *ag, int layer, float *w, float *b, void 
   GCRL_CUDA(cudaSetDevice(ag->device));
   int rows, cols, ld, woff, boff;
   actor_linear_geom(ag, layer, &rows, &cols, &ld, &woff, &boff);
-  if (w) download_padded(w, ag->actor.p + woff, rows, cols, ld, as_stream(stream));
-  if (b) download_padded(b, ag->actor.p + boff, 1, rows, rows, as_stream(stream));
+  if (w) download_rows(w, ag->actor.p + woff, rows, cols, ld, as_stream(stream));
+  if (b) download_rows(b, ag->actor.p + boff, 1, rows, rows, as_stream(stream));
   GCRL_API_END
 }
 
@@ -1790,10 +1683,10 @@ int gcrl_sac_set_actor_bn(gcrl_sac *ag, int layer, const float *weight, const fl
   GCRL_CUDA(cudaSetDevice(ag->device));
   cudaStream_t st = as_stream(stream);
   ActorNet &a = ag->actor;
-  if (weight) upload_padded(a.p + a.gam_off[layer], weight, 1, ag->H, ag->H, st);
-  if (bias) upload_padded(a.p + a.bet_off[layer], bias, 1, ag->H, ag->H, st);
-  if (rm) upload_padded(a.rmean + size_t(layer) * ag->ldh, rm, 1, ag->H, ag->H, st);
-  if (rv) upload_padded(a.rvar + size_t(layer) * ag->ldh, rv, 1, ag->H, ag->H, st);
+  if (weight) upload_rows(a.p + a.gam_off[layer], weight, 1, ag->H, ag->H, st);
+  if (bias) upload_rows(a.p + a.bet_off[layer], bias, 1, ag->H, ag->H, st);
+  if (rm) upload_rows(a.rmean + size_t(layer) * ag->ldh, rm, 1, ag->H, ag->H, st);
+  if (rv) upload_rows(a.rvar + size_t(layer) * ag->ldh, rv, 1, ag->H, ag->H, st);
   GCRL_API_END
 }
 
@@ -1804,10 +1697,10 @@ int gcrl_sac_get_actor_bn(gcrl_sac *ag, int layer, float *weight, float *bias, f
   GCRL_CUDA(cudaSetDevice(ag->device));
   cudaStream_t st = as_stream(stream);
   ActorNet &a = ag->actor;
-  if (weight) download_padded(weight, a.p + a.gam_off[layer], 1, ag->H, ag->H, st);
-  if (bias) download_padded(bias, a.p + a.bet_off[layer], 1, ag->H, ag->H, st);
-  if (rm) download_padded(rm, a.rmean + size_t(layer) * ag->ldh, 1, ag->H, ag->H, st);
-  if (rv) download_padded(rv, a.rvar + size_t(layer) * ag->ldh, 1, ag->H, ag->H, st);
+  if (weight) download_rows(weight, a.p + a.gam_off[layer], 1, ag->H, ag->H, st);
+  if (bias) download_rows(bias, a.p + a.bet_off[layer], 1, ag->H, ag->H, st);
+  if (rm) download_rows(rm, a.rmean + size_t(layer) * ag->ldh, 1, ag->H, ag->H, st);
+  if (rv) download_rows(rv, a.rvar + size_t(layer) * ag->ldh, 1, ag->H, ag->H, st);
   GCRL_API_END
 }
 
@@ -1816,12 +1709,12 @@ int gcrl_sac_set_critic_layer(gcrl_sac *ag, int critic, int target, int layer, c
   GCRL_API_BEGIN
   require_handle(ag);
   GCRL_REQUIRE(ag && w && b && critic >= 0 && critic < ag->n, "bad critic index / NULL data");
-  CriticNet &c = target ? ag->target[critic] : ag->critic[critic];
+  MlpParams &c = target ? ag->target[critic] : ag->critic[critic];
   GCRL_REQUIRE(layer >= 0 && layer < c.layers, "bad layer index");
   GCRL_CUDA(cudaSetDevice(ag->device));
-  upload_padded(c.p + c.w_off[layer], w, c.out_d[layer], c.in_d[layer], c.ldw[layer], as_stream(stream));
-  upload_padded(c.p + c.b_off[layer], b, 1, c.out_d[layer], c.out_d[layer], as_stream(stream));
-  c.tc.weights_changed(c.p, as_stream(stream));
+  upload_rows(c.p + c.w_off[layer], w, c.out_d[layer], c.in_d[layer], c.ldw[layer], as_stream(stream));
+  upload_rows(c.p + c.b_off[layer], b, 1, c.out_d[layer], c.out_d[layer], as_stream(stream));
+  c.copies.weights_changed(c.p, as_stream(stream));
   GCRL_API_END
 }
 
@@ -1829,11 +1722,11 @@ int gcrl_sac_get_critic_layer(gcrl_sac *ag, int critic, int target, int layer, f
   GCRL_API_BEGIN
   require_handle(ag);
   GCRL_REQUIRE(ag && critic >= 0 && critic < ag->n, "bad critic index");
-  CriticNet &c = target ? ag->target[critic] : ag->critic[critic];
+  MlpParams &c = target ? ag->target[critic] : ag->critic[critic];
   GCRL_REQUIRE(layer >= 0 && layer < c.layers, "bad layer index");
   GCRL_CUDA(cudaSetDevice(ag->device));
-  if (w) download_padded(w, c.p + c.w_off[layer], c.out_d[layer], c.in_d[layer], c.ldw[layer], as_stream(stream));
-  if (b) download_padded(b, c.p + c.b_off[layer], 1, c.out_d[layer], c.out_d[layer], as_stream(stream));
+  if (w) download_rows(w, c.p + c.w_off[layer], c.out_d[layer], c.in_d[layer], c.ldw[layer], as_stream(stream));
+  if (b) download_rows(b, c.p + c.b_off[layer], 1, c.out_d[layer], c.out_d[layer], as_stream(stream));
   GCRL_API_END
 }
 
@@ -1845,7 +1738,7 @@ int gcrl_sac_hard_update(gcrl_sac *ag, void *stream) {
   for (int i = 0; i < ag->n; ++i) {
     GCRL_CUDA(cudaMemcpyAsync(ag->target[i].p, ag->critic[i].p, size_t(ag->critic[i].total) * 4,
                               cudaMemcpyDeviceToDevice, as_stream(stream)));
-    ag->target[i].tc.weights_changed(ag->target[i].p, as_stream(stream));
+    ag->target[i].copies.weights_changed(ag->target[i].p, as_stream(stream));
   }
   GCRL_API_END
 }
