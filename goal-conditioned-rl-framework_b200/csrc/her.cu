@@ -18,7 +18,8 @@
 //
 // The sampler is a chain of dependent gathers, so its latency is the number of HBM round trips on that chain:
 // bucket record -> (packed row || future-offset word) -> future goal = 3 (round 1: header -> bucket -> episode
-// record -> binary search -> two rounds of row loads -> future goal = 6-7).
+// record -> binary search -> two rounds of row loads -> future goal = 6-7).  Online relabelling and eager `final`
+// know the goal step after the bucket record, so there the goal gather runs beside the row gather: 2.
 #include <algorithm>
 #include <cstring>
 #include <deque>
@@ -160,7 +161,8 @@ her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg,
       }
     }
   }
-  // ---- round trip 3: the future achieved goal (issued before the barrier: it overlaps the tail of the gather)
+  // ---- round trip 3: the relabel goal (issued before the barrier: it overlaps the tail of the gather; where
+  //      her_resolve knew the goal step without the offset word, it does not depend on round trip 2)
   float gf[4] = {0.f, 0.f, 0.f, 0.f};
   const float *agf = nullptr;
   if (tid < n && ref.j > 0) {
@@ -177,8 +179,7 @@ her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg,
     float *row = tile + tid * g.row_f;
     if (g.G <= 4) {
       her_relabel_row(g, row, gf);
-    } else {                       // wide goals: the future goal is staged behind the (already consumed) future offsets
-      float *tmp = row + g.off_fut;
+    } else {                       // wide goals: read from the compact copy one column at a time
       float acc = 0.f;
       for (int c = 0; c < g.G; ++c) {
         const float gfc = __ldg(agf + c);
@@ -188,7 +189,6 @@ her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg,
         row[g.D - g.G + c] = gfc;
         row[g.off_ns + g.D - g.G + c] = gfc;
       }
-      (void)tmp;
       const float dist = __fsqrt_rn(acc);
       reinterpret_cast<uint32_t *>(row)[g.off_r] = 0x80000000u | ((dist > g.threshold) ? 0x3F800000u : 0u);
       row[g.off_d] = 0.0f;
@@ -220,7 +220,7 @@ struct gcrl_her {
   int64_t total_entries = 0, total_tr = 0, next_eid = 0, ep_first = 0, tr_live_first = 0;
   std::deque<std::pair<int64_t, int>> live;  // (entry_end, T) of live episodes, oldest first
   uint64_t seed = 0, host_ctr = 0;
-  unsigned long long draw_epoch = 0;         // device index stream: one epoch per launch that draws its own positions
+  unsigned long long draw_epoch = 0;         // one per launch that draws its own positions; online store: every launch
   PinnedRing stage;
   char *d_stage[PinnedRing::kSlots] = {};
   size_t blob_max = 0;
@@ -243,7 +243,8 @@ SampleScalars her_next_scalars(gcrl_her *h, bool positions_given) {
   sc.len = h->len();
   sc.draw_epoch = h->draw_epoch;
   sc.use_idx = positions_given ? 1 : 0;
-  if (!positions_given) h->draw_epoch += 1;     // device index stream: one epoch per draw
+  // device index stream: one epoch per draw; online relabelling draws its coins from the epoch on every call
+  if (!positions_given || h->g.online_k > 0) h->draw_epoch += 1;
   return sc;
 }
 const HerGeom &her_geom(const gcrl_her *h) { return h->g; }
@@ -334,7 +335,9 @@ int gcrl_her_create(gcrl_her **out, int device, int64_t max_entries, int64_t cap
   GCRL_REQUIRE(max_entries >= 1, "max_entries must be >= 1");
   GCRL_REQUIRE(goal_dim >= 1 && state_dim > goal_dim, "need state_dim > goal_dim >= 1");
   GCRL_REQUIRE(act_dim >= 1 && k_future >= 0 && k_future <= 64, "bad act_dim / k_future");
-  if (cap_transitions <= 0) cap_transitions = max_entries;
+  // the live window holds at most max_entries - 1 entries besides the oldest live episode's, which may keep up to
+  // 254 transitions whose entries are already evicted (a K = 0 / online store has one entry per transition)
+  if (cap_transitions <= 0) cap_transitions = max_entries + 254;
   GCRL_REQUIRE(cap_transitions < (int64_t(1) << 31), "cap_transitions must be < 2^31");
   GCRL_CUDA(cudaSetDevice(device));
   auto *h = new gcrl_her();
@@ -419,6 +422,7 @@ int gcrl_her_push_episode(gcrl_her *h, int T, const float *s, const float *a, co
   GCRL_REQUIRE(h != nullptr, "handle is NULL");
   GCRL_REQUIRE(T >= 1 && T <= 255, "episode length must be in [1, 255]");
   GCRL_REQUIRE(s && a && ns && r && d && ag, "NULL episode array");
+  GCRL_REQUIRE(fut == nullptr || h->g.online_k == 0, "an online-relabelling store draws its goals at sample time (fut must be NULL)");
   GCRL_CUDA(cudaSetDevice(h->device));
   const HerGeom &g = h->g;
   const int k = g.K;
@@ -468,13 +472,17 @@ int gcrl_her_push_episode(gcrl_her *h, int T, const float *s, const float *a, co
     std::memcpy(row + g.off_ag, ag + size_t(t) * g.G, size_t(g.G) * 4);
     uint8_t *fb = reinterpret_cast<uint8_t *>(row + g.off_fut);
     if (t < T - 1) {
+      // the strategy's goal range [lo, T-1]: future [t+1, T-1], final {T-1}, episode [0, T-1]
+      const int lo = g.strategy == GCRL_HER_EPISODE ? 0 : (g.strategy == GCRL_HER_FINAL ? T - 1 : t + 1);
       for (int j = 0; j < k; ++j) {
         int f;
         if (fut != nullptr) {
           f = fut[size_t(t) * k + j];
-          if (f <= t || f >= T) throw Error(GCRL_ERR_INVALID, "future index outside [t+1, T-1]");
+          if (f < lo || f >= T) throw Error(GCRL_ERR_INVALID, "relabel goal index outside the strategy's range");
+        } else if (lo == T - 1) {
+          f = lo;
         } else {
-          f = t + 1 + int(splitmix64(h->seed ^ (0xA5A5A5A5ull + h->host_ctr++)) % uint64_t(T - 1 - t));
+          f = lo + int(splitmix64(h->seed ^ (0xA5A5A5A5ull + h->host_ctr++)) % uint64_t(T - lo));
         }
         fb[j] = uint8_t(f);
       }
@@ -506,6 +514,28 @@ int gcrl_her_set_threshold(gcrl_her *h, float threshold) {
   GCRL_REQUIRE(h != nullptr, "handle is NULL");
   GCRL_REQUIRE(threshold >= 0.f, "the distance threshold must be >= 0");
   h->g.threshold = threshold;
+  GCRL_API_END
+}
+
+int gcrl_her_set_goal_selection(gcrl_her *h, int strategy, int online_k) {
+  GCRL_API_BEGIN
+  GCRL_REQUIRE(h != nullptr, "handle is NULL");
+  GCRL_REQUIRE(strategy == GCRL_HER_FUTURE || strategy == GCRL_HER_FINAL || strategy == GCRL_HER_EPISODE,
+               "unknown goal-selection strategy");
+  GCRL_REQUIRE(online_k >= 0 && online_k <= 64, "online_k must be in [0, 64]");
+  GCRL_REQUIRE(online_k == 0 || h->g.K == 0, "online relabelling needs a store created with k_future = 0");
+  GCRL_REQUIRE(h->next_eid == 0, "the goal selection cannot change once an episode has been committed");
+  h->g.strategy = strategy;
+  h->g.online_k = online_k;
+  GCRL_API_END
+}
+
+uint64_t gcrl_her_get_draw_epoch(const gcrl_her *h) { return h ? h->draw_epoch : 0; }
+
+int gcrl_her_set_draw_epoch(gcrl_her *h, uint64_t epoch) {
+  GCRL_API_BEGIN
+  GCRL_REQUIRE(h != nullptr, "handle is NULL");
+  h->draw_epoch = epoch;
   GCRL_API_END
 }
 

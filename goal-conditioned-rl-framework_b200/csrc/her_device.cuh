@@ -1,6 +1,7 @@
 // Device-side view of the HER episode store (csrc/her.cu), shared with the row-slab update kernel (fused.cu), which
-// samples its own rows: position -> (episode, t, j) -> packed row + future goal, the mapping SURVEY.md 8(a-3) proves
-// equal to apply_her entry for entry (reference src/buffer.py:143-179).
+// samples its own rows: position -> (episode, t, j) -> packed row + relabel goal, the mapping SURVEY.md 8(a-3) proves
+// equal to apply_her entry for entry (reference src/buffer.py:143-179).  Online relabelling (online_k > 0, a store
+// with K = 0) draws the relabel coin and goal step per sampled row instead (DESIGN.md section 2).
 #pragma once
 #include "common.cuh"
 
@@ -46,6 +47,8 @@ struct HerGeom {
   FastDiv div_k1, div_D, div_A, div_rf4;
   uint64_t seed;
   float threshold;          // sparse reward: -(||ag - g|| > threshold), 0.05 for the Panda tasks
+  int strategy;             // goal selection: GCRL_HER_FUTURE / _FINAL / _EPISODE
+  int online_k;             // > 0: online relabelling, each sampled row relabelled with probability k / (k + 1)
 };
 
 // totals by value (or through a small device struct for graph-captured consumers): the host mirrors the deque
@@ -88,8 +91,16 @@ __host__ __device__ inline int64_t feistel_position(uint64_t x, uint64_t n, uint
   return int64_t(x);
 }
 
+// Online relabelling: the 64-bit hash of (buffer seed, draw epoch, batch row i).  Row i is relabelled iff
+// h % (k + 1) != 0, to goal step lo + (h >> 32) % (T - lo) (lo = t + 1 for `future`, 0 for `episode`).
+__host__ __device__ inline uint64_t her_relabel_hash(uint64_t seed, uint64_t epoch, uint64_t i) {
+  return splitmix64(splitmix64(seed ^ 0x6A09E667F3BCC909ull ^ (epoch * 0xD1B54A32D192ED03ull)) + i);
+}
+
 // One sample: deque position -> bucket record -> (episode, t, j) -> ring slot.  `futw` receives the 4 packed
-// future offsets that contain this relabel's (j > 0), loaded here so that it travels with the row gather.
+// future offsets that contain this relabel's (j > 0), loaded here so that it travels with the row gather.  Where
+// the goal step f is known without that load (online mode, eager `final`), futw carries f in every byte instead
+// (online mode: j = 1 and f in the low byte), so her_future_slot reads it the same way.
 struct SampleRef {
   uint32_t slot, ep0, j, futw;
 };
@@ -124,11 +135,22 @@ __device__ __forceinline__ SampleRef her_resolve(const HerGeom &g, const SampleS
   uint32_t slot = tr_slot + t;
   if (slot >= g.cap_tr) slot -= g.cap_tr;
   SampleRef r{slot, tr_slot, j, 0u};
-  if (j > 0) r.futw = __ldg(reinterpret_cast<const uint32_t *>(g.rows + size_t(slot) * g.row_f + g.off_fut) + ((j - 1) >> 2));
+  if (g.online_k > 0) {            // K == 0 store: j == 0 above; the goal's slot is known after this round trip
+    const uint64_t h = her_relabel_hash(g.seed, sc.draw_epoch, uint64_t(i));
+    const uint32_t lo = g.strategy == GCRL_HER_EPISODE ? 0u : t + 1;
+    if (lo < T && h % uint64_t(g.online_k + 1) != 0) {
+      r.j = 1;
+      r.futw = g.strategy == GCRL_HER_FINAL ? T - 1 : lo + uint32_t(h >> 32) % (T - lo);
+    }
+  } else if (j > 0) {
+    r.futw = g.strategy == GCRL_HER_FINAL
+                 ? (T - 1) * 0x01010101u
+                 : __ldg(reinterpret_cast<const uint32_t *>(g.rows + size_t(slot) * g.row_f + g.off_fut) + ((j - 1) >> 2));
+  }
   return r;
 }
 
-// ring slot of the future transition whose achieved goal relabels this sample (j > 0)
+// ring slot of the transition whose achieved goal relabels this sample (j > 0)
 __device__ __forceinline__ uint32_t her_future_slot(const HerGeom &g, const SampleRef &r) {
   uint32_t fs = r.ep0 + ((r.futw >> (8 * ((r.j - 1) & 3))) & 0xffu);
   if (fs >= g.cap_tr) fs -= g.cap_tr;

@@ -19,6 +19,7 @@ class GcrlError(RuntimeError):
 
 
 OK, ERR_INVALID, ERR_UNDERFILLED, ERR_CUDA, ERR_CAPACITY = 0, 1, 2, 3, 4
+HER_FUTURE, HER_FINAL, HER_EPISODE = 0, 1, 2          # GCRL_HER_* goal-selection strategies
 
 c_i32, c_i64, c_u64, c_f32, c_f64 = C.c_int32, C.c_int64, C.c_uint64, C.c_float, C.c_double
 vp = C.c_void_p
@@ -52,6 +53,9 @@ SIGNATURES = {
     "gcrl_her_destroy": (C.c_int, [vp]),
     "gcrl_her_push_episode": (C.c_int, [vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp]),
     "gcrl_her_set_threshold": (C.c_int, [vp, C.c_float]),
+    "gcrl_her_set_goal_selection": (C.c_int, [vp, C.c_int, C.c_int]),
+    "gcrl_her_get_draw_epoch": (c_u64, [vp]),
+    "gcrl_her_set_draw_epoch": (C.c_int, [vp, c_u64]),
     "gcrl_her_len": (c_i64, [vp]),
     "gcrl_her_total_entries": (c_i64, [vp]),
     "gcrl_her_live_transitions": (c_i64, [vp]),

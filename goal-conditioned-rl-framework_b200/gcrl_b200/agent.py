@@ -117,11 +117,14 @@ class _AgentBase:
     WEIGHT_DECAY = 0.0
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, *,
-                 index_source="host", device=0, max_batch=None, seed=1898, precision=1):
+                 index_source="host", device=0, max_batch=None, seed=1898, precision=1,
+                 goal_selection_strategy="future", online_sampling=False):
         """precision: 1 (default) runs the hidden-layer GEMMs of batches >= 2048 on the tcgen05 tensor
         cores with the 3xTF32 split (fp32-level accuracy, rel ~2e-6 per layer); 2 does so for every
-        batch >= 128; 0 keeps every GEMM on the fp32 FFMA tiles."""
-        self._init_common(obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed)
+        batch >= 128; 0 keeps every GEMM on the fp32 FFMA tiles.
+        goal_selection_strategy / online_sampling: passed to the HER buffer (HERBuffer)."""
+        self._init_common(obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed,
+                          goal_selection_strategy, online_sampling)
         cfg = AgentConfig(algo=self.ALGO, state_dim=self.obs_dim, act_dim=self.ac_dim,
                           hidden_dim=config.hidden_dim, layer_count=config.layer_count,
                           max_batch=int(max_batch or config.batch_size), gamma=config.gamma,
@@ -135,7 +138,8 @@ class _AgentBase:
         self._max_batch = int(max_batch or config.batch_size)
         self._metrics = (C.c_float * 8)()
 
-    def _init_common(self, obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed):
+    def _init_common(self, obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed,
+                     goal_selection_strategy, online_sampling):
         _lib.require_cuda()
         self.device_index = int(device)
         self.device = f"cuda:{self.device_index}"
@@ -147,7 +151,8 @@ class _AgentBase:
         if config.buffer_type == "HER":
             self.buffer = HERBuffer(config.max_len, config.max_eps_len, nenvs,
                                     k_future=config.k_future, index_source=index_source,
-                                    seed=seed, device=device)
+                                    seed=seed, device=device, goal_selection_strategy=goal_selection_strategy,
+                                    online_sampling=online_sampling)
         elif config.buffer_type == "PER":                                  # src/agent.py:67-68
             self.buffer = PERBuffer(config.max_len, config.alpha, device=device)
         elif config.buffer_type == "REPLAY":                               # :69-70

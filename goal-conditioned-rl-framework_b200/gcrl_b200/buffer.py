@@ -11,7 +11,8 @@ from . import _lib
 from ._lib import check, lib, np_ptr, vp
 
 _FLUSH_LEN = 50  # the reference flushes on `done or len >= 50` (literal, src/buffer.py:117)
-_RANDINT_BOUNDS = {}  # (T, k) -> (lo, hi) arrays of apply_her's randint calls, in its draw order
+_RANDINT_BOUNDS = {}  # (T, k, strategy) -> (lo, hi) arrays of apply_her's randint calls, in its draw order
+_STRATEGIES = {"future": _lib.HER_FUTURE, "final": _lib.HER_FINAL, "episode": _lib.HER_EPISODE}
 
 
 def _to_np(x, dtype=np.float32):
@@ -36,13 +37,35 @@ class HERBuffer:
     PROBED on known-answer points around the threshold (as soon as the goal width is known) and must agree
     with that rule exactly; any other reward function raises ``ValueError`` instead of silently training on
     different rewards.  ``threshold`` (default 0.05, src/buffer.py:93) is passed to the kernel.
+
+    goal_selection_strategy (Andrychowicz et al. 2017): the step f whose achieved goal relabels a transition at
+    step t of an episode of T steps --
+      "future"  -- f in [t+1, T-1] (the reference's strategy, the default);
+      "final"   -- f = T-1;
+      "episode" -- f in [0, T-1].
+    online_sampling:
+      False -- each episode is expanded into the reference's deque entries (the original and, for t < T-1,
+               ``k_future`` relabelled copies whose f are drawn at commit: ``random.randint`` in apply_her's order
+               with the "host" index source, "final" draws nothing).
+      True  -- each transition is stored once (``len()`` counts transitions, so ``max_mem_len`` holds
+               ``k_future + 1`` times as many episodes) and every sampled row is relabelled with probability
+               k_future / (k_future + 1) to a freshly drawn f (none at t = T-1 for "future" / "final"): coin and f
+               come from a hash of (seed, draw epoch, batch row), drawn on the GPU whatever the index source.
     """
+    goal_selection_strategy = "future"
+    online_sampling = False
 
     def __init__(self, max_mem_len, max_eps_len, nenvs, threshold=0.05, k_future=4, *,
-                 index_source="host", seed=1898, cap_transitions=0, device=0):
+                 index_source="host", seed=1898, cap_transitions=0, device=0,
+                 goal_selection_strategy="future", online_sampling=False):
         _lib.require_cuda()
         if index_source not in ("host", "device"):
             raise ValueError(f"index_source must be 'host' or 'device', got {index_source!r}")
+        if goal_selection_strategy not in _STRATEGIES:
+            raise ValueError(f"goal_selection_strategy must be one of {sorted(_STRATEGIES)}, "
+                             f"got {goal_selection_strategy!r}")
+        if not isinstance(online_sampling, (bool, np.bool_)):
+            raise ValueError(f"online_sampling must be True or False, got {online_sampling!r}")
         if not 1 <= int(max_eps_len) <= 255:
             raise ValueError(f"max_eps_len must be in [1, 255] (future offsets are stored as uint8), got {max_eps_len}")
         if float(threshold) < 0:
@@ -58,6 +81,8 @@ class HERBuffer:
         self.obs_normalizer = None
         self.dg_normalizer = None
         self.index_source = index_source
+        self.goal_selection_strategy = goal_selection_strategy
+        self.online_sampling = bool(online_sampling)
         self.seed = int(seed)
         self.cap_transitions = int(cap_transitions)
         self._h = None
@@ -107,18 +132,29 @@ class HERBuffer:
     def _ensure(self, D, A, G):
         if self._h is None:
             h = vp()
-            check(lib.gcrl_her_create(C.byref(h), self.device_index, self.max_mem_len,
-                                      self.cap_transitions, D, G, A, self.k_future, self.seed))
+            # an online store holds each transition once: the K = 0 entry mapping, relabelled at sample time
+            check(lib.gcrl_her_create(C.byref(h), self.device_index, self.max_mem_len, self.cap_transitions, D, G, A,
+                                      self._stored_k(), self.seed))
             self._h, self._dims = h, (D, A, G)
             check(lib.gcrl_her_set_threshold(h, float(self.threshold)))
+            check(lib.gcrl_her_set_goal_selection(h, _STRATEGIES[self.goal_selection_strategy],
+                                                  self.k_future if self.online_sampling else 0))
         elif self._dims != (D, A, G):
             raise ValueError(f"transition shape changed: {self._dims} -> {(D, A, G)}")
         if not self._reward_checked:
             self._check_reward(G)
 
+    def _stored_k(self):
+        return 0 if self.online_sampling else self.k_future
+
     @property
     def handle(self):
         return self._h
+
+    @property
+    def draw_epoch(self):
+        """Sample calls drawn so far on the device index stream (online sampling: every sample call)."""
+        return int(lib.gcrl_her_get_draw_epoch(self._h)) if self._h else 0
 
     def _stream(self):
         return _lib.current_stream(self.device_index)
@@ -141,26 +177,33 @@ class HERBuffer:
         d = np.ascontiguousarray(d, np.float32).reshape(-1)
         ag = np.ascontiguousarray(ag, np.float32)
         T = s.shape[0]
+        if self.online_sampling and fut is not None:
+            raise ValueError("an online-sampling HERBuffer draws relabel goals at sample time: fut must be None")
         self._ensure(s.shape[1], a.shape[1], ag.shape[1])
-        if fut is None and self.index_source == "host" and self.k_future > 0:
+        k = self._stored_k()
+        if fut is None and self.index_source == "host" and k > 0:
             fut = self._draw_future(T)
         fptr = None
-        if fut is not None and self.k_future > 0:
-            fut = np.ascontiguousarray(fut, np.uint8).reshape(T, -1)[:, :self.k_future]
+        if fut is not None and k > 0:
+            fut = np.ascontiguousarray(fut, np.uint8).reshape(T, -1)[:, :k]
             fut = np.ascontiguousarray(fut)
             fptr = np_ptr(fut)
         check(lib.gcrl_her_push_episode(self._h, T, np_ptr(s), np_ptr(a), np_ptr(ns), np_ptr(r),
                                         np_ptr(d), np_ptr(ag), fptr, self._stream()))
 
     def _draw_future(self, T):
-        """random.randint(t+1, T-1) in apply_her's order (src/buffer.py:145-153)."""
-        k = self.k_future
+        """random.randint(t+1, T-1) in apply_her's order (src/buffer.py:145-153); "episode" draws
+        random.randint(0, T-1) in the same order, "final" takes T-1 and draws nothing."""
+        k, strategy = self.k_future, self.goal_selection_strategy
         fut = np.zeros((T, max(k, 1)), np.uint8)
-        if T > 1 and k > 0:   # the same (T - 1) * k draws, in the same order, through the C mirror of CPython's MT
-            bounds = _RANDINT_BOUNDS.get((T, k))
+        if T > 1 and k > 0 and strategy == "final":
+            fut[:T - 1, :k] = T - 1
+        elif T > 1 and k > 0:   # the same (T - 1) * k draws, in the same order, through the C mirror of CPython's MT
+            bounds = _RANDINT_BOUNDS.get((T, k, strategy))
             if bounds is None:
-                lo = np.repeat(np.arange(1, T, dtype=np.int32), k)
-                bounds = _RANDINT_BOUNDS[(T, k)] = (lo, np.full(lo.shape, T - 1, np.int32))
+                lo = np.repeat(np.arange(1, T, dtype=np.int32), k) if strategy == "future" else \
+                    np.zeros((T - 1) * k, np.int32)
+                bounds = _RANDINT_BOUNDS[(T, k, strategy)] = (lo, np.full(lo.shape, T - 1, np.int32))
             fut[:T - 1, :k] = _lib.py_randint_seq(*bounds).reshape(T - 1, k)
         return fut
 
@@ -212,12 +255,13 @@ class HERBuffer:
     def state_dict(self):
         """Every episode that still holds a live entry (oldest first, with the future indices that were
         drawn) and the transitions staged per env.  ``load_state_dict`` on a fresh buffer with the same
-        ``max_mem_len`` / ``k_future`` reproduces every deque position, so a resumed run samples the same
-        batches from the same ``random`` stream."""
+        ``max_mem_len`` / ``k_future`` / goal selection reproduces every deque position, so a resumed run samples
+        the same batches from the same ``random`` stream.  An online-sampling buffer stores no future indices; it
+        records its draw epoch instead, so the resumed run draws the same relabels."""
         eps = []
         if self._h:
             D, A, G = self._dims
-            k = self.k_future
+            k = self._stored_k()
             for i in range(int(lib.gcrl_her_live_episodes(self._h))):
                 T = C.c_int()
                 check(lib.gcrl_her_get_episode(self._h, i, C.byref(T), *([None] * 7), self._stream()))
@@ -231,17 +275,29 @@ class HERBuffer:
                                                np_ptr(arrs["ag"]), np_ptr(fut) if k else None, self._stream()))
                 if k:
                     arrs["fut"] = fut
+                elif self.online_sampling:
+                    arrs["fut"] = None
                 eps.append(arrs)
-        return {"max_mem_len": self.max_mem_len, "k_future": self.k_future, "dims": self._dims, "episodes": eps,
-                "staging": [list(ep) for ep in self.episodes]}
+        sd = {"max_mem_len": self.max_mem_len, "k_future": self.k_future, "dims": self._dims, "episodes": eps,
+              "staging": [list(ep) for ep in self.episodes]}
+        if self.goal_selection_strategy != "future" or self.online_sampling:
+            sd.update(goal_selection_strategy=self.goal_selection_strategy, online_sampling=self.online_sampling)
+        if self.online_sampling:
+            sd["draw_epoch"] = self.draw_epoch
+        return sd
 
     def load_state_dict(self, sd):
         if sd["max_mem_len"] != self.max_mem_len or sd["k_future"] != self.k_future:
             raise ValueError("buffer checkpoint was written with a different max_mem_len / k_future")
+        if (sd.get("goal_selection_strategy", "future") != self.goal_selection_strategy
+                or bool(sd.get("online_sampling", False)) != self.online_sampling):
+            raise ValueError("buffer checkpoint was written with a different goal_selection_strategy / online_sampling")
         if self._h:
             check(lib.gcrl_her_clear(self._h))
         for ep in sd["episodes"]:
             self.push_episode(ep["s"], ep["a"], ep["ns"], ep["r"], ep["d"], ep["ag"], ep["fut"])
+        if self.online_sampling and self._h:
+            check(lib.gcrl_her_set_draw_epoch(self._h, int(sd["draw_epoch"])))
         for dq, items in zip(self.episodes, sd["staging"]):
             dq.clear()
             dq.extend(items)

@@ -184,12 +184,15 @@ class _SacBase(_AgentBase):
     _sync_bn = None          # set by enable_data_parallel(sync_bn=True): the BatchNorm statistics all-gather
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, *,
-                 index_source="host", device=0, max_batch=None, seed=1898, precision=0):
+                 index_source="host", device=0, max_batch=None, seed=1898, precision=0,
+                 goal_selection_strategy="future", online_sampling=False):
         """precision: 0 (default) runs every GEMM on the fp32 FFMA tiles; 1 runs the hidden-layer GEMMs of the
         critics and the actor on the tcgen05 tensor cores (3xTF32 split, the critic ensemble batched into one launch
         per layer) once batch * hidden_dim**2 >= 2048 * 256**2 (2048 rows at hidden_dim 256, 512 at 512, 8192 at
-        128); 2 does so for every batch >= 128 (tests).  select_action stays on fp32."""
-        self._init_common(obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed)
+        128); 2 does so for every batch >= 128 (tests).  select_action stays on fp32.
+        goal_selection_strategy / online_sampling: passed to the HER buffer (HERBuffer)."""
+        self._init_common(obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed,
+                          goal_selection_strategy, online_sampling)
         self.alpha_min = getattr(config, "alpha_min", 0.05)
         self.alpha_min_steps = getattr(config, "alpha_min_steps", 10000)
         self.target_entropy = self._target_entropy(ac_dim)

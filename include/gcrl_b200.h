@@ -51,7 +51,7 @@ uint64_t gcrl_kernel_launches(void);
  * Entries are never materialised: gcrl_her_sample() maps a deque position to
  * (episode, t, j) and relabels on the fly.  `max_entries` is the deque's maxlen
  * (per-ENTRY FIFO eviction, src/buffer.py:101); `cap_transitions` sizes the ring of
- * stored transitions (<= 0: max_entries, always sufficient).
+ * stored transitions (<= 0: max_entries + 254, always sufficient).
  */
 typedef struct gcrl_her gcrl_her;
 
@@ -65,8 +65,9 @@ int gcrl_her_destroy(gcrl_her *h);
  * src/env.py:215-224: s[t] = state, ns[t] = next_state (both [D], goal in the last
  * goal_dim columns), a[t], r[t], d[t] (0/1), ag[t] = achieved goal of the NEXT
  * observation.  fut[t*k + j] (t < T-1) is the absolute future index f in [t+1, T-1]
- * drawn by `random.randint(t+1, T-1)` at src/buffer.py:153; NULL = draw them from the
- * handle's own counter-based generator.  All pointers are host memory.  1 <= T <= 255. */
+ * drawn by `random.randint(t+1, T-1)` at src/buffer.py:153 (other goal-selection strategies: their
+ * range, gcrl_her_set_goal_selection); NULL = draw them from the handle's own counter-based generator.
+ * All pointers are host memory.  1 <= T <= 255. */
 int gcrl_her_push_episode(gcrl_her *h, int T, const float *s, const float *a, const float *ns,
                           const float *r, const float *d, const float *ag, const uint8_t *fut,
                           void *stream);
@@ -75,6 +76,28 @@ int gcrl_her_push_episode(gcrl_her *h, int T, const float *s, const float *a, co
  * constructor argument, src/buffer.py:93; panda-gym's tasks use 0.05, the default).  Takes effect for the
  * following samples. */
 int gcrl_her_set_threshold(gcrl_her *h, float threshold);
+
+/* Goal selection (Andrychowicz et al. 2017).  A relabelled transition at step t of an episode of T steps takes the
+ * achieved goal of step f as its goal:
+ *   GCRL_HER_FUTURE  (default) f in [t+1, T-1] -- random.randint(t+1, T-1), the reference's only strategy
+ *   GCRL_HER_FINAL   f = T-1
+ *   GCRL_HER_EPISODE f in [0, T-1]
+ * online_k == 0 (eager, the default): the k_future relabelled copies of the store's entry mapping; fut[] of
+ * gcrl_her_push_episode must lie in the strategy's range (f == T-1 for FINAL), and fut == NULL draws it there.
+ * online_k > 0 (online relabelling): the store holds each transition once (it must be created with k_future = 0,
+ * so len() counts transitions), and each sampled row is relabelled at sample time with probability
+ * online_k / (online_k + 1) to a goal step drawn uniformly from the strategy's range (FUTURE / FINAL: none at
+ * t = T-1); coin and goal step come from a hash of (seed, draw epoch, batch row), and every sample call of an
+ * online store advances the draw epoch.  gcrl_her_push_episode then takes no fut (fut != NULL: GCRL_ERR_INVALID).
+ * Refused (GCRL_ERR_INVALID) once an episode has been committed. */
+#define GCRL_HER_FUTURE 0
+#define GCRL_HER_FINAL 1
+#define GCRL_HER_EPISODE 2
+int gcrl_her_set_goal_selection(gcrl_her *h, int strategy, int online_k);
+/* The draw epoch of the device index stream and of online relabelling (one per sample call that draws on the
+ * device; in online mode one per sample call).  A checkpoint saves it so that a resumed run draws the same rows. */
+uint64_t gcrl_her_get_draw_epoch(const gcrl_her *h);
+int gcrl_her_set_draw_epoch(gcrl_her *h, uint64_t epoch);
 int64_t gcrl_her_len(const gcrl_her *h);            /* __len__, src/buffer.py:137-138   */
 int64_t gcrl_her_total_entries(const gcrl_her *h);  /* entries ever appended            */
 int64_t gcrl_her_live_transitions(const gcrl_her *h);
