@@ -432,6 +432,174 @@ actor_trunc_kernel(const float *__restrict__ q, int64_t ldq, int n, int keep, co
   if (threadIdx.x == 0) *loss_out = t / float(M);
 }
 
+// ---- quantile critics (TQC with n_quantiles M per critic) ------------------------------------------------
+// Atoms of critic i live at z + i * zstride as rows [B][ldm] (ldm = pad4(M)).  Every reduction below runs in a fixed
+// order (warp trees, block trees, serial loops), no atomics.
+
+// Target (sb3-contrib order): the n * M atoms of a row sorted ascending, the K smallest kept,
+// y[b][j] = r + gamma (1 - d) (z_(j) - coef log pi').  One warp per row; the 32 * KPL keys (+inf past n * M) sit
+// KPL per lane (key e = lane * KPL + r) and go through a bitonic network: partners closer than KPL are registers of
+// the same lane, the others one shuffle away.
+template <int KPL>
+__global__ void __launch_bounds__(256)
+quantile_target_kernel(const float *__restrict__ zt, int64_t zstride, int ldm, int n, int M, int keep,
+                       const float *__restrict__ logp, const float *__restrict__ r, const float *__restrict__ d,
+                       float gamma, float coef_const, const float *__restrict__ alpha_dev, float *__restrict__ y,
+                       int ldy, int B) {
+  const float coef = coef_const >= 0.f ? coef_const : *alpha_dev;
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int nwarps = (gridDim.x * blockDim.x) >> 5;
+  const int total = n * M;
+  for (int b = warp; b < B; b += nwarps) {
+    float v[KPL];
+#pragma unroll
+    for (int q = 0; q < KPL; ++q) {
+      const int e = lane * KPL + q;
+      const int i = e / M;
+      v[q] = e < total ? zt[int64_t(i) * zstride + int64_t(b) * ldm + (e - i * M)] : INFINITY;
+    }
+#pragma unroll
+    for (int k = 2; k <= 32 * KPL; k <<= 1) {
+#pragma unroll
+      for (int j = k >> 1; j > 0; j >>= 1) {
+        if (j >= KPL) {
+#pragma unroll
+          for (int q = 0; q < KPL; ++q) {
+            const int e = lane * KPL + q;
+            const float o = __shfl_xor_sync(0xffffffffu, v[q], j / KPL);
+            const bool up = (e & k) == 0, low = (e & j) == 0;
+            v[q] = up == low ? fminf(v[q], o) : fmaxf(v[q], o);
+          }
+        } else {
+#pragma unroll
+          for (int q = 0; q < KPL; ++q)
+            if ((q & j) == 0) {
+              const bool up = ((lane * KPL + q) & k) == 0;
+              const float a = v[q], c = v[q + j];
+              v[q] = up ? fminf(a, c) : fmaxf(a, c);
+              v[q + j] = up ? fmaxf(a, c) : fminf(a, c);
+            }
+        }
+      }
+    }
+    const float ent = coef * logp[b], rb = r[b], disc = gamma * (1.0f - d[b]);
+#pragma unroll
+    for (int q = 0; q < KPL; ++q) {
+      const int e = lane * KPL + q;
+      if (e < keep) y[int64_t(b) * ldy + e] = rb + disc * (v[q] - ent);
+    }
+  }
+}
+
+// Critic loss, forward and backward in one pass: blockIdx.y = critic i, blockIdx.x = a block of `rows` batch rows,
+// thread t owns (row t / M, atom k = t % M).  With u = y_j - Z_ik, tau_k = (k + 0.5) / M and Huber kappa = 1:
+//   dZ_ik = -w_b sum_j |tau_k - 1{u < 0}| clamp(u, -1, 1) / (B M K)          -> dz (the head's input of the backward)
+//   loss partial of the block = sum over its (row, k, j) of w_b |tau_k - 1{u < 0}| h(u)   -> loss_part[i][blockIdx.x]
+//   |mean_k Z_ik - mean_j y_j| per row                                       -> td_part[i][b]
+constexpr int kQhThreads = 256;
+constexpr int kQhMaxTargets = 2048;   // rows * K <= (256 / M) * n M <= 8 * 256
+__global__ void __launch_bounds__(kQhThreads)
+quantile_huber_kernel(const float *__restrict__ z, int64_t zstride, int ldm, int M, const float *__restrict__ y,
+                      int ldy, int K, const float *__restrict__ is_w, float *__restrict__ dz,
+                      float *__restrict__ loss_part, float *__restrict__ td_part, int B, int rows) {
+  __shared__ float ys[kQhMaxTargets];
+  __shared__ float zs[kQhThreads];
+  __shared__ float red[kQhThreads];
+  const int i = blockIdx.y, b0 = blockIdx.x * rows, tid = threadIdx.x;
+  const int nrows = min(rows, B - b0);
+  for (int t = tid; t < nrows * K; t += kQhThreads) {
+    const int rr = t / K;
+    ys[t] = y[int64_t(b0 + rr) * ldy + (t - rr * K)];
+  }
+  const int rr = tid / M, k = tid - rr * M, b = b0 + rr;
+  const bool own = rr < nrows;
+  const int64_t at = int64_t(i) * zstride + int64_t(b) * ldm + k;
+  const float zv = own ? z[at] : 0.f;
+  zs[tid] = zv;
+  __syncthreads();
+  float l = 0.f;
+  if (own) {
+    const float tau = (float(k) + 0.5f) / float(M);
+    const float *yr = ys + rr * K;
+    float g = 0.f;
+    for (int j = 0; j < K; ++j) {
+      const float u = yr[j] - zv;
+      const float wt = u < 0.f ? 1.0f - tau : tau;
+      const float au = fabsf(u);
+      l = fmaf(wt, au > 1.0f ? au - 0.5f : 0.5f * u * u, l);
+      g = fmaf(wt, fminf(fmaxf(u, -1.0f), 1.0f), g);
+    }
+    const float w = is_w != nullptr ? is_w[b] : 1.0f;
+    dz[at] = -(w * g) / (float(B) * float(M) * float(K));
+    l *= w;
+    if (k == 0) {
+      float sz = 0.f, sy = 0.f;
+      for (int kk = 0; kk < M; ++kk) sz += zs[rr * M + kk];
+      for (int j = 0; j < K; ++j) sy += yr[j];
+      td_part[int64_t(i) * B + b] = fabsf(sz / float(M) - sy / float(K));
+    }
+  }
+  red[tid] = l;
+  __syncthreads();
+  for (int s = kQhThreads / 2; s >= 1; s >>= 1) {
+    if (tid < s) red[tid] += red[tid + s];
+    __syncthreads();
+  }
+  if (tid == 0) loss_part[int64_t(i) * gridDim.x + blockIdx.x] = red[0];
+}
+
+// out[M_CLOSS + i] = (sum of critic i's loss partials) / (B M K); per row the max over the critics of the td parts
+// -> td_out (prioritised replay) and their batch mean -> out[M_TD]
+__global__ void __launch_bounds__(1024)
+quantile_metrics_kernel(const float *__restrict__ loss_part, int nblk, const float *__restrict__ td_part, int n, int B,
+                        float count, float *__restrict__ out, int slot_loss, int slot_td, float *__restrict__ td_out) {
+  __shared__ float sm[1024];
+  for (int i = 0; i < n; ++i) {
+    float s = 0.f;
+    for (int t = threadIdx.x; t < nblk; t += 1024) s += loss_part[int64_t(i) * nblk + t];
+    const float tot = cta_sum_1024(s, sm);
+    if (threadIdx.x == 0) out[slot_loss + i] = tot / count;
+  }
+  float td = 0.f;
+  for (int m = threadIdx.x; m < B; m += 1024) {
+    float mx = 0.f;
+    for (int i = 0; i < n; ++i) mx = fmaxf(mx, td_part[int64_t(i) * B + m]);
+    td += mx;
+    if (td_out != nullptr) td_out[m] = mx;
+  }
+  const float tot = cta_sum_1024(td, sm);
+  if (threadIdx.x == 0) out[slot_td] = tot / float(B);
+}
+
+// Per row b: the mean of the n * M atoms, or coef log pi_b - that mean (the actor loss's row term) when logp is
+// given; with dz != nullptr every atom's gradient slot of the row gets dz_value (the actor's backward through the
+// critics: d loss / d Z_ik = -1 / (B n M)).  One warp per row.
+__global__ void __launch_bounds__(256)
+quantile_row_mean_kernel(const float *__restrict__ z, int64_t zstride, int ldm, int n, int M,
+                         const float *__restrict__ logp, float coef_const, const float *__restrict__ alpha_dev,
+                         float *__restrict__ row_out, float *__restrict__ dz, float dz_value, int B) {
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int nwarps = (gridDim.x * blockDim.x) >> 5;
+  const int total = n * M;
+  for (int b = warp; b < B; b += nwarps) {
+    float s = 0.f;
+    for (int e = lane; e < total; e += 32) {
+      const int i = e / M;
+      const int64_t at = int64_t(i) * zstride + int64_t(b) * ldm + (e - i * M);
+      s += z[at];
+      if (dz != nullptr) dz[at] = dz_value;
+    }
+#pragma unroll
+    for (int o = 16; o >= 1; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) {
+      const float mean = s / float(total);
+      row_out[b] = logp != nullptr ? (coef_const >= 0.f ? coef_const : *alpha_dev) * logp[b] - mean : mean;
+    }
+  }
+}
+
 // dact[m, j] (+)= sum_n dZ0[m, n] W0[n, col0 + j]   (critic layer-1 input gradient, action columns)
 __global__ void __launch_bounds__(256)
 action_grad_acc_kernel(const float *__restrict__ dZ0, int lddz, const float *__restrict__ W0, int ldw, int col0,
@@ -671,6 +839,11 @@ struct gcrl_sac {
   float *eps_next = nullptr, *eps_cur = nullptr;
   float *per_w = nullptr, *per_td = nullptr;     // prioritised replay: importance weights in, TD errors out [maxB]
   bool per_on = false;                           // flags bit3 of the update being issued
+  // quantile critics (gcrl_sac_create_quantile; nq == 0: scalar critics): M atoms per critic, d dropped per critic,
+  // K = n (M - d) kept target atoms.  q / qt / dq then hold [n][maxB][ldm] (qstride floats per critic), y [maxB][ldy]
+  int nq = 0, nq_drop = 0, nq_keep = 0, ldm = 0, ldy = 0;
+  int64_t qstride = 0;
+  float *qloss = nullptr, *qtd = nullptr, *qrow = nullptr;   // loss partials [n][maxB], td parts [n][maxB], rows [maxB]
   float *partials = nullptr;
   int64_t slab = 0;
   float *sumsq = nullptr;
@@ -768,6 +941,13 @@ void critics_fwd(gcrl_sac *ag, const MlpParams *nets, const float *X, float *q_o
       pr[i] = LinearFwdProblem{l == 0 ? X : ag->ch[i][l - 1], l == 0 ? ag->ldc : ag->ldh, nets[i].W(l), nets[i].ldw[l],
                                nets[i].b(l), ag->ch[i][l], ag->ldh};
     launch_linear_fwd_batched(pr, n, B, ag->H, l == 0 ? ag->D + ag->A : ag->H, ACT_LEAKY, st);
+  }
+  if (ag->nq > 0) {           // quantile critics: the H -> M head on the fp32 tiles, atoms [B][ldm] per critic
+    for (int i = 0; i < n; ++i)
+      pr[i] = LinearFwdProblem{ag->ch[i][L - 1], ag->ldh, nets[i].W(L), nets[i].ldw[L], nets[i].b(L),
+                               q_out + int64_t(i) * ag->qstride, ag->ldm};
+    launch_linear_fwd_batched(pr, n, B, ag->nq, ag->H, ACT_NONE, st);
+    return;
   }
   HeadFwdProblem hp[kMaxBatchedLinear];
   for (int i = 0; i < n; ++i)
@@ -872,6 +1052,64 @@ void rereduce(gcrl_sac *ag, float *g, int total, cudaStream_t st) {
   launch_reduce_grads(r, st);
 }
 
+// ---- quantile critics: the launches around the loss kernels and the head's backward ----------------------------
+// target atoms in qt -> y; critic atoms in q -> dZ in dq, per-critic losses, td (and the prioritised TD rows)
+void quantile_critic_loss(gcrl_sac *ag, int B, cudaStream_t st) {
+  const int n = ag->n, M = ag->nq, total = n * M;
+  auto target = total <= 32 ? quantile_target_kernel<1>
+              : total <= 64 ? quantile_target_kernel<2> : total <= 128 ? quantile_target_kernel<4> : quantile_target_kernel<8>;
+  target<<<blocks_for(B, 8), 256, 0, st>>>(ag->qt, ag->qstride, ag->ldm, n, M, ag->nq_keep, ag->logp, ag->br, ag->bd,
+                                          ag->cfg.gamma, ag->cfg.entropy_coef, ag->alpha_state + 1, ag->y, ag->ldy, B);
+  GCRL_LAUNCHED();
+  const int rows = std::max(1, kQhThreads / M);
+  const int nblk = (B + rows - 1) / rows;
+  quantile_huber_kernel<<<dim3(nblk, n), kQhThreads, 0, st>>>(ag->q, ag->qstride, ag->ldm, M, ag->y, ag->ldy,
+                                                              ag->nq_keep, ag->per_on ? ag->per_w : nullptr, ag->dq,
+                                                              ag->qloss, ag->qtd, B, rows);
+  GCRL_LAUNCHED();
+  quantile_metrics_kernel<<<1, 1024, 0, st>>>(ag->qloss, nblk, ag->qtd, n, B,
+                                              float(B) * float(M) * float(ag->nq_keep), ag->mdev, M_CLOSS, M_TD,
+                                              ag->per_on ? ag->per_td : nullptr);
+  GCRL_LAUNCHED();
+}
+
+// *out = mean over the batch of quantile_row_mean_kernel's row values of the atoms z (see there for logp / dz)
+void quantile_row_mean(gcrl_sac *ag, const float *z, const float *logp, float *dz, float *out, int B, cudaStream_t st) {
+  quantile_row_mean_kernel<<<blocks_for(B, 8), 256, 0, st>>>(z, ag->qstride, ag->ldm, ag->n, ag->nq, logp,
+                                                             ag->cfg.entropy_coef, ag->alpha_state + 1, ag->qrow, dz,
+                                                             -1.0f / (float(B) * float(ag->n * ag->nq)), B);
+  GCRL_LAUNCHED();
+  alpha_mean_kernel<<<1, 1024, 0, st>>>(ag->qrow, B, 0.f, out);
+  GCRL_LAUNCHED();
+}
+
+// The H -> M head of critics first .. first + m - 1, from dZ [B][ldm] in dq: with wgrad, the weight-gradient partial
+// slabs into each critic's partial set (pset_stride floats apart); always dX = dZ W (.) leaky'(h) into
+// dz_out[j * dz_step].  Returns the weight gradient's number of batch slabs.
+int quantile_head_bwd(gcrl_sac *ag, int first, int m, float *const *dz_out, bool wgrad, int64_t pset_stride, int B,
+                      cudaStream_t st, int dz_step = 1) {
+  const int L = ag->L;
+  int splits = 0;
+  if (wgrad) {
+    WgradProblem wp[kMaxWgradProblems];
+    for (int j = 0; j < m; ++j) {
+      const MlpParams &c = ag->critic[first + j];
+      float *part = ag->partials + j * pset_stride;
+      wp[j] = WgradProblem{ag->dq + (first + j) * ag->qstride, ag->ldm, ag->ch[first + j][L - 1], ag->ldh,
+                           part + c.w_off[L], c.ldw[L], part + c.b_off[L], ag->nq, ag->H};
+    }
+    splits = launch_multi_wgrad(wp, m, B, ag->slab, kSplits, st);
+  }
+  LinearDgradProblem dg[kMaxBatchedLinear];
+  for (int j = 0; j < m; ++j) {
+    const MlpParams &c = ag->critic[first + j];
+    dg[j] = LinearDgradProblem{ag->dq + (first + j) * ag->qstride, ag->ldm, c.W(L), c.ldw[L], ag->ch[first + j][L - 1],
+                               ag->ldh, dz_out[j * dz_step], ag->ldh};
+  }
+  launch_linear_dgrad_batched(dg, m, B, ag->nq, ag->H, st);
+  return splits;
+}
+
 enum : int { PH_CGRAD = 1, PH_CSTEP = 2, PH_AGRAD = 4, PH_ASTEP = 8, PH_ALL = 15 };
 
 // critic_update (SAC :548-639, TQC :951-1042).  mask PH_ALL: every critic is stepped right after its own
@@ -885,6 +1123,10 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   // next action and log-probability = actor.sample(next_state) in train mode (batch statistics; running statistics move)
   actor_fwd(ag, ag->nsa, ag->eps_next, B, true, false, nullptr, st);
   critics_fwd(ag, ag->target, ag->nsa, ag->qt, B, st);         // ch[i] as scratch: overwritten by the critic forward
+  if (ag->nq > 0) {
+    critics_fwd(ag, ag->critic, ag->sa, ag->q, B, st);
+    quantile_critic_loss(ag, B, st);
+  } else {
   sac_target_kernel<<<blocks_for(B, 256), 256, 0, st>>>(ag->qt, ag->maxB, n, ag->keep, ag->logp, ag->br, ag->bd,
                                                        ag->cfg.gamma, ag->cfg.entropy_coef, ag->alpha_state + 1,
                                                        ag->y, B);
@@ -893,6 +1135,7 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   critic_metrics_kernel<<<1, 1024, 0, st>>>(ag->q, ag->maxB, n, ag->y, B, ag->mdev + M_CLOSS, 0,
                                             ag->per_on ? ag->per_w : nullptr, ag->per_on ? ag->per_td : nullptr);
   GCRL_LAUNCHED();
+  }
   if (B <= kEnsembleBatchMax) {
     // the ensemble's backward passes share their launches: one head launch, one weight-gradient and one
     // input-gradient launch per layer (per-critic gradient buffers and partial sets), then reduce + AdamW per critic
@@ -913,7 +1156,8 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
       h.M = B; h.K = ag->H;
       hs[i] = h;
     }
-    const int head_splits = launch_head_bwd_batched(hs, n, kSplits, st);
+    const int head_splits = ag->nq > 0 ? quantile_head_bwd(ag, 0, n, ag->dzc.data(), true, ag->pset, B, st, 2)
+                                       : launch_head_bwd_batched(hs, n, kSplits, st);
     int splits[8] = {};
     int cur = 0;
     for (int l = L - 1; l >= 0; --l) {
@@ -965,7 +1209,7 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     h.pB = ag->partials + c.b_off[L]; h.b_split_stride = ag->slab;
     h.metric_partials = ag->partials + ag->slab * kSplits;      // scratch tail, unused
     h.M = B; h.K = ag->H;
-    const int head_splits = launch_head_bwd(h, kSplits, st);
+    const int head_splits = ag->nq > 0 ? quantile_head_bwd(ag, i, 1, ag->dz, true, 0, B, st) : launch_head_bwd(h, kSplits, st);
     int splits[8] = {};
     int cur = 0;
     for (int l = L - 1; l >= 0; --l) {
@@ -997,6 +1241,10 @@ void critic_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   }
   if (tqc && (mask & PH_CSTEP)) {   // logged Q = mean over the STEPPED critics (:1016-1019)
     critics_fwd(ag, ag->critic, ag->sa, ag->qt, B, st);        // the backward pass is done with ch[i]
+    if (ag->nq > 0) {
+      quantile_row_mean(ag, ag->qt, nullptr, nullptr, ag->mdev + M_Q, B, st);
+      return;
+    }
     critic_metrics_kernel<<<1, 1024, 0, st>>>(ag->qt, ag->maxB, n, nullptr, B, ag->mdev + M_CLOSS, 1, nullptr, nullptr);
     GCRL_LAUNCHED();
   }
@@ -1010,9 +1258,13 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
   if (mask & PH_AGRAD) {
   actor_fwd(ag, ag->spi, ag->eps_cur, B, true, true, nullptr, st);
   critics_fwd(ag, ag->critic, ag->spi, ag->q, B, st);
+  if (ag->nq > 0) {     // no truncation: loss mean_b(coef log pi - mean_ik Z_ik), every atom's gradient -1 / (B n M)
+    quantile_row_mean(ag, ag->q, ag->logp, ag->dq, ag->mdev + M_ALOSS, B, st);
+  } else {
   actor_trunc_kernel<<<1, 1024, 0, st>>>(ag->q, ag->maxB, n, ag->keep, ag->logp, ag->cfg.entropy_coef,
                                         ag->alpha_state + 1, ag->dq, ag->mdev + M_ALOSS, B);
   GCRL_LAUNCHED();
+  }
   if (B <= kEnsembleBatchMax) {        // the ensemble's input-gradient chains share their launches
     HeadBwdArgs hs[kMaxBatchedLinear];
     for (int i = 0; i < n; ++i) {
@@ -1026,7 +1278,8 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
       h.M = B; h.K = ag->H;
       hs[i] = h;
     }
-    launch_head_bwd_batched(hs, n, kSplits, st);
+    if (ag->nq > 0) quantile_head_bwd(ag, 0, n, ag->dzc.data(), false, 0, B, st, 2);
+    else launch_head_bwd_batched(hs, n, kSplits, st);
     int cur = 0;
     for (int l = L - 1; l >= 1; --l) {
       if (ag->tc_update) {
@@ -1061,7 +1314,8 @@ void actor_update(gcrl_sac *ag, int B, int flags, int mask, cudaStream_t st) {
     h.dZprev = ag->dz[0]; h.lddz = ag->ldh;
     h.pW = nullptr; h.pB = nullptr;              // critic weight gradients are discarded
     h.M = B; h.K = ag->H;
-    launch_head_bwd(h, kSplits, st);
+    if (ag->nq > 0) quantile_head_bwd(ag, i, 1, ag->dz, false, 0, B, st);
+    else launch_head_bwd(h, kSplits, st);
     int cur = 0;
     for (int l = L - 1; l >= 1; --l) {
       if (ag->tc_update)
@@ -1544,17 +1798,22 @@ static void update_many(gcrl_sac *ag, gcrl_her *her, gcrl_replay *rb, int64_t B,
   read_many_rows(ag, n, B, flags, metrics_host, per ? td_host : nullptr, st);
 }
 
-extern "C" {
-
-int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
-  GCRL_API_BEGIN
+// gcrl_sac_create (nq == 0: scalar critics) and gcrl_sac_create_quantile (nq atoms per critic, nq_drop dropped)
+static void sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg, int nq, int nq_drop) {
   GCRL_REQUIRE(out != nullptr && cfg != nullptr, "NULL argument");
   GCRL_REQUIRE(cfg->algo == GCRL_ALGO_SAC || cfg->algo == GCRL_ALGO_TQC, "unknown algo");
   GCRL_REQUIRE(cfg->state_dim >= 1 && cfg->act_dim >= 1 && cfg->act_dim <= 4, "need state_dim >= 1 and 1 <= act_dim <= 4");
   GCRL_REQUIRE(cfg->hidden_dim >= 1 && cfg->hidden_dim <= 4096, "hidden_dim outside [1, 4096]");
   GCRL_REQUIRE(cfg->layer_count >= 1 && cfg->layer_count <= 6, "layer_count outside [1, 6]");
   GCRL_REQUIRE(cfg->n_critics >= 1 && cfg->n_critics <= kMaxCritics, "n_critics outside [1, 8]");
-  GCRL_REQUIRE(cfg->drop_top >= 0 && cfg->drop_top < cfg->n_critics, "drop_top outside [0, n_critics)");
+  if (nq == 0) {
+    GCRL_REQUIRE(cfg->drop_top >= 0 && cfg->drop_top < cfg->n_critics, "drop_top outside [0, n_critics)");
+  } else {
+    GCRL_REQUIRE(cfg->algo == GCRL_ALGO_TQC, "quantile critics need algo GCRL_ALGO_TQC");
+    GCRL_REQUIRE(nq >= 1 && nq_drop >= 0 && nq_drop < nq,
+                 "quantile critics need n_quantiles >= 1 and 0 <= drop_per_net < n_quantiles");
+    GCRL_REQUIRE(cfg->n_critics * nq <= 256, "quantile critics need n_critics * n_quantiles <= 256");
+  }
   GCRL_REQUIRE(cfg->max_batch >= 2 && cfg->max_batch <= kSplits * 256, "max_batch outside [2, 32768]");
   GCRL_REQUIRE(cfg->precision >= 0 && cfg->precision <= 2, "precision must be 0 (fp32 FFMA), 1 (tensor cores for large batches) or 2 (tensor cores whenever supported)");
   GCRL_CUDA(cudaSetDevice(device));
@@ -1564,11 +1823,15 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
     ag->D = cfg->state_dim; ag->A = cfg->act_dim; ag->H = cfg->hidden_dim; ag->L = cfg->layer_count;
     ag->n = cfg->n_critics; ag->keep = cfg->n_critics - cfg->drop_top;
     ag->ldh = pad4(ag->H); ag->ldc = pad4(ag->D + ag->A); ag->maxB = cfg->max_batch;
+    ag->nq = nq; ag->nq_drop = nq_drop; ag->nq_keep = cfg->n_critics * (nq - nq_drop);
+    ag->ldm = pad4(nq); ag->ldy = pad4(ag->nq_keep);
+    ag->qstride = nq > 0 ? ag->maxB * ag->ldm : ag->maxB;
     GCRL_REQUIRE(4 * ag->L + 4 <= kMaxSegs, "layer_count too large for the reduction descriptor");
     const int D = ag->D, A = ag->A, H = ag->H, L = ag->L, n = ag->n;
     const size_t mb = size_t(ag->maxB), act = mb * ag->ldh;
     ag->actor.init(D, H, A, L);
-    for (int i = 0; i < n; ++i) { ag->critic[i].layout(D + A, H, 1, L); ag->target[i].layout(D + A, H, 1, L); }
+    const int nout = nq > 0 ? nq : 1;
+    for (int i = 0; i < n; ++i) { ag->critic[i].layout(D + A, H, nout, L); ag->target[i].layout(D + A, H, nout, L); }
     ag->critic_stride = ag->critic[0].total;
     ag->critic_grads = dev_alloc<float>(size_t(n) * ag->critic_stride);
     GCRL_CUDA(cudaMemset(ag->critic_grads, 0, size_t(n) * ag->critic_stride * 4));
@@ -1585,9 +1848,16 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
     for (auto &p : ag->dz) p = dev_alloc<float>(act);
     for (int i = 0; i < 2 * n; ++i) ag->dzc.push_back(dev_alloc<float>(size_t(std::min<int64_t>(mb, kEnsembleBatchMax)) * ag->ldh));
     for (float **p : {&ag->sa, &ag->nsa, &ag->spi}) *p = dev_alloc<float>(mb * ag->ldc);
-    for (float **p : {&ag->br, &ag->bd, &ag->br0, &ag->bd0, &ag->y, &ag->logp, &ag->per_w, &ag->per_td}) *p = dev_alloc<float>(mb);
+    for (float **p : {&ag->br, &ag->bd, &ag->br0, &ag->bd0, &ag->logp, &ag->per_w, &ag->per_td}) *p = dev_alloc<float>(mb);
+    ag->y = dev_alloc<float>(mb * (nq > 0 ? ag->ldy : 1));
     ag->bs = dev_alloc<float>(mb * D); ag->bns = dev_alloc<float>(mb * D); ag->ba = dev_alloc<float>(mb * A);
-    ag->q = dev_alloc<float>(mb * n); ag->qt = dev_alloc<float>(mb * n); ag->dq = dev_alloc<float>(mb * n * 4);
+    ag->q = dev_alloc<float>(n * ag->qstride); ag->qt = dev_alloc<float>(n * ag->qstride);
+    ag->dq = dev_alloc<float>(n * std::max<int64_t>(ag->qstride, mb * 4));
+    if (nq > 0) {
+      ag->qloss = dev_alloc<float>(mb * (2 * n + 1));
+      ag->qtd = ag->qloss + mb * n;
+      ag->qrow = ag->qtd + mb * n;
+    }
     for (float **p : {&ag->act4, &ag->std4, &ag->gate4, &ag->dact, &ag->eps_next, &ag->eps_cur}) *p = dev_alloc<float>(mb * 4);
     ag->dzh = dev_alloc<float>(mb * 8);
     ag->slab = std::max(ag->actor.total, ag->critic[0].total);
@@ -1619,6 +1889,21 @@ int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
     throw;
   }
   *out = ag;
+}
+
+extern "C" {
+
+int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg) {
+  GCRL_API_BEGIN
+  sac_create(out, device, cfg, 0, 0);
+  GCRL_API_END
+}
+
+int gcrl_sac_create_quantile(gcrl_sac **out, int device, const gcrl_sac_config *cfg, int n_quantiles,
+                             int drop_per_net) {
+  GCRL_API_BEGIN
+  GCRL_REQUIRE(n_quantiles >= 1, "quantile critics need n_quantiles >= 1");
+  sac_create(out, device, cfg, n_quantiles, drop_per_net);
   GCRL_API_END
 }
 
@@ -1635,7 +1920,7 @@ int gcrl_sac_destroy(gcrl_sac *ag) {
   for (float *p : {ag->invstd, ag->dz[0], ag->dz[1], ag->sa, ag->nsa, ag->spi, ag->br, ag->bd, ag->bs, ag->ba, ag->bns,
                    ag->br0, ag->bd0, ag->q, ag->qt, ag->y, ag->dq, ag->logp, ag->act4, ag->std4, ag->gate4, ag->dact,
                    ag->dzh, ag->eps_next, ag->eps_cur, ag->partials, ag->sumsq, ag->mdev, ag->d_io,
-                   ag->critic_grads, ag->per_w, ag->per_td})
+                   ag->critic_grads, ag->per_w, ag->per_td, ag->qloss})
     if (p) cudaFree(p);
   for (auto &kv : ag->graphs) cudaGraphExecDestroy(kv.second.exec);
   ag->many.graphs.clear();
@@ -1819,6 +2104,7 @@ int gcrl_sac_update_phase(gcrl_sac *ag, int phase, gcrl_her *buf, int64_t B, con
   GCRL_NVTX("gcrl_sac_update_phase");
   require_handle(ag);
   GCRL_REQUIRE(ag != nullptr && phase >= 0 && phase <= 3, "NULL handle / phase outside 0..3");
+  GCRL_REQUIRE(ag->nq == 0, "data parallelism is not available for quantile critics (gcrl_sac_create_quantile)");
   GCRL_CUDA(cudaSetDevice(ag->device));
   sac_update(ag, phase, buf, B, idx_host, s, a, r, ns, d, eps_next, eps_cur, lr_c, lr_a, flags, nullptr,
              as_stream(stream));
@@ -1828,6 +2114,7 @@ int gcrl_sac_update_phase(gcrl_sac *ag, int phase, gcrl_her *buf, int64_t B, con
 int gcrl_sac_set_sync_bn(gcrl_sac *ag, int world, int rank) {
   GCRL_API_BEGIN
   require_handle(ag);
+  GCRL_REQUIRE(ag->nq == 0, "data parallelism is not available for quantile critics (gcrl_sac_create_quantile)");
   GCRL_REQUIRE(world >= 0 && world <= 1024 && (world == 0 || (rank >= 0 && rank < world)),
                "need 0 <= world <= 1024 and 0 <= rank < world (world 0 switches sync-BN off)");
   GCRL_CUDA(cudaSetDevice(ag->device));
@@ -1851,6 +2138,7 @@ int gcrl_sac_update_segment(gcrl_sac *ag, int segment, gcrl_her *buf, int64_t B,
   GCRL_NVTX("gcrl_sac_update_segment");
   require_handle(ag);
   GCRL_REQUIRE(segment >= 0 && collective != nullptr, "segment < 0 / NULL collective");
+  GCRL_REQUIRE(ag->nq == 0, "data parallelism is not available for quantile critics (gcrl_sac_create_quantile)");
   GCRL_REQUIRE(ag->sync_world > 0, "gcrl_sac_set_sync_bn first");
   GCRL_CUDA(cudaSetDevice(ag->device));
   sac_update(ag, -1, buf, B, idx_host, s, a, r, ns, d, eps_next, eps_cur, lr_c, lr_a, flags, nullptr,

@@ -108,6 +108,7 @@ SIGNATURES = {
     "gcrl_agent_metrics_buffer": (C.c_int, [vp, pp]),
     # SAC / TQC
     "gcrl_sac_create": (C.c_int, [pp, C.c_int, C.POINTER(SacConfig)]),
+    "gcrl_sac_create_quantile": (C.c_int, [pp, C.c_int, C.POINTER(SacConfig), C.c_int, C.c_int]),
     "gcrl_sac_destroy": (C.c_int, [vp]),
     "gcrl_sac_set_actor_linear": (C.c_int, [vp, C.c_int, vp, vp, vp]),
     "gcrl_sac_get_actor_linear": (C.c_int, [vp, C.c_int, vp, vp, vp]),

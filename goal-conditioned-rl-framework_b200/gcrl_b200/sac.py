@@ -123,7 +123,7 @@ class _SacCriticView:
     def _shape(self, layer):
         a = self._a
         L, H = a.config.layer_count, a.config.hidden_dim
-        return (1 if layer == L else H, a.obs_dim + a.ac_dim if layer == 0 else H)
+        return (a._head_width() if layer == L else H, a.obs_dim + a.ac_dim if layer == 0 else H)
 
     def layers(self):
         a, out = self._a, []
@@ -182,6 +182,7 @@ class _SacBase(_AgentBase):
     N_CRITICS, DROP_TOP = 2, 1
     ENTROPY_COEF = 0.2
     _sync_bn = None          # set by enable_data_parallel(sync_bn=True): the BatchNorm statistics all-gather
+    _nq, _nq_drop = None, 0  # quantile critics (TQCAgent(n_quantiles=...)): atoms per critic, dropped per critic
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, *,
                  index_source="host", device=0, max_batch=None, seed=1898, precision=0,
@@ -204,7 +205,10 @@ class _SacBase(_AgentBase):
                         target_entropy=self.target_entropy, alpha_lr=getattr(config, "alpha_lr", 3e-4),
                         precision=int(precision))
         h = vp()
-        check(lib.gcrl_sac_create(C.byref(h), self.device_index, C.byref(cfg)))
+        if self._nq is None:
+            check(lib.gcrl_sac_create(C.byref(h), self.device_index, C.byref(cfg)))
+        else:
+            check(lib.gcrl_sac_create_quantile(C.byref(h), self.device_index, C.byref(cfg), self._nq, self._nq_drop))
         self._h = h
         self._max_batch = int(max_batch or config.batch_size)
         self._metrics = (C.c_float * 12)()
@@ -238,11 +242,15 @@ class _SacBase(_AgentBase):
         self.actor.set_linear(L, *xavier(A, H))
         self.actor.set_linear(L + 1, *xavier(A, H))
         for view in self._critic_views:
-            view.set_layers([xavier(1 if l == L else H, D + A if l == 0 else H) for l in range(L + 1)])
+            view.set_layers([xavier(self._head_width() if l == L else H, D + A if l == 0 else H) for l in range(L + 1)])
         self._bn_batches = 0
 
     def _target_entropy(self, ac_dim):
         raise NotImplementedError
+
+    def _head_width(self):
+        """Rows of every critic's last Linear: 1, or n_quantiles for quantile critics."""
+        return 1 if self._nq is None else self._nq
 
     def update_target_network(self):
         check(lib.gcrl_sac_hard_update(self._h, self._stream()))
@@ -298,7 +306,11 @@ class _SacBase(_AgentBase):
         whole batch).  Every rank must use the same local batch size.  ``sync_bn=False`` keeps local statistics
         (torch DDP's default without SyncBatchNorm: 4 phases, 3 collectives per update instead of 3 + 3 per
         BatchNorm layer) and averages the running statistics after every update.
-        ``world`` / ``rank`` / ``allgather(slots_tensor)`` override torch.distributed (tests)."""
+        ``world`` / ``rank`` / ``allgather(slots_tensor)`` override torch.distributed (tests).  Not available for
+        quantile critics (TQCAgent(n_quantiles=...)): ValueError."""
+        if self._nq is not None:
+            raise ValueError(f"{type(self).__name__}: data parallelism is not available for quantile critics "
+                             "(n_quantiles); train on one GPU")
         dp = super().enable_data_parallel(process_group, allreduce_mean)
         self._sync_bn = None
         if not sync_bn:
@@ -455,7 +467,7 @@ class _SacBase(_AgentBase):
         self.actor.set_linear(L, *xavier(A, H))
         self.actor.set_linear(L + 1, *xavier(A, H))
         for view in list(self._critic_views) + list(self._target_views):
-            view.set_layers([xavier(1 if l == L else H, D + A if l == 0 else H) for l in range(L + 1)])
+            view.set_layers([xavier(self._head_width() if l == L else H, D + A if l == 0 else H) for l in range(L + 1)])
         self.set_log_alpha(0.0)          # also re-creates alpha's AdamW state (gcrl_sac_set_log_alpha)
 
     # -- what the DDPG / TD3 base offers through gcrl_agent_* does not exist for this handle type ---------------
@@ -536,14 +548,24 @@ class SACAgent(_SacBase):
 
 
 class TQCAgent(_SacBase):
-    """Reference src/agent.py:773-1171 (5 scalar critics, drop the top 2; see SURVEY 0.4)."""
+    """Reference src/agent.py:773-1171 (5 scalar critics, drop the top 2; see SURVEY 0.4).
+
+    ``n_quantiles=None`` (the default) is that agent.  An integer M gives Truncated Quantile Critics as
+    sb3-contrib's ``TQC(n_quantiles=M, top_quantiles_to_drop_per_net=d)`` runs them (Kuznetsov et al., 2020):
+    every critic ends in an H -> M Linear (M quantile atoms), the target pools the 5 M atoms of the target critics
+    at (s', a'), keeps the 5 (M - d) smallest and each critic fits all its atoms to them with the quantile Huber
+    loss (kappa 1); the actor maximises the mean of all atoms, without truncation.  Checkpoints hold an [M, H] head
+    in ``net.{2L}.weight``; data parallelism is not available for quantile critics."""
     ALGO = ALGO_TQC
     N_CRITICS, DROP_TOP = 5, 2           # getattr defaults, :789-790 (the YAML keys never reach the config)
     ENTROPY_COEF = -1.0                  # use the learned alpha (:928, :978)
 
-    def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw):
+    def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, *, n_quantiles=None,
+                 top_quantiles_to_drop_per_net=2, **kw):
+        self._nq, self._nq_drop = self._check_quantiles(n_quantiles, top_quantiles_to_drop_per_net)
         super().__init__(obs_dim, ac_dim, config, weights, nenvs, gradient_step, **kw)
         self.num_critics, self.top_quantiles_to_drop = self.N_CRITICS, self.DROP_TOP
+        self.n_quantiles, self.top_quantiles_to_drop_per_net = self._nq, self._nq_drop
         self.critics, self.target_critics = list(self._critic_views), list(self._target_views)
         if weights:
             import torch
@@ -556,6 +578,24 @@ class TQCAgent(_SacBase):
             if os.path.exists(p):
                 self.set_log_alpha(float(torch.load(p, map_location="cpu").reshape(-1)[0]))
         self.update_target_network()
+
+    @classmethod
+    def _check_quantiles(cls, n_quantiles, drop):
+        """(M, d) of the quantile critics, or (None, 0); ValueError before anything touches the device."""
+        if n_quantiles is None:
+            return None, 0
+
+        def whole(x):
+            return isinstance(x, (int, np.integer)) and not isinstance(x, (bool, np.bool_))
+        if not whole(n_quantiles) or n_quantiles < 1:
+            raise ValueError(f"n_quantiles must be None or an integer >= 1, got {n_quantiles!r}")
+        if cls.N_CRITICS * int(n_quantiles) > 256:
+            raise ValueError(f"n_quantiles = {n_quantiles}: {cls.N_CRITICS} critics x n_quantiles must be <= 256 "
+                             f"(n_quantiles <= {256 // cls.N_CRITICS})")
+        if not whole(drop) or not 0 <= drop < n_quantiles:
+            raise ValueError(f"top_quantiles_to_drop_per_net must be an integer in [0, n_quantiles) = "
+                             f"[0, {n_quantiles}), got {drop!r}")
+        return int(n_quantiles), int(drop)
 
     def _target_entropy(self, ac_dim):
         return float(-ac_dim)            # :815

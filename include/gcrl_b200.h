@@ -349,6 +349,15 @@ typedef struct gcrl_sac_config {
 } gcrl_sac_config;
 
 int gcrl_sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg);
+/* TQC with quantile critics: as gcrl_sac_create, but every critic ends in an H -> n_quantiles Linear, the target
+ * keeps the n_critics * (n_quantiles - drop_per_net) smallest pooled atoms and the critics minimise the quantile
+ * Huber loss.  cfg->algo must be GCRL_ALGO_TQC; cfg->drop_top is not used.  1 <= n_quantiles,
+ * 0 <= drop_per_net < n_quantiles, n_critics * n_quantiles <= 256; otherwise GCRL_ERR_INVALID.
+ * Every other gcrl_sac_* call works on such a handle (gcrl_sac_get / set_critic_layer move an [n_quantiles, H]
+ * head) except data parallelism: gcrl_sac_set_sync_bn, gcrl_sac_update_phase and gcrl_sac_update_segment refuse
+ * it with GCRL_ERR_INVALID. */
+int gcrl_sac_create_quantile(gcrl_sac **out, int device, const gcrl_sac_config *cfg, int n_quantiles,
+                             int drop_per_net);
 int gcrl_sac_destroy(gcrl_sac *h);
 
 /* Parameter exchange in the reference's state_dict layout (fp32, weight [out, in] row-major).
