@@ -843,7 +843,7 @@ struct gcrl_sac {
   // K = n (M - d) kept target atoms.  q / qt / dq then hold [n][maxB][ldm] (qstride floats per critic), y [maxB][ldy]
   int nq = 0, nq_drop = 0, nq_keep = 0, ldm = 0, ldy = 0;
   int64_t qstride = 0;
-  float *qloss = nullptr, *qtd = nullptr, *qrow = nullptr;   // loss partials [n][maxB], td parts [n][maxB], rows [maxB]
+  float *qscratch = nullptr, *qrow = nullptr;   // quantile_critic_loss's scratch [2 n maxB], rows [maxB]
   float *partials = nullptr;
   int64_t slab = 0;
   float *sumsq = nullptr;
@@ -1053,24 +1053,36 @@ void rereduce(gcrl_sac *ag, float *g, int total, cudaStream_t st) {
 }
 
 // ---- quantile critics: the launches around the loss kernels and the head's backward ----------------------------
-// target atoms in qt -> y; critic atoms in q -> dZ in dq, per-critic losses, td (and the prioritised TD rows)
-void quantile_critic_loss(gcrl_sac *ag, int B, cudaStream_t st) {
-  const int n = ag->n, M = ag->nq, total = n * M;
+// The loss of n critics of M atoms with K kept targets, on any buffers (the agent's and gcrl_quantile_critic_loss):
+// target atoms zt -> y [B][ldy]; critic atoms z -> dZ in dz (same layout as z), the per-critic losses into
+// out[slot_loss + i], the batch-mean TD into out[slot_td] and the per-row TD into td_rows (or nullptr).
+// scratch: n * (B + ceil(B / rows)) floats, the TD parts [n][B] then the loss partials [n][nblk].
+void quantile_critic_loss(const float *zt, const float *z, int64_t zstride, int ldm, int n, int M, int K,
+                          const float *logp, const float *r, const float *d, const float *w, float gamma, float coef,
+                          const float *alpha_dev, float *y, int ldy, float *dz, float *out, int slot_loss, int slot_td,
+                          float *td_rows, float *scratch, int B, cudaStream_t st) {
+  const int total = n * M;
   auto target = total <= 32 ? quantile_target_kernel<1>
               : total <= 64 ? quantile_target_kernel<2> : total <= 128 ? quantile_target_kernel<4> : quantile_target_kernel<8>;
-  target<<<blocks_for(B, 8), 256, 0, st>>>(ag->qt, ag->qstride, ag->ldm, n, M, ag->nq_keep, ag->logp, ag->br, ag->bd,
-                                          ag->cfg.gamma, ag->cfg.entropy_coef, ag->alpha_state + 1, ag->y, ag->ldy, B);
+  target<<<blocks_for(B, 8), 256, 0, st>>>(zt, zstride, ldm, n, M, K, logp, r, d, gamma, coef, alpha_dev, y, ldy, B);
   GCRL_LAUNCHED();
   const int rows = std::max(1, kQhThreads / M);
   const int nblk = (B + rows - 1) / rows;
-  quantile_huber_kernel<<<dim3(nblk, n), kQhThreads, 0, st>>>(ag->q, ag->qstride, ag->ldm, M, ag->y, ag->ldy,
-                                                              ag->nq_keep, ag->per_on ? ag->per_w : nullptr, ag->dq,
-                                                              ag->qloss, ag->qtd, B, rows);
+  float *td_part = scratch, *loss_part = scratch + int64_t(n) * B;
+  quantile_huber_kernel<<<dim3(nblk, n), kQhThreads, 0, st>>>(z, zstride, ldm, M, y, ldy, K, w, dz, loss_part, td_part,
+                                                              B, rows);
   GCRL_LAUNCHED();
-  quantile_metrics_kernel<<<1, 1024, 0, st>>>(ag->qloss, nblk, ag->qtd, n, B,
-                                              float(B) * float(M) * float(ag->nq_keep), ag->mdev, M_CLOSS, M_TD,
-                                              ag->per_on ? ag->per_td : nullptr);
+  quantile_metrics_kernel<<<1, 1024, 0, st>>>(loss_part, nblk, td_part, n, B, float(B) * float(M) * float(K), out,
+                                              slot_loss, slot_td, td_rows);
   GCRL_LAUNCHED();
+}
+
+// target atoms in qt -> y; critic atoms in q -> dZ in dq, per-critic losses, td (and the prioritised TD rows)
+void quantile_critic_loss(gcrl_sac *ag, int B, cudaStream_t st) {
+  quantile_critic_loss(ag->qt, ag->q, ag->qstride, ag->ldm, ag->n, ag->nq, ag->nq_keep, ag->logp, ag->br, ag->bd,
+                       ag->per_on ? ag->per_w : nullptr, ag->cfg.gamma, ag->cfg.entropy_coef, ag->alpha_state + 1,
+                       ag->y, ag->ldy, ag->dq, ag->mdev, M_CLOSS, M_TD, ag->per_on ? ag->per_td : nullptr,
+                       ag->qscratch, B, st);
 }
 
 // *out = mean over the batch of quantile_row_mean_kernel's row values of the atoms z (see there for logp / dz)
@@ -1854,9 +1866,8 @@ static void sac_create(gcrl_sac **out, int device, const gcrl_sac_config *cfg, i
     ag->q = dev_alloc<float>(n * ag->qstride); ag->qt = dev_alloc<float>(n * ag->qstride);
     ag->dq = dev_alloc<float>(n * std::max<int64_t>(ag->qstride, mb * 4));
     if (nq > 0) {
-      ag->qloss = dev_alloc<float>(mb * (2 * n + 1));
-      ag->qtd = ag->qloss + mb * n;
-      ag->qrow = ag->qtd + mb * n;
+      ag->qscratch = dev_alloc<float>(mb * (2 * n + 1));
+      ag->qrow = ag->qscratch + 2 * mb * n;
     }
     for (float **p : {&ag->act4, &ag->std4, &ag->gate4, &ag->dact, &ag->eps_next, &ag->eps_cur}) *p = dev_alloc<float>(mb * 4);
     ag->dzh = dev_alloc<float>(mb * 8);
@@ -1920,7 +1931,7 @@ int gcrl_sac_destroy(gcrl_sac *ag) {
   for (float *p : {ag->invstd, ag->dz[0], ag->dz[1], ag->sa, ag->nsa, ag->spi, ag->br, ag->bd, ag->bs, ag->ba, ag->bns,
                    ag->br0, ag->bd0, ag->q, ag->qt, ag->y, ag->dq, ag->logp, ag->act4, ag->std4, ag->gate4, ag->dact,
                    ag->dzh, ag->eps_next, ag->eps_cur, ag->partials, ag->sumsq, ag->mdev, ag->d_io,
-                   ag->critic_grads, ag->per_w, ag->per_td, ag->qloss})
+                   ag->critic_grads, ag->per_w, ag->per_td, ag->qscratch})
     if (p) cudaFree(p);
   for (auto &kv : ag->graphs) cudaGraphExecDestroy(kv.second.exec);
   ag->many.graphs.clear();
@@ -2214,6 +2225,28 @@ int gcrl_sac_act(gcrl_sac *ag, int64_t n, const float *obs_host, const float *ep
   actor_fwd(ag, ag->spi, eps, int(n), false, false, out, st);     // set_eval(): running statistics
   GCRL_CUDA(cudaMemcpyAsync(act_host, out, size_t(n) * A * 4, cudaMemcpyDeviceToHost, st));
   GCRL_CUDA(cudaStreamSynchronize(st));
+  GCRL_API_END
+}
+
+int gcrl_quantile_critic_loss(int device, int n, int M, int drop, int64_t B, const float *zt_dev, const float *z_dev,
+                              int ldm, int64_t zstride, const float *logp_dev, const float *r_dev, const float *d_dev,
+                              const float *w_dev, float gamma, float coef, const float *alpha_dev, float *y_dev, int ldy,
+                              float *dz_dev, float *out_dev, float *td_rows_dev, float *scratch_dev, void *stream) {
+  GCRL_API_BEGIN
+  GCRL_REQUIRE(n >= 1 && n <= kMaxCritics, "n_critics outside [1, 8]");
+  GCRL_REQUIRE(M >= 1 && n * M <= 256, "need n_quantiles >= 1 and n_critics * n_quantiles <= 256");
+  GCRL_REQUIRE(drop >= 0 && drop < M, "drop_per_net outside [0, n_quantiles)");
+  GCRL_REQUIRE(B >= 1 && B < (int64_t(1) << 31), "batch size outside [1, 2^31)");
+  const int K = n * (M - drop);
+  GCRL_REQUIRE(ldm >= M && ldm % 4 == 0, "ldm must be >= n_quantiles and a multiple of 4");
+  GCRL_REQUIRE(zstride >= B * ldm, "zstride must be >= B * ldm");
+  GCRL_REQUIRE(ldy >= K && ldy % 4 == 0, "ldy must be >= n_critics * (n_quantiles - drop_per_net) and a multiple of 4");
+  GCRL_REQUIRE(coef >= 0.f || alpha_dev != nullptr, "coef < 0 reads the coefficient from alpha_dev: NULL");
+  GCRL_REQUIRE(zt_dev && z_dev && logp_dev && r_dev && d_dev && y_dev && dz_dev && out_dev && scratch_dev,
+               "NULL argument");
+  GCRL_CUDA(cudaSetDevice(device));
+  quantile_critic_loss(zt_dev, z_dev, zstride, ldm, n, M, K, logp_dev, r_dev, d_dev, w_dev, gamma, coef, alpha_dev,
+                       y_dev, ldy, dz_dev, out_dev, 0, n, td_rows_dev, scratch_dev, int(B), as_stream(stream));
   GCRL_API_END
 }
 

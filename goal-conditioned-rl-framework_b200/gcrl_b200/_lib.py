@@ -159,6 +159,8 @@ SIGNATURES = {
                                    vp, c_i64, C.c_int, C.POINTER(C.c_int), vp]),
     "gcrl_dense_layer": (C.c_int, [C.c_int, C.c_int, C.c_int, c_i64, C.c_int, C.c_int, vp, C.c_int, vp, C.c_int, vp,
                                    vp, C.c_int, vp, C.c_int, vp]),
+    "gcrl_quantile_critic_loss": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, c_i64, vp, vp, C.c_int, c_i64, vp, vp,
+                                            vp, vp, c_f32, c_f32, vp, vp, C.c_int, vp, vp, vp, vp, vp]),
 }
 
 

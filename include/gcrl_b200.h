@@ -578,6 +578,21 @@ int gcrl_dense_wgrad(int device, int engine, int64_t M, int N, int K, const floa
                      const float *x_dev, int ldx, float *pw_dev, int ldw, int64_t w_split_stride,
                      float *pb_dev, int64_t b_split_stride, int max_splits, int *splits_out, void *stream);
 
+/* The quantile-critic loss of a TQC update on caller buffers: the same three launches
+ * (quantile_target_kernel<KPL> -> quantile_huber_kernel -> quantile_metrics_kernel) an update issues.
+ *   1 <= n <= 8 critics of M >= 1 atoms, n * M <= 256, 0 <= drop < M dropped per critic, K = n (M - drop) kept
+ *   zt, z : [n][B][ldm] target / current atoms, critic i at + i * zstride (ldm >= M, multiple of 4; the agent's is
+ *           pad4(M); zstride >= B * ldm)
+ *   logp, r, d : [B];  w : [B] importance weights or NULL;  coef >= 0: entropy coefficient, < 0: *alpha_dev
+ *   y  : [B][ldy] sorted, truncated targets, ldy >= K, multiple of 4
+ *   dz : [n][B][ldm] (same layout as z);  out : float[n + 1], per-critic losses then the batch-mean TD;
+ *   td_rows : [B] or NULL;  scratch : n * (B + ceil(B / max(1, 256 / M))) floats
+ * Only columns < M of z / zt and < K of y, and rows < B, are read or written. */
+int gcrl_quantile_critic_loss(int device, int n, int M, int drop, int64_t B, const float *zt_dev, const float *z_dev,
+                              int ldm, int64_t zstride, const float *logp_dev, const float *r_dev, const float *d_dev,
+                              const float *w_dev, float gamma, float coef, const float *alpha_dev, float *y_dev, int ldy,
+                              float *dz_dev, float *out_dev, float *td_rows_dev, float *scratch_dev, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

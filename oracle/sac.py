@@ -174,6 +174,7 @@ class ScalarAdamW:
 
 class SACOracle:
     """algo = 'sac' | 'tqc'."""
+    ENSEMBLE = {"sac": 2, "tqc": 5}      # the reference's critic counts; None: any count (a subclass's own critics)
 
     def __init__(self, algo, actor, actor_stats, critics, *, act_dim, gamma, tau, grad_clip, actor_lr,
                  critic_lr, alpha_lr, alpha_min_steps, gradient_step, actor_lr_min=None, critic_lr_min=None,
@@ -186,7 +187,7 @@ class SACOracle:
         self.target_critics = [clone_params(c) for c in critics]
         self.n = len(critics)
         self.drop = 1 if algo == "sac" else 2
-        assert self.n == (2 if algo == "sac" else 5)
+        assert self.ENSEMBLE is None or self.n == self.ENSEMBLE[algo]
         self.actor_opt = AdamState(self.actor, ADAMW_WD)
         self.critic_opts = [AdamState(c, ADAMW_WD) for c in self.critics]
         self.actor_sched = CosineAnnealingLR(actor_lr, ac_scheduler_steps,

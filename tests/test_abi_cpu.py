@@ -77,6 +77,23 @@ def test_header_compiles_as_plain_c_and_struct_sizes_agree(tmp_path):
     assert [int(x) for x in out] == [ctypes.sizeof(AgentConfig), ctypes.sizeof(SacConfig), 5]
 
 
+def test_quantile_critic_loss_refuses_bad_arguments():
+    """gcrl_quantile_critic_loss checks its sizes, leading dimensions and operands before it touches a device (every
+    buffer is NULL: nothing here can launch)."""
+    from gcrl_b200._lib import ERR_INVALID, lib
+
+    def call(n=5, M=25, drop=2, B=64, ldm=28, zstride=64 * 28, ldy=116, coef=0.2):
+        return lib.gcrl_quantile_critic_loss(0, n, M, drop, B, None, None, ldm, zstride, None, None, None, None, 0.98,
+                                             coef, None, None, ldy, None, None, None, None, None)
+    for kw, msg in [(dict(n=0), b"n_critics"), (dict(n=9), b"n_critics"), (dict(M=0), b"n_quantiles"),
+                    (dict(n=8, M=33, ldm=36, zstride=64 * 36), b"256"), (dict(drop=25), b"drop"),
+                    (dict(drop=-1), b"drop"), (dict(B=0), b"batch"), (dict(ldm=24), b"ldm"), (dict(ldm=30), b"ldm"),
+                    (dict(zstride=64 * 28 - 1), b"zstride"), (dict(ldy=112), b"ldy"), (dict(ldy=118), b"ldy"),
+                    (dict(coef=-1.0), b"alpha_dev"), ({}, b"NULL")]:
+        assert call(**kw) == ERR_INVALID, kw
+        assert msg in lib.gcrl_last_error(), (kw, lib.gcrl_last_error())
+
+
 def test_no_cpu_fallback_without_device():
     """Without a GPU the product must fail loudly, never compute on the host."""
     from gcrl_b200 import _lib

@@ -22,8 +22,8 @@ pytestmark = pytest.mark.gpu
 ENG = 4.0
 
 
-def make_pair(B, H, L, D, A, M, drop, seed=5, precision=0, reference=True, **over):
-    """A quantile TQCAgent and the reference on the same seeded initial networks."""
+def make_pair(B, H, L, D, A, M, drop, seed=5, precision=0, reference=True, n=5, **over):
+    """A quantile TQCAgent with n critics and the reference on the same seeded initial networks."""
     from gcrl_b200 import TQCAgent
     from oracle import ddpg as OD
     from oracle import sac as OS
@@ -31,8 +31,12 @@ def make_pair(B, H, L, D, A, M, drop, seed=5, precision=0, reference=True, **ove
     cfg = sac_config(hidden_dim=H, layer_count=L, batch_size=B, grad_clip=0.5, tau=0.05, alpha_min_steps=1,
                      alpha_lr=1e-2, **over)
     actor0, stats0 = OS.init_sac_actor(rng, D, H, A, L, head_scale=0.1, log_std_bias=-1.0)
-    critics0 = [OD.init_mlp(rng, D + A, H, M, L) for _ in range(5)]
-    ag = TQCAgent(D, A, cfg, None, 1, 2, n_quantiles=M, top_quantiles_to_drop_per_net=drop, precision=precision)
+    critics0 = [OD.init_mlp(rng, D + A, H, M, L) for _ in range(n)]
+
+    class _TQC8(TQCAgent):
+        N_CRITICS = 8
+    cls = {5: TQCAgent, 8: _TQC8}[n]
+    ag = cls(D, A, cfg, None, 1, 2, n_quantiles=M, top_quantiles_to_drop_per_net=drop, precision=precision)
     load_initial(ag, actor0, stats0, critics0)
     orc = None
     if reference:
@@ -101,15 +105,22 @@ def assert_within_adam_bound(ag, orc, lr, n):
 
 
 # ---- 1. three updates against the reference ----------------------------------------------------------------------
-SHAPES = [(33, 64, 1, 7, 1, 5, 0), (256, 256, 3, 21, 3, 25, 2), (512, 512, 3, 22, 4, 25, 2),
-          (64, 64, 2, 10, 2, 1, 0), (4608, 64, 2, 10, 2, 25, 2)]
+# (B, H, L, D, A, M, drop, critics).  The target kernel sorts n M keys in a warp at KPL = 1, 2, 4, 8 keys per lane
+# (n M up to 32, 64, 128, 256): M = 12 runs KPL 2, M = 51 KPL 8 with a head two 32-wide fp32 tiles tall (d = 50
+# keeps K = 5 targets, fewer than a warp's lanes), eight critics of 32 atoms fill the 256 keys and every loss slot.
+# B = 10000 is more rows than the 64 x 148 warps of the capped grids of the target and row-mean kernels.
+SHAPES = [(33, 64, 1, 7, 1, 5, 0, 5), (256, 256, 3, 21, 3, 25, 2, 5), (512, 512, 3, 22, 4, 25, 2, 5),
+          (64, 64, 2, 10, 2, 1, 0, 5), (4608, 64, 2, 10, 2, 25, 2, 5), (256, 64, 2, 10, 2, 12, 2, 5),
+          (512, 256, 2, 22, 3, 51, 0, 5), (512, 256, 2, 22, 3, 51, 50, 5), (10000, 64, 2, 10, 2, 25, 2, 5),
+          (256, 64, 2, 10, 2, 32, 0, 8)]
 
 
-@pytest.mark.parametrize("B,H,L,D,A,M,drop", SHAPES, ids=[f"B{s[0]}_H{s[1]}_M{s[5]}_d{s[6]}" for s in SHAPES])
-def test_updates_match_reference(B, H, L, D, A, M, drop):
+@pytest.mark.parametrize("B,H,L,D,A,M,drop,n", SHAPES,
+                         ids=[f"B{s[0]}_H{s[1]}_M{s[5]}_d{s[6]}" + (f"_n{s[7]}" if s[7] != 5 else "") for s in SHAPES])
+def test_updates_match_reference(B, H, L, D, A, M, drop, n):
     """Actor and alpha steps included (alpha from step 2); M = 1 is the quantile rule with one atom (tau 0.5, Huber),
     not the scalar MSE path; B = 4608 runs the per-critic backward above the ensemble's batch limit."""
-    ag, orc, rng = make_pair(B, H, L, D, A, M, drop)
+    ag, orc, rng = make_pair(B, H, L, D, A, M, drop, n=n)
     for step in (1, 2, 3):
         batch, e1, e2 = rand_batch(rng, B, D, A)
         want = np.array(orc.update_on_batch(step, *batch, e1, e2), np.float64)

@@ -48,7 +48,8 @@ def quantile_huber(z, y, w=None):
 
 
 class QuantileTQCOracle(SACOracle):
-    """SACOracle('tqc', ...) with critics whose last Linear is H -> n_quantiles."""
+    """SACOracle('tqc', ...) with critics whose last Linear is H -> n_quantiles, as many as the critic list holds."""
+    ENSEMBLE = None
 
     def __init__(self, actor, actor_stats, critics, *, n_quantiles, drop_per_net, **kw):
         super().__init__("tqc", actor, actor_stats, critics, **kw)
