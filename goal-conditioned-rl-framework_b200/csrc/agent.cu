@@ -1552,4 +1552,17 @@ int gcrl_agent_metrics_buffer(gcrl_agent *ag, float **metrics_dev) {
   GCRL_API_END
 }
 
+int gcrl_agent_param_buffers(gcrl_agent *ag, int net, const float **flat_dev, int64_t *count,
+                             const float **flat_t_dev, int64_t *count_t) {
+  GCRL_API_BEGIN
+  require_handle(ag);
+  GCRL_REQUIRE(ag && net >= 0 && net < NUM_NETS && ag->has[net] && ag->net[net].p, "bad network id");
+  const MlpParams &n = ag->net[net];
+  if (flat_dev) *flat_dev = n.p;
+  if (count) *count = n.total;
+  if (flat_t_dev) *flat_t_dev = n.copies.pT;
+  if (count_t) *count_t = n.copies.pT ? n.copies.total_t : 0;
+  GCRL_API_END
+}
+
 }  // extern "C"

@@ -539,6 +539,17 @@ int gcrl_her_set_draw_epoch(gcrl_her *h, uint64_t epoch) {
   GCRL_API_END
 }
 
+int gcrl_her_index_tables(gcrl_her *h, const void **eps_dev, int64_t *eps_bytes, const void **buckets_dev,
+                          int64_t *bucket_bytes) {
+  GCRL_API_BEGIN
+  GCRL_REQUIRE(h != nullptr, "handle is NULL");
+  if (eps_dev) *eps_dev = h->g.eps;
+  if (eps_bytes) *eps_bytes = h->cap_ep * int64_t(sizeof(EpRec));
+  if (buckets_dev) *buckets_dev = h->g.buckets;
+  if (bucket_bytes) *bucket_bytes = h->nb * int64_t(sizeof(BucketRec));
+  GCRL_API_END
+}
+
 int64_t gcrl_her_len(const gcrl_her *h) { return h ? h->len() : 0; }
 int64_t gcrl_her_total_entries(const gcrl_her *h) { return h ? h->total_entries : 0; }
 int64_t gcrl_her_live_transitions(const gcrl_her *h) {

@@ -56,6 +56,7 @@ SIGNATURES = {
     "gcrl_her_set_goal_selection": (C.c_int, [vp, C.c_int, C.c_int]),
     "gcrl_her_get_draw_epoch": (c_u64, [vp]),
     "gcrl_her_set_draw_epoch": (C.c_int, [vp, c_u64]),
+    "gcrl_her_index_tables": (C.c_int, [vp, pp, C.POINTER(c_i64), pp, C.POINTER(c_i64)]),
     "gcrl_her_len": (c_i64, [vp]),
     "gcrl_her_total_entries": (c_i64, [vp]),
     "gcrl_her_live_transitions": (c_i64, [vp]),
@@ -106,6 +107,7 @@ SIGNATURES = {
     "gcrl_agent_dp_barrier": (C.c_int, [vp, vp]),
     "gcrl_agent_grad_buffer": (C.c_int, [vp, C.c_int, pp, C.POINTER(c_i64)]),
     "gcrl_agent_metrics_buffer": (C.c_int, [vp, pp]),
+    "gcrl_agent_param_buffers": (C.c_int, [vp, C.c_int, pp, C.POINTER(c_i64), pp, C.POINTER(c_i64)]),
     # SAC / TQC
     "gcrl_sac_create": (C.c_int, [pp, C.c_int, C.POINTER(SacConfig)]),
     "gcrl_sac_create_quantile": (C.c_int, [pp, C.c_int, C.POINTER(SacConfig), C.c_int, C.c_int]),

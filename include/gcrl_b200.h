@@ -98,6 +98,10 @@ int gcrl_her_set_goal_selection(gcrl_her *h, int strategy, int online_k);
  * device; in online mode one per sample call).  A checkpoint saves it so that a resumed run draws the same rows. */
 uint64_t gcrl_her_get_draw_epoch(const gcrl_her *h);
 int gcrl_her_set_draw_epoch(gcrl_her *h, uint64_t epoch);
+/* Diagnostics (cache experiments, profiles/cold_start.py): the device episode and bucket index tables that map a
+ * deque position to its row, with their sizes in bytes. */
+int gcrl_her_index_tables(gcrl_her *h, const void **eps_dev, int64_t *eps_bytes, const void **buckets_dev,
+                          int64_t *bucket_bytes);
 int64_t gcrl_her_len(const gcrl_her *h);            /* __len__, src/buffer.py:137-138   */
 int64_t gcrl_her_total_entries(const gcrl_her *h);  /* entries ever appended            */
 int64_t gcrl_her_live_transitions(const gcrl_her *h);
@@ -309,6 +313,10 @@ int gcrl_agent_grad_buffer(gcrl_agent *h, int net, float **grad_dev, int64_t *co
 /* device float[8] holding the metrics of the most recent update (averaged across ranks by the
  * caller when a data-parallel run wants global losses) */
 int gcrl_agent_metrics_buffer(gcrl_agent *h, float **metrics_dev);
+/* Diagnostics (cache experiments, profiles/cold_start.py): a network's flat parameter buffer and its transposed
+ * copy, device pointers and element counts (NULL and 0 when the network keeps no transposed copy). */
+int gcrl_agent_param_buffers(gcrl_agent *h, int net, const float **flat_dev, int64_t *count,
+                             const float **flat_t_dev, int64_t *count_t);
 
 /* ------------------------------------------------------------------------------------
  * Stochastic-actor agents -- replace SACAgent (src/agent.py:388-770) and TQCAgent (:773-1171)
