@@ -734,9 +734,10 @@ void run_many(gcrl_agent *ag, gcrl_her *her, gcrl_replay *rb, int B, int n, cons
                          ag->use_graphs, ag->cap_stream);
 }
 
-// The row-slab critic kernel draws the batch itself from `buf` (else the sampler is a launch of its own)
+// The row-slab critic kernel draws the batch itself from `buf` (else the sampler is a launch of its own).  Its
+// in-kernel sampler draws one-step rows only: an n-step buffer always takes the standalone sampler.
 bool samples_in_kernel(const gcrl_agent *ag, const gcrl_her *buf, int64_t B) {
-  return fused_ok(ag, int(B)) && ag->fuse_sampler && fused_sample_supported(her_geom(buf));
+  return fused_ok(ag, int(B)) && ag->fuse_sampler && her_n_step(buf) == 1 && fused_sample_supported(her_geom(buf));
 }
 
 // Stage one batch (sampled from `buf`, or the caller's dense device batch) into the operand rows.

@@ -13,6 +13,7 @@ void her_sample_into(gcrl_her *h, int64_t B, const int64_t *idx_host, float *s, 
 int her_state_dim(const gcrl_her *h);
 int her_act_dim(const gcrl_her *h);
 int her_device(const gcrl_her *h);
+int her_n_step(const gcrl_her *h);
 void her_sample_graphed(gcrl_her *h, int64_t B, const SampleScalars *sc_dev, const int64_t *idx_dev, float *s,
                         float *a, float *r, float *ns, float *d, cudaStream_t st);
 unsigned long long &her_draw_epoch(gcrl_her *h);

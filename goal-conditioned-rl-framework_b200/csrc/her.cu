@@ -113,18 +113,62 @@ __device__ __forceinline__ void write_field(float *__restrict__ out, const float
   }
 }
 
-template <bool VEC, int SPB>
+// sparse reward of achieved goal `a` against goal `gf` (her_relabel_row's rule): -1.0f, or -0.0f on success
+__device__ __forceinline__ float her_sparse_reward(const HerGeom &g, const float *a, const float *gf) {
+  float acc = 0.f;
+  for (int c = 0; c < g.G; ++c) {
+    const float diff = __fsub_rn(a[c], gf[c]);
+    const float sq = __fmul_rn(diff, diff);
+    acc = (c == 0) ? sq : __fadd_rn(acc, sq);
+  }
+  // the word goes through an opaque move: seen as a float select of {-1.0f, -0.0f}, nvcc 12.9 rewrites it into
+  // int->float(-(int)pred), which yields +0.0f (see her_relabel_row)
+  const uint32_t w = 0x80000000u | ((__fsqrt_rn(acc) > g.threshold) ? 0x3F800000u : 0u);
+  float r;
+  asm("mov.b32 %0, %1;" : "=f"(r) : "r"(w));
+  return r;
+}
+
+// window steps whose reward word / achieved goal one thread has in flight at once: n <= 7 takes one round of loads
+// (a chunk of 8 spills in the 16 B-store instantiation, 6 uses 82 registers and none)
+constexpr int kNStepChunk = 6;
+
+// ring slot of window step t+i (i < T - t <= cap_tr: one wrap at most)
+__device__ __forceinline__ uint32_t her_window_slot(const HerGeom &g, const SampleRef &r, uint32_t i) {
+  uint32_t s = r.slot + i;
+  if (s >= g.cap_tr) s -= g.cap_tr;
+  return s;
+}
+
+// what window step t+i contributes to an n-step reward: its stored reward word (j = 0, in .x), or its achieved goal
+// from the compact copy (relabelled, G <= 4; wider goals are read column by column where they are used)
+__device__ __forceinline__ float4 her_window_load(const HerGeom &g, const SampleRef &r, uint32_t i) {
+  const uint32_t s = her_window_slot(g, r, i);
+  if (r.j == 0) return make_float4(__ldg(g.rows + size_t(s) * g.row_f + g.off_r), 0.f, 0.f, 0.f);
+  if (g.G <= 4) return __ldg(reinterpret_cast<const float4 *>(g.ag + size_t(s) * g.gpad));
+  return make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
+// NSTEP: n-step rows (DESIGN.md section 2).  Sample i at step t of an episode of T steps takes the window
+// t .. t+k-1, k = min(n, T - t): r <- r_t + gamma (r_{t+1} + gamma (... + gamma r_{t+k-1})) (unfused fp32, from the
+// back), s' <- ns of row t+k-1 (goal columns <- the sample's goal), d <- 1 - gamma^(k-1) (1 - done_{t+k-1}), so that
+// gamma (1 - d) is the bootstrap weight gamma^k (1 - done).  Relabelled rows recompute every r_{t+i} for their goal
+// from the compact ag array and take done = 0.  k = 1 rows are the one-step rows.
+template <bool VEC, int SPB, bool NSTEP>
 __global__ void __launch_bounds__(kSampleThreads)
 her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg, const SampleScalars *__restrict__ sc_dev,
                   int64_t B, const int64_t *__restrict__ idx,
                   float *__restrict__ out_s, float *__restrict__ out_a, float *__restrict__ out_r,
-                  float *__restrict__ out_ns, float *__restrict__ out_d, int64_t *__restrict__ idx_out) {
+                  float *__restrict__ out_ns, float *__restrict__ out_d, int64_t *__restrict__ idx_out,
+                  const NStepArgs nst) {
   // sc_dev: the totals and draw epoch of this launch's update, written by the host before a replayed graph runs
   // (a value captured into the graph would freeze them); otherwise they come by value
   const SampleScalars sc = sc_dev != nullptr ? *sc_dev : sc_arg;
   extern __shared__ float4 smem4[];
   float *tile = reinterpret_cast<float *>(smem4);
   uint32_t *m_row = reinterpret_cast<uint32_t *>(tile + SPB * g.row_f);
+  uint32_t *m_last = m_row + SPB;                                  // NSTEP: ring slot of row t+k-1
+  float *tile_ns = reinterpret_cast<float *>(m_last + SPB);        // NSTEP: [SPB][D] s' of row t+k-1
 
   const int tid = threadIdx.x;
   const int64_t base = int64_t(blockIdx.x) * SPB;
@@ -132,8 +176,18 @@ her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg,
 
   // ---- round trip 1: deque position -> bucket record -> (episode, t, j) -> ring slot (her_device.cuh) ----
   SampleRef ref{0u, 0u, 0u, 0u};
+  uint32_t k = 1;
   if (tid < n) {
-    ref = her_resolve(g, sc, base + tid, sc.use_idx ? idx : nullptr, idx_out);
+    if constexpr (NSTEP) {
+      const SampleRefN rn = her_resolve_n(g, sc, base + tid, sc.use_idx ? idx : nullptr, idx_out);
+      ref = rn.r;
+      k = min(uint32_t(nst.n), rn.T - rn.t);
+      uint32_t last = ref.slot + k - 1;
+      if (last >= g.cap_tr) last -= g.cap_tr;
+      m_last[tid] = last;
+    } else {
+      ref = her_resolve(g, sc, base + tid, sc.use_idx ? idx : nullptr, idx_out);
+    }
     m_row[tid] = ref.slot;
   }
   __syncthreads();
@@ -160,6 +214,25 @@ her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg,
         if (c < nchunks) smem4[c] = v[u];
       }
     }
+    if constexpr (NSTEP) {       // s' segment of row t+k-1, into its own tile
+      const int total = n * g.D;
+      for (int e0 = tid; e0 < total; e0 += kSampleThreads * U) {
+        float v[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+          const int e = e0 + u * kSampleThreads;
+          if (e < total) {
+            const uint32_t i = g.div_D.div(e), c = e - i * g.D;
+            v[u] = __ldg(g.rows + size_t(m_last[i]) * g.row_f + g.off_ns + c);
+          }
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+          const int e = e0 + u * kSampleThreads;
+          if (e < total) tile_ns[e] = v[u];
+        }
+      }
+    }
   }
   // ---- round trip 3: the relabel goal (issued before the barrier: it overlaps the tail of the gather; where
   //      her_resolve knew the goal step without the offset word, it does not depend on round trip 2)
@@ -170,6 +243,20 @@ her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg,
     if (g.G <= 4) {
       const float4 v = __ldg(reinterpret_cast<const float4 *>(agf));
       gf[0] = v.x; gf[1] = v.y; gf[2] = v.z; gf[3] = v.w;
+    }
+  }
+  // NSTEP: the last kNStepChunk window steps' reward words (or, relabelled, achieved goals) and the done word of row
+  // t+k-1 ride with the goal: none of them depends on it
+  float4 wv[NSTEP ? kNStepChunk : 1];
+  float done_last = 0.f;
+  if constexpr (NSTEP) {
+    if (tid < n && k > 1) {
+      if (ref.j == 0) done_last = __ldg(g.rows + size_t(m_last[tid]) * g.row_f + g.off_d);
+#pragma unroll
+      for (int u = 0; u < kNStepChunk; ++u) {
+        const int i = int(k) - 1 - u;
+        if (i >= 1) wv[u] = her_window_load(g, ref, uint32_t(i));
+      }
     }
   }
   __syncthreads();
@@ -194,12 +281,52 @@ her_sample_kernel(const __grid_constant__ HerGeom g, const SampleScalars sc_arg,
       row[g.off_d] = 0.0f;
     }
   }
+  if constexpr (NSTEP) {
+    if (tid < n) {
+      float *row = tile + tid * g.row_f;
+      if (ref.j > 0)
+        for (int c = 0; c < g.G; ++c) tile_ns[tid * g.D + g.D - g.G + c] = g.G <= 4 ? gf[c] : __ldg(agf + c);
+      if (k > 1) {
+        // window steps k-1 .. 1, from the back, kNStepChunk per round of loads (the first round was issued above)
+        float acc = 0.f;
+        for (int hi = int(k) - 1; hi >= 1; hi -= kNStepChunk) {
+          if (hi != int(k) - 1) {
+#pragma unroll
+            for (int u = 0; u < kNStepChunk; ++u)
+              if (hi - u >= 1) wv[u] = her_window_load(g, ref, uint32_t(hi - u));
+          }
+#pragma unroll
+          for (int u = 0; u < kNStepChunk; ++u) {
+            const int i = hi - u;
+            if (i < 1) break;
+            float ri;
+            if (ref.j == 0) {
+              ri = wv[u].x;
+            } else if (g.G <= 4) {
+              const float a4[4] = {wv[u].x, wv[u].y, wv[u].z, wv[u].w};
+              ri = her_sparse_reward(g, a4, gf);
+            } else {
+              ri = her_sparse_reward(g, g.ag + size_t(her_window_slot(g, ref, uint32_t(i))) * g.gpad, agf);
+            }
+            acc = (i == int(k) - 1) ? ri : __fadd_rn(ri, __fmul_rn(nst.gamma, acc));
+          }
+        }
+        float p = 1.f;                                    // gamma^(k-1), k-1 rounded products
+        for (uint32_t i = 1; i < k; ++i) p = __fmul_rn(p, nst.gamma);
+        row[g.off_r] = __fadd_rn(row[g.off_r], __fmul_rn(nst.gamma, acc));
+        row[g.off_d] = __fsub_rn(1.f, __fmul_rn(p, __fsub_rn(1.f, ref.j > 0 ? 0.f : done_last)));
+      }
+    }
+  }
   __syncthreads();
 
   // ---- coalesced write-out of the five output tensors ---------------------------------------------------
   const FastDiv one(1);
   write_field<VEC>(out_s + base * g.D, tile, n, g.D, 0, g.row_f, g.div_D, tid);
-  write_field<VEC>(out_ns + base * g.D, tile, n, g.D, g.off_ns, g.row_f, g.div_D, tid);
+  if constexpr (NSTEP)
+    write_field<VEC>(out_ns + base * g.D, tile_ns, n, g.D, 0, g.D, g.div_D, tid);
+  else
+    write_field<VEC>(out_ns + base * g.D, tile, n, g.D, g.off_ns, g.row_f, g.div_D, tid);
   write_field<VEC>(out_a + base * g.A, tile, n, g.A, g.off_a, g.row_f, g.div_A, tid);
   write_field<VEC>(out_r + base, tile, n, 1, g.off_r, g.row_f, one, tid);
   write_field<VEC>(out_d + base, tile, n, 1, g.off_d, g.row_f, one, tid);
@@ -232,6 +359,7 @@ struct gcrl_her {
   int64_t *d_idx_out = nullptr;
   size_t out_cap = 0;
   size_t smem_bytes = 0;
+  NStepArgs nstep{1, 1.f};                   // gcrl_her_set_n_step
 
   int64_t len() const { return std::min(total_entries, max_entries); }
 };
@@ -253,6 +381,8 @@ int64_t her_len(const gcrl_her *h) { return h->len(); }
 
 static constexpr int kSmallTile = 32;      // samples per CTA while the batch is too small to fill the SMs with 128
 static size_t sample_smem(const gcrl_her *h, int spb) { return size_t(spb) * h->g.row_f * 4 + size_t(spb) * 4; }
+// the n-step tile adds the slot of each sample's last window row and that row's s'
+static size_t sample_smem_nstep(const gcrl_her *h, int spb) { return sample_smem(h, spb) + size_t(spb) * (4 + h->g.D * 4); }
 
 // sc_dev == nullptr: this call draws the scalars (her_next_scalars) and passes them by value
 static void her_launch_sample(gcrl_her *h, int64_t B, const int64_t *idx_dev, float *s, float *a,
@@ -265,14 +395,14 @@ static void her_launch_sample(gcrl_her *h, int64_t B, const int64_t *idx_dev, fl
   const bool small = B <= int64_t(sm_count()) * 4 * kSmallTile;
   const int spb = small ? kSmallTile : kSamplesPerBlock;
   const unsigned blocks = unsigned((B + spb - 1) / spb);
-  const size_t smem = sample_smem(h, spb);
-  if (small) {
-    if (vec) her_sample_kernel<true, kSmallTile><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out);
-    else her_sample_kernel<false, kSmallTile><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out);
-  } else {
-    if (vec) her_sample_kernel<true, kSamplesPerBlock><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out);
-    else her_sample_kernel<false, kSamplesPerBlock><<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out);
-  }
+  const bool nstep = h->nstep.n > 1;
+  const size_t smem = nstep ? sample_smem_nstep(h, spb) : sample_smem(h, spb);
+  const NStepArgs nst = h->nstep;
+  auto kernel = small ? (nstep ? (vec ? her_sample_kernel<true, kSmallTile, true> : her_sample_kernel<false, kSmallTile, true>)
+                               : (vec ? her_sample_kernel<true, kSmallTile, false> : her_sample_kernel<false, kSmallTile, false>))
+                      : (nstep ? (vec ? her_sample_kernel<true, kSamplesPerBlock, true> : her_sample_kernel<false, kSamplesPerBlock, true>)
+                               : (vec ? her_sample_kernel<true, kSamplesPerBlock, false> : her_sample_kernel<false, kSamplesPerBlock, false>));
+  kernel<<<blocks, kSampleThreads, smem, st>>>(h->g, sc, sc_dev, B, idx_dev, s, a, r, ns, d, idx_out, nst);
   GCRL_LAUNCHED();
 }
 
@@ -318,6 +448,7 @@ unsigned long long &her_draw_epoch(gcrl_her *h) { return h->draw_epoch; }
 int her_state_dim(const gcrl_her *h) { return h->g.D; }
 int her_act_dim(const gcrl_her *h) { return h->g.A; }
 int her_device(const gcrl_her *h) { return h->device; }
+int her_n_step(const gcrl_her *h) { return h->nstep.n; }
 }  // namespace gcrl
 
 static int64_t next_pow2(int64_t x) {
@@ -381,13 +512,13 @@ int gcrl_her_create(gcrl_her **out, int device, int64_t max_entries, int64_t cap
     h->stage.init(h->blob_max);
     for (int i = 0; i < PinnedRing::kSlots; ++i) h->d_stage[i] = dev_alloc<char>(h->blob_max);
     h->idx_stage.init(size_t(1) << 16);
-    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<true, kSamplesPerBlock>,
+    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<true, kSamplesPerBlock, false>,
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, int(h->smem_bytes)));
-    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<false, kSamplesPerBlock>,
+    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<false, kSamplesPerBlock, false>,
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, int(h->smem_bytes)));
-    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<true, kSmallTile>,
+    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<true, kSmallTile, false>,
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, int(sample_smem(h, kSmallTile))));
-    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<false, kSmallTile>,
+    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<false, kSmallTile, false>,
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, int(sample_smem(h, kSmallTile))));
   } catch (...) {
     delete h;
@@ -527,6 +658,29 @@ int gcrl_her_set_goal_selection(gcrl_her *h, int strategy, int online_k) {
   GCRL_REQUIRE(h->next_eid == 0, "the goal selection cannot change once an episode has been committed");
   h->g.strategy = strategy;
   h->g.online_k = online_k;
+  GCRL_API_END
+}
+
+int gcrl_her_set_n_step(gcrl_her *h, int n, float gamma) {
+  GCRL_API_BEGIN
+  GCRL_REQUIRE(h != nullptr, "handle is NULL");
+  GCRL_REQUIRE(n >= 1 && n <= 255, "n_step must be in [1, 255]");
+  GCRL_REQUIRE(n == 1 || (gamma > 0.f && gamma <= 1.f), "n-step returns need a discount gamma in (0, 1]");
+  GCRL_REQUIRE(h->next_eid == 0, "n_step cannot change once an episode has been committed");
+  GCRL_REQUIRE(n == 1 || sample_smem_nstep(h, kSamplesPerBlock) <= 227 * 1024,
+               "transition row too wide for the n-step sampler tile");
+  if (n > 1) {
+    GCRL_CUDA(cudaSetDevice(h->device));
+    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<true, kSamplesPerBlock, true>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, int(sample_smem_nstep(h, kSamplesPerBlock))));
+    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<false, kSamplesPerBlock, true>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, int(sample_smem_nstep(h, kSamplesPerBlock))));
+    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<true, kSmallTile, true>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, int(sample_smem_nstep(h, kSmallTile))));
+    GCRL_CUDA(cudaFuncSetAttribute(her_sample_kernel<false, kSmallTile, true>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, int(sample_smem_nstep(h, kSmallTile))));
+  }
+  h->nstep = NStepArgs{n, n > 1 ? gamma : 1.f};
   GCRL_API_END
 }
 

@@ -105,8 +105,14 @@ struct SampleRef {
   uint32_t slot, ep0, j, futw;
 };
 
-__device__ __forceinline__ SampleRef her_resolve(const HerGeom &g, const SampleScalars &sc, int64_t i,
-                                                 const int64_t *__restrict__ idx, int64_t *__restrict__ idx_out) {
+// The n-step sampler also needs the sample's step t and its episode's length T (the window is t .. t+k-1).
+struct SampleRefN {
+  SampleRef r;
+  uint32_t t, T;
+};
+
+__device__ __forceinline__ SampleRefN her_resolve_n(const HerGeom &g, const SampleScalars &sc, int64_t i,
+                                                    const int64_t *__restrict__ idx, int64_t *__restrict__ idx_out) {
   int64_t p;
   if (idx != nullptr) {
     p = idx[i];
@@ -147,8 +153,20 @@ __device__ __forceinline__ SampleRef her_resolve(const HerGeom &g, const SampleS
                  ? (T - 1) * 0x01010101u
                  : __ldg(reinterpret_cast<const uint32_t *>(g.rows + size_t(slot) * g.row_f + g.off_fut) + ((j - 1) >> 2));
   }
-  return r;
+  return SampleRefN{r, t, T};
 }
+
+__device__ __forceinline__ SampleRef her_resolve(const HerGeom &g, const SampleScalars &sc, int64_t i,
+                                                 const int64_t *__restrict__ idx, int64_t *__restrict__ idx_out) {
+  return her_resolve_n(g, sc, i, idx, idx_out).r;
+}
+
+// n-step returns (gcrl_her_set_n_step): fixed for the buffer's lifetime, passed beside HerGeom so that the row-slab
+// kernel, which embeds HerGeom in its arguments, keeps its parameter layout
+struct NStepArgs {
+  int n;          // 1: one-step rows
+  float gamma;
+};
 
 // ring slot of the transition whose achieved goal relabels this sample (j > 0)
 __device__ __forceinline__ uint32_t her_future_slot(const HerGeom &g, const SampleRef &r) {

@@ -54,6 +54,7 @@ SIGNATURES = {
     "gcrl_her_push_episode": (C.c_int, [vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp]),
     "gcrl_her_set_threshold": (C.c_int, [vp, C.c_float]),
     "gcrl_her_set_goal_selection": (C.c_int, [vp, C.c_int, C.c_int]),
+    "gcrl_her_set_n_step": (C.c_int, [vp, C.c_int, C.c_float]),
     "gcrl_her_get_draw_epoch": (c_u64, [vp]),
     "gcrl_her_set_draw_epoch": (C.c_int, [vp, c_u64]),
     "gcrl_her_index_tables": (C.c_int, [vp, pp, C.POINTER(c_i64), pp, C.POINTER(c_i64)]),

@@ -118,13 +118,16 @@ class _AgentBase:
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, *,
                  index_source="host", device=0, max_batch=None, seed=1898, precision=1,
-                 goal_selection_strategy="future", online_sampling=False):
+                 goal_selection_strategy="future", online_sampling=False, n_step=1):
         """precision: 1 (default) runs the hidden-layer GEMMs of batches >= 2048 on the tcgen05 tensor
         cores with the 3xTF32 split (fp32-level accuracy, rel ~2e-6 per layer); 2 does so for every
         batch >= 128; 0 keeps every GEMM on the fp32 FFMA tiles.
-        goal_selection_strategy / online_sampling: passed to the HER buffer (HERBuffer)."""
+        goal_selection_strategy / online_sampling / n_step: passed to the HER buffer (HERBuffer), n_step with
+        config.gamma.  n_step > 1 needs buffer_type "HER" (ValueError otherwise).  The buffer's rows carry the n-step
+        reward and a done column whose gamma*(1 - done) is gamma**k*(1 - done), so every update computes the n-step
+        target unchanged; SAC / TQC take the entropy term at the bootstrap state only, as Stable-Baselines3 does."""
         self._init_common(obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed,
-                          goal_selection_strategy, online_sampling)
+                          goal_selection_strategy, online_sampling, n_step)
         cfg = AgentConfig(algo=self.ALGO, state_dim=self.obs_dim, act_dim=self.ac_dim,
                           hidden_dim=config.hidden_dim, layer_count=config.layer_count,
                           max_batch=int(max_batch or config.batch_size), gamma=config.gamma,
@@ -139,7 +142,7 @@ class _AgentBase:
         self._metrics = (C.c_float * 8)()
 
     def _init_common(self, obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed,
-                     goal_selection_strategy, online_sampling):
+                     goal_selection_strategy, online_sampling, n_step):
         _lib.require_cuda()
         self.device_index = int(device)
         self.device = f"cuda:{self.device_index}"
@@ -148,11 +151,14 @@ class _AgentBase:
         self.obs_dim, self.ac_dim = int(obs_dim), int(ac_dim)
         self.index_source = index_source
 
+        if n_step != 1 and config.buffer_type != "HER":
+            raise ValueError(f"n_step > 1 needs the HER buffer (its episodes bound the window), got buffer_type "
+                             f"{config.buffer_type!r}")
         if config.buffer_type == "HER":
             self.buffer = HERBuffer(config.max_len, config.max_eps_len, nenvs,
                                     k_future=config.k_future, index_source=index_source,
                                     seed=seed, device=device, goal_selection_strategy=goal_selection_strategy,
-                                    online_sampling=online_sampling)
+                                    online_sampling=online_sampling, n_step=n_step, gamma=config.gamma)
         elif config.buffer_type == "PER":                                  # src/agent.py:67-68
             self.buffer = PERBuffer(config.max_len, config.alpha, device=device)
         elif config.buffer_type == "REPLAY":                               # :69-70

@@ -21,6 +21,20 @@ def _to_np(x, dtype=np.float32):
     return np.asarray(x, dtype=dtype)
 
 
+def _check_n_step(n_step, gamma):
+    """-> (n_step, gamma as a float32 value, None when n_step == 1); ValueError on anything else."""
+    if isinstance(n_step, (bool, np.bool_)) or not isinstance(n_step, (int, np.integer)) or not 1 <= n_step <= 255:
+        raise ValueError(f"n_step must be an integer in [1, 255], got {n_step!r}")
+    if n_step == 1:
+        return 1, None
+    if gamma is None:
+        raise ValueError("n_step > 1 needs the discount gamma")
+    g = float(np.float32(gamma))
+    if not 0.0 < g <= 1.0:
+        raise ValueError(f"gamma must be in (0, 1], got {gamma!r}")
+    return int(n_step), g
+
+
 class HERBuffer:
     """Same constructor, ``push`` / ``sample`` / ``__len__`` and attributes as the
     reference class.  Transitions are staged per env on the host and committed to the GPU
@@ -51,14 +65,24 @@ class HERBuffer:
                ``k_future + 1`` times as many episodes) and every sampled row is relabelled with probability
                k_future / (k_future + 1) to a freshly drawn f (none at t = T-1 for "future" / "final"): coin and f
                come from a hash of (seed, draw epoch, batch row), drawn on the GPU whatever the index source.
+    n_step (Stable-Baselines3's ``n_steps``; 1, the default, samples one-step rows): a sampled row at step t of an
+    episode of T stored steps, with goal g (the original or its relabel), covers the window t .. t+k-1,
+    k = min(n_step, T - t).  ``rewards`` is r_t + gamma*(r_{t+1} + gamma*(... + gamma*r_{t+k-1})) in unfused float32
+    from the back (relabelled rows recompute every r_{t+i} for g with the sparse rule), ``next_states`` is the next
+    state of step t+k-1 (goal columns <- g), and ``dones`` is d' = 1 - gamma**(k-1) * (1 - done_{t+k-1}) (0 for the
+    done of relabelled rows; gamma**(k-1) as k-1 rounded float32 products).  Any learner's gamma*(1 - d') is then the
+    n-step bootstrap weight gamma**k * (1 - done): bit for bit fl(gamma * gamma**(k-1)) while gamma**(k-1) >= 1/2
+    (gamma = 0.98: n_step <= 35), and within 2**-25 of it below.  The window does not stop at the relabel step.
+    ``gamma`` in (0, 1] is required when n_step > 1; n_step is in [1, 255].
     """
     goal_selection_strategy = "future"
     online_sampling = False
 
     def __init__(self, max_mem_len, max_eps_len, nenvs, threshold=0.05, k_future=4, *,
                  index_source="host", seed=1898, cap_transitions=0, device=0,
-                 goal_selection_strategy="future", online_sampling=False):
+                 goal_selection_strategy="future", online_sampling=False, n_step=1, gamma=None):
         _lib.require_cuda()
+        n_step, gamma = _check_n_step(n_step, gamma)
         if index_source not in ("host", "device"):
             raise ValueError(f"index_source must be 'host' or 'device', got {index_source!r}")
         if goal_selection_strategy not in _STRATEGIES:
@@ -85,6 +109,7 @@ class HERBuffer:
         self.online_sampling = bool(online_sampling)
         self.seed = int(seed)
         self.cap_transitions = int(cap_transitions)
+        self.n_step, self.gamma = n_step, gamma
         self._h = None
         self._dims = None
 
@@ -139,6 +164,8 @@ class HERBuffer:
             check(lib.gcrl_her_set_threshold(h, float(self.threshold)))
             check(lib.gcrl_her_set_goal_selection(h, _STRATEGIES[self.goal_selection_strategy],
                                                   self.k_future if self.online_sampling else 0))
+            if self.n_step > 1:
+                check(lib.gcrl_her_set_n_step(h, self.n_step, self.gamma))
         elif self._dims != (D, A, G):
             raise ValueError(f"transition shape changed: {self._dims} -> {(D, A, G)}")
         if not self._reward_checked:
@@ -284,6 +311,8 @@ class HERBuffer:
             sd.update(goal_selection_strategy=self.goal_selection_strategy, online_sampling=self.online_sampling)
         if self.online_sampling:
             sd["draw_epoch"] = self.draw_epoch
+        if self.n_step > 1:
+            sd.update(n_step=self.n_step, gamma=self.gamma)
         return sd
 
     def load_state_dict(self, sd):
@@ -292,6 +321,9 @@ class HERBuffer:
         if (sd.get("goal_selection_strategy", "future") != self.goal_selection_strategy
                 or bool(sd.get("online_sampling", False)) != self.online_sampling):
             raise ValueError("buffer checkpoint was written with a different goal_selection_strategy / online_sampling")
+        if (int(sd.get("n_step", 1)), sd.get("gamma")) != (self.n_step, self.gamma):
+            raise ValueError(f"buffer checkpoint was written with n_step={sd.get('n_step', 1)} / gamma={sd.get('gamma')}, "
+                             f"this buffer has n_step={self.n_step} / gamma={self.gamma}")
         if self._h:
             check(lib.gcrl_her_clear(self._h))
         for ep in sd["episodes"]:

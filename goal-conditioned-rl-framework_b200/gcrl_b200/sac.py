@@ -186,14 +186,17 @@ class _SacBase(_AgentBase):
 
     def __init__(self, obs_dim, ac_dim, config, weights, nenvs, gradient_step, *,
                  index_source="host", device=0, max_batch=None, seed=1898, precision=0,
-                 goal_selection_strategy="future", online_sampling=False):
+                 goal_selection_strategy="future", online_sampling=False, n_step=1):
         """precision: 0 (default) runs every GEMM on the fp32 FFMA tiles; 1 runs the hidden-layer GEMMs of the
         critics and the actor on the tcgen05 tensor cores (3xTF32 split, the critic ensemble batched into one launch
         per layer) once batch * hidden_dim**2 >= 2048 * 256**2 (2048 rows at hidden_dim 256, 512 at 512, 8192 at
         128); 2 does so for every batch >= 128 (tests).  select_action stays on fp32.
-        goal_selection_strategy / online_sampling: passed to the HER buffer (HERBuffer)."""
+        goal_selection_strategy / online_sampling / n_step: passed to the HER buffer (HERBuffer), n_step with
+        config.gamma.  n_step > 1 needs buffer_type "HER" (ValueError otherwise).  The buffer's rows carry the n-step
+        reward and a done column whose gamma*(1 - done) is gamma**k*(1 - done), so every update computes the n-step
+        target unchanged; SAC / TQC take the entropy term at the bootstrap state only, as Stable-Baselines3 does."""
         self._init_common(obs_dim, ac_dim, config, nenvs, gradient_step, index_source, device, seed,
-                          goal_selection_strategy, online_sampling)
+                          goal_selection_strategy, online_sampling, n_step)
         self.alpha_min = getattr(config, "alpha_min", 0.05)
         self.alpha_min_steps = getattr(config, "alpha_min_steps", 10000)
         self.target_entropy = self._target_entropy(ac_dim)

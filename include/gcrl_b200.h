@@ -94,6 +94,14 @@ int gcrl_her_set_threshold(gcrl_her *h, float threshold);
 #define GCRL_HER_FINAL 1
 #define GCRL_HER_EPISODE 2
 int gcrl_her_set_goal_selection(gcrl_her *h, int strategy, int online_k);
+/* n-step returns, as Stable-Baselines3's `n_steps` for its off-policy algorithms (1: one-step rows, the default).
+ * A sampled row at step t of an episode of T stored steps, with goal g (original or relabelled), covers the window
+ * t .. t+k-1, k = min(n, T - t): reward R = r_t + gamma (r_{t+1} + ... + gamma r_{t+k-1}) (unfused fp32, from the
+ * back; relabelled rows recompute every r_{t+i} for g), next state = ns of row t+k-1 (goal columns <- g), done =
+ * 1 - gamma^(k-1) (1 - done_{t+k-1}) (relabelled rows: done_{t+k-1} = 0).  A learner's gamma (1 - done) is then the
+ * n-step bootstrap weight gamma^k (1 - done_{t+k-1}), exactly while gamma^(k-1) >= 1/2 and within 2^-25 beyond.
+ * 1 <= n <= 255; 0 < gamma <= 1 when n > 1.  Refused (GCRL_ERR_INVALID) once an episode has been committed. */
+int gcrl_her_set_n_step(gcrl_her *h, int n, float gamma);
 /* The draw epoch of the device index stream and of online relabelling (one per sample call that draws on the
  * device; in online mode one per sample call).  A checkpoint saves it so that a resumed run draws the same rows. */
 uint64_t gcrl_her_get_draw_epoch(const gcrl_her *h);
